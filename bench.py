@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]          # B200 arm (one process per GPU under torchrun)
     python bench.py --impl reference [...]                       # the reference arm: CPU port on the host cores
+    python bench.py --dump-outputs DIR [...]                     # also write the last timed step's outputs to DIR/<name>.npy
 
 A step = one forward + backward of spatial_transformer3.transformer over one batch of synthetic frames at
 BASELINE.json configs[1]: 32 x 288 x 512 x 3 fp32 per GPU, 4x4 mesh (weak scaling: every rank gets its own 32).
@@ -60,6 +61,23 @@ def synth_inputs(n, seed=0):
     import synth
     return dict(U=synth.noise_image(n, H, W, C, 900 + seed), theta=synth.random_mesh(n, GH, GW, 0.05, 901 + seed),
                 d_out=synth.randn((n, H, W, C), 902 + seed), d_img=synth.randn((n, H, W, 2), 903 + seed, 0.1))
+
+
+DUMP_BYTES = 60 << 20      # --dump-outputs writes at most this much
+
+
+def dump_outputs(path, outputs):
+    """Writes the arrays one step handed its caller as path/<name>.npy (float32).  Every array is cut to the same frames: a
+    fixed, seeded sample of the batch, as many as fit in DUMP_BYTES.  Returns the frame indices."""
+    n = next(iter(outputs.values())).shape[0]
+    per_frame = sum(t[0].numel() * t.element_size() for t in outputs.values())
+    k = max(1, min(n, DUMP_BYTES // per_frame))
+    frames = np.sort(np.random.RandomState(0).choice(n, k, replace=False))
+    idx = torch.as_tensor(frames, device=next(iter(outputs.values())).device)
+    os.makedirs(path, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(path, name + '.npy'), t.index_select(0, idx).float().cpu().numpy())
+    return frames.tolist()
 
 
 class ClockSampler:
@@ -127,7 +145,7 @@ def run_reference(args):
     inp = synth_inputs(ns)
     for _ in range(max(args.warmup, 1)):
         cpu_port_step(inp, ns)
-    steps = max(1, min(args.steps, 60))
+    steps = args.steps
     t = sum(cpu_port_step(inp, ns) for _ in range(steps))
     val = ns * H * W * steps / t / 1e6
     sample = '%d of 32 frames of configs[1] per step (fwd+bwd, dU+dtheta), %d steps' % (ns, steps)
@@ -161,6 +179,7 @@ def pin_to_gpu_cores(local):
 
 
 def main():
+    sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (which may be read-only)
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
     ap.add_argument('--steps', type=int, default=50)
@@ -173,7 +192,11 @@ def main():
     ap.add_argument('--kernel-impl', default='auto', choices=['auto', 'generic', 'tma', 'pipe'])
     ap.add_argument('--no-graph', action='store_true', help='launch the step eagerly instead of replaying CUDA graphs')
     ap.add_argument('--no-l2-keep', action='store_true', help='zero-fill dU without the L2 evict_last policy')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step returned (out, black, img, Hs, dU, dtheta; '
+                                                          'a seeded sample of its frames) to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         return run_reference(args)
 
@@ -182,6 +205,7 @@ def main():
     import torch.distributed as dist
     assert torch.cuda.is_available(), 'bench.py needs a CUDA device: the product has no CPU path'
     rank, world, local = mgw.parallel.init_from_env()
+    torch.manual_seed(rank)          # the torch-generated inputs (mesh-head features, config #3) are the same from run to run
     assert world == args.gpus or world == 1, 'launch with torchrun --nproc-per-node %d' % args.gpus
     ncores = pin_to_gpu_cores(local)
     dev = torch.device('cuda', local)
@@ -271,9 +295,10 @@ def main():
                 cur.wait_stream(side)
             if world > 1:
                 reducer.wait()                          # join: fork and join both lie inside the step (CUDA-graph capturable)
-            return dtheta
+            return dict(out=out, black=black, img=img, Hs=Hs, dU=dU, dtheta=dtheta)
 
         graphs = None
+        captured = []         # what the capture of graph i returned: every replay of graph i rewrites these tensors
         if not args.no_graph:
             # The step is launch-bound on the host once NCCL is in it (a dozen launches for ~100 us of GPU work): capture one
             # CUDA graph per rotating input set and replay.  Same kernels, same work; eager launches if capture is not possible.
@@ -288,7 +313,7 @@ def main():
                     gph = torch.cuda.CUDAGraph()
                     # thread_local: the NCCL watchdog thread polls CUDA events while we capture
                     with torch.cuda.graph(gph, capture_error_mode='thread_local'):
-                        step_eager(i)
+                        captured.append(step_eager(i))
                     graphs.append(gph)
                 torch.cuda.synchronize()
             except Exception as e:      # noqa: BLE001
@@ -296,7 +321,9 @@ def main():
                 graphs = None
                 torch.cuda.synchronize()
 
-        state = {'k': 0}      # the steps follow each other whatever index the caller passes (the dU buffers alternate)
+        # the steps follow each other whatever index the caller passes (the dU buffers alternate); 'eager' = what the last
+        # eager step() returned
+        state = {'k': 0, 'eager': None}
 
         def step(_i):
             k = state['k']
@@ -304,8 +331,12 @@ def main():
             if graphs is not None:
                 graphs[k % ngraph].replay()
             else:
-                step_eager(k)
-        return step, step_eager, graphs, dU_buf
+                state['eager'] = step_eager(k)
+
+        def last_outputs():
+            """the tensors the last call of step() wrote (calls of step_eager outside step() do not change them)"""
+            return captured[(state['k'] - 1) % ngraph] if graphs is not None else state['eager']
+        return step, step_eager, graphs, dU_buf, last_outputs
 
     def timed(fn, steps, warm, before_stop=None):
         for i in range(warm):
@@ -330,7 +361,7 @@ def main():
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item())
 
-    step, step_eager, graphs, dU_buf = make_step(sets, feats, reducer)
+    step, step_eager, graphs, dU_buf, last_outputs = make_step(sets, feats, reducer)
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
@@ -348,6 +379,9 @@ def main():
     ms_total = timed(step, K, Wm)
     launches_timed = launches_per_step * K
     clocks = sampler.stop() if rank == 0 else None
+    dumped = None
+    if args.dump_outputs and rank == 0:      # before the legs below reuse dU_buf and replay the step again
+        dumped = {'dir': args.dump_outputs, 'frames': dump_outputs(args.dump_outputs, last_outputs())}
 
     # --- the same step sustained: >= 1 s of replay (the K-step figure above lasts a few milliseconds)
     sustained = None
@@ -364,7 +398,7 @@ def main():
     # (mgw_mesh_warp_bwd_acc): what a training loop that owns two dU buffers gets.  One GPU only (see FILL_MODE above).
     double_buffered = None
     if not args.no_configs and fill_mode == 'fused' and world == 1:
-        step_db, _, _, _ = make_step(sets, feats, reducer, fill_mode='pipelined')
+        step_db, _, _, _, _ = make_step(sets, feats, reducer, fill_mode='pipelined')
         ms_db = timed(step_db, K, Wm) / K
         double_buffered = {'ms_per_step': ms_db, 'value': P / (ms_db * 1e-3) / 1e6, 'unit': 'Mpix/s',
                            'note': 'one zero-fill per step inside the timed region, of the buffer the NEXT step accumulates into, next to '
@@ -532,6 +566,8 @@ def main():
         line['e2e_u8_fused'] = e2e_u8
     if configs is not None:
         line['configs'] = configs
+    if dumped is not None:
+        line['dump_outputs'] = dumped
     if world == 1 and not args.no_cpu_baseline:
         torch.set_num_threads(os.cpu_count() or 1)
         ns = args.cpu_sample
@@ -651,7 +687,7 @@ def other_configs(mgw, ops, dev, rank, world, timed, make_step, keep):
             continue
         mode5 = FILL_MODE or ('pipelined' if nb >= 64 else 'fused')
         rec5['dU_zero_fill'] = mode5
-        step5, _, _, _ = make_step(set5 * 2, feats5, red5, sync_reduce=sync, fill_mode=mode5)
+        step5, _, _, _, _ = make_step(set5 * 2, feats5, red5, sync_reduce=sync, fill_mode=mode5)
         k5 = 20
         ms5 = timed(step5, k5, 3)
         rec5['ms_per_step_' + name] = ms5 / k5
