@@ -103,7 +103,7 @@ def launch_count():
 
 def set_impl(mode):
     """'auto' (pipeline / TMA tiles when the shape allows, else generic) | 'generic' | 'tma' (one TMA tile per CTA, error if the
-    shape does not fit) | 'pipe' (the persistent pipelines, error if the shape does not fit)"""
+    shape does not fit) | 'pipe' (the persistent forward pipeline, the backward as 'tma'; error if the shape does not fit)"""
     if mode not in ('auto', 'generic', 'tma', 'pipe'):
         raise ValueError('unknown kernel family %r' % (mode,))
     os.environ['MGW_IMPL'] = mode          # the library reads the variable at every call: a test / tuning hook, not an ABI entry

@@ -14,7 +14,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 SO = os.path.join(HERE, os.environ.get('MGW_SO_NAME', 'libmgw_b200.so'))       # MGW_SO_NAME / MGW_EXTRA_FLAGS: A/B builds for tuning
-SOURCES = ['mgw_capi.cu', 'mgw_solve.cu', 'mgw_warp_generic.cu', 'mgw_warp_tma.cu', 'mgw_warp_pipe.cu', 'mgw_warp_bwd_pipe.cu', 'mgw_interp.cu', 'mgw_loss.cu', 'mgw_loss_tile.cu', 'mgw_pass.cu', 'mgw_deploy.cu', 'mgw_stream.cu', 'mgw_crop.cu', 'mgw_vertex_loss.cu']
+SOURCES = ['mgw_capi.cu', 'mgw_solve.cu', 'mgw_warp_generic.cu', 'mgw_warp_tma.cu', 'mgw_warp_pipe.cu', 'mgw_interp.cu', 'mgw_loss.cu', 'mgw_loss_tile.cu', 'mgw_pass.cu', 'mgw_deploy.cu', 'mgw_stream.cu', 'mgw_crop.cu', 'mgw_vertex_loss.cu']
 FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17', '-fmad=false',
          '--expt-relaxed-constexpr', '-Xcompiler', '-fPIC,-O2,-fvisibility=hidden', '-cudart', 'static']
 

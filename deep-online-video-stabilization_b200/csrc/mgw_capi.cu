@@ -161,9 +161,7 @@ int mgw_warp_fwd(const float* U, const float* Hs, int N, int H, int W, int C, in
 
 size_t mgw_warp_bwd_workspace_bytes(int N, int H, int W, int C, int gh, int gw)
 {
-    const WarpShape s{N, H, W, C, H, W, gh, gw};
-    const size_t a = tma_bwd_supported(s) ? tma_bwd_workspace_bytes(s) : 0, b = pipe_bwd_supported(s) ? pipe_bwd_workspace_bytes(s) : 0;
-    return a > b ? a : b;
+    return tma_bwd_workspace_bytes(WarpShape{N, H, W, C, H, W, gh, gw});      // 0 when the tile kernels cannot serve the shape
 }
 
 // shared by mgw_warp_bwd and mgw_mesh_warp_bwd: produces dH partials; returns their layout
@@ -174,17 +172,9 @@ static int warp_bwd_core(const float* U, const float* Hs, const float* d_out, co
 {
     const size_t ncell = (size_t)s.N * s.gh * s.gw;
     const int mode = impl_mode();
+    // the one-tile-per-CTA kernels serve every backward they can take (MGW_IMPL=tma and =pipe: or fail), the generic kernels the rest
     const bool tma_ok = mode != 1 && workspace && tma_bwd_supported(s) && aligned(U, 16) && (!dU || aligned(dU, 16)) &&
                         (!d_img || aligned(d_img, 8));
-    // the persistent pipeline serves the calls that want dU (modes auto / pipe); dH-only calls and mode 2 take the tile kernels
-    // auto takes the one-tile-per-CTA backward: 61-63 us at config #2 against the pipeline's 77 (they were equally fast until the
-    // tile kernel got its gradients by TMA and its drain by vector reductions), and its 3072 short CTAs share the SMs gracefully
-    // with a concurrent NCCL kernel, while a CTA of the persistent pipeline that starts late finishes late.
-    // MGW_IMPL=pipe or MGW_BWD=pipe selects the pipeline.
-    static const bool prefer_pipe = [] { const char* v = getenv("MGW_BWD"); return v && v[0] == 'p'; }();
-    // (a fused img_loss with a second gradient on `output` is served by the tile kernels)
-    const bool pipe_ok = mode != 1 && mode != 2 && (prefer_pipe || mode == 3) && dU && workspace && pipe_bwd_supported(s) && aligned(U, 16) && aligned(dU, 16) &&
-                         (!d_img || aligned(d_img, 8)) && !(fl && d_out);
     bool own_fill = false;          // the tile backward then runs NEXT TO the fill up to its first access to dU (programmatic launch)
     if (dU && zero_dU) {
         // the library's own fill (evict_last: the lines are still in L2 when the reductions arrive) where its 16-byte granularity
@@ -193,13 +183,6 @@ static int warp_bwd_core(const float* U, const float* Hs, const float* d_out, co
         if (bytes % 16 == 0 && aligned(dU, 16)) { TRY(launch_fill_zero(dU, bytes, true, st)); own_fill = true; }
         else TRY(check_memset(cudaMemsetAsync(dU, 0, bytes, st), "memset dU"));
     }
-    if (pipe_ok) {
-        int np = 0;
-        TRY(launch_warp_bwd_pipe(U, Hs, d_out, d_img, s, dU, (float*)workspace, &np, fl, st));
-        *parts = (const float*)workspace; *nparts = np; *part_stride = 8;
-        return MGW_OK;
-    }
-    // (MGW_IMPL=pipe: the backward pipeline has one tile shape (cells of at least 24 x 32 px); smaller cells take the tile kernels)
     if (!tma_ok && mode >= 2)
         return set_error(MGW_ERR_UNSUPPORTED, "TMA path required (MGW_IMPL=tma|pipe) but shape/alignment/workspace does not allow it");
     if (tma_ok) {

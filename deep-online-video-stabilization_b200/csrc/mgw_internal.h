@@ -12,7 +12,7 @@ namespace mgw {
 int set_error(int code, const char* fmt, ...);
 int check_launch(const char* what);          // counts the launch, maps cudaGetLastError() to MGW_ERR_CUDA
 void count_launches(int n);
-int impl_mode();                             // MGW_IMPL environment override: 0 auto, 1 generic, 2 tma tiles, 3 pipelines
+int impl_mode();                             // MGW_IMPL environment override: 0 auto, 1 generic, 2 tma tiles, 3 forward pipeline (backward: tma tiles)
 
 // Launch with (pdl = true) the programmatic-stream-serialization attribute: the kernel may be scheduled while the previous
 // kernel of the stream is still running and synchronises with it through griddep_wait() (mgw_device.cuh).
@@ -106,12 +106,6 @@ int launch_warp_bwd_tma(const float* U, const float* Hs, const float* d_out, con
 // out + black + img)
 bool pipe_fwd_supported(const WarpShape& s);
 int launch_warp_fwd_pipe(const float* U, const float* Hs, const WarpShape& s, float* out, float* black, float* img, cudaStream_t st);
-
-// mgw_warp_bwd_pipe.cu : backward (dU + dH partials) as a persistent warp-specialised pipeline; needs dU != nullptr
-bool pipe_bwd_supported(const WarpShape& s);
-size_t pipe_bwd_workspace_bytes(const WarpShape& s);
-int launch_warp_bwd_pipe(const float* U, const float* Hs, const float* d_out, const float* d_img, const WarpShape& s,
-                         float* dU, float* dHs_part, int* nparts, const FusedImgLoss* fl, cudaStream_t st);
 
 // mgw_deploy.cu : deploy-side colour-frame warp (deploy_bundle.py:136-146)
 size_t remap_bundle_workspace_bytes(int N, int H, int W);

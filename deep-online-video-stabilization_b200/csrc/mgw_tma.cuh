@@ -1,7 +1,6 @@
 // Minimal sm_100a TMA / mbarrier wrappers (inline PTX) used by the tile kernels.
 //   loads  : cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes   (SASS UTMALDG)
 //   stores : cp.async.bulk.tensor.3d.global.shared::cta.bulk_group                          (SASS UTMASTG)
-//   reduce : cp.reduce.async.bulk.tensor.3d.global.shared::cta.add.tile.bulk_group          (SASS UTMAREDG)
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -20,7 +19,7 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count)
 // make the barrier init visible to the async proxy before a TMA targets it
 __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 
-// generic-proxy smem writes -> visible to the async proxy (before a TMA store / reduce reads them)
+// generic-proxy smem writes -> visible to the async proxy (before a TMA store reads them)
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes)
@@ -78,12 +77,6 @@ __device__ __forceinline__ void load_3d(void* smem_dst, const CUtensorMap* map, 
 __device__ __forceinline__ void store_3d(const CUtensorMap* map, const void* smem_src, int c0, int c1, int c2)
 {
     asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-                 ::"l"(map), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-
-__device__ __forceinline__ void reduce_add_3d(const CUtensorMap* map, const void* smem_src, int c0, int c1, int c2)
-{
-    asm volatile("cp.reduce.async.bulk.tensor.3d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3, %4}], [%1];"
                  ::"l"(map), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "r"(c2) : "memory");
 }
 

@@ -15,8 +15,7 @@
 //             scale is a power of two chosen per tile from max|d_out|, kBits = 31 - ceil(log2(TH*TW)) <= 22 bits per term,
 //             so the int32 sums provably cannot overflow.  The box leaves as fp32 by 16-byte reductions
 //             (red.global.add.v4.f32, REDG; all-zero groups skipped) straight from the fixed-point words -- no conversion
-//             back into shared memory, no third barrier, no TMA read wait before the CTA exits (MGW_BWD_DRAIN_RED=0 brings
-//             the round-1 drain back: ONE TMA reduce-add of the converted box, cp.reduce.async.bulk.tensor / UTMAREDG).
+//             back into shared memory, no third barrier, no TMA read wait before the CTA exits.
 //             Launched programmatically behind the library's zero-fill of dU, the kernel runs next to it up to its first
 //             access to dU (griddepcontrol.wait).  The 8 dH terms are reduced warp-shuffle -> shared -> one deterministic
 //             partial per tile (no global atomics).
@@ -340,18 +339,6 @@ struct LossBwd {
     const float* kscale_dev;    // nullable device factor on kscale
 };
 
-#ifndef MGW_BWD_SKIP_ZERO
-#define MGW_BWD_SKIP_ZERO 1
-#endif
-#ifndef MGW_BWD_STAGE_IMG
-#define MGW_BWD_STAGE_IMG 1
-#endif
-#ifndef MGW_BWD_STAGE
-#define MGW_BWD_STAGE 1
-#endif
-#ifndef MGW_BWD_DRAIN_RED
-#define MGW_BWD_DRAIN_RED 1
-#endif
 #ifndef MGW_BWD_MINB
 #define MGW_BWD_MINB (NT == 256 ? (K <= 3 ? 4 : 3) : 2)
 #endif
@@ -362,8 +349,8 @@ struct LossBwd {
 // accumulator box, no scatter code, fewer registers -> one more CTA per SM.
 template <int C, int TW, int K, int NT, bool LOSS, bool DU>
 __global__ void __launch_bounds__(NT, DU ? MGW_BWD_MINB : MGW_BWD_NODU_MINB)
-warp_bwd_tma_kernel(const __grid_constant__ CUtensorMap mapU, const __grid_constant__ CUtensorMap mapDU,
-                    const __grid_constant__ CUtensorMap mapG, const __grid_constant__ CUtensorMap mapGI, const float* __restrict__ U, const float* __restrict__ Hs, const float* __restrict__ d_out,
+warp_bwd_tma_kernel(const __grid_constant__ CUtensorMap mapU, const __grid_constant__ CUtensorMap mapG,
+                    const __grid_constant__ CUtensorMap mapGI, const float* __restrict__ U, const float* __restrict__ Hs, const float* __restrict__ d_out,
                     const float* __restrict__ d_img, const __grid_constant__ TileCfg cfg, float* __restrict__ dU,
                     float* __restrict__ parts, const LossBwd loss)
 {
@@ -379,7 +366,7 @@ warp_bwd_tma_kernel(const __grid_constant__ CUtensorMap mapU, const __grid_const
     // pixels up from shared memory (12-byte lane stride: conflict free).  As 24 LDGs per thread with a 12-byte lane stride
     // (three lines per request) they queued in the LSU for ~3500 cycles next to the other CTAs' shared-memory traffic and
     // the CTA spent more than half of its life before its first pixel.
-    constexpr bool STAGE = MGW_BWD_STAGE && DU && !LOSS && (G::kBoxF >= G::TH * TW * (C + 2));
+    constexpr bool STAGE = DU && !LOSS && (G::kBoxF >= G::TH * TW * (C + 2));
     constexpr int kStageOut = G::TH * TW * C;         // floats of the staged d_out tile; the d_img tile follows it
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 #ifdef MGW_PROBE
@@ -397,9 +384,9 @@ warp_bwd_tma_kernel(const __grid_constant__ CUtensorMap mapU, const __grid_const
     PROBE(12);     // tile decode
     if (STAGE && tid == 0) {
         float* sg = reinterpret_cast<float*>(s_acc);
-        tma::mbar_expect_tx(bar + 1, (uint32_t)((kStageOut + ((MGW_BWD_STAGE_IMG && d_img) ? G::TH * TW * 2 : 0)) * sizeof(float)));
+        tma::mbar_expect_tx(bar + 1, (uint32_t)((kStageOut + (d_img ? G::TH * TW * 2 : 0)) * sizeof(float)));
         tma::load_3d(sg, &mapG, bar + 1, tl.c0 * C, tl.r0, tl.n);
-        if (MGW_BWD_STAGE_IMG && d_img) tma::load_3d(sg + kStageOut, &mapGI, bar + 1, tl.c0 * 2, tl.r0, tl.n);
+        if (d_img) tma::load_3d(sg + kStageOut, &mapGI, bar + 1, tl.c0 * 2, tl.r0, tl.n);
     }
     float Hc[9];
 #pragma unroll
@@ -424,16 +411,6 @@ warp_bwd_tma_kernel(const __grid_constant__ CUtensorMap mapU, const __grid_const
     PROBE(13);     // Hs loads issued, lin_step
     float gout[K][C], gimg[K][2];
     if (STAGE) {
-#if !MGW_BWD_STAGE_IMG
-        {   // d_img: 8 contiguous bytes per lane (two lines per request), wanted only at the end of a pixel: plain loads
-            const float2* pi = reinterpret_cast<const float2*>(d_img) + ((size_t)tl.n * cfg.H + tl.r0 + g * K) * cfg.W + col;
-#pragma unroll
-            for (int k = 0; k < K; ++k) {
-                const float2 di = d_img ? __ldg(pi + (size_t)k * cfg.W) : make_float2(0.0f, 0.0f);
-                gimg[k][0] = di.x; gimg[k][1] = di.y;
-            }
-        }
-#endif
         __syncthreads();                              // the barriers thread 0 initialised are visible to everybody
         tma::mbar_wait(bar + 1, 0);
         const float* sg = reinterpret_cast<const float*>(s_acc) + (g * K * TW + tx) * C;
@@ -442,7 +419,6 @@ warp_bwd_tma_kernel(const __grid_constant__ CUtensorMap mapU, const __grid_const
         for (int k = 0; k < K; ++k) {
 #pragma unroll
             for (int ch = 0; ch < C; ++ch) gout[k][ch] = sg[k * TW * C + ch];
-            if (!MGW_BWD_STAGE_IMG) continue;
             if (d_img) {
                 const float2 di = si[k * TW];
                 gimg[k][0] = di.x; gimg[k][1] = di.y;
@@ -653,7 +629,7 @@ warp_bwd_tma_kernel(const __grid_constant__ CUtensorMap mapU, const __grid_const
         if ((lane & 3) == 0) s_red[warp * 8 + ((lane >> 4) & 1) * 4 + ((lane >> 3) & 1) * 2 + ((lane >> 2) & 1)] = v1;
     }
     PROBE(6);      // dH shuffles
-    __syncthreads();                                  // also orders every shared atomic before the conversion below
+    __syncthreads();                                  // also orders every shared atomic before the drain below
     PROBE(7);      // barrier 2
     if (tid < 8) {
         float v = 0.0f;
@@ -665,7 +641,6 @@ warp_bwd_tma_kernel(const __grid_constant__ CUtensorMap mapU, const __grid_const
         // Launched programmatically behind the zero-fill of dU (mgw_capi.cu), this kernel has run up to here NEXT TO it: nothing
         // above reads or writes dU.  From here on the fill must be complete and visible (a no-op under a plain launch).
         griddep_wait();
-#if MGW_BWD_DRAIN_RED
         // fixed point -> fp32 straight from the accumulator into dU by 16-byte reductions (red.global.add.v4.f32, fire and
         // forget through the LSU): no conversion back into shared memory, no proxy fence, no third barrier, and nothing of this
         // CTA waits in the SM's TMA unit in front of the next CTA's box load
@@ -681,37 +656,12 @@ warp_bwd_tma_kernel(const __grid_constant__ CUtensorMap mapU, const __grid_const
             const int row = j / kQ, q = j % kQ;
             if (row < rows && q < nq) {
                 const int4 v = a4[j];
-#if MGW_BWD_SKIP_ZERO
                 if ((v.x | v.y | v.z | v.w) != 0)      // most of the box outside the tile's own footprint received nothing: no traffic for +0
-#endif
-                tma::red_add_v4(base + row * pitch + q * 4, float_of_fixed(v.x) * inv_scale, float_of_fixed(v.y) * inv_scale,
-                                float_of_fixed(v.z) * inv_scale, float_of_fixed(v.w) * inv_scale);
+                    tma::red_add_v4(base + row * pitch + q * 4, float_of_fixed(v.x) * inv_scale, float_of_fixed(v.y) * inv_scale,
+                                    float_of_fixed(v.z) * inv_scale, float_of_fixed(v.w) * inv_scale);
             }
         }
         PROBE(8);
-#else
-        // fixed point -> fp32 in place, then ONE TMA reduce-add of the whole box into dU
-        int4* a4 = reinterpret_cast<int4*>(s_acc);
-#pragma unroll
-        for (int i = 0; i < (G::kBoxF / 4 + NT - 1) / NT; ++i) {
-            const int j = i * NT + tid;
-            if (j < G::kBoxF / 4) {
-                const int4 v = a4[j];
-                reinterpret_cast<float4*>(s_acc)[j] = make_float4(float_of_fixed(v.x) * inv_scale, float_of_fixed(v.y) * inv_scale,
-                                                                  float_of_fixed(v.z) * inv_scale, float_of_fixed(v.w) * inv_scale);
-            }
-        }
-        PROBE(8);      // convert
-        tma::fence_proxy_async();
-        __syncthreads();
-        PROBE(9);      // barrier 3
-        if (tid == 0) {
-            tma::reduce_add_3d(&mapDU, s_acc, bx0 * C, by0, tl.n);
-            tma::commit_group();
-            tma::wait_group_read0();
-        }
-        PROBE(10);     // TMA reduce issued and read (thread 0 only)
-#endif
     }
 }
 
@@ -802,9 +752,8 @@ static int launch_bwd_v(const float* U, const float* Hs, const float* d_out, con
 {
     using G = Geo<C, TW, K, NT>;
     const TileCfg& c = p.cfg;
-    CUtensorMap mU, mDU;
+    CUtensorMap mU;
     TRY_RC(make_map(&mU, U, c.W * C, c.H, c.N, G::kRowF, G::SBH));
-    if (dU) TRY_RC(make_map(&mDU, dU, c.W * C, c.H, c.N, G::kRowF, G::SBH)); else mDU = mU;
     CUtensorMap mG = mU, mGI = mU;                  // staged d_out / d_img tiles (plain backward with dU only)
     if (dU && !loss) {
         TRY_RC(make_map(&mG, d_out, c.W * C, c.H, c.N, TW * C, G::TH));
@@ -816,21 +765,21 @@ static int launch_bwd_v(const float* U, const float* Hs, const float* d_out, con
     if (loss && dU) {
         static bool attr[64] = {};
         TRY_RC(allow_smem(warp_bwd_tma_kernel<C, TW, K, NT, true, true>, attr, "warp_bwd_tma(loss)"));
-        warp_bwd_tma_kernel<C, TW, K, NT, true, true><<<grid, NT, smem, st>>>(mU, mDU, mG, mGI, U, Hs, d_out, d_img, c, dU, parts, *loss);
+        warp_bwd_tma_kernel<C, TW, K, NT, true, true><<<grid, NT, smem, st>>>(mU, mG, mGI, U, Hs, d_out, d_img, c, dU, parts, *loss);
     } else if (loss) {
         static bool attr[64] = {};
         TRY_RC(allow_smem(warp_bwd_tma_kernel<C, TW, K, NT, true, false>, attr, "warp_bwd_tma(loss, no dU)"));
-        warp_bwd_tma_kernel<C, TW, K, NT, true, false><<<grid, NT, smem, st>>>(mU, mDU, mG, mGI, U, Hs, d_out, d_img, c, nullptr, parts, *loss);
+        warp_bwd_tma_kernel<C, TW, K, NT, true, false><<<grid, NT, smem, st>>>(mU, mG, mGI, U, Hs, d_out, d_img, c, nullptr, parts, *loss);
     } else if (dU) {
         static bool attr[64] = {};
         TRY_RC(allow_smem(warp_bwd_tma_kernel<C, TW, K, NT, false, true>, attr, "warp_bwd_tma"));
         const cudaError_t e = launch_ex(warp_bwd_tma_kernel<C, TW, K, NT, false, true>, grid, dim3(NT), smem, st, behind_own_fill && pdl_enabled(),
-                                        mU, mDU, mG, mGI, U, Hs, d_out, d_img, c, dU, parts, LossBwd{});
+                                        mU, mG, mGI, U, Hs, d_out, d_img, c, dU, parts, LossBwd{});
         if (e != cudaSuccess) { count_launches(1); return set_error(MGW_ERR_CUDA, "warp_bwd_tma: %s", cudaGetErrorString(e)); }
     } else {
         static bool attr[64] = {};
         TRY_RC(allow_smem(warp_bwd_tma_kernel<C, TW, K, NT, false, false>, attr, "warp_bwd_tma(no dU)"));
-        warp_bwd_tma_kernel<C, TW, K, NT, false, false><<<grid, NT, smem, st>>>(mU, mDU, mG, mGI, U, Hs, d_out, d_img, c, nullptr, parts, LossBwd{});
+        warp_bwd_tma_kernel<C, TW, K, NT, false, false><<<grid, NT, smem, st>>>(mU, mG, mGI, U, Hs, d_out, d_img, c, nullptr, parts, LossBwd{});
     }
     return check_launch("warp_bwd_tma");
 }

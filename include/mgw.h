@@ -44,9 +44,10 @@ MGW_API const char* mgw_last_error(void);
 /* Number of kernels this library has launched on the calling process so far (bench.py's gpu_launches). */
 MGW_API uint64_t mgw_launch_count(void);
 
-/* Kernel family: chosen per call from shape and alignment (persistent TMA pipelines, else one TMA tile per CTA, else the
- * generic global-gather kernels).  Tests and tuning runs can force one through the environment variable
- * MGW_IMPL = auto | generic | tma | pipe ("tma" / "pipe" fail instead of falling back); the library keeps no such state. */
+/* Kernel family: chosen per call from shape and alignment (forward: a persistent TMA pipeline, else one TMA tile per CTA;
+ * backward: one TMA tile per CTA; else the generic global-gather kernels).  Tests and tuning runs can force one through the
+ * environment variable MGW_IMPL = auto | generic | tma | pipe ("tma" / "pipe" fail instead of falling back; "pipe" selects the
+ * forward pipeline and, for the backward, the tile kernels like "tma"); the library keeps no such state. */
 
 /* ---- a0: get_4_pts, s_net_bundle_nobm.py:29-71 --------------------------------------------------------
  * head [N, 2*(gh+1)*(gw+1)] -> pts2 [N,gh+1,gw+1,2] (absolute clamped vertices, (x,y) last),

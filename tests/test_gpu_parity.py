@@ -187,7 +187,7 @@ def test_pipe_path_is_taken_and_matches_generic(mgw, name):
     o_t, b_t, i_t, _ = mgw.ops.warp_fwd(Ud, Hd)
     assert torch.equal(o_g.view(torch.int32), o_t.view(torch.int32)) and torch.equal(b_g, b_t)
     assert torch.equal(i_g.view(torch.int32), i_t.view(torch.int32))
-    # the backward pipeline (fixed-point shared accumulation, 16-byte reductions) vs fp32 atomics (generic)
+    # the backward under 'pipe' runs the tile kernels (fixed-point shared accumulation, 16-byte reductions) vs fp32 atomics (generic)
     dU_t, dH_t = mgw.ops.warp_bwd(Ud, Hd, dev(d_out), dev(d_img))
     s0 = 1 if 'fold' in name else 0      # a folded cell scatters 1e5-weighted terms: order-dependent garbage in any implementation
     assert relmax(dU_t[s0:].cpu().numpy(), dU_g[s0:].cpu().numpy()) < 2e-5

@@ -1,5 +1,5 @@
-"""Randomised agreement soak (GPU): many random shapes / meshes, `auto` (pipeline / TMA tiles) against the generic kernels --
-forward bit for bit, backward to rounding -- plus the no-dU and fused-loss variants against their unfused forms.
+"""Randomised agreement soak (GPU): many random shapes / meshes, `auto` (forward: pipeline / TMA tiles; backward: TMA tiles)
+against the generic kernels -- forward bit for bit, backward to rounding -- plus the no-dU and fused-loss variants against their unfused forms.
 usage: soak.py [cases] [seed].  Not part of the test suite (minutes of GPU time at a few hundred cases)."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
