@@ -85,7 +85,7 @@ using namespace mgw;
 
 extern "C" {
 
-int mgw_version(void) { return 100; }
+int mgw_version(void) { return 101; }
 
 const char* mgw_last_error(void) { return g_err; }
 
@@ -536,7 +536,7 @@ int mgw_resize_linear_u8(const uint8_t* img, int H, int W, int C, const int32_t*
     REQUIRE(H > 0 && W > 0 && out_h > 0 && out_w > 0 && (long long)H * W * 4 < (1LL << 31) && (long long)out_h * out_w < (1LL << 29),
             "mgw_resize_linear_u8: bad sizes");
     REQUIRE((!xtab || aligned(xtab, 16)) && (!ytab || aligned(ytab, 16)), "mgw_resize_linear_u8: tables must be 16-byte aligned");
-    return launch_resize_linear_u8(img, H, W, C, xtab, ytab, out_h, out_w, dst, (cudaStream_t)stream);
+    return launch_resize_linear_u8(img, 1, H, W, C, xtab, ytab, out_h, out_w, dst, (cudaStream_t)stream);
 }
 
 int mgw_cvt_img2train_u8(const uint8_t* bgr, int H, int W, const int32_t* kx, const int32_t* x0, const int32_t* xn, int ksx,
@@ -546,7 +546,7 @@ int mgw_cvt_img2train_u8(const uint8_t* bgr, int H, int W, const int32_t* kx, co
     REQUIRE(bgr && kx && x0 && xn && ky && y0 && yn && tmp && out, "mgw_cvt_img2train_u8: null pointer");
     REQUIRE(H > 0 && W > 0 && out_h > 0 && out_w > 0 && ksx > 0 && ksy > 0 && (long long)H * out_w < (1LL << 31) &&
             (long long)H * W < (1LL << 29), "mgw_cvt_img2train_u8: bad sizes");
-    return launch_cvt_img2train_u8(bgr, H, W, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w, tmp, out, (cudaStream_t)stream);
+    return launch_cvt_img2train_u8(bgr, 1, H, W, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w, tmp, out, (cudaStream_t)stream);
 }
 
 int mgw_warp_rev_bundle_u8(const uint8_t* img, const double* Hs_cvt, int N, int H, int W, int C, int gh, int gw, uint8_t* dst,
@@ -612,6 +612,66 @@ int mgw_stream_push_dev(float* frames, float* masks, int depth, int32_t* head_de
     REQUIRE(depth > 0 && H > 0 && W > 0 && (long long)H * W < (1LL << 31), "mgw_stream_push_dev: bad sizes");
     TRY(launch_stream_push(frames, masks, depth, 0, img, black, H, W, nullptr, 1, (cudaStream_t)stream, reinterpret_cast<const int*>(head_dev)));
     return launch_stream_advance(reinterpret_cast<int*>(head_dev), depth, (cudaStream_t)stream);
+}
+
+// Batched deploy calls: S streams (frames) of one size, the stream index in gridDim.y (hence S <= 65535).  The sizes are checked
+// first: S = 0 returns MGW_OK before the pointers are looked at (an empty batch may come with null buffers) and launches nothing.
+int mgw_cvt_img2train_u8_batch(const uint8_t* bgr, int S, int H, int W, const int32_t* kx, const int32_t* x0, const int32_t* xn, int ksx,
+                               const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h, int out_w, uint8_t* tmp,
+                               float* out, void* stream)
+{
+    REQUIRE(S >= 0 && S <= 65535 && H > 0 && W > 0 && out_h > 0 && out_w > 0 && ksx > 0 && ksy > 0 &&
+            (long long)S * H * out_w < (1LL << 31) && (long long)S * out_h * out_w < (1LL << 31) && (long long)S * H * W < (1LL << 29),
+            "mgw_cvt_img2train_u8_batch: bad sizes (S=%d H=%d W=%d out %dx%d)", S, H, W, out_h, out_w);
+    if (S == 0) return MGW_OK;
+    REQUIRE(bgr && kx && x0 && xn && ky && y0 && yn && tmp && out, "mgw_cvt_img2train_u8_batch: null pointer");
+    return launch_cvt_img2train_u8(bgr, S, H, W, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w, tmp, out, (cudaStream_t)stream);
+}
+
+int mgw_resize_linear_u8_batch(const uint8_t* img, int S, int H, int W, int C, const int32_t* xtab, const int32_t* ytab, int out_h,
+                               int out_w, uint8_t* dst, void* stream)
+{
+    REQUIRE(S >= 0 && S <= 65535 && H > 0 && W > 0 && out_h > 0 && out_w > 0 && (long long)S * H * W * 4 < (1LL << 31) &&
+            (long long)S * out_h * out_w < (1LL << 29), "mgw_resize_linear_u8_batch: bad sizes (S=%d H=%d W=%d out %dx%d)", S, H, W,
+            out_h, out_w);
+    REQUIRE(C == 1 || C == 3 || C == 4, "mgw_resize_linear_u8_batch: C must be 1, 3 or 4 (got %d)", C);
+    if (S == 0) return MGW_OK;
+    REQUIRE(img && dst, "mgw_resize_linear_u8_batch: null pointer");
+    REQUIRE((W == 2 * out_w && H == 2 * out_h) || (xtab && ytab), "mgw_resize_linear_u8_batch: coefficient tables are required");
+    REQUIRE((!xtab || aligned(xtab, 16)) && (!ytab || aligned(ytab, 16)), "mgw_resize_linear_u8_batch: tables must be 16-byte aligned");
+    return launch_resize_linear_u8(img, S, H, W, C, xtab, ytab, out_h, out_w, dst, (cudaStream_t)stream);
+}
+
+static int validate_streams(const char* fn, int S, int depth, int H, int W, int nch)
+{
+    REQUIRE(S >= 0 && S <= 65535 && depth > 0 && H > 0 && W > 0 && (long long)S * depth * H * W < (1LL << 31) &&
+            (long long)S * H * W * nch < (1LL << 31), "%s: bad sizes (S=%d depth=%d H=%d W=%d)", fn, S, depth, H, W);
+    return MGW_OK;
+}
+
+int mgw_streams_assemble(const float* frames, const float* masks, int S, int depth, const int32_t* heads_dev, const int* taps, int ntaps,
+                         int use_masks, const float* cur, int H, int W, float* in_x, void* stream)
+{
+    REQUIRE(taps || ntaps == 0, "mgw_streams_assemble: null pointer");
+    REQUIRE(ntaps >= 0 && ntaps <= 32, "mgw_streams_assemble: at most 32 taps (got %d)", ntaps);
+    for (int k = 0; k < ntaps; ++k)
+        REQUIRE(taps[k] >= 1 && taps[k] <= depth, "mgw_streams_assemble: tap %d outside [1, depth = %d]", taps[k], depth);
+    TRY(validate_streams("mgw_streams_assemble", S, depth, H, W, (use_masks ? 2 : 1) * ntaps + 1));
+    if (S == 0) return MGW_OK;
+    REQUIRE(frames && cur && in_x && heads_dev && (masks || !use_masks), "mgw_streams_assemble: null pointer");
+    return launch_stream_assemble(frames, masks, depth, 0, taps, ntaps, use_masks, cur, H, W, in_x, (cudaStream_t)stream,
+                                  reinterpret_cast<const int*>(heads_dev), S);
+}
+
+int mgw_streams_push(float* frames, float* masks, int S, int depth, int32_t* heads_dev, const float* img, const float* black, int H, int W,
+                     void* stream)
+{
+    TRY(validate_streams("mgw_streams_push", S, depth, H, W, 1));
+    if (S == 0) return MGW_OK;
+    REQUIRE(img && black && frames && heads_dev, "mgw_streams_push: null pointer");
+    TRY(launch_stream_push(frames, masks, depth, 0, img, black, H, W, nullptr, 1, (cudaStream_t)stream,
+                           reinterpret_cast<const int*>(heads_dev), S));
+    return launch_stream_advance(reinterpret_cast<int*>(heads_dev), depth, (cudaStream_t)stream, S);
 }
 
 int mgw_img_loss_fwd(const float* out, const float* y, const float* black, int N, int H, int W, int C, float* sums, void* stream)

@@ -184,6 +184,8 @@ int launch_remap_bundle_u8(const uint8_t* img, const float* xy, int N, int H, in
 // cvt_img2train (config.py:6-21): BGR uint8 frame -> cv2 BGR2GRAY -> Pillow resize(BILINEAR) [-> crop] -> v*(1/255) - 0.5.
 // The host binding computes Pillow's 22-bit fixed-point coefficient tables (double arithmetic, Resample.c) once per shape
 // and slices them for the crop; the two passes below are Pillow's: horizontal first into a uint8 image, then vertical.
+// A batch of S frames of one size shares the tables; blockIdx.y is the frame (the stream index of a StreamBatch): each block
+// offsets its base pointers once, the per-pixel index arithmetic is the single-frame one, and S = 1 is the single-frame call.
 namespace {
 
 __global__ void __launch_bounds__(256)
@@ -192,6 +194,8 @@ gray_hpass_kernel(const uint8_t* __restrict__ bgr, int H, int W, const int32_t* 
 {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= H * out_w) return;
+    bgr += (size_t)blockIdx.y * H * W * 3;
+    tmp += (size_t)blockIdx.y * H * out_w;
     const int xx = t % out_w, row = t / out_w;
     const uint8_t* p = bgr + ((size_t)row * W + __ldg(x0 + xx)) * 3;
     const int n = __ldg(xn + xx);
@@ -205,11 +209,13 @@ gray_hpass_kernel(const uint8_t* __restrict__ bgr, int H, int W, const int32_t* 
 }
 
 __global__ void __launch_bounds__(256)
-vpass_norm_kernel(const uint8_t* __restrict__ tmp, int out_w, const int32_t* __restrict__ ky, const int32_t* __restrict__ y0,
+vpass_norm_kernel(const uint8_t* __restrict__ tmp, int H, int out_w, const int32_t* __restrict__ ky, const int32_t* __restrict__ y0,
                   const int32_t* __restrict__ yn, int ks, int out_h, float* __restrict__ out)
 {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= out_h * out_w) return;
+    tmp += (size_t)blockIdx.y * H * out_w;
+    out += (size_t)blockIdx.y * out_h * out_w;
     const int xx = t % out_w, yy = t / out_w;
     const uint8_t* p = tmp + (size_t)__ldg(y0 + yy) * out_w + xx;
     const int n = __ldg(yn + yy);
@@ -222,13 +228,13 @@ vpass_norm_kernel(const uint8_t* __restrict__ tmp, int out_w, const int32_t* __r
 
 }  // namespace
 
-int launch_cvt_img2train_u8(const uint8_t* bgr, int H, int W, const int32_t* kx, const int32_t* x0, const int32_t* xn, int ksx,
+int launch_cvt_img2train_u8(const uint8_t* bgr, int S, int H, int W, const int32_t* kx, const int32_t* x0, const int32_t* xn, int ksx,
                             const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h, int out_w, uint8_t* tmp,
                             float* out, cudaStream_t st)
 {
-    gray_hpass_kernel<<<(H * out_w + 255) / 256, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp);
+    gray_hpass_kernel<<<dim3((H * out_w + 255) / 256, S), 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp);
     if (int rc = check_launch("gray_hpass")) return rc;
-    vpass_norm_kernel<<<(out_h * out_w + 255) / 256, 256, 0, st>>>(tmp, out_w, ky, y0, yn, ksy, out_h, out);
+    vpass_norm_kernel<<<dim3((out_h * out_w + 255) / 256, S), 256, 0, st>>>(tmp, H, out_w, ky, y0, yn, ksy, out_h, out);
     return check_launch("vpass_norm");
 }
 
@@ -236,6 +242,7 @@ int launch_cvt_img2train_u8(const uint8_t* bgr, int H, int W, const int32_t* kx,
 // cv2.resize(frame, (width, height)) of the uint8 colour frame (deploy_bundle.py:301; INTER_LINEAR): OpenCV's 8-bit path --
 // 11-bit fixed-point weights (tables from the host binding: x0, x1, a0, a1 per output column / row), int32 horizontal sums,
 // ((b0*(S0>>4))>>16) + ((b1*(S1>>4))>>16) + 2) >> 2 vertically; an exact 2x2 decimation is OpenCV's INTER_AREA shortcut.
+// blockIdx.y is the frame of a batch of S frames of one size (as for cvt_img2train above).
 namespace {
 
 template <int C>
@@ -245,6 +252,8 @@ resize_u8_kernel(const uint8_t* __restrict__ img, int H, int W, const int4* __re
 {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= out_h * out_w) return;
+    img += (size_t)blockIdx.y * H * W * C;
+    dst += (size_t)blockIdx.y * out_h * out_w * C;
     const int x = t % out_w, y = t / out_w;
     uint8_t* o = dst + (size_t)t * C;
     if (area2) {
@@ -269,12 +278,12 @@ resize_u8_kernel(const uint8_t* __restrict__ img, int H, int W, const int4* __re
 
 }  // namespace
 
-int launch_resize_linear_u8(const uint8_t* img, int H, int W, int C, const int32_t* xtab, const int32_t* ytab, int out_h, int out_w,
+int launch_resize_linear_u8(const uint8_t* img, int S, int H, int W, int C, const int32_t* xtab, const int32_t* ytab, int out_h, int out_w,
                             uint8_t* dst, cudaStream_t st)
 {
     const int area2 = (W == 2 * out_w && H == 2 * out_h) ? 1 : 0;
     if (!area2 && (!xtab || !ytab)) return set_error(MGW_ERR_INVALID, "resize_linear_u8: coefficient tables are required");
-    const int grid = (out_h * out_w + 255) / 256;
+    const dim3 grid((out_h * out_w + 255) / 256, S);
     const int4* xt = reinterpret_cast<const int4*>(xtab);
     const int4* yt = reinterpret_cast<const int4*>(ytab);
     switch (C) {

@@ -112,9 +112,10 @@ size_t remap_bundle_workspace_bytes(int N, int H, int W);
 int launch_remap_bundle_u8(const uint8_t* img, const float* xy, int N, int H, int W, int C, uint8_t* dst, void* workspace,
                            cudaStream_t st);
 
-int launch_resize_linear_u8(const uint8_t* img, int H, int W, int C, const int32_t* xtab, const int32_t* ytab, int out_h, int out_w,
+// S frames of one size ([S,H,W,C] -> [S,out_h,out_w,C]; S >= 1, the single-frame calls pass 1)
+int launch_resize_linear_u8(const uint8_t* img, int S, int H, int W, int C, const int32_t* xtab, const int32_t* ytab, int out_h, int out_w,
                             uint8_t* dst, cudaStream_t st);
-int launch_cvt_img2train_u8(const uint8_t* bgr, int H, int W, const int32_t* kx, const int32_t* x0, const int32_t* xn, int ksx,
+int launch_cvt_img2train_u8(const uint8_t* bgr, int S, int H, int W, const int32_t* kx, const int32_t* x0, const int32_t* xn, int ksx,
                             const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h, int out_w, uint8_t* tmp,
                             float* out, cudaStream_t st);
 int launch_warp_rev_bundle_u8(const uint8_t* img, const double* Hs_cvt, int N, int H, int W, int C, int gh, int gw, uint8_t* dst,
@@ -158,10 +159,11 @@ size_t crop_rect_workspace_bytes(int H, int W);
 int launch_crop_rect(const int32_t* all_black, int H, int W, int step, void* workspace, int32_t* rect, cudaStream_t st);
 
 // mgw_stream.cu : deploy-side streaming state (device-resident history rings, deploy_bundle.py:204-232,259-295,319-327)
+// S > 1 (device heads only): S independent streams, rings [S][depth][H][W], heads head_dev[S], pixels [S][H][W]
 int launch_stream_assemble(const float* frames, const float* masks, int depth, int head, const int* taps_host, int ntaps, int use_masks,
-                           const float* cur, int H, int W, float* in_x, cudaStream_t st, const int* head_dev = nullptr);
+                           const float* cur, int H, int W, float* in_x, cudaStream_t st, const int* head_dev = nullptr, int S = 1);
 int launch_stream_push(float* frames, float* masks, int depth, int slot, const float* img, const float* black, int H, int W,
-                       float* frame_out, int out_stride, cudaStream_t st, const int* head_dev = nullptr);
-int launch_stream_advance(int* head_dev, int depth, cudaStream_t st);
+                       float* frame_out, int out_stride, cudaStream_t st, const int* head_dev = nullptr, int S = 1);
+int launch_stream_advance(int* head_dev, int depth, cudaStream_t st, int S = 1);
 
 }  // namespace mgw

@@ -5,13 +5,16 @@
 `warpRevBundle2` keeps the reference signature -- one uint8 frame [H,W,3] and the operator's x_map / y_map [H,W] -- and
 accepts numpy arrays (as the reference's caller passes; the result comes back as a numpy array) or CUDA tensors (batched
 [N,H,W,C] / [N,H,W] too; the result stays on the device).  The work is one C-ABI call, mgw_remap_bundle_u8.
+
+StreamBatch runs the whole per-frame loop for S videos of one size at once: one set of launches per frame, capturable as one
+CUDA graph, every video's result bit-identical to its own StreamState / CropState pipeline.
 """
 import numpy as np
 import torch
 
 from . import ops
 
-__all__ = ['warpRevBundle2', 'warpRevBundle', 'warpRev', 'cvt_theta_mat_bundle', 'cvt_img2train', 'cv2_resize', 'StreamState', 'CropState']
+__all__ = ['warpRevBundle2', 'warpRevBundle', 'warpRev', 'cvt_theta_mat_bundle', 'cvt_img2train', 'cv2_resize', 'StreamState', 'CropState', 'StreamBatch']
 
 
 def warpRevBundle2(img, x_map, y_map, device=None):
@@ -87,34 +90,36 @@ _CVT_TABLES = {}
 _RESIZE_TABLES = {}
 
 
-def cv2_resize(img, dsize, device='cuda'):
-    """cv2.resize(img, dsize) for a uint8 frame [H,W,C] (reference deploy_bundle.py:301 resizes the unstable colour frame to the
-    network size before warpRevBundle2), byte-exact with OpenCV's INTER_LINEAR; dsize = (width, height) as in OpenCV.
-    numpy in -> numpy out; a CUDA frame stays on the device."""
-    as_numpy = isinstance(img, np.ndarray)
-    im = (torch.as_tensor(np.ascontiguousarray(img)) if as_numpy else img).to(device=device if as_numpy else img.device, dtype=torch.uint8)
-    H, W = int(im.shape[0]), int(im.shape[1])
-    ow, oh = int(dsize[0]), int(dsize[1])
-    key = (H, W, oh, ow, str(im.device))
+def _resize_tables(H, W, oh, ow, device):
+    key = (H, W, oh, ow, str(device))
     if key not in _RESIZE_TABLES:
         if W == 2 * ow and H == 2 * oh:
             _RESIZE_TABLES[key] = (None, None)
         else:
-            _RESIZE_TABLES[key] = (torch.as_tensor(_cv_linear_table(ow, W, True)).to(im.device),
-                                   torch.as_tensor(_cv_linear_table(oh, H, False)).to(im.device))
-    dst = ops.resize_linear_u8(im.contiguous(), _RESIZE_TABLES[key][0], _RESIZE_TABLES[key][1], oh, ow)
+            _RESIZE_TABLES[key] = (torch.as_tensor(_cv_linear_table(ow, W, True)).to(device),
+                                   torch.as_tensor(_cv_linear_table(oh, H, False)).to(device))
+    return _RESIZE_TABLES[key]
+
+
+def cv2_resize(img, dsize, device='cuda'):
+    """cv2.resize(img, dsize) for a uint8 frame [H,W,C] (reference deploy_bundle.py:301 resizes the unstable colour frame to the
+    network size before warpRevBundle2), byte-exact with OpenCV's INTER_LINEAR; dsize = (width, height) as in OpenCV.
+    A batch [S,H,W,C] of frames of one size gives [S,height,width,C], each frame as its own call would (one launch).
+    numpy in -> numpy out; a CUDA frame stays on the device."""
+    as_numpy = isinstance(img, np.ndarray)
+    im = (torch.as_tensor(np.ascontiguousarray(img)) if as_numpy else img).to(device=device if as_numpy else img.device, dtype=torch.uint8)
+    H, W = int(im.shape[-3]), int(im.shape[-2])
+    ow, oh = int(dsize[0]), int(dsize[1])
+    xtab, ytab = _resize_tables(H, W, oh, ow, im.device)
+    if im.dim() == 4:
+        dst = ops.resize_linear_u8_batch(im.contiguous(), xtab, ytab, oh, ow)
+    else:
+        dst = ops.resize_linear_u8(im.contiguous(), xtab, ytab, oh, ow)
     return dst.cpu().numpy() if as_numpy else dst
 
 
-def cvt_img2train(img, crop_rate=1, height=288, width=512, device='cuda', as_numpy=False):
-    """reference config.py:6-21 (`height`, `width` are its config globals): one BGR uint8 frame [H,W,3] -> the network's frame
-    format, exact: cv2 BGR2GRAY, Pillow resize(BILINEAR) (to (width, height), or to the 1/crop_rate larger size followed by
-    the centre crop), v * (1/255) - 0.5.  Returns a CUDA fp32 tensor [1,height,width,1]; as_numpy=True gives the reference's
-    float64 numpy array (same values: the network's placeholder casts to fp32).  The coefficient tables are built once per
-    shape on the host and kept on the device."""
-    im = (torch.as_tensor(np.ascontiguousarray(img)) if isinstance(img, np.ndarray) else img).to(device=device, dtype=torch.uint8)
-    H, W = int(im.shape[0]), int(im.shape[1])
-    key = (H, W, height, width, float(crop_rate), str(im.device))
+def _cvt_tables(H, W, height, width, crop_rate, device):
+    key = (H, W, height, width, float(crop_rate), str(device))
     if key not in _CVT_TABLES:
         if crop_rate != 1:
             h = int(height / crop_rate); dh = int((h - height) / 2)
@@ -124,8 +129,24 @@ def cvt_img2train(img, crop_rate=1, height=288, width=512, device='cuda', as_num
         kx, x0, xn = _pil_bilinear_windows(W, w)
         ky, y0, yn = _pil_bilinear_windows(H, h)
         tabs = (kx[dw:dw + width], x0[dw:dw + width], xn[dw:dw + width], ky[dh:dh + height], y0[dh:dh + height], yn[dh:dh + height])
-        _CVT_TABLES[key] = tuple(torch.as_tensor(np.ascontiguousarray(t)).to(im.device) for t in tabs)
-    out = ops.cvt_img2train_u8(im.contiguous(), _CVT_TABLES[key], height, width).reshape(1, height, width, 1)
+        _CVT_TABLES[key] = tuple(torch.as_tensor(np.ascontiguousarray(t)).to(device) for t in tabs)
+    return _CVT_TABLES[key]
+
+
+def cvt_img2train(img, crop_rate=1, height=288, width=512, device='cuda', as_numpy=False):
+    """reference config.py:6-21 (`height`, `width` are its config globals): one BGR uint8 frame [H,W,3] -> the network's frame
+    format, exact: cv2 BGR2GRAY, Pillow resize(BILINEAR) (to (width, height), or to the 1/crop_rate larger size followed by
+    the centre crop), v * (1/255) - 0.5.  Returns a CUDA fp32 tensor [1,height,width,1]; as_numpy=True gives the reference's
+    float64 numpy array (same values: the network's placeholder casts to fp32).  The coefficient tables are built once per
+    shape on the host and kept on the device.  A batch [S,H,W,3] of frames of one size gives [S,height,width,1], each frame
+    as its own call would (one pair of launches for the batch)."""
+    im = (torch.as_tensor(np.ascontiguousarray(img)) if isinstance(img, np.ndarray) else img).to(device=device, dtype=torch.uint8)
+    H, W = int(im.shape[-3]), int(im.shape[-2])
+    tabs = _cvt_tables(H, W, height, width, crop_rate, im.device)
+    if im.dim() == 4:
+        out = ops.cvt_img2train_u8_batch(im.contiguous(), tabs, height, width).reshape(-1, height, width, 1)
+    else:
+        out = ops.cvt_img2train_u8(im.contiguous(), tabs, height, width).reshape(1, height, width, 1)
     if not as_numpy:
         return out
     v = np.rint((out.cpu().numpy().astype(np.float64) + 0.5) * 255)          # the resampled byte, recovered exactly
@@ -216,6 +237,13 @@ class StreamState:
         return self.frames[order], self.masks[order]
 
 
+def _crop_rect(all_black, step):
+    r = [int(v) for v in ops.crop_rect(all_black, step).cpu()]
+    if r[0] < 0:
+        raise IndexError('no black-free rectangle: every lattice corner has been black (the reference fails on ans[3] here)')
+    return r
+
+
 class CropState:
     """The crop bookkeeping of deploy_bundle.py: `all_black` (:240) gathers every black mask the network produced (:291),
     and after the last frame the largest never-black rectangle on the 10-pixel corner lattice (:344-365) is cut out of
@@ -234,11 +262,136 @@ class CropState:
         ops.black_accumulate(self.all_black, black)
 
     def rect(self, step=10):
-        r = [int(v) for v in ops.crop_rect(self.all_black, step).cpu()]
-        if r[0] < 0:
-            raise IndexError('no black-free rectangle: every lattice corner has been black (the reference fails on ans[3] here)')
-        return r
+        return _crop_rect(self.all_black, step)
 
     def cut(self, frame, step=10):
         t, l, b, r = self.rect(step)
         return frame[..., t:b + 1, l:r + 1, :]
+
+
+class StreamBatch:
+    """S videos of one source size stabilised side by side.  Slot s holds what StreamState + CropState hold for one video (the
+    history rings, a device-resident ring head, `all_black`), and one step advances every slot by one frame with one set of
+    launches: the deploy loop of deploy_bundle.py:259-328 for all slots at once, each slot bit-identical to its own pipeline.
+
+        sb = StreamBatch(4, (1080, 1920))               # 4 slots of 1080p BGR frames, network size 288x512
+        sb.join(0, first_bgr)                           # slot 0 starts a video: [1080,1920,3] uint8
+        for raw in frames:                              # raw: [4,1080,1920,3] uint8 on the device, one frame per slot
+            colour = sb.step(raw, net)                  # [4,288,512,3] uint8: the stabilised frames
+        top, left, bottom, right = sb.leave(0)          # slot 0's video ends: its crop rectangle
+
+    net(in_x) takes the assembled input [S,h,w,nch] and returns (out [S,h,w,1], black [S,h,w], xy [S,h,w,2]): the network plus
+    the multi-grid warp (out / black / img of the transformer), as StreamState's `net` does for one video.
+
+    Every slot is computed at every step.  A slot that carries no video (never joined, or left and not joined again) runs on
+    whatever frame the caller puts there and its output means nothing: the caller decides which slots carry a video and
+    ignores the others.  All buffers are allocated here and never reallocated, so a step can be captured once as a CUDA graph
+    (capture()) and replayed; join / leave between replays act on the same buffers."""
+
+    def __init__(self, S, src_size, height=288, width=512, depth=32, taps=(1, 2, 4, 8, 16, 32), use_masks=True, crop_rate=1, refine=1,
+                 device='cuda'):
+        S, H, W, h, w = int(S), int(src_size[0]), int(src_size[1]), int(height), int(width)
+        if S < 1 or refine < 1:
+            raise ValueError('StreamBatch needs S >= 1 and refine >= 1 (got S=%d, refine=%d)' % (S, refine))
+        self.taps = tuple(int(t) for t in taps)
+        if not 1 <= len(self.taps) <= 32 or any(t < 1 or t > depth for t in self.taps):
+            raise ValueError('taps %s: 1 to 32 distances in [1, depth = %d]' % (self.taps, depth))
+        dev = torch.device(device)
+        self.S, self.src_size, self.height, self.width, self.depth = S, (H, W), h, w, int(depth)
+        self.use_masks, self.crop_rate, self.refine = bool(use_masks), crop_rate, int(refine)
+        self.nch = (2 if use_masks else 1) * len(self.taps) + 1
+        f32 = dict(device=dev, dtype=torch.float32)
+        self.frames = torch.zeros((S, depth, h, w), **f32)
+        self.masks = torch.zeros((S, depth, h, w), **f32)
+        self.heads_dev = torch.full((S,), depth - 1, device=dev, dtype=torch.int32)
+        self.all_black = torch.zeros((S, h, w), device=dev, dtype=torch.int32)
+        # per-step buffers: the network frames, the horizontal pass of cvt_img2train, the network input, the resized and the
+        # stabilised colour frames, the /4 maps of warpRevBundle2
+        self.cur = torch.empty((S, h, w), **f32)
+        self.cvt_tmp = torch.empty((S, H, w), device=dev, dtype=torch.uint8)
+        self.in_x = torch.empty((S, h, w, self.nch), **f32)
+        self.small = torch.empty((S, h, w, 3), device=dev, dtype=torch.uint8)
+        self.colour = torch.empty((S, h, w, 3), device=dev, dtype=torch.uint8)
+        self.remap_ws = torch.empty(ops.remap_bundle_workspace_floats(S, h, w), **f32)
+        self._cvt = _cvt_tables(H, W, h, w, crop_rate, dev)
+        self._resize = _resize_tables(H, W, h, w, dev)
+
+    def _slot(self, slot):
+        if not isinstance(slot, (int, np.integer)) or not 0 <= slot < self.S:
+            raise ValueError('slot %r outside [0, %d)' % (slot, self.S))
+        return int(slot)
+
+    def join(self, slot, first):
+        """A new video starts in `slot`: its first frame (a BGR uint8 frame [H,W,3], or a network frame [h,w] fp32 already in
+        cvt_img2train's format) fills the frames ring, the masks ring and all_black are zeroed and the head is reset -- what
+        StreamState(first) and CropState() construct for one video."""
+        s = self._slot(slot)
+        dev = self.frames.device
+        f = torch.as_tensor(np.ascontiguousarray(first)) if isinstance(first, np.ndarray) else first
+        if f.dtype == torch.uint8:
+            if tuple(f.shape) != self.src_size + (3,):
+                raise ValueError('first frame must be [%d,%d,3] uint8 (got %s)' % (self.src_size + (tuple(f.shape),)))
+            f = cvt_img2train(f.to(dev), self.crop_rate, self.height, self.width).reshape(self.height, self.width)
+        elif tuple(f.shape) != (self.height, self.width):
+            raise ValueError('a network frame must be [%d,%d] (got %s)' % (self.height, self.width, tuple(f.shape)))
+        self.frames[s].copy_(f.to(device=dev, dtype=torch.float32).expand(self.depth, self.height, self.width))
+        self.masks[s].zero_()
+        self.heads_dev[s].fill_(self.depth - 1)
+        self.all_black[s].zero_()
+
+    def leave(self, slot, step=10):
+        """The video in `slot` has ended: its crop rectangle [top, left, bottom, right] (CropState.rect).  The slot's state is
+        left as it is until the next join."""
+        return _crop_rect(self.all_black[self._slot(slot)], step)
+
+    def advance(self, cur, net):
+        """One frame of every slot from network frames cur [S,h,w] (cvt_img2train's format): input assembly from the rings,
+        `refine` x (net, black accumulation, re-feed of the current-frame channel), ring push.  Returns the last xy [S,h,w,2]."""
+        S, h, w, nch = self.S, self.height, self.width, self.nch
+        masks = self.masks if self.use_masks else None
+        in_x = ops.streams_assemble(self.frames, masks, self.heads_dev, self.taps, cur, self.use_masks, out=self.in_x)
+        for _ in range(self.refine):
+            out, black, xy = net(in_x)
+            if out.numel() != S * h * w or black.numel() != S * h * w or tuple(xy.shape) != (S, h, w, 2):
+                raise ValueError('net must return out [S,h,w,1], black [S,h,w] and xy [S,h,w,2] (S=%d, %dx%d)' % (S, h, w))
+            ops.black_accumulate(self.all_black, black)
+            ops.stream_push(None, None, 0, out.reshape(S * h, w), black.reshape(S * h, w), refeed_into=in_x.view(1, S * h, w, nch))
+        ops.streams_push(self.frames, self.masks, self.heads_dev, out.reshape(S, h, w), black.reshape(S, h, w))
+        return xy
+
+    def step(self, raw_bgr, net):
+        """One frame of every slot from raw_bgr [S,H,W,3] uint8 on the device: cvt_img2train, advance(), cv2_resize of the
+        colour frames and warpRevBundle2 with the last xy.  Returns the stabilised colour frames [S,h,w,3] uint8 (self.colour,
+        overwritten by the next step)."""
+        raw = ops._chk(raw_bgr, 'raw_bgr', torch.uint8)
+        if tuple(raw.shape) != (self.S,) + self.src_size + (3,):
+            raise ValueError('raw_bgr must be [%d,%d,%d,3] uint8 (got %s)' % ((self.S,) + self.src_size + (tuple(raw.shape),)))
+        h, w = self.height, self.width
+        cur = ops.cvt_img2train_u8_batch(raw, self._cvt, h, w, out=self.cur, tmp=self.cvt_tmp)
+        xy = self.advance(cur, net)
+        small = ops.resize_linear_u8_batch(raw, self._resize[0], self._resize[1], h, w, out=self.small)
+        return ops.remap_bundle_u8(small, xy, out=self.colour, workspace=self.remap_ws)
+
+    def capture(self, raw_bgr, net, upload_from=None, download_to=None):
+        """Records step(raw_bgr, net) as a CUDA graph and returns it: graph.replay() runs one step on whatever raw_bgr holds and
+        leaves the frames in self.colour.  upload_from / download_to: optional host buffers ([S,H,W,3] / [S,h,w,3] uint8,
+        pinned) copied into raw_bgr before and out of self.colour after the step, inside the graph.  One eager step runs first
+        on a side stream as a warm-up (a network may select algorithms or allocate on its first call); the state it changed
+        is restored, so capturing leaves every slot as it was."""
+        state = (self.frames, self.masks, self.heads_dev, self.all_black)
+        snap = [t.clone() for t in state]
+        side = torch.cuda.Stream(device=self.frames.device)
+        side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(side):
+            self.step(raw_bgr, net)
+        torch.cuda.current_stream().wait_stream(side)
+        for t, v in zip(state, snap):
+            t.copy_(v)
+        graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(graph):
+            if upload_from is not None:
+                raw_bgr.copy_(upload_from, non_blocking=True)
+            self.step(raw_bgr, net)
+            if download_to is not None:
+                download_to.copy_(self.colour, non_blocking=True)
+        return graph

@@ -424,18 +424,26 @@ def temp_loss_bwd(out1, black1, out2, black2, flow, sums, upstream):
     return d1, d2
 
 
-def remap_bundle_u8(img, xy):
+def remap_bundle_u8(img, xy, out=None, workspace=None):
     """deploy_bundle.py:136-146 on the device: img [N,H,W,C] uint8, xy [N,H,W,2] fp32 (x_map,y_map interleaved, the `img`
-    output of warp_fwd) -> [N,H,W,C] uint8.  One C-ABI call (two launches)."""
+    output of warp_fwd) -> [N,H,W,C] uint8.  One C-ABI call (two launches).  out / workspace: optional preallocated result and
+    fp32 scratch of remap_bundle_workspace_floats(N, H, W) (static buffers for CUDA-graph capture)."""
     img, xy = _chk(img, 'img', torch.uint8), _chk(xy, 'xy')
     if img.dim() != 4 or xy.dim() != 4 or xy.shape[3] != 2 or xy.shape[:3] != img.shape[:3]:
         raise ValueError('img must be [N,H,W,C] uint8 and xy [N,H,W,2] (got %s, %s)' % (tuple(img.shape), tuple(xy.shape)))
     n, h, w, c = img.shape
-    dst = torch.empty_like(img)
-    ws = torch.empty(max(lib.mgw_remap_bundle_u8_workspace_bytes(n, h, w) // 4, 2), device=img.device, dtype=torch.float32)
+    dst = _out(out, tuple(img.shape), img.device, torch.uint8, 'out')
+    ws = (torch.empty(remap_bundle_workspace_floats(n, h, w), device=img.device, dtype=torch.float32) if workspace is None
+          else _chk_out(workspace, 'workspace'))
+    if ws.numel() < remap_bundle_workspace_floats(n, h, w):
+        raise ValueError('workspace needs %d floats' % remap_bundle_workspace_floats(n, h, w))
     with torch.cuda.device(img.device):
         check(lib.mgw_remap_bundle_u8(_p(img), _p(xy), n, h, w, c, _p(dst), _p(ws), _st()), 'mgw_remap_bundle_u8')
     return dst
+
+
+def remap_bundle_workspace_floats(n, h, w):
+    return max(lib.mgw_remap_bundle_u8_workspace_bytes(n, h, w) // 4, 2)
 
 
 def stream_assemble(frames, masks, head, taps, cur, use_masks=True):
@@ -623,3 +631,83 @@ def stream_push_dev(frames, masks, head_dev, img, black):
     depth, h, w = frames.shape
     with torch.cuda.device(frames.device):
         check(lib.mgw_stream_push_dev(_p(frames), _p(masks), depth, _p(head_dev), _p(img), _p(black), h, w, _st()), 'mgw_stream_push_dev')
+
+
+# ---- several videos of one size at once (deploy.StreamBatch): one launch per stage for all S streams, each stream's result
+# bit-identical to the single-stream call on its slice.  `out` / `tmp`: optional preallocated buffers (CUDA-graph capture).
+def _out(out, shape, dev, dtype, name):
+    if out is None:
+        return torch.empty(shape, device=dev, dtype=dtype)
+    out = _chk_out(out, name, dtype)
+    if tuple(out.shape) != tuple(shape):
+        raise ValueError('%s must be %s (got %s)' % (name, tuple(shape), tuple(out.shape)))
+    return out
+
+
+def cvt_img2train_u8_batch(bgr, tables, out_h, out_w, out=None, tmp=None):
+    """cvt_img2train_u8 for bgr [S,H,W,3] uint8 (one size, shared tables) -> [S,out_h,out_w] fp32."""
+    bgr = _chk(bgr, 'bgr', torch.uint8)
+    kx, x0, xn, ky, y0, yn = (_chk(t, 'table', torch.int32) for t in tables)
+    if bgr.dim() != 4 or bgr.shape[3] != 3 or kx.shape[0] != out_w or ky.shape[0] != out_h:
+        raise ValueError('bgr must be [S,H,W,3] and the tables must cover the %dx%d output (got %s)' % (out_h, out_w, tuple(bgr.shape)))
+    s, h, w, _ = bgr.shape
+    tmp = _out(tmp, (s, h, out_w), bgr.device, torch.uint8, 'tmp')
+    out = _out(out, (s, out_h, out_w), bgr.device, torch.float32, 'out')
+    with torch.cuda.device(bgr.device):
+        check(lib.mgw_cvt_img2train_u8_batch(_p(bgr), s, h, w, _p(kx), _p(x0), _p(xn), kx.shape[1], _p(ky), _p(y0), _p(yn), ky.shape[1],
+                                             out_h, out_w, _p(tmp), _p(out), _st()), 'mgw_cvt_img2train_u8_batch')
+    return out
+
+
+def resize_linear_u8_batch(img, xtab, ytab, out_h, out_w, out=None):
+    """resize_linear_u8 for img [S,H,W,C] uint8 (one size, shared tables) -> [S,out_h,out_w,C]."""
+    img = _chk(img, 'img', torch.uint8)
+    if img.dim() != 4:
+        raise ValueError('img must be [S,H,W,C] (got %s)' % (tuple(img.shape),))
+    s, h, w, c = img.shape
+    xtab = None if xtab is None else _chk(xtab, 'xtab', torch.int32)
+    ytab = None if ytab is None else _chk(ytab, 'ytab', torch.int32)
+    dst = _out(out, (s, out_h, out_w, c), img.device, torch.uint8, 'out')
+    with torch.cuda.device(img.device):
+        check(lib.mgw_resize_linear_u8_batch(_p(img), s, h, w, c, _p(xtab), _p(ytab), out_h, out_w, _p(dst), _st()),
+              'mgw_resize_linear_u8_batch')
+    return dst
+
+
+def _streams_dims(frames, heads_dev, what):
+    if frames.dim() != 4:
+        raise ValueError('%s must be [S,depth,H,W] rings (got %s)' % (what, tuple(frames.shape)))
+    s, depth, h, w = frames.shape
+    if tuple(heads_dev.shape) != (s,):
+        raise ValueError('heads_dev must be [%d] (got %s)' % (s, tuple(heads_dev.shape)))
+    return s, depth, h, w
+
+
+def streams_assemble(frames, masks, heads_dev, taps, cur, use_masks=True, out=None):
+    """stream_assemble_dev for S streams: frames / masks [S,depth,H,W], heads_dev int32 [S], cur [S,H,W] -> in_x [S,H,W,nch]."""
+    import ctypes
+    frames, cur, heads_dev = _chk(frames, 'frames'), _chk(cur, 'cur'), _chk(heads_dev, 'heads_dev', torch.int32)
+    s, depth, h, w = _streams_dims(frames, heads_dev, 'frames')
+    masks = _chk(masks, 'masks') if use_masks else None
+    if (masks is not None and masks.shape != frames.shape) or tuple(cur.shape) != (s, h, w):
+        raise ValueError('masks must have the shape of frames and cur must be [%d,%d,%d]' % (s, h, w))
+    nch = (2 if use_masks else 1) * len(taps) + 1
+    in_x = _out(out, (s, h, w, nch), frames.device, torch.float32, 'out')
+    arr = (ctypes.c_int * len(taps))(*[int(t) for t in taps])
+    with torch.cuda.device(frames.device):
+        check(lib.mgw_streams_assemble(_p(frames), _p(masks), s, depth, _p(heads_dev), arr, len(taps), 1 if use_masks else 0, _p(cur),
+                                       h, w, _p(in_x), _st()), 'mgw_streams_assemble')
+    return in_x
+
+
+def streams_push(frames, masks, heads_dev, img, black):
+    """stream_push_dev for S streams: frame = img + black*(-1) and black [S,H,W] into the slot after each stream's head, then
+    every head advances."""
+    frames, heads_dev = _chk_out(frames, 'frames'), _chk_out(heads_dev, 'heads_dev', torch.int32)
+    img, black = _chk(img, 'img'), _chk(black, 'black')
+    masks = None if masks is None else _chk_out(masks, 'masks')
+    s, depth, h, w = _streams_dims(frames, heads_dev, 'frames')
+    if (masks is not None and masks.shape != frames.shape) or img.numel() != s * h * w or black.numel() != s * h * w:
+        raise ValueError('masks must have the shape of frames and img / black %d x %d x %d pixels' % (s, h, w))
+    with torch.cuda.device(frames.device):
+        check(lib.mgw_streams_push(_p(frames), _p(masks), s, depth, _p(heads_dev), _p(img), _p(black), h, w, _st()), 'mgw_streams_push')

@@ -246,6 +246,27 @@ MGW_API int mgw_stream_assemble_dev(const float* frames, const float* masks, int
 MGW_API int mgw_stream_push_dev(float* frames, float* masks, int depth, int32_t* head_dev, const float* img, const float* black,
                         int H, int W, void* stream);
 
+/* ---- f1/f2 batched: S independent videos of one source size advanced by one set of launches ----------------------------
+ * Every per-stream result is bit-identical to the single-stream call on that stream's slice.  0 <= S <= 65535; S = 0 returns
+ * MGW_OK and launches nothing.
+ * mgw_cvt_img2train_u8_batch: bgr [S,H,W,3] -> out [S,out_h,out_w]; the tables as for mgw_cvt_img2train_u8 (shared by all S
+ *   frames), tmp: S*H*out_w bytes.
+ * mgw_resize_linear_u8_batch: img [S,H,W,C] -> dst [S,out_h,out_w,C]; the tables as for mgw_resize_linear_u8.
+ * mgw_streams_assemble: frames, masks [S,depth,H,W] (stream s's rings are byte for byte those of mgw_stream_assemble_dev),
+ *   heads_dev [S] int32 (device), cur [S,H,W] -> in_x [S,H,W,nch].
+ * mgw_streams_push: img, black [S,H,W]: writes slot heads_dev[s]+1 of every stream, then advances all S heads (two launches).
+ * The refine re-feed and mgw_black_accumulate are element-wise: call mgw_stream_push (frame_out, H = S*H) and
+ * mgw_black_accumulate (n = S*H*W) on the [S,H,W] buffers as they are. */
+MGW_API int mgw_cvt_img2train_u8_batch(const uint8_t* bgr, int S, int H, int W, const int32_t* kx, const int32_t* x0, const int32_t* xn,
+                               int ksx, const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h, int out_w,
+                               uint8_t* tmp, float* out, void* stream);
+MGW_API int mgw_resize_linear_u8_batch(const uint8_t* img, int S, int H, int W, int C, const int32_t* xtab, const int32_t* ytab,
+                               int out_h, int out_w, uint8_t* dst, void* stream);
+MGW_API int mgw_streams_assemble(const float* frames, const float* masks, int S, int depth, const int32_t* heads_dev, const int* taps,
+                         int ntaps, int use_masks, const float* cur, int H, int W, float* in_x, void* stream);
+MGW_API int mgw_streams_push(float* frames, float* masks, int S, int depth, int32_t* heads_dev, const float* img, const float* black,
+                     int H, int W, void* stream);
+
 /* ---- a6: interpolate(im, x, y, out_size), spatial_transformer.py:200-281 ------------------------------
  * im [N,IH,IW,C]; x,y [N,OH,OW] normalised coords -> out [N,OH,OW,C]. */
 MGW_API int mgw_interp_fwd(const float* im, const float* x, const float* y, int N, int IH, int IW, int C, int OH, int OW,
