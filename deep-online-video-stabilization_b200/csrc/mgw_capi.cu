@@ -85,7 +85,7 @@ using namespace mgw;
 
 extern "C" {
 
-int mgw_version(void) { return 101; }
+int mgw_version(void) { return 102; }
 
 const char* mgw_last_error(void) { return g_err; }
 
@@ -640,6 +640,38 @@ int mgw_resize_linear_u8_batch(const uint8_t* img, int S, int H, int W, int C, c
     REQUIRE((W == 2 * out_w && H == 2 * out_h) || (xtab && ytab), "mgw_resize_linear_u8_batch: coefficient tables are required");
     REQUIRE((!xtab || aligned(xtab, 16)) && (!ytab || aligned(ytab, 16)), "mgw_resize_linear_u8_batch: tables must be 16-byte aligned");
     return launch_resize_linear_u8(img, S, H, W, C, xtab, ytab, out_h, out_w, dst, (cudaStream_t)stream);
+}
+
+// YUV 4:2:0 frames [S,3H/2,W]: the BGR batch calls' checks in the same order, their 32-bit index limit taken over the YUV bytes
+static int validate_yuv420(const char* fn, int format, int S, int H, int W, int out_h, int out_w)
+{
+    REQUIRE(S >= 0 && S <= 65535 && H > 0 && W > 0 && H % 2 == 0 && W % 2 == 0 && out_h > 0 && out_w > 0 &&
+            (long long)S * (H + H / 2) * W < (1LL << 31) && (long long)S * H * out_w < (1LL << 31) && (long long)S * out_h * out_w < (1LL << 29),
+            "%s: bad sizes (S=%d H=%d W=%d out %dx%d; H and W must be even)", fn, S, H, W, out_h, out_w);
+    REQUIRE(format == MGW_YUV420_NV12 || format == MGW_YUV420_I420, "%s: unknown format %d", fn, format);
+    return MGW_OK;
+}
+
+int mgw_cvt_img2train_yuv420_batch(const uint8_t* yuv, int format, int S, int H, int W, const int32_t* kx, const int32_t* x0,
+                                   const int32_t* xn, int ksx, const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h,
+                                   int out_w, uint8_t* tmp, float* out, void* stream)
+{
+    TRY(validate_yuv420("mgw_cvt_img2train_yuv420_batch", format, S, H, W, out_h, out_w));
+    REQUIRE(ksx > 0 && ksy > 0, "mgw_cvt_img2train_yuv420_batch: bad sizes (ksx=%d ksy=%d)", ksx, ksy);
+    if (S == 0) return MGW_OK;
+    REQUIRE(yuv && kx && x0 && xn && ky && y0 && yn && tmp && out, "mgw_cvt_img2train_yuv420_batch: null pointer");
+    return launch_cvt_img2train_u8(yuv, S, H, W, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w, tmp, out, (cudaStream_t)stream, format);
+}
+
+int mgw_resize_linear_yuv420_batch(const uint8_t* yuv, int format, int S, int H, int W, const int32_t* xtab, const int32_t* ytab,
+                                   int out_h, int out_w, uint8_t* dst, void* stream)
+{
+    TRY(validate_yuv420("mgw_resize_linear_yuv420_batch", format, S, H, W, out_h, out_w));
+    if (S == 0) return MGW_OK;
+    REQUIRE(yuv && dst, "mgw_resize_linear_yuv420_batch: null pointer");
+    REQUIRE((W == 2 * out_w && H == 2 * out_h) || (xtab && ytab), "mgw_resize_linear_yuv420_batch: coefficient tables are required");
+    REQUIRE((!xtab || aligned(xtab, 16)) && (!ytab || aligned(ytab, 16)), "mgw_resize_linear_yuv420_batch: tables must be 16-byte aligned");
+    return launch_resize_linear_u8(yuv, S, H, W, 3, xtab, ytab, out_h, out_w, dst, (cudaStream_t)stream, format);
 }
 
 static int validate_streams(const char* fn, int S, int depth, int H, int W, int nch)

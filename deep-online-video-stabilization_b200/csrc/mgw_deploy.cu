@@ -186,24 +186,83 @@ int launch_remap_bundle_u8(const uint8_t* img, const float* xy, int N, int H, in
 // and slices them for the crop; the two passes below are Pillow's: horizontal first into a uint8 image, then vertical.
 // A batch of S frames of one size shares the tables; blockIdx.y is the frame (the stream index of a StreamBatch): each block
 // offsets its base pointers once, the per-pixel index arithmetic is the single-frame one, and S = 1 is the single-frame call.
+// The source frame is BGR (SRC_BGR) or YUV 4:2:0 in OpenCV's layout (MGW_YUV420_NV12 / MGW_YUV420_I420): the kernels then read
+// the BGR frame cv2.cvtColor would make of it, converted per pixel on the fly.
 namespace {
 
+constexpr int SRC_BGR = 0;
+
+// cv2.cvtColor(COLOR_YUV2BGR_NV12 / _I420), color_yuv.simd.hpp: BT.601 limited range in 20-bit fixed point, one chroma sample per
+// 2x2 block, no chroma interpolation.  The chroma terms (rounding constant included) are formed once per chroma sample.
+struct Chroma { int r, g, b; };
+
+__device__ __forceinline__ Chroma yuv_chroma(int U, int V)
+{
+    const int u = U - 128, v = V - 128;
+    return Chroma{(1 << 19) + 1673527 * v, (1 << 19) - 852492 * v - 409993 * u, (1 << 19) + 2116026 * u};
+}
+
+// the per-pixel half: y = max(0, Y-16)*CY, channel = sat8((y + chroma term) >> 20); every sum fits int32
+__device__ __forceinline__ int3 yuv_to_bgr(int Y, const Chroma& c)
+{
+    const int y = max(Y - 16, 0) * 1220542;
+    return make_int3(min(max((y + c.b) >> 20, 0), 255), min(max((y + c.g) >> 20, 0), 255), min(max((y + c.r) >> 20, 0), 255));
+}
+
+// the chroma sample of pixel (row, x) in a frame [3H/2, W]: after the H*W bytes of the Y plane, NV12 interleaves U,V in rows of W
+// bytes; I420 has the U plane (H/2 rows of W/2) and then the V plane -- contiguous planes, so byte offsets, not row offsets
+template <int FMT>
+__device__ __forceinline__ Chroma yuv_chroma_at(const uint8_t* __restrict__ f, int H, int W, int row, int x)
+{
+    const uint8_t* c = f + (size_t)H * W;
+    if constexpr (FMT == MGW_YUV420_NV12) {
+        const uint8_t* p = c + (size_t)(row >> 1) * W + (x & ~1);
+        return yuv_chroma(__ldg(p), __ldg(p + 1));
+    } else {
+        const uint8_t* p = c + (size_t)(row >> 1) * (W >> 1) + (x >> 1);
+        return yuv_chroma(__ldg(p), __ldg(p + (size_t)(H >> 1) * (W >> 1)));
+    }
+}
+
+// bytes of one source frame: a batch's frames are contiguous
+template <int FMT>
+__device__ __forceinline__ size_t src_frame_bytes(int H, int W)
+{
+    return FMT == SRC_BGR ? (size_t)H * W * 3 : (size_t)H * W * 3 / 2;
+}
+
+template <int FMT>
 __global__ void __launch_bounds__(256)
 gray_hpass_kernel(const uint8_t* __restrict__ bgr, int H, int W, const int32_t* __restrict__ kx, const int32_t* __restrict__ x0,
                   const int32_t* __restrict__ xn, int ks, int out_w, uint8_t* __restrict__ tmp)
 {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= H * out_w) return;
-    bgr += (size_t)blockIdx.y * H * W * 3;
     tmp += (size_t)blockIdx.y * H * out_w;
     const int xx = t % out_w, row = t / out_w;
-    const uint8_t* p = bgr + ((size_t)row * W + __ldg(x0 + xx)) * 3;
     const int n = __ldg(xn + xx);
     int acc = 1 << 21;
-    for (int k = 0; k < n; ++k, p += 3) {
-        // RGB2Gray<uchar>: (B*3735 + G*19235 + R*9798 + 2^14) >> 15
-        const int g = ((int)__ldg(p) * 3735 + (int)__ldg(p + 1) * 19235 + (int)__ldg(p + 2) * 9798 + (1 << 14)) >> 15;
-        acc += g * __ldg(kx + (size_t)xx * ks + k);
+    if constexpr (FMT == SRC_BGR) {
+        bgr += (size_t)blockIdx.y * H * W * 3;
+        const uint8_t* p = bgr + ((size_t)row * W + __ldg(x0 + xx)) * 3;
+        for (int k = 0; k < n; ++k, p += 3) {
+            // RGB2Gray<uchar>: (B*3735 + G*19235 + R*9798 + 2^14) >> 15
+            const int g = ((int)__ldg(p) * 3735 + (int)__ldg(p + 1) * 19235 + (int)__ldg(p + 2) * 9798 + (1 << 14)) >> 15;
+            acc += g * __ldg(kx + (size_t)xx * ks + k);
+        }
+    } else {
+        // the BGR pixel cvtColor makes, then the same gray; a pair of pixels (even x, x+1) shares one chroma sample
+        const uint8_t* f = bgr + (size_t)blockIdx.y * src_frame_bytes<FMT>(H, W);
+        const int xs = __ldg(x0 + xx);
+        const uint8_t* py = f + (size_t)row * W + xs;
+        Chroma c;
+#pragma unroll 1        // unrolled, the NV12 loop spills at 40 registers; rolled, both formats take 32 and none
+        for (int k = 0; k < n; ++k) {
+            if (k == 0 || ((xs + k) & 1) == 0) c = yuv_chroma_at<FMT>(f, H, W, row, xs + k);
+            const int3 p = yuv_to_bgr(__ldg(py + k), c);
+            const int g = (p.x * 3735 + p.y * 19235 + p.z * 9798 + (1 << 14)) >> 15;
+            acc += g * __ldg(kx + (size_t)xx * ks + k);
+        }
     }
     tmp[t] = (uint8_t)min(max(acc >> 22, 0), 255);
 }
@@ -230,9 +289,15 @@ vpass_norm_kernel(const uint8_t* __restrict__ tmp, int H, int out_w, const int32
 
 int launch_cvt_img2train_u8(const uint8_t* bgr, int S, int H, int W, const int32_t* kx, const int32_t* x0, const int32_t* xn, int ksx,
                             const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h, int out_w, uint8_t* tmp,
-                            float* out, cudaStream_t st)
+                            float* out, cudaStream_t st, int src_fmt)
 {
-    gray_hpass_kernel<<<dim3((H * out_w + 255) / 256, S), 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp);
+    const dim3 g1((H * out_w + 255) / 256, S);
+    switch (src_fmt) {
+    case SRC_BGR: gray_hpass_kernel<SRC_BGR><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp); break;
+    case MGW_YUV420_NV12: gray_hpass_kernel<MGW_YUV420_NV12><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp); break;
+    case MGW_YUV420_I420: gray_hpass_kernel<MGW_YUV420_I420><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp); break;
+    default: return set_error(MGW_ERR_INVALID, "cvt_img2train: unknown source format %d", src_fmt);
+    }
     if (int rc = check_launch("gray_hpass")) return rc;
     vpass_norm_kernel<<<dim3((out_h * out_w + 255) / 256, S), 256, 0, st>>>(tmp, H, out_w, ky, y0, yn, ksy, out_h, out);
     return check_launch("vpass_norm");
@@ -245,13 +310,51 @@ int launch_cvt_img2train_u8(const uint8_t* bgr, int S, int H, int W, const int32
 // blockIdx.y is the frame of a batch of S frames of one size (as for cvt_img2train above).
 namespace {
 
-template <int C>
+// a YUV 4:2:0 source (FMT = MGW_YUV420_*, C = 3) is resampled as the BGR frame cvtColor makes of it: each tap is converted
+template <int FMT>
+__device__ __forceinline__ int3 yuv_bgr_at(const uint8_t* __restrict__ f, int H, int W, int row, int x)
+{
+    return yuv_to_bgr(__ldg(f + (size_t)row * W + x), yuv_chroma_at<FMT>(f, H, W, row, x));
+}
+
+__device__ __forceinline__ int ch_of(const int3& p, int ch) { return ch == 0 ? p.x : (ch == 1 ? p.y : p.z); }
+
+template <int C, int FMT = SRC_BGR>
 __global__ void __launch_bounds__(256)
 resize_u8_kernel(const uint8_t* __restrict__ img, int H, int W, const int4* __restrict__ xtab, const int4* __restrict__ ytab,
                  int out_h, int out_w, int area2, uint8_t* __restrict__ dst)
 {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= out_h * out_w) return;
+    if constexpr (FMT != SRC_BGR) {
+        static_assert(C == 3, "a YUV 4:2:0 source resizes to BGR");
+        const uint8_t* f = img + (size_t)blockIdx.y * src_frame_bytes<FMT>(H, W);
+        dst += (size_t)blockIdx.y * out_h * out_w * 3;
+        const int x = t % out_w, y = t / out_w;
+        uint8_t* o = dst + (size_t)t * 3;
+        if (area2) {
+            // the 2x2 block starts at even coordinates: four Y samples, one chroma sample
+            const uint8_t* py = f + (size_t)(2 * y) * W + 2 * x;
+            const Chroma c = yuv_chroma_at<FMT>(f, H, W, 2 * y, 2 * x);
+            const int3 p00 = yuv_to_bgr(__ldg(py), c), p01 = yuv_to_bgr(__ldg(py + 1), c);
+            const int3 p10 = yuv_to_bgr(__ldg(py + W), c), p11 = yuv_to_bgr(__ldg(py + W + 1), c);
+            o[0] = (uint8_t)((p00.x + p01.x + p10.x + p11.x + 2) >> 2);
+            o[1] = (uint8_t)((p00.y + p01.y + p10.y + p11.y + 2) >> 2);
+            o[2] = (uint8_t)((p00.z + p01.z + p10.z + p11.z + 2) >> 2);
+            return;
+        }
+        const int4 xt = __ldg(xtab + x), yt = __ldg(ytab + y);        // {i0, i1, a0, a1}
+        const int3 p00 = yuv_bgr_at<FMT>(f, H, W, yt.x, xt.x), p01 = yuv_bgr_at<FMT>(f, H, W, yt.x, xt.y);
+        const int3 p10 = yuv_bgr_at<FMT>(f, H, W, yt.y, xt.x), p11 = yuv_bgr_at<FMT>(f, H, W, yt.y, xt.y);
+#pragma unroll
+        for (int ch = 0; ch < 3; ++ch) {
+            const int h0 = ch_of(p00, ch) * xt.z + ch_of(p01, ch) * xt.w;
+            const int h1 = ch_of(p10, ch) * xt.z + ch_of(p11, ch) * xt.w;
+            const int v = (((yt.z * (h0 >> 4)) >> 16) + ((yt.w * (h1 >> 4)) >> 16) + 2) >> 2;
+            o[ch] = (uint8_t)min(max(v, 0), 255);
+        }
+        return;
+    }
     img += (size_t)blockIdx.y * H * W * C;
     dst += (size_t)blockIdx.y * out_h * out_w * C;
     const int x = t % out_w, y = t / out_w;
@@ -279,13 +382,22 @@ resize_u8_kernel(const uint8_t* __restrict__ img, int H, int W, const int4* __re
 }  // namespace
 
 int launch_resize_linear_u8(const uint8_t* img, int S, int H, int W, int C, const int32_t* xtab, const int32_t* ytab, int out_h, int out_w,
-                            uint8_t* dst, cudaStream_t st)
+                            uint8_t* dst, cudaStream_t st, int src_fmt)
 {
     const int area2 = (W == 2 * out_w && H == 2 * out_h) ? 1 : 0;
     if (!area2 && (!xtab || !ytab)) return set_error(MGW_ERR_INVALID, "resize_linear_u8: coefficient tables are required");
     const dim3 grid((out_h * out_w + 255) / 256, S);
     const int4* xt = reinterpret_cast<const int4*>(xtab);
     const int4* yt = reinterpret_cast<const int4*>(ytab);
+    if (src_fmt != SRC_BGR) {
+        if (C != 3) return set_error(MGW_ERR_UNSUPPORTED, "resize_linear_u8: a YUV 4:2:0 source gives C = 3 (got %d)", C);
+        switch (src_fmt) {
+        case MGW_YUV420_NV12: resize_u8_kernel<3, MGW_YUV420_NV12><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst); break;
+        case MGW_YUV420_I420: resize_u8_kernel<3, MGW_YUV420_I420><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst); break;
+        default: return set_error(MGW_ERR_INVALID, "resize_linear_u8: unknown source format %d", src_fmt);
+        }
+        return check_launch("resize_u8");
+    }
     switch (C) {
     case 1: resize_u8_kernel<1><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst); break;
     case 3: resize_u8_kernel<3><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst); break;

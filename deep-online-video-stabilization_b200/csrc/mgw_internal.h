@@ -112,12 +112,13 @@ size_t remap_bundle_workspace_bytes(int N, int H, int W);
 int launch_remap_bundle_u8(const uint8_t* img, const float* xy, int N, int H, int W, int C, uint8_t* dst, void* workspace,
                            cudaStream_t st);
 
-// S frames of one size ([S,H,W,C] -> [S,out_h,out_w,C]; S >= 1, the single-frame calls pass 1)
+// S frames of one size ([S,H,W,C] -> [S,out_h,out_w,C]; S >= 1, the single-frame calls pass 1).  src_fmt: 0 for the BGR / C-channel
+// frames, MGW_YUV420_NV12 or MGW_YUV420_I420 for YUV 4:2:0 frames [S,3H/2,W] read as the BGR frames cvtColor makes of them (C = 3)
 int launch_resize_linear_u8(const uint8_t* img, int S, int H, int W, int C, const int32_t* xtab, const int32_t* ytab, int out_h, int out_w,
-                            uint8_t* dst, cudaStream_t st);
+                            uint8_t* dst, cudaStream_t st, int src_fmt = 0);
 int launch_cvt_img2train_u8(const uint8_t* bgr, int S, int H, int W, const int32_t* kx, const int32_t* x0, const int32_t* xn, int ksx,
                             const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h, int out_w, uint8_t* tmp,
-                            float* out, cudaStream_t st);
+                            float* out, cudaStream_t st, int src_fmt = 0);
 int launch_warp_rev_bundle_u8(const uint8_t* img, const double* Hs_cvt, int N, int H, int W, int C, int gh, int gw, uint8_t* dst,
                               cudaStream_t st);
 

@@ -101,15 +101,42 @@ def _resize_tables(H, W, oh, ow, device):
     return _RESIZE_TABLES[key]
 
 
-def cv2_resize(img, dsize, device='cuda'):
+def _yuv420_frames(img, src_format):
+    """src_format 'bgr' -> None.  'nv12' / 'i420': img is a YUV 4:2:0 frame [3H/2,W] or a batch [S,3H/2,W] (uint8, OpenCV's
+    layout) -> (the frames as a uint8 tensor [S,3H/2,W] where they are, single, H, W).  Anything else is a ValueError."""
+    if src_format == 'bgr':
+        return None
+    if src_format not in ops.YUV420_FORMATS:
+        raise ValueError("src_format must be 'bgr', 'nv12' or 'i420' (got %r)" % (src_format,))
+    is_np = isinstance(img, np.ndarray)
+    if not is_np and not isinstance(img, torch.Tensor) or img.dtype != (np.uint8 if is_np else torch.uint8):
+        raise ValueError('a %s frame must be a uint8 array or tensor (got %s)' % (src_format, getattr(img, 'dtype', type(img))))
+    shape = tuple(img.shape)
+    if len(shape) not in (2, 3) or shape[-2] % 3 != 0 or shape[-2] == 0 or shape[-1] % 2 != 0 or shape[-1] == 0:
+        raise ValueError('a %s frame must be [3H/2,W] or [S,3H/2,W] with H and W even (got %s)' % (src_format, shape))
+    t = torch.as_tensor(np.ascontiguousarray(img)) if is_np else img
+    return (t.unsqueeze(0) if len(shape) == 2 else t), len(shape) == 2, shape[-2] // 3 * 2, shape[-1]
+
+
+def cv2_resize(img, dsize, device='cuda', src_format='bgr'):
     """cv2.resize(img, dsize) for a uint8 frame [H,W,C] (reference deploy_bundle.py:301 resizes the unstable colour frame to the
     network size before warpRevBundle2), byte-exact with OpenCV's INTER_LINEAR; dsize = (width, height) as in OpenCV.
     A batch [S,H,W,C] of frames of one size gives [S,height,width,C], each frame as its own call would (one launch).
-    numpy in -> numpy out; a CUDA frame stays on the device."""
+    src_format 'nv12' / 'i420': img is a YUV 4:2:0 frame [3H/2,W] (or a batch [S,3H/2,W]) in OpenCV's layout, and the result
+    is the BGR call's on cv2.cvtColor(img, COLOR_YUV2BGR_NV12 / _I420), [height,width,3] ([S,height,width,3]), with the
+    conversion done inside the kernel.  numpy in -> numpy out; a CUDA frame stays on the device."""
     as_numpy = isinstance(img, np.ndarray)
+    ow, oh = int(dsize[0]), int(dsize[1])
+    yuv = _yuv420_frames(img, src_format)
+    if yuv is not None:
+        yuv, single, H, W = yuv
+        yuv = yuv.to(device=device if as_numpy else img.device).contiguous()
+        xtab, ytab = _resize_tables(H, W, oh, ow, yuv.device)
+        dst = ops.resize_linear_yuv420_batch(yuv, src_format, xtab, ytab, oh, ow)
+        dst = dst[0] if single else dst
+        return dst.cpu().numpy() if as_numpy else dst
     im = (torch.as_tensor(np.ascontiguousarray(img)) if as_numpy else img).to(device=device if as_numpy else img.device, dtype=torch.uint8)
     H, W = int(im.shape[-3]), int(im.shape[-2])
-    ow, oh = int(dsize[0]), int(dsize[1])
     xtab, ytab = _resize_tables(H, W, oh, ow, im.device)
     if im.dim() == 4:
         dst = ops.resize_linear_u8_batch(im.contiguous(), xtab, ytab, oh, ow)
@@ -133,20 +160,30 @@ def _cvt_tables(H, W, height, width, crop_rate, device):
     return _CVT_TABLES[key]
 
 
-def cvt_img2train(img, crop_rate=1, height=288, width=512, device='cuda', as_numpy=False):
+def cvt_img2train(img, crop_rate=1, height=288, width=512, device='cuda', as_numpy=False, src_format='bgr'):
     """reference config.py:6-21 (`height`, `width` are its config globals): one BGR uint8 frame [H,W,3] -> the network's frame
     format, exact: cv2 BGR2GRAY, Pillow resize(BILINEAR) (to (width, height), or to the 1/crop_rate larger size followed by
     the centre crop), v * (1/255) - 0.5.  Returns a CUDA fp32 tensor [1,height,width,1]; as_numpy=True gives the reference's
     float64 numpy array (same values: the network's placeholder casts to fp32).  The coefficient tables are built once per
     shape on the host and kept on the device.  A batch [S,H,W,3] of frames of one size gives [S,height,width,1], each frame
-    as its own call would (one pair of launches for the batch)."""
-    im = (torch.as_tensor(np.ascontiguousarray(img)) if isinstance(img, np.ndarray) else img).to(device=device, dtype=torch.uint8)
-    H, W = int(im.shape[-3]), int(im.shape[-2])
-    tabs = _cvt_tables(H, W, height, width, crop_rate, im.device)
-    if im.dim() == 4:
-        out = ops.cvt_img2train_u8_batch(im.contiguous(), tabs, height, width).reshape(-1, height, width, 1)
+    as its own call would (one pair of launches for the batch).
+    src_format 'nv12' / 'i420': img is a YUV 4:2:0 frame [3H/2,W] (or a batch [S,3H/2,W]) in OpenCV's layout, as video
+    decoders emit it, and the result is the BGR call's on cv2.cvtColor(img, COLOR_YUV2BGR_NV12 / _I420): the conversion runs
+    inside the kernel, and the gray frame is BGR2GRAY of the converted frame (not the Y plane)."""
+    yuv = _yuv420_frames(img, src_format)
+    if yuv is not None:
+        yuv, _, H, W = yuv
+        yuv = yuv.to(device=device).contiguous()
+        tabs = _cvt_tables(H, W, height, width, crop_rate, yuv.device)
+        out = ops.cvt_img2train_yuv420_batch(yuv, src_format, tabs, height, width).reshape(-1, height, width, 1)
     else:
-        out = ops.cvt_img2train_u8(im.contiguous(), tabs, height, width).reshape(1, height, width, 1)
+        im = (torch.as_tensor(np.ascontiguousarray(img)) if isinstance(img, np.ndarray) else img).to(device=device, dtype=torch.uint8)
+        H, W = int(im.shape[-3]), int(im.shape[-2])
+        tabs = _cvt_tables(H, W, height, width, crop_rate, im.device)
+        if im.dim() == 4:
+            out = ops.cvt_img2train_u8_batch(im.contiguous(), tabs, height, width).reshape(-1, height, width, 1)
+        else:
+            out = ops.cvt_img2train_u8(im.contiguous(), tabs, height, width).reshape(1, height, width, 1)
     if not as_numpy:
         return out
     v = np.rint((out.cpu().numpy().astype(np.float64) + 0.5) * 255)          # the resampled byte, recovered exactly
@@ -280,6 +317,11 @@ class StreamBatch:
             colour = sb.step(raw, net)                  # [4,288,512,3] uint8: the stabilised frames
         top, left, bottom, right = sb.leave(0)          # slot 0's video ends: its crop rectangle
 
+    src_format='nv12' or 'i420' takes the frames as video decoders emit them, YUV 4:2:0 [3H/2,W] uint8 in OpenCV's layout
+    (src_size stays the picture's (H, W)): step() then takes [S,3H/2,W], join() a frame of that format, and every result is the
+    BGR batch's on the frames cv2.cvtColor(COLOR_YUV2BGR_NV12 / _I420) makes of them -- half the bytes to upload, and the
+    conversion runs inside the two kernels that read the source frame.
+
     net(in_x) takes the assembled input [S,h,w,nch] and returns (out [S,h,w,1], black [S,h,w], xy [S,h,w,2]): the network plus
     the multi-grid warp (out / black / img of the transformer), as StreamState's `net` does for one video.
 
@@ -289,10 +331,19 @@ class StreamBatch:
     (capture()) and replayed; join / leave between replays act on the same buffers."""
 
     def __init__(self, S, src_size, height=288, width=512, depth=32, taps=(1, 2, 4, 8, 16, 32), use_masks=True, crop_rate=1, refine=1,
-                 device='cuda'):
+                 device='cuda', src_format='bgr'):
         S, H, W, h, w = int(S), int(src_size[0]), int(src_size[1]), int(height), int(width)
         if S < 1 or refine < 1:
             raise ValueError('StreamBatch needs S >= 1 and refine >= 1 (got S=%d, refine=%d)' % (S, refine))
+        if src_format == 'bgr':
+            self.frame_shape = (H, W, 3)
+        elif src_format in ops.YUV420_FORMATS:
+            if H % 2 or W % 2:
+                raise ValueError('a %s source needs an even size (got %dx%d)' % (src_format, H, W))
+            self.frame_shape = (H * 3 // 2, W)
+        else:
+            raise ValueError("src_format must be 'bgr', 'nv12' or 'i420' (got %r)" % (src_format,))
+        self.src_format = src_format
         self.taps = tuple(int(t) for t in taps)
         if not 1 <= len(self.taps) <= 32 or any(t < 1 or t > depth for t in self.taps):
             raise ValueError('taps %s: 1 to 32 distances in [1, depth = %d]' % (self.taps, depth))
@@ -322,16 +373,16 @@ class StreamBatch:
         return int(slot)
 
     def join(self, slot, first):
-        """A new video starts in `slot`: its first frame (a BGR uint8 frame [H,W,3], or a network frame [h,w] fp32 already in
-        cvt_img2train's format) fills the frames ring, the masks ring and all_black are zeroed and the head is reset -- what
+        """A new video starts in `slot`: its first frame (a uint8 frame in the batch's format -- BGR [H,W,3], or YUV 4:2:0
+        [3H/2,W] --, or a network frame [h,w] fp32 already in cvt_img2train's format) fills the frames ring, the masks ring and all_black are zeroed and the head is reset -- what
         StreamState(first) and CropState() construct for one video."""
         s = self._slot(slot)
         dev = self.frames.device
         f = torch.as_tensor(np.ascontiguousarray(first)) if isinstance(first, np.ndarray) else first
         if f.dtype == torch.uint8:
-            if tuple(f.shape) != self.src_size + (3,):
-                raise ValueError('first frame must be [%d,%d,3] uint8 (got %s)' % (self.src_size + (tuple(f.shape),)))
-            f = cvt_img2train(f.to(dev), self.crop_rate, self.height, self.width).reshape(self.height, self.width)
+            if tuple(f.shape) != self.frame_shape:
+                raise ValueError('first frame must be %s uint8 (got %s)' % (list(self.frame_shape), tuple(f.shape)))
+            f = cvt_img2train(f.to(dev), self.crop_rate, self.height, self.width, src_format=self.src_format).reshape(self.height, self.width)
         elif tuple(f.shape) != (self.height, self.width):
             raise ValueError('a network frame must be [%d,%d] (got %s)' % (self.height, self.width, tuple(f.shape)))
         self.frames[s].copy_(f.to(device=dev, dtype=torch.float32).expand(self.depth, self.height, self.width))
@@ -360,22 +411,28 @@ class StreamBatch:
         return xy
 
     def step(self, raw_bgr, net):
-        """One frame of every slot from raw_bgr [S,H,W,3] uint8 on the device: cvt_img2train, advance(), cv2_resize of the
-        colour frames and warpRevBundle2 with the last xy.  Returns the stabilised colour frames [S,h,w,3] uint8 (self.colour,
-        overwritten by the next step)."""
+        """One frame of every slot from raw_bgr [S,H,W,3] uint8 on the device ([S,3H/2,W] for a YUV 4:2:0 batch): cvt_img2train,
+        advance(), cv2_resize of the colour frames and warpRevBundle2 with the last xy.  Returns the stabilised colour frames
+        [S,h,w,3] uint8 BGR (self.colour, overwritten by the next step)."""
         raw = ops._chk(raw_bgr, 'raw_bgr', torch.uint8)
-        if tuple(raw.shape) != (self.S,) + self.src_size + (3,):
-            raise ValueError('raw_bgr must be [%d,%d,%d,3] uint8 (got %s)' % ((self.S,) + self.src_size + (tuple(raw.shape),)))
+        if tuple(raw.shape) != (self.S,) + self.frame_shape:
+            raise ValueError('raw_bgr must be %s uint8 (got %s)' % ([self.S] + list(self.frame_shape), tuple(raw.shape)))
         h, w = self.height, self.width
-        cur = ops.cvt_img2train_u8_batch(raw, self._cvt, h, w, out=self.cur, tmp=self.cvt_tmp)
+        if self.src_format == 'bgr':
+            cur = ops.cvt_img2train_u8_batch(raw, self._cvt, h, w, out=self.cur, tmp=self.cvt_tmp)
+        else:
+            cur = ops.cvt_img2train_yuv420_batch(raw, self.src_format, self._cvt, h, w, out=self.cur, tmp=self.cvt_tmp)
         xy = self.advance(cur, net)
-        small = ops.resize_linear_u8_batch(raw, self._resize[0], self._resize[1], h, w, out=self.small)
+        if self.src_format == 'bgr':
+            small = ops.resize_linear_u8_batch(raw, self._resize[0], self._resize[1], h, w, out=self.small)
+        else:
+            small = ops.resize_linear_yuv420_batch(raw, self.src_format, self._resize[0], self._resize[1], h, w, out=self.small)
         return ops.remap_bundle_u8(small, xy, out=self.colour, workspace=self.remap_ws)
 
     def capture(self, raw_bgr, net, upload_from=None, download_to=None):
         """Records step(raw_bgr, net) as a CUDA graph and returns it: graph.replay() runs one step on whatever raw_bgr holds and
-        leaves the frames in self.colour.  upload_from / download_to: optional host buffers ([S,H,W,3] / [S,h,w,3] uint8,
-        pinned) copied into raw_bgr before and out of self.colour after the step, inside the graph.  One eager step runs first
+        leaves the frames in self.colour.  upload_from / download_to: optional host buffers ([S,H,W,3] or, for a YUV 4:2:0
+        batch, [S,3H/2,W] / [S,h,w,3] uint8, pinned) copied into raw_bgr before and out of self.colour after the step, inside the graph.  One eager step runs first
         on a side stream as a warm-up (a network may select algorithms or allocate on its first call); the state it changed
         is restored, so capturing leaves every slot as it was."""
         state = (self.frames, self.masks, self.heads_dev, self.all_black)

@@ -674,6 +674,50 @@ def resize_linear_u8_batch(img, xtab, ytab, out_h, out_w, out=None):
     return dst
 
 
+YUV420_FORMATS = {'nv12': 1, 'i420': 2}          # MGW_YUV420_NV12, MGW_YUV420_I420
+
+
+def _yuv420_dims(yuv, fmt):
+    """yuv [S,3H/2,W] uint8 in OpenCV's 4:2:0 layout -> (format constant, S, H, W)"""
+    if fmt not in YUV420_FORMATS:
+        raise ValueError('YUV 4:2:0 format must be one of %s (got %r)' % (sorted(YUV420_FORMATS), fmt))
+    # 3H/2 rows: a row count that is a multiple of 3 is exactly an even H
+    if yuv.dim() != 3 or yuv.shape[1] % 3 != 0 or yuv.shape[2] % 2 != 0:
+        raise ValueError('yuv must be [S,3H/2,W] with H and W even (got %s)' % (tuple(yuv.shape),))
+    s, rows, w = yuv.shape
+    return YUV420_FORMATS[fmt], s, rows // 3 * 2, w
+
+
+def cvt_img2train_yuv420_batch(yuv, fmt, tables, out_h, out_w, out=None, tmp=None):
+    """cvt_img2train_u8_batch of the BGR frames cv2.cvtColor(COLOR_YUV2BGR_NV12 / _I420) makes of yuv [S,3H/2,W] uint8
+    (fmt 'nv12' / 'i420'), converted inside the kernel -> [S,out_h,out_w] fp32."""
+    yuv = _chk(yuv, 'yuv', torch.uint8)
+    code, s, h, w = _yuv420_dims(yuv, fmt)
+    kx, x0, xn, ky, y0, yn = (_chk(t, 'table', torch.int32) for t in tables)
+    if kx.shape[0] != out_w or ky.shape[0] != out_h:
+        raise ValueError('the tables must cover the %dx%d output' % (out_h, out_w))
+    tmp = _out(tmp, (s, h, out_w), yuv.device, torch.uint8, 'tmp')
+    out = _out(out, (s, out_h, out_w), yuv.device, torch.float32, 'out')
+    with torch.cuda.device(yuv.device):
+        check(lib.mgw_cvt_img2train_yuv420_batch(_p(yuv), code, s, h, w, _p(kx), _p(x0), _p(xn), kx.shape[1], _p(ky), _p(y0), _p(yn),
+                                                 ky.shape[1], out_h, out_w, _p(tmp), _p(out), _st()), 'mgw_cvt_img2train_yuv420_batch')
+    return out
+
+
+def resize_linear_yuv420_batch(yuv, fmt, xtab, ytab, out_h, out_w, out=None):
+    """resize_linear_u8_batch of the BGR frames cv2.cvtColor makes of yuv [S,3H/2,W] uint8 (fmt 'nv12' / 'i420'), converted
+    inside the kernel -> [S,out_h,out_w,3] BGR."""
+    yuv = _chk(yuv, 'yuv', torch.uint8)
+    code, s, h, w = _yuv420_dims(yuv, fmt)
+    xtab = None if xtab is None else _chk(xtab, 'xtab', torch.int32)
+    ytab = None if ytab is None else _chk(ytab, 'ytab', torch.int32)
+    dst = _out(out, (s, out_h, out_w, 3), yuv.device, torch.uint8, 'out')
+    with torch.cuda.device(yuv.device):
+        check(lib.mgw_resize_linear_yuv420_batch(_p(yuv), code, s, h, w, _p(xtab), _p(ytab), out_h, out_w, _p(dst), _st()),
+              'mgw_resize_linear_yuv420_batch')
+    return dst
+
+
 def _streams_dims(frames, heads_dev, what):
     if frames.dim() != 4:
         raise ValueError('%s must be [S,depth,H,W] rings (got %s)' % (what, tuple(frames.shape)))

@@ -267,6 +267,26 @@ MGW_API int mgw_streams_assemble(const float* frames, const float* masks, int S,
 MGW_API int mgw_streams_push(float* frames, float* masks, int S, int depth, int32_t* heads_dev, const float* img, const float* black,
                      int H, int W, void* stream);
 
+/* ---- f1/f2 from YUV 4:2:0 frames, as video decoders emit them ----------------------------------------------------------
+ * yuv [S,3H/2,W] uint8 in OpenCV's 4:2:0 layout, H and W even: the Y plane (H rows of W), then
+ *   MGW_YUV420_NV12: H/2 rows of W bytes of interleaved U,V;
+ *   MGW_YUV420_I420: the U plane, then the V plane (H/2 x W/2 bytes each, contiguous: byte offsets H*W and H*W + H*W/4).
+ * Each call gives byte for byte what its BGR batch call gives on cv2.cvtColor(yuv, COLOR_YUV2BGR_NV12 / _I420) of every frame:
+ * OpenCV's BT.601 limited-range 20-bit fixed point, one chroma sample per 2x2 block, converted inside the kernels that read the
+ * source.  The frame the network sees is BGR2GRAY of that BGR frame, not the Y plane.  (cv2.VideoCapture converts with FFmpeg's
+ * swscale, which is not byte-identical to cvtColor.)  Pitched decoder surfaces are copied to contiguous frames by the caller.
+ * mgw_cvt_img2train_yuv420_batch: -> out [S,out_h,out_w]; tables and tmp (S*H*out_w bytes) as for mgw_cvt_img2train_u8_batch.
+ * mgw_resize_linear_yuv420_batch: -> dst [S,out_h,out_w,3] BGR; tables as for mgw_resize_linear_u8_batch.
+ * Checked in the order of the BGR batch calls: sizes and format (S <= 65535, H, W even and positive, S*(3H/2)*W < 2^31), then
+ * S = 0 returns MGW_OK and launches nothing, then the pointers and the 16-byte table alignment. */
+#define MGW_YUV420_NV12 1
+#define MGW_YUV420_I420 2
+MGW_API int mgw_cvt_img2train_yuv420_batch(const uint8_t* yuv, int format, int S, int H, int W, const int32_t* kx, const int32_t* x0,
+                               const int32_t* xn, int ksx, const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h,
+                               int out_w, uint8_t* tmp, float* out, void* stream);
+MGW_API int mgw_resize_linear_yuv420_batch(const uint8_t* yuv, int format, int S, int H, int W, const int32_t* xtab, const int32_t* ytab,
+                               int out_h, int out_w, uint8_t* dst, void* stream);
+
 /* ---- a6: interpolate(im, x, y, out_size), spatial_transformer.py:200-281 ------------------------------
  * im [N,IH,IW,C]; x,y [N,OH,OW] normalised coords -> out [N,OH,OW,C]. */
 MGW_API int mgw_interp_fwd(const float* im, const float* x, const float* y, int N, int IH, int IW, int C, int OH, int OW,

@@ -10,6 +10,9 @@ Per S:
   and the bytes each frame moves over PCIe.
 First the S = 1 step against the single-stream graph loop of tools/bench_configs.py (one stream, one refine pass, fixed mesh; that
 loop has no refine re-feed, so it is also timed with one), timed alternately in rounds.  refine = 1 throughout.
+--src-format nv12 / i420: the same legs (a), (b), (c) with YUV 4:2:0 frames [S,1620,1920] uploaded instead of BGR (half the bytes;
+the conversion runs inside the kernels that read the source), no single-stream comparison, and at S = 1 and S = 64 the BGR batch's
+(a) and (b) timed alternately with the YUV batch's in rounds, in the same process.
 Prints one JSON object (the GPU's name and power limit included); --out also writes it to a file."""
 import argparse, json, os, subprocess, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -75,11 +78,15 @@ def stabnet_net(model):
     return net
 
 
-def make_batch(S, rs):
-    sb = mgw.StreamBatch(S, (H, W), height=h, width=w, refine=1)
+def frame_shape(fmt):
+    return (H, W, 3) if fmt == 'bgr' else (H * 3 // 2, W)
+
+
+def make_batch(S, rs, fmt='bgr'):
+    sb = mgw.StreamBatch(S, (H, W), height=h, width=w, refine=1, src_format=fmt)
     for s in range(S):
-        sb.join(s, torch.as_tensor(rs.randint(0, 256, (H, W, 3)).astype(np.uint8)).to(dev))
-    raw_h = torch.as_tensor(rs.randint(0, 256, (S, H, W, 3)).astype(np.uint8)).pin_memory()
+        sb.join(s, torch.as_tensor(rs.randint(0, 256, frame_shape(fmt)).astype(np.uint8)).to(dev))
+    raw_h = torch.as_tensor(rs.randint(0, 256, (S,) + frame_shape(fmt)).astype(np.uint8)).pin_memory()
     raw_d = raw_h.to(dev)
     out_h = torch.empty((S, h, w, 3), dtype=torch.uint8).pin_memory()
     return sb, raw_h, raw_d, out_h
@@ -121,20 +128,47 @@ def single_stream_graph(rs, refeed=False):
     return g
 
 
+def yuv_vs_bgr_rounds(S, rs, fmt, rounds, reps):
+    """(a) and (b) of a YUV batch and of a BGR batch at the same S, alternately in rounds: per round and format the device step
+    with the frames resident and the host-to-host p50 with the copies inside the graph"""
+    arms = {}
+    for f in (fmt, 'bgr'):
+        sb, raw_h, raw_d, out_h = make_batch(S, rs, f)
+        net = fixed_mesh_net(sb)
+        arms[f] = (sb.capture(raw_d, net), sb.capture(raw_d, net, upload_from=raw_h, download_to=out_h), sb, raw_h, raw_d, out_h)
+    out = {f: {'a_us_device_step_per_round': [], 'b_us_p50_host_to_host_per_round': []} for f in arms}
+    for _ in range(rounds):
+        for f, (g_res, g_io, *_) in arms.items():
+            out[f]['a_us_device_step_per_round'].append(dev_time(g_res.replay, reps))
+            out[f]['b_us_p50_host_to_host_per_round'].append(float(np.percentile(host_times(g_io.replay, reps), 50)))
+    for f in out:
+        a_med, b_med = float(np.median(out[f]['a_us_device_step_per_round'])), float(np.median(out[f]['b_us_p50_host_to_host_per_round']))
+        out[f].update(a_us_device_per_frame_median=a_med / S, b_frames_per_s_median=S * 1e6 / b_med)
+    del arms
+    torch.cuda.empty_cache()
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--streams', default='1,4,16,64')
     ap.add_argument('--reps', type=int, default=300, help='timed replays per measurement (the StabNet leg takes a sixth)')
     ap.add_argument('--ab-rounds', type=int, default=6)
+    ap.add_argument('--src-format', default='bgr', choices=('bgr', 'nv12', 'i420'))
     ap.add_argument('--out')
     a = ap.parse_args()
     assert torch.cuda.is_available(), 'bench_streams.py measures on the GPU; there is nothing to measure without one'
     torch.backends.cudnn.benchmark = True
-    res = {'gpu': gpu_info(), 'source': '%dx%d BGR uint8' % (H, W), 'network_size': '%dx%d' % (h, w), 'refine': 1,
-           'bytes_pcie_per_frame': {'h2d_raw_bgr': H * W * 3, 'd2h_colour': h * w * 3, 'total': H * W * 3 + h * w * 3}, 'per_S': {}}
+    fmt = a.src_format
+    raw_bytes = int(np.prod(frame_shape(fmt)))
+    res = {'gpu': gpu_info(), 'source': '%dx%d %s uint8' % (H, W, fmt.upper()), 'network_size': '%dx%d' % (h, w), 'refine': 1,
+           'bytes_pcie_per_frame': {'h2d_raw_' + fmt: raw_bytes, 'd2h_colour': h * w * 3, 'total': raw_bytes + h * w * 3}, 'per_S': {}}
     rs = np.random.RandomState(0)
     torch.manual_seed(0)
     model = mgw.StabNet(in_ch=13, grid=(4, 4)).to(dev).eval().to(memory_format=torch.channels_last)
+    if fmt != 'bgr':
+        measure_format(a, res, rs, model, fmt)
+        return emit(res, a.out)
     # S = 1 against the single-stream loop, alternately
     sb, raw_h, raw_d, out_h = make_batch(1, rs)
     with torch.no_grad():
@@ -150,34 +184,56 @@ def main():
     del sb, raw_h, raw_d, out_h, g_batch, arms
     torch.cuda.empty_cache()
     for S in [int(v) for v in a.streams.split(',')]:
-        r = {}
-        sb, raw_h, raw_d, out_h = make_batch(S, rs)
-        with torch.no_grad():
-            net = fixed_mesh_net(sb)
-            g_res = sb.capture(raw_d, net)
-            t = dev_time(g_res.replay, a.reps)
-            r['a_us_device_step_fixed_mesh_resident'] = t
-            r['a_us_device_per_frame'] = t / S
-            g_io = sb.capture(raw_d, net, upload_from=raw_h, download_to=out_h)
-            r['b_host_to_host_fixed_mesh'] = summary(host_times(g_io.replay, a.reps), S)
+        res['per_S'][str(S)] = legs(S, rs, model, a.reps)
+    emit(res, a.out)
 
-            def copies():
-                raw_d.copy_(raw_h, non_blocking=True); out_h.copy_(sb.colour, non_blocking=True)
-            r['b_host_to_host_copies_only'] = summary(host_times(copies, a.reps), S)
-            r['h2d_GB_per_s'] = S * H * W * 3 / (dev_time(lambda: raw_d.copy_(raw_h, non_blocking=True), a.reps) * 1e3)
-            del g_res, g_io
-            g_net = sb.capture(raw_d, stabnet_net(model), upload_from=raw_h, download_to=out_h)
-            reps = max(a.reps // 6, 20)
-            r['c_host_to_host_stabnet'] = summary(host_times(g_net.replay, reps), S)
-            r['c_us_device_step_stabnet'] = dev_time(g_net.replay, reps)
-            del g_net
-        res['per_S'][str(S)] = r
-        del sb, raw_h, raw_d, out_h
-        torch.cuda.empty_cache()
-        print(json.dumps({S: r}), file=sys.stderr)
+
+def legs(S, rs, model, reps, fmt='bgr'):
+    """(a), (b) with the copies alone and the upload rate, (c) for one S"""
+    r = {}
+    raw_bytes = int(np.prod(frame_shape(fmt)))
+    sb, raw_h, raw_d, out_h = make_batch(S, rs, fmt)
+    with torch.no_grad():
+        net = fixed_mesh_net(sb)
+        g_res = sb.capture(raw_d, net)
+        t = dev_time(g_res.replay, reps)
+        r['a_us_device_step_fixed_mesh_resident'] = t
+        r['a_us_device_per_frame'] = t / S
+        g_io = sb.capture(raw_d, net, upload_from=raw_h, download_to=out_h)
+        r['b_host_to_host_fixed_mesh'] = summary(host_times(g_io.replay, reps), S)
+
+        def copies():
+            raw_d.copy_(raw_h, non_blocking=True); out_h.copy_(sb.colour, non_blocking=True)
+        r['b_host_to_host_copies_only'] = summary(host_times(copies, reps), S)
+        r['h2d_GB_per_s'] = S * raw_bytes / (dev_time(lambda: raw_d.copy_(raw_h, non_blocking=True), reps) * 1e3)
+        del g_res, g_io
+        g_net = sb.capture(raw_d, stabnet_net(model), upload_from=raw_h, download_to=out_h)
+        reps_c = max(reps // 6, 20)
+        r['c_host_to_host_stabnet'] = summary(host_times(g_net.replay, reps_c), S)
+        r['c_us_device_step_stabnet'] = dev_time(g_net.replay, reps_c)
+        del g_net
+    del sb, raw_h, raw_d, out_h
+    torch.cuda.empty_cache()
+    print(json.dumps({S: r}), file=sys.stderr)
+    return r
+
+
+def measure_format(a, res, rs, model, fmt):
+    """--src-format nv12 / i420: every leg with YUV input, and the BGR batch alongside at S = 1 and S = 64"""
+    res['bytes_pcie_per_frame_bgr'] = {'h2d_raw_bgr': H * W * 3, 'd2h_colour': h * w * 3, 'total': H * W * 3 + h * w * 3}
+    res['yuv_vs_bgr_alternating'] = {}
+    for S in [int(v) for v in a.streams.split(',')]:
+        res['per_S'][str(S)] = legs(S, rs, model, a.reps, fmt)
+        if S in (1, 64):
+            with torch.no_grad():
+                res['yuv_vs_bgr_alternating'][str(S)] = yuv_vs_bgr_rounds(S, rs, fmt, a.ab_rounds, a.reps)
+            print(json.dumps({'alternating': {S: res['yuv_vs_bgr_alternating'][str(S)]}}), file=sys.stderr)
+
+
+def emit(res, out):
     print(json.dumps(res, indent=1))
-    if a.out:
-        with open(a.out, 'w') as f:
+    if out:
+        with open(out, 'w') as f:
             json.dump(res, f, indent=1)
 
 
