@@ -62,6 +62,8 @@ SIGNATURES = {
     'mgw_streams_push': (c_i, [c_f, c_f, c_i, c_i, c_f, c_f, c_f, c_i, c_i, c_st]),
     'mgw_cvt_img2train_yuv420_batch': (c_i, [c_f, c_i, c_i, c_i, c_i, c_f, c_f, c_f, c_i, c_f, c_f, c_f, c_i, c_i, c_i, c_f, c_f, c_st]),
     'mgw_resize_linear_yuv420_batch': (c_i, [c_f, c_i, c_i, c_i, c_i, c_f, c_f, c_i, c_i, c_f, c_st]),
+    'mgw_cvt_img2train_mixed': (c_i, [c_f, c_i, c_i, c_i, c_i, c_f, c_f, c_f, c_f, c_i, c_f, c_f, c_f, c_i, c_i, c_i, c_f, c_f, c_st]),
+    'mgw_resize_linear_mixed': (c_i, [c_f, c_i, c_i, c_i, c_i, c_f, c_f, c_f, c_i, c_i, c_f, c_st]),
     'mgw_interp_fwd': (c_i, [c_f, c_f, c_f] + [c_i] * 6 + [c_f, c_st]),
     'mgw_interp_bwd': (c_i, [c_f, c_f, c_f, c_f] + [c_i] * 6 + [c_f, c_f, c_f, c_st]),
     'mgw_homography_warp_fwd': (c_i, [c_f, c_f] + [c_i] * 6 + [c_f, c_f, c_f, c_st]),

@@ -674,6 +674,42 @@ int mgw_resize_linear_yuv420_batch(const uint8_t* yuv, int format, int S, int H,
     return launch_resize_linear_u8(yuv, S, H, W, 3, xtab, ytab, out_h, out_w, dst, (cudaStream_t)stream, format);
 }
 
+// Per-slot source geometry: the capacity (max_h, max_w) takes the place of the uniform batch's H, W in its size checks (every
+// slot's region and tmp rows are laid out for it); the 8-byte alignment of sizes is that of the int2 each block loads.
+static int validate_mixed(const char* fn, int format, int S, int max_h, int max_w, int out_h, int out_w)
+{
+    REQUIRE(format == MGW_BGR24 || format == MGW_YUV420_NV12 || format == MGW_YUV420_I420, "%s: unknown format %d", fn, format);
+    if (format != MGW_BGR24) return validate_yuv420(fn, format, S, max_h, max_w, out_h, out_w);
+    REQUIRE(S >= 0 && S <= 65535 && max_h > 0 && max_w > 0 && out_h > 0 && out_w > 0 && (long long)S * max_h * max_w < (1LL << 29) &&
+            (long long)S * max_h * out_w < (1LL << 31) && (long long)S * out_h * out_w < (1LL << 29),
+            "%s: bad sizes (S=%d capacity %dx%d out %dx%d)", fn, S, max_h, max_w, out_h, out_w);
+    return MGW_OK;
+}
+
+int mgw_cvt_img2train_mixed(const uint8_t* src, int format, int S, int max_h, int max_w, const int32_t* sizes, const int32_t* kx,
+                            const int32_t* x0, const int32_t* xn, int ksx, const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy,
+                            int out_h, int out_w, uint8_t* tmp, float* out, void* stream)
+{
+    TRY(validate_mixed("mgw_cvt_img2train_mixed", format, S, max_h, max_w, out_h, out_w));
+    REQUIRE(ksx > 0 && ksy > 0, "mgw_cvt_img2train_mixed: bad sizes (ksx=%d ksy=%d)", ksx, ksy);
+    if (S == 0) return MGW_OK;
+    REQUIRE(src && sizes && kx && x0 && xn && ky && y0 && yn && tmp && out, "mgw_cvt_img2train_mixed: null pointer");
+    REQUIRE(aligned(sizes, 8), "mgw_cvt_img2train_mixed: sizes must be 8-byte aligned");
+    return launch_cvt_img2train_mixed(src, format, S, max_h, max_w, sizes, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w, tmp, out,
+                                      (cudaStream_t)stream);
+}
+
+int mgw_resize_linear_mixed(const uint8_t* src, int format, int S, int max_h, int max_w, const int32_t* sizes, const int32_t* xtab,
+                            const int32_t* ytab, int out_h, int out_w, uint8_t* dst, void* stream)
+{
+    TRY(validate_mixed("mgw_resize_linear_mixed", format, S, max_h, max_w, out_h, out_w));
+    if (S == 0) return MGW_OK;
+    REQUIRE(src && sizes && xtab && ytab && dst, "mgw_resize_linear_mixed: null pointer");
+    REQUIRE(aligned(xtab, 16) && aligned(ytab, 16), "mgw_resize_linear_mixed: tables must be 16-byte aligned");
+    REQUIRE(aligned(sizes, 8), "mgw_resize_linear_mixed: sizes must be 8-byte aligned");
+    return launch_resize_linear_mixed(src, format, S, max_h, max_w, sizes, xtab, ytab, out_h, out_w, dst, (cudaStream_t)stream);
+}
+
 static int validate_streams(const char* fn, int S, int depth, int H, int W, int nch)
 {
     REQUIRE(S >= 0 && S <= 65535 && depth > 0 && H > 0 && W > 0 && (long long)S * depth * H * W < (1LL << 31) &&

@@ -188,6 +188,10 @@ int launch_remap_bundle_u8(const uint8_t* img, const float* xy, int N, int H, in
 // offsets its base pointers once, the per-pixel index arithmetic is the single-frame one, and S = 1 is the single-frame call.
 // The source frame is BGR (SRC_BGR) or YUV 4:2:0 in OpenCV's layout (MGW_YUV420_NV12 / MGW_YUV420_I420): the kernels then read
 // the BGR frame cv2.cvtColor would make of it, converted per pixel on the fly.
+// MIXED = per-slot source geometry (a batch of videos of different sizes): H, W are the batch's capacity, slot s owns the region
+// [s * frame_bytes(H, W), +frame_bytes(H, W)) of the source and its frame of size sizes[s] lies at the start of it, and the slot
+// has its own tables (kx [S,out_w,ks], ...) and tmp rows [S,H,out_w].  Block (., s) reads sizes[s] once, offsets its pointers to
+// the slot, and then runs the per-pixel code of the uniform batch at the slot's size with frame index 0.
 namespace {
 
 constexpr int SRC_BGR = 0;
@@ -231,19 +235,38 @@ __device__ __forceinline__ size_t src_frame_bytes(int H, int W)
     return FMT == SRC_BGR ? (size_t)H * W * 3 : (size_t)H * W * 3 / 2;
 }
 
+// A slot is idle -- its blocks return before they write anything -- when its size is 0, larger than the capacity, or odd for a
+// YUV format: never-joined slots, and a bad device-side size cannot move a read outside the slot's region.
 template <int FMT>
+__device__ __forceinline__ bool slot_active(int2 sz, int max_h, int max_w)
+{
+    return sz.x > 0 && sz.y > 0 && sz.x <= max_h && sz.y <= max_w && (FMT == SRC_BGR || ((sz.x | sz.y) & 1) == 0);
+}
+
+template <int FMT, bool MIXED = false>
 __global__ void __launch_bounds__(256)
 gray_hpass_kernel(const uint8_t* __restrict__ bgr, int H, int W, const int32_t* __restrict__ kx, const int32_t* __restrict__ x0,
-                  const int32_t* __restrict__ xn, int ks, int out_w, uint8_t* __restrict__ tmp)
+                  const int32_t* __restrict__ xn, int ks, int out_w, uint8_t* __restrict__ tmp, const int2* __restrict__ sizes)
 {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if constexpr (MIXED) {
+        const int2 sz = __ldg(sizes + blockIdx.y);
+        if (!slot_active<FMT>(sz, H, W)) return;
+        bgr += (size_t)blockIdx.y * src_frame_bytes<FMT>(H, W);
+        tmp += (size_t)blockIdx.y * H * out_w;
+        kx += (size_t)blockIdx.y * out_w * ks;
+        x0 += (size_t)blockIdx.y * out_w;
+        xn += (size_t)blockIdx.y * out_w;
+        H = sz.x; W = sz.y;                                 // launched over the capacity's rows: rows >= H return below
+    }
+    const unsigned s = MIXED ? 0u : blockIdx.y;             // the frame index of a uniform batch
     if (t >= H * out_w) return;
-    tmp += (size_t)blockIdx.y * H * out_w;
+    tmp += (size_t)s * H * out_w;
     const int xx = t % out_w, row = t / out_w;
     const int n = __ldg(xn + xx);
     int acc = 1 << 21;
     if constexpr (FMT == SRC_BGR) {
-        bgr += (size_t)blockIdx.y * H * W * 3;
+        bgr += (size_t)s * H * W * 3;
         const uint8_t* p = bgr + ((size_t)row * W + __ldg(x0 + xx)) * 3;
         for (int k = 0; k < n; ++k, p += 3) {
             // RGB2Gray<uchar>: (B*3735 + G*19235 + R*9798 + 2^14) >> 15
@@ -252,7 +275,7 @@ gray_hpass_kernel(const uint8_t* __restrict__ bgr, int H, int W, const int32_t* 
         }
     } else {
         // the BGR pixel cvtColor makes, then the same gray; a pair of pixels (even x, x+1) shares one chroma sample
-        const uint8_t* f = bgr + (size_t)blockIdx.y * src_frame_bytes<FMT>(H, W);
+        const uint8_t* f = bgr + (size_t)s * src_frame_bytes<FMT>(H, W);
         const int xs = __ldg(x0 + xx);
         const uint8_t* py = f + (size_t)row * W + xs;
         Chroma c;
@@ -267,11 +290,19 @@ gray_hpass_kernel(const uint8_t* __restrict__ bgr, int H, int W, const int32_t* 
     tmp[t] = (uint8_t)min(max(acc >> 22, 0), 255);
 }
 
+// MIXED: H is the capacity's height (the tmp rows of a slot), max_w its width; the slot's rows of ky / y0 / yn
+template <int FMT = SRC_BGR, bool MIXED = false>
 __global__ void __launch_bounds__(256)
 vpass_norm_kernel(const uint8_t* __restrict__ tmp, int H, int out_w, const int32_t* __restrict__ ky, const int32_t* __restrict__ y0,
-                  const int32_t* __restrict__ yn, int ks, int out_h, float* __restrict__ out)
+                  const int32_t* __restrict__ yn, int ks, int out_h, float* __restrict__ out, const int2* __restrict__ sizes, int max_w)
 {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if constexpr (MIXED) {
+        if (!slot_active<FMT>(__ldg(sizes + blockIdx.y), H, max_w)) return;
+        ky += (size_t)blockIdx.y * out_h * ks;
+        y0 += (size_t)blockIdx.y * out_h;
+        yn += (size_t)blockIdx.y * out_h;
+    }
     if (t >= out_h * out_w) return;
     tmp += (size_t)blockIdx.y * H * out_w;
     out += (size_t)blockIdx.y * out_h * out_w;
@@ -293,14 +324,39 @@ int launch_cvt_img2train_u8(const uint8_t* bgr, int S, int H, int W, const int32
 {
     const dim3 g1((H * out_w + 255) / 256, S);
     switch (src_fmt) {
-    case SRC_BGR: gray_hpass_kernel<SRC_BGR><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp); break;
-    case MGW_YUV420_NV12: gray_hpass_kernel<MGW_YUV420_NV12><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp); break;
-    case MGW_YUV420_I420: gray_hpass_kernel<MGW_YUV420_I420><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp); break;
+    case SRC_BGR: gray_hpass_kernel<SRC_BGR><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp, nullptr); break;
+    case MGW_YUV420_NV12: gray_hpass_kernel<MGW_YUV420_NV12><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp, nullptr); break;
+    case MGW_YUV420_I420: gray_hpass_kernel<MGW_YUV420_I420><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp, nullptr); break;
     default: return set_error(MGW_ERR_INVALID, "cvt_img2train: unknown source format %d", src_fmt);
     }
     if (int rc = check_launch("gray_hpass")) return rc;
-    vpass_norm_kernel<<<dim3((out_h * out_w + 255) / 256, S), 256, 0, st>>>(tmp, H, out_w, ky, y0, yn, ksy, out_h, out);
+    vpass_norm_kernel<<<dim3((out_h * out_w + 255) / 256, S), 256, 0, st>>>(tmp, H, out_w, ky, y0, yn, ksy, out_h, out, nullptr, 0);
     return check_launch("vpass_norm");
+}
+
+template <int FMT>
+static int cvt_mixed(const uint8_t* src, int S, int max_h, int max_w, const int2* sizes, const int32_t* kx, const int32_t* x0,
+                     const int32_t* xn, int ksx, const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h, int out_w,
+                     uint8_t* tmp, float* out, cudaStream_t st)
+{
+    gray_hpass_kernel<FMT, true><<<dim3((max_h * out_w + 255) / 256, S), 256, 0, st>>>(src, max_h, max_w, kx, x0, xn, ksx, out_w, tmp, sizes);
+    if (int rc = check_launch("gray_hpass")) return rc;
+    vpass_norm_kernel<FMT, true><<<dim3((out_h * out_w + 255) / 256, S), 256, 0, st>>>(tmp, max_h, out_w, ky, y0, yn, ksy, out_h, out,
+                                                                                      sizes, max_w);
+    return check_launch("vpass_norm");
+}
+
+int launch_cvt_img2train_mixed(const uint8_t* src, int src_fmt, int S, int max_h, int max_w, const int32_t* sizes, const int32_t* kx,
+                               const int32_t* x0, const int32_t* xn, int ksx, const int32_t* ky, const int32_t* y0, const int32_t* yn,
+                               int ksy, int out_h, int out_w, uint8_t* tmp, float* out, cudaStream_t st)
+{
+    const int2* sz = reinterpret_cast<const int2*>(sizes);
+    switch (src_fmt) {
+    case SRC_BGR: return cvt_mixed<SRC_BGR>(src, S, max_h, max_w, sz, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w, tmp, out, st);
+    case MGW_YUV420_NV12: return cvt_mixed<MGW_YUV420_NV12>(src, S, max_h, max_w, sz, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w, tmp, out, st);
+    case MGW_YUV420_I420: return cvt_mixed<MGW_YUV420_I420>(src, S, max_h, max_w, sz, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w, tmp, out, st);
+    default: return set_error(MGW_ERR_INVALID, "cvt_img2train_mixed: unknown source format %d", src_fmt);
+    }
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -319,16 +375,28 @@ __device__ __forceinline__ int3 yuv_bgr_at(const uint8_t* __restrict__ f, int H,
 
 __device__ __forceinline__ int ch_of(const int3& p, int ch) { return ch == 0 ? p.x : (ch == 1 ? p.y : p.z); }
 
-template <int C, int FMT = SRC_BGR>
+// MIXED: H, W are the capacity (see cvt_img2train above); xtab [S,out_w], ytab [S,out_h]; the 2x2 shortcut is the slot's own
+template <int C, int FMT = SRC_BGR, bool MIXED = false>
 __global__ void __launch_bounds__(256)
 resize_u8_kernel(const uint8_t* __restrict__ img, int H, int W, const int4* __restrict__ xtab, const int4* __restrict__ ytab,
-                 int out_h, int out_w, int area2, uint8_t* __restrict__ dst)
+                 int out_h, int out_w, int area2, uint8_t* __restrict__ dst, const int2* __restrict__ sizes)
 {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= out_h * out_w) return;
+    if constexpr (MIXED) {
+        static_assert(C == 3, "a slot's frame is BGR or YUV 4:2:0");
+        const int2 sz = __ldg(sizes + blockIdx.y);
+        if (!slot_active<FMT>(sz, H, W)) return;
+        img += (size_t)blockIdx.y * src_frame_bytes<FMT>(H, W);
+        xtab += (size_t)blockIdx.y * out_w;
+        ytab += (size_t)blockIdx.y * out_h;
+        H = sz.x; W = sz.y;
+        area2 = W == 2 * out_w && H == 2 * out_h;
+    }
+    const unsigned s = MIXED ? 0u : blockIdx.y;             // the source frame index of a uniform batch
     if constexpr (FMT != SRC_BGR) {
         static_assert(C == 3, "a YUV 4:2:0 source resizes to BGR");
-        const uint8_t* f = img + (size_t)blockIdx.y * src_frame_bytes<FMT>(H, W);
+        const uint8_t* f = img + (size_t)s * src_frame_bytes<FMT>(H, W);
         dst += (size_t)blockIdx.y * out_h * out_w * 3;
         const int x = t % out_w, y = t / out_w;
         uint8_t* o = dst + (size_t)t * 3;
@@ -355,7 +423,7 @@ resize_u8_kernel(const uint8_t* __restrict__ img, int H, int W, const int4* __re
         }
         return;
     }
-    img += (size_t)blockIdx.y * H * W * C;
+    img += (size_t)s * H * W * C;
     dst += (size_t)blockIdx.y * out_h * out_w * C;
     const int x = t % out_w, y = t / out_w;
     uint8_t* o = dst + (size_t)t * C;
@@ -392,17 +460,35 @@ int launch_resize_linear_u8(const uint8_t* img, int S, int H, int W, int C, cons
     if (src_fmt != SRC_BGR) {
         if (C != 3) return set_error(MGW_ERR_UNSUPPORTED, "resize_linear_u8: a YUV 4:2:0 source gives C = 3 (got %d)", C);
         switch (src_fmt) {
-        case MGW_YUV420_NV12: resize_u8_kernel<3, MGW_YUV420_NV12><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst); break;
-        case MGW_YUV420_I420: resize_u8_kernel<3, MGW_YUV420_I420><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst); break;
+        case MGW_YUV420_NV12: resize_u8_kernel<3, MGW_YUV420_NV12><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr); break;
+        case MGW_YUV420_I420: resize_u8_kernel<3, MGW_YUV420_I420><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr); break;
         default: return set_error(MGW_ERR_INVALID, "resize_linear_u8: unknown source format %d", src_fmt);
         }
         return check_launch("resize_u8");
     }
     switch (C) {
-    case 1: resize_u8_kernel<1><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst); break;
-    case 3: resize_u8_kernel<3><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst); break;
-    case 4: resize_u8_kernel<4><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst); break;
+    case 1: resize_u8_kernel<1><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr); break;
+    case 3: resize_u8_kernel<3><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr); break;
+    case 4: resize_u8_kernel<4><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr); break;
     default: return set_error(MGW_ERR_UNSUPPORTED, "resize_linear_u8: C must be 1, 3 or 4 (got %d)", C);
+    }
+    return check_launch("resize_u8");
+}
+
+int launch_resize_linear_mixed(const uint8_t* src, int src_fmt, int S, int max_h, int max_w, const int32_t* sizes, const int32_t* xtab,
+                               const int32_t* ytab, int out_h, int out_w, uint8_t* dst, cudaStream_t st)
+{
+    const dim3 grid((out_h * out_w + 255) / 256, S);
+    const int2* sz = reinterpret_cast<const int2*>(sizes);
+    const int4* xt = reinterpret_cast<const int4*>(xtab);
+    const int4* yt = reinterpret_cast<const int4*>(ytab);
+    switch (src_fmt) {
+    case SRC_BGR: resize_u8_kernel<3, SRC_BGR, true><<<grid, 256, 0, st>>>(src, max_h, max_w, xt, yt, out_h, out_w, 0, dst, sz); break;
+    case MGW_YUV420_NV12:
+        resize_u8_kernel<3, MGW_YUV420_NV12, true><<<grid, 256, 0, st>>>(src, max_h, max_w, xt, yt, out_h, out_w, 0, dst, sz); break;
+    case MGW_YUV420_I420:
+        resize_u8_kernel<3, MGW_YUV420_I420, true><<<grid, 256, 0, st>>>(src, max_h, max_w, xt, yt, out_h, out_w, 0, dst, sz); break;
+    default: return set_error(MGW_ERR_INVALID, "resize_linear_mixed: unknown source format %d", src_fmt);
     }
     return check_launch("resize_u8");
 }

@@ -119,6 +119,13 @@ int launch_resize_linear_u8(const uint8_t* img, int S, int H, int W, int C, cons
 int launch_cvt_img2train_u8(const uint8_t* bgr, int S, int H, int W, const int32_t* kx, const int32_t* x0, const int32_t* xn, int ksx,
                             const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h, int out_w, uint8_t* tmp,
                             float* out, cudaStream_t st, int src_fmt = 0);
+// per-slot source geometry: slot s's frame of size sizes[s] (int32 [S,2], 8-byte aligned) at src + s * frame_bytes(max_h, max_w),
+// per-slot tables; BGR (src_fmt 0) or YUV 4:2:0, C = 3.  Slots with a size of 0, above the capacity or odd (YUV) write nothing.
+int launch_cvt_img2train_mixed(const uint8_t* src, int src_fmt, int S, int max_h, int max_w, const int32_t* sizes, const int32_t* kx,
+                               const int32_t* x0, const int32_t* xn, int ksx, const int32_t* ky, const int32_t* y0, const int32_t* yn,
+                               int ksy, int out_h, int out_w, uint8_t* tmp, float* out, cudaStream_t st);
+int launch_resize_linear_mixed(const uint8_t* src, int src_fmt, int S, int max_h, int max_w, const int32_t* sizes, const int32_t* xtab,
+                               const int32_t* ytab, int out_h, int out_w, uint8_t* dst, cudaStream_t st);
 int launch_warp_rev_bundle_u8(const uint8_t* img, const double* Hs_cvt, int N, int H, int W, int C, int gh, int gw, uint8_t* dst,
                               cudaStream_t st);
 

@@ -7,14 +7,16 @@ accepts numpy arrays (as the reference's caller passes; the result comes back as
 [N,H,W,C] / [N,H,W] too; the result stays on the device).  The work is one C-ABI call, mgw_remap_bundle_u8.
 
 StreamBatch runs the whole per-frame loop for S videos of one size at once: one set of launches per frame, capturable as one
-CUDA graph, every video's result bit-identical to its own StreamState / CropState pipeline.
+CUDA graph, every video's result bit-identical to its own StreamState / CropState pipeline.  MixedStreamBatch does the same for
+videos of different source sizes up to a capacity.
 """
 import numpy as np
 import torch
 
 from . import ops
 
-__all__ = ['warpRevBundle2', 'warpRevBundle', 'warpRev', 'cvt_theta_mat_bundle', 'cvt_img2train', 'cv2_resize', 'StreamState', 'CropState', 'StreamBatch']
+__all__ = ['warpRevBundle2', 'warpRevBundle', 'warpRev', 'cvt_theta_mat_bundle', 'cvt_img2train', 'cv2_resize', 'StreamState', 'CropState', 'StreamBatch',
+           'MixedStreamBatch', 'mixed_slot_tables']
 
 
 def warpRevBundle2(img, x_map, y_map, device=None):
@@ -44,7 +46,7 @@ def _pil_bilinear_windows(in_size, out_size):
     scale = in_size / float(out_size)
     filterscale = max(scale, 1.0)
     support = 1.0 * filterscale
-    ksize = int(math.ceil(support)) * 2 + 1
+    ksize = _pil_ksize(in_size, out_size)
     first = np.zeros(out_size, np.int32)
     count = np.zeros(out_size, np.int32)
     kk = np.zeros((out_size, ksize), np.int32)
@@ -62,6 +64,12 @@ def _pil_bilinear_windows(in_size, out_size):
             kk[xx, x] = int(v * (1 << 22) + 0.5)
         first[xx], count[xx] = xmin, xmax
     return kk, first, count
+
+
+def _pil_ksize(in_size, out_size):
+    """the window length of _pil_bilinear_windows: 2*ceil(max(in/out, 1)) + 1, which does not decrease as in_size grows"""
+    import math
+    return int(math.ceil(1.0 * max(in_size / float(out_size), 1.0))) * 2 + 1
 
 
 def _cv_linear_table(n_out, n_in, horizontal):
@@ -145,19 +153,48 @@ def cv2_resize(img, dsize, device='cuda', src_format='bgr'):
     return dst.cpu().numpy() if as_numpy else dst
 
 
+def _resample_size(height, width, crop_rate):
+    """(h, w, dh, dw): the size cvt_img2train resizes to and the offset of the centre crop"""
+    if crop_rate != 1:
+        h = int(height / crop_rate); dh = int((h - height) / 2)
+        w = int(width / crop_rate); dw = int((w - width) / 2)
+        return h, w, dh, dw
+    return height, width, 0, 0
+
+
+def _cvt_windows(H, W, height, width, crop_rate):
+    """cvt_img2train's tables (kx, x0, xn, ky, y0, yn) for an H x W source, numpy int32"""
+    h, w, dh, dw = _resample_size(height, width, crop_rate)
+    kx, x0, xn = _pil_bilinear_windows(W, w)
+    ky, y0, yn = _pil_bilinear_windows(H, h)
+    return kx[dw:dw + width], x0[dw:dw + width], xn[dw:dw + width], ky[dh:dh + height], y0[dh:dh + height], yn[dh:dh + height]
+
+
 def _cvt_tables(H, W, height, width, crop_rate, device):
     key = (H, W, height, width, float(crop_rate), str(device))
     if key not in _CVT_TABLES:
-        if crop_rate != 1:
-            h = int(height / crop_rate); dh = int((h - height) / 2)
-            w = int(width / crop_rate); dw = int((w - width) / 2)
-        else:
-            h, w, dh, dw = height, width, 0, 0
-        kx, x0, xn = _pil_bilinear_windows(W, w)
-        ky, y0, yn = _pil_bilinear_windows(H, h)
-        tabs = (kx[dw:dw + width], x0[dw:dw + width], xn[dw:dw + width], ky[dh:dh + height], y0[dh:dh + height], yn[dh:dh + height])
+        tabs = _cvt_windows(H, W, height, width, crop_rate)
         _CVT_TABLES[key] = tuple(torch.as_tensor(np.ascontiguousarray(t)).to(device) for t in tabs)
     return _CVT_TABLES[key]
+
+
+def mixed_slot_tables(src_size, max_src_size, height=288, width=512, crop_rate=1):
+    """One slot's tables for the per-slot calls (ops.cvt_img2train_mixed / ops.resize_linear_mixed), numpy int32:
+    (kx [width,ksx], x0, xn [width], ky [height,ksy], y0, yn [height], xtab [width,4], ytab [height,4]).  They are the uniform
+    tables at the slot's size src_size = (H, W), with the Pillow windows zero-padded to the lengths ksx, ksy of the capacity
+    max_src_size; xtab / ytab are given even where the slot takes the 2x2 shortcut."""
+    (H, W), (mh, mw) = (int(v) for v in src_size), (int(v) for v in max_src_size)
+    if not (0 < H <= mh and 0 < W <= mw):
+        raise ValueError('source size %dx%d outside the capacity %dx%d' % (H, W, mh, mw))
+    rh, rw, _, _ = _resample_size(height, width, crop_rate)
+    kx, x0, xn, ky, y0, yn = _cvt_windows(H, W, height, width, crop_rate)
+    ksx, ksy = _pil_ksize(mw, rw), _pil_ksize(mh, rh)
+    if kx.shape[1] > ksx or ky.shape[1] > ksy:
+        raise ValueError('a %dx%d source needs longer windows than its capacity %dx%d' % (H, W, mh, mw))
+    kxp, kyp = np.zeros((width, ksx), np.int32), np.zeros((height, ksy), np.int32)
+    kxp[:, :kx.shape[1]], kyp[:, :ky.shape[1]] = kx, ky
+    return (kxp, np.ascontiguousarray(x0), np.ascontiguousarray(xn), kyp, np.ascontiguousarray(y0), np.ascontiguousarray(yn),
+            _cv_linear_table(width, W, True), _cv_linear_table(height, H, False))
 
 
 def cvt_img2train(img, crop_rate=1, height=288, width=512, device='cuda', as_numpy=False, src_format='bgr'):
@@ -364,7 +401,12 @@ class StreamBatch:
         self.small = torch.empty((S, h, w, 3), device=dev, dtype=torch.uint8)
         self.colour = torch.empty((S, h, w, 3), device=dev, dtype=torch.uint8)
         self.remap_ws = torch.empty(ops.remap_bundle_workspace_floats(S, h, w), **f32)
-        self._cvt = _cvt_tables(H, W, h, w, crop_rate, dev)
+        self._init_front_end(dev)
+
+    def _init_front_end(self, dev):
+        """the coefficient tables of the two stages that read the source frame: the uniform ones of src_size"""
+        (H, W), h, w = self.src_size, self.height, self.width
+        self._cvt = _cvt_tables(H, W, h, w, self.crop_rate, dev)
         self._resize = _resize_tables(H, W, h, w, dev)
 
     def _slot(self, slot):
@@ -452,3 +494,104 @@ class StreamBatch:
             if download_to is not None:
                 download_to.copy_(self.colour, non_blocking=True)
         return graph
+
+
+class MixedStreamBatch(StreamBatch):
+    """A StreamBatch whose slots carry videos of different source sizes, up to the capacity max_src_size = (H, W).  Every size
+    is resized to the same network frame, so everything after the front end is the StreamBatch's; the two kernels that read the
+    source frame take each slot's size and tables from device memory.  Every slot is bit-identical to its own pipeline at its
+    own size (and so to a StreamBatch of that size).
+
+        mb = MixedStreamBatch(4, (1080, 1920))          # capacity 1080p, BGR
+        pool = torch.empty(mb.pool_shape, dtype=torch.uint8, device='cuda')
+        mb.join(0, first_720p)                          # [720,1280,3] uint8: slot 0 is now a 720p video
+        mb.join(1, first_1080p)
+        for ...:
+            mb.slot_frame(pool, 0).copy_(next_720p)     # each slot's frame goes to the start of its region of the pool
+            mb.slot_frame(pool, 1).copy_(next_1080p)
+            colour = mb.step(pool, net)                 # [4,288,512,3] uint8
+
+    pool: [S, frame_bytes(max_src_size)] uint8 (frame_bytes = 3*H*W for BGR, 3H/2*W for YUV 4:2:0); slot s's frame lies contiguous
+    at the start of pool[s], BGR [H_s,W_s,3] or YUV [3H_s/2,W_s].  slot_frame() gives that view of any pool-shaped buffer (device
+    or pinned host).  capture(pool, net, upload_from=, download_to=) is StreamBatch.capture: the upload inside the graph copies
+    the whole pool, capacity bytes per slot whatever the slots' sizes.  A slot can join again at another size between replays of
+    a captured graph: join writes the slot's size and tables with stream-ordered device copies, and the graph reads them.
+    Slots that never joined are idle: the front end writes nothing for them and the network sees zero frames.  A slot that left
+    keeps its size and runs on whatever its region holds, as in StreamBatch."""
+
+    def __init__(self, S, max_src_size, height=288, width=512, depth=32, taps=(1, 2, 4, 8, 16, 32), use_masks=True, crop_rate=1,
+                 refine=1, device='cuda', src_format='bgr'):
+        super().__init__(S, max_src_size, height, width, depth, taps, use_masks, crop_rate, refine, device, src_format)
+
+    def _init_front_end(self, dev):
+        """per-slot sizes and tables, all zero (every slot idle) until a slot joins"""
+        (H, W), h, w = self.src_size, self.height, self.width
+        rh, rw, _, _ = _resample_size(h, w, self.crop_rate)
+        i32 = dict(device=dev, dtype=torch.int32)
+        self.pool_shape = (self.S, int(np.prod(self.frame_shape)))
+        self.sizes = torch.zeros((self.S, 2), **i32)
+        self.tables = (torch.zeros((self.S, w, _pil_ksize(W, rw)), **i32), torch.zeros((self.S, w), **i32),
+                       torch.zeros((self.S, w), **i32), torch.zeros((self.S, h, _pil_ksize(H, rh)), **i32),
+                       torch.zeros((self.S, h), **i32), torch.zeros((self.S, h), **i32))
+        self.xtab, self.ytab = torch.zeros((self.S, w, 4), **i32), torch.zeros((self.S, h, 4), **i32)
+        self.slot_sizes = [None] * self.S
+        self.cur.zero_()
+        self.small.zero_()
+
+    def _frame_size(self, f):
+        if not isinstance(f, torch.Tensor) or f.dtype != torch.uint8:
+            raise ValueError('a source frame must be a uint8 array or tensor (got %s)' % (getattr(f, 'dtype', type(f)),))
+        if self.src_format == 'bgr':
+            if f.dim() != 3 or f.shape[2] != 3:
+                raise ValueError('a BGR frame must be [H,W,3] (got %s)' % (tuple(f.shape),))
+            H, W = int(f.shape[0]), int(f.shape[1])
+        else:
+            if f.dim() != 2 or f.shape[0] % 3 or f.shape[1] % 2:
+                raise ValueError('a %s frame must be [3H/2,W] with H and W even (got %s)' % (self.src_format, tuple(f.shape)))
+            H, W = int(f.shape[0]) // 3 * 2, int(f.shape[1])
+        if not (0 < H <= self.src_size[0] and 0 < W <= self.src_size[1]):
+            raise ValueError('a %dx%d frame does not fit the capacity %dx%d' % (H, W, self.src_size[0], self.src_size[1]))
+        return H, W
+
+    def _frame_shape_of(self, H, W):
+        return (H, W, 3) if self.src_format == 'bgr' else (H * 3 // 2, W)
+
+    def join(self, slot, first):
+        """A new video starts in `slot` at the size of its first frame (BGR [H,W,3] or YUV 4:2:0 [3H/2,W] uint8, up to the
+        capacity): the slot's size and tables are written, then everything StreamBatch.join does, with the first frame converted
+        by cvt_img2train at its own size."""
+        s = self._slot(slot)
+        f = torch.as_tensor(np.ascontiguousarray(first)) if isinstance(first, np.ndarray) else first
+        H, W = self._frame_size(f)
+        # host-built tables (about 15 ms at 2160x3840), copied into the slot's rows on the current stream; nothing is kept per size
+        tabs = mixed_slot_tables((H, W), self.src_size, self.height, self.width, self.crop_rate)
+        for dst, src in zip((self.sizes,) + self.tables + (self.xtab, self.ytab), (np.array([H, W], np.int32),) + tabs):
+            dst[s].copy_(torch.as_tensor(src))
+        self.slot_sizes[s] = (H, W)
+        cur = cvt_img2train(f.to(self.frames.device), self.crop_rate, self.height, self.width, src_format=self.src_format)
+        super().join(s, cur.reshape(self.height, self.width))
+
+    def slot_frame(self, buf, slot):
+        """The view of slot `slot`'s current frame inside a pool-shaped buffer buf [S, frame_bytes(capacity)] uint8 (the pool on
+        the device, or a pinned host buffer that is uploaded into it): BGR [H_s,W_s,3] or YUV [3H_s/2,W_s] at the slot's size."""
+        s = self._slot(slot)
+        if self.slot_sizes[s] is None:
+            raise ValueError('slot %d carries no video' % s)
+        if tuple(buf.shape) != self.pool_shape or buf.dtype != torch.uint8:
+            raise ValueError('buf must be %s uint8 (got %s %s)' % (list(self.pool_shape), tuple(buf.shape), buf.dtype))
+        shape = self._frame_shape_of(*self.slot_sizes[s])
+        return buf[s, :int(np.prod(shape))].view(shape)
+
+    def step(self, pool, net):
+        """One frame of every slot from pool [S, frame_bytes(capacity)] uint8 on the device: cvt_img2train and cv2.resize of each
+        slot at its own size, and the StreamBatch step around them.  Returns the stabilised colour frames [S,h,w,3] uint8 BGR
+        (self.colour, overwritten by the next step)."""
+        if not isinstance(pool, torch.Tensor) or pool.dtype != torch.uint8 or tuple(pool.shape) != self.pool_shape:
+            raise ValueError('pool must be a %s uint8 tensor (got %s %s)' % (list(self.pool_shape), tuple(getattr(pool, 'shape', ())),
+                                                                           getattr(pool, 'dtype', type(pool))))
+        pool = ops._chk(pool, 'pool', torch.uint8).view((self.S,) + self.frame_shape)
+        h, w = self.height, self.width
+        cur = ops.cvt_img2train_mixed(pool, self.src_format, self.sizes, self.tables, h, w, out=self.cur, tmp=self.cvt_tmp)
+        xy = self.advance(cur, net)
+        small = ops.resize_linear_mixed(pool, self.src_format, self.sizes, self.xtab, self.ytab, h, w, out=self.small)
+        return ops.remap_bundle_u8(small, xy, out=self.colour, workspace=self.remap_ws)

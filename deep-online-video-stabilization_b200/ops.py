@@ -755,3 +755,56 @@ def streams_push(frames, masks, heads_dev, img, black):
         raise ValueError('masks must have the shape of frames and img / black %d x %d x %d pixels' % (s, h, w))
     with torch.cuda.device(frames.device):
         check(lib.mgw_streams_push(_p(frames), _p(masks), s, depth, _p(heads_dev), _p(img), _p(black), h, w, _st()), 'mgw_streams_push')
+
+
+# ---- several videos of different source sizes at once (deploy.MixedStreamBatch): per-slot source geometry
+SRC_FORMATS = {'bgr': 0, 'nv12': 1, 'i420': 2}    # MGW_BGR24, MGW_YUV420_NV12, MGW_YUV420_I420
+
+
+def _mixed_dims(pool, fmt, sizes):
+    """pool [S,max_h,max_w,3] (BGR) or [S,3max_h/2,max_w] (YUV 4:2:0) uint8: slot s's frame lies at the start of pool[s] in its
+    own size sizes[s] (int32 device [S,2]) -> (format constant, S, max_h, max_w)"""
+    if fmt not in SRC_FORMATS:
+        raise ValueError('source format must be one of %s (got %r)' % (sorted(SRC_FORMATS), fmt))
+    if fmt == 'bgr':
+        if pool.dim() != 4 or pool.shape[3] != 3:
+            raise ValueError('a BGR pool must be [S,max_h,max_w,3] (got %s)' % (tuple(pool.shape),))
+        s, mh, mw, _ = pool.shape
+    else:
+        code, s, mh, mw = _yuv420_dims(pool, fmt)
+    if tuple(sizes.shape) != (s, 2):
+        raise ValueError('sizes must be [%d,2] (got %s)' % (s, tuple(sizes.shape)))
+    return SRC_FORMATS[fmt], s, mh, mw
+
+
+def cvt_img2train_mixed(pool, fmt, sizes, tables, out_h, out_w, out=None, tmp=None):
+    """cvt_img2train of every slot of a pool at the slot's own size -> [S,out_h,out_w] fp32; tables = (kx [S,out_w,ksx], x0, xn
+    [S,out_w], ky [S,out_h,ksy], y0, yn [S,out_h]) int32 (deploy.mixed_slot_tables per slot).  Idle slots (size 0, above the
+    capacity, odd for YUV) leave their rows of out / tmp [S,max_h,out_w] untouched."""
+    pool, sizes = _chk(pool, 'pool', torch.uint8), _chk(sizes, 'sizes', torch.int32)
+    code, s, mh, mw = _mixed_dims(pool, fmt, sizes)
+    kx, x0, xn, ky, y0, yn = (_chk(t, 'table', torch.int32) for t in tables)
+    if (kx.dim() != 3 or tuple(kx.shape[:2]) != (s, out_w) or ky.dim() != 3 or tuple(ky.shape[:2]) != (s, out_h) or
+            any(tuple(t.shape) != (s, out_w) for t in (x0, xn)) or any(tuple(t.shape) != (s, out_h) for t in (y0, yn))):
+        raise ValueError('the tables must be [%d,%d,ksx], [%d,%d] x2, [%d,%d,ksy], [%d,%d] x2' % (s, out_w, s, out_w, s, out_h, s, out_h))
+    tmp = _out(tmp, (s, mh, out_w), pool.device, torch.uint8, 'tmp')
+    out = _out(out, (s, out_h, out_w), pool.device, torch.float32, 'out')
+    with torch.cuda.device(pool.device):
+        check(lib.mgw_cvt_img2train_mixed(_p(pool), code, s, mh, mw, _p(sizes), _p(kx), _p(x0), _p(xn), kx.shape[2], _p(ky), _p(y0),
+                                          _p(yn), ky.shape[2], out_h, out_w, _p(tmp), _p(out), _st()), 'mgw_cvt_img2train_mixed')
+    return out
+
+
+def resize_linear_mixed(pool, fmt, sizes, xtab, ytab, out_h, out_w, out=None):
+    """cv2.resize of every slot of a pool at the slot's own size -> [S,out_h,out_w,3] BGR; xtab [S,out_w,4], ytab [S,out_h,4]
+    int32 (also for slots that take the 2x2 shortcut).  Idle slots leave their rows of out untouched."""
+    pool, sizes = _chk(pool, 'pool', torch.uint8), _chk(sizes, 'sizes', torch.int32)
+    code, s, mh, mw = _mixed_dims(pool, fmt, sizes)
+    xtab, ytab = _chk(xtab, 'xtab', torch.int32), _chk(ytab, 'ytab', torch.int32)
+    if tuple(xtab.shape) != (s, out_w, 4) or tuple(ytab.shape) != (s, out_h, 4):
+        raise ValueError('xtab / ytab must be [%d,%d,4] / [%d,%d,4]' % (s, out_w, s, out_h))
+    dst = _out(out, (s, out_h, out_w, 3), pool.device, torch.uint8, 'out')
+    with torch.cuda.device(pool.device):
+        check(lib.mgw_resize_linear_mixed(_p(pool), code, s, mh, mw, _p(sizes), _p(xtab), _p(ytab), out_h, out_w, _p(dst), _st()),
+              'mgw_resize_linear_mixed')
+    return dst

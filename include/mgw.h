@@ -287,6 +287,29 @@ MGW_API int mgw_cvt_img2train_yuv420_batch(const uint8_t* yuv, int format, int S
 MGW_API int mgw_resize_linear_yuv420_batch(const uint8_t* yuv, int format, int S, int H, int W, const int32_t* xtab, const int32_t* ytab,
                                int out_h, int out_w, uint8_t* dst, void* stream);
 
+/* ---- f1/f2 for a batch of videos of different source sizes: per-slot source geometry ----------------------------------
+ * The batch has a capacity (max_h, max_w); slot s owns the region src + s * frame_bytes(max_h, max_w) of the pool (frame_bytes =
+ * 3*H*W for MGW_BGR24, 3H/2*W for YUV 4:2:0), and its frame lies contiguous at the start of that region in the slot's own size
+ * sizes[s] = (H_s, W_s): BGR [H_s,W_s,3] or YUV [3H_s/2,W_s] in the layouts above.  sizes: device int32 [S,2], 8-byte aligned.
+ * Per-slot tables, each slot's rows those of the uniform call at the slot's size:
+ *   mgw_cvt_img2train_mixed: kx [S,out_w,ksx], x0 / xn [S,out_w], ky [S,out_h,ksy], y0 / yn [S,out_h]; ksx / ksy are the window
+ *     lengths of the capacity (Pillow's 2*ceil(max(in/out,1))+1 does not decrease as the input grows), a slot's shorter rows
+ *     zero-padded; tmp [S,max_h,out_w] bytes; -> out [S,out_h,out_w].
+ *   mgw_resize_linear_mixed: xtab [S,out_w,4], ytab [S,out_h,4] (16-byte aligned, required even where a slot takes the 2x2
+ *     shortcut, which is chosen per slot: H_s == 2*out_h and W_s == 2*out_w); -> dst [S,out_h,out_w,3] BGR.
+ * Every active slot's result is bit-identical to the uniform batch call (mgw_*_u8_batch / mgw_*_yuv420_batch) at that slot's size.
+ * A slot whose size is 0, larger than the capacity, or odd for a YUV format is idle: its blocks write nothing (out / tmp / dst rows
+ * keep what they held).  The tables' contents are trusted, as in the uniform calls.
+ * Checked in the order of the batch calls: sizes and format (0 <= S <= 65535, capacity positive and even for YUV, the uniform
+ * calls' 32-bit limits over the capacity: S*max_h*max_w < 2^29 for BGR, S*(3max_h/2)*max_w < 2^31 for YUV; ksx, ksy > 0), then
+ * S = 0 returns MGW_OK and launches nothing, then the pointers and their alignment. */
+#define MGW_BGR24 0
+MGW_API int mgw_cvt_img2train_mixed(const uint8_t* src, int format, int S, int max_h, int max_w, const int32_t* sizes,
+                               const int32_t* kx, const int32_t* x0, const int32_t* xn, int ksx, const int32_t* ky, const int32_t* y0,
+                               const int32_t* yn, int ksy, int out_h, int out_w, uint8_t* tmp, float* out, void* stream);
+MGW_API int mgw_resize_linear_mixed(const uint8_t* src, int format, int S, int max_h, int max_w, const int32_t* sizes,
+                               const int32_t* xtab, const int32_t* ytab, int out_h, int out_w, uint8_t* dst, void* stream);
+
 /* ---- a6: interpolate(im, x, y, out_size), spatial_transformer.py:200-281 ------------------------------
  * im [N,IH,IW,C]; x,y [N,OH,OW] normalised coords -> out [N,OH,OW,C]. */
 MGW_API int mgw_interp_fwd(const float* im, const float* x, const float* y, int N, int IH, int IW, int C, int OH, int OW,
