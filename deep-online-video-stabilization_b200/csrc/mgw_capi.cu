@@ -512,6 +512,28 @@ int mgw_remap_bundle_u8(const uint8_t* img, const float* xy, int N, int H, int W
     return launch_remap_bundle_u8(img, xy, N, H, W, C, dst, workspace, (cudaStream_t)stream);
 }
 
+size_t mgw_remap_bundle_frame_workspace_bytes(int S, int h, int w, int H, int W)
+{
+    (void)H; (void)W;       // the workspace holds the /4 maps, whose size is the network's
+    return mgw_remap_bundle_u8_workspace_bytes(S, h, w);
+}
+
+// The batch calls' order: sizes and format, then S = 0, then pointers.  H, W <= 32767: OpenCV clamps the taps to int16.
+int mgw_remap_bundle_frame(const uint8_t* src, int format, const float* xy, int S, int h, int w, int H, int W, uint8_t* dst,
+                           void* workspace, void* stream)
+{
+    REQUIRE(S >= 0 && S <= 65535 && h >= 8 && w >= 8 && H >= 1 && W >= 1 && H <= 32767 && W <= 32767 &&
+            (format == MGW_BGR24 || (H % 2 == 0 && W % 2 == 0)) && (long long)S * H * W * 3 < (1LL << 31) &&
+            (long long)S * h * w < (1LL << 31),
+            "mgw_remap_bundle_frame: bad sizes (S=%d maps %dx%d frame %dx%d; h, w >= 8, H and W even for YUV)", S, h, w, H, W);
+    REQUIRE(format == MGW_BGR24 || format == MGW_YUV420_NV12 || format == MGW_YUV420_I420, "mgw_remap_bundle_frame: unknown format %d",
+            format);
+    if (S == 0) return MGW_OK;
+    REQUIRE(src && xy && dst && workspace, "mgw_remap_bundle_frame: null pointer");
+    REQUIRE(aligned(xy, 8) && aligned(workspace, 8), "mgw_remap_bundle_frame: xy and workspace must be 8-byte aligned");
+    return launch_remap_bundle(src, format, 3, xy, S, h, w, H, W, dst, workspace, (cudaStream_t)stream);
+}
+
 int mgw_stream_assemble(const float* frames, const float* masks, int depth, int head, const int* taps, int ntaps, int use_masks,
                         const float* cur, int H, int W, float* in_x, void* stream)
 {

@@ -14,17 +14,17 @@ namespace {
 
 struct Lin { int i0, i1; float a0, a1; };
 
-// resize.cpp: inv_scale = dsize / (double)ssize, scale = 1. / inv_scale, fx = (float)((d + 0.5) * scale - 0.5)
-__device__ __forceinline__ float src_pos(int d, int n_out, int n_in)
-{
-    const double scale = 1.0 / ((double)n_out / (double)n_in);
-    return (float)(((double)d + 0.5) * scale - 0.5);
-}
+// resize.cpp: inv_scale = dsize / (double)ssize, scale = 1. / inv_scale, fx = (float)((d + 0.5) * scale - 0.5).  The scale is the
+// same IEEE double on the host and the device, so a kernel may take it as a launch argument (resize_scale) instead of dividing.
+__host__ __device__ __forceinline__ double resize_scale(int n_out, int n_in) { return 1.0 / ((double)n_out / (double)n_in); }
+
+__device__ __forceinline__ float src_pos_s(int d, double scale) { return (float)(((double)d + 0.5) * scale - 0.5); }
+
+__device__ __forceinline__ float src_pos(int d, int n_out, int n_in) { return src_pos_s(d, resize_scale(n_out, n_in)); }
 
 // horizontal taps: a tap outside the row is folded onto the border with weight 0
-__device__ __forceinline__ Lin hcoef(int d, int n_out, int n_in)
+__device__ __forceinline__ Lin hcoef_at(float fx, int n_in)
 {
-    float fx = src_pos(d, n_out, n_in);
     int sx = (int)floorf(fx);
     fx = __fsub_rn(fx, (float)sx);
     if (sx < 0) { sx = 0; fx = 0.0f; }
@@ -35,15 +35,17 @@ __device__ __forceinline__ Lin hcoef(int d, int n_out, int n_in)
 }
 
 // vertical taps: row indices clamped, weights kept
-__device__ __forceinline__ Lin vcoef(int d, int n_out, int n_in)
+__device__ __forceinline__ Lin vcoef_at(float fy, int n_in)
 {
-    float fy = src_pos(d, n_out, n_in);
     const int sy = (int)floorf(fy);
     fy = __fsub_rn(fy, (float)sy);
     Lin l;
     l.i0 = min(max(sy, 0), n_in - 1); l.i1 = min(max(sy + 1, 0), n_in - 1); l.a0 = __fsub_rn(1.0f, fy); l.a1 = fy;
     return l;
 }
+
+__device__ __forceinline__ Lin hcoef(int d, int n_out, int n_in) { return hcoef_at(src_pos(d, n_out, n_in), n_in); }
+__device__ __forceinline__ Lin vcoef(int d, int n_out, int n_in) { return vcoef_at(src_pos(d, n_out, n_in), n_in); }
 
 // one bilinear resize sample of an interleaved (x,y) map: rows first horizontally, then vertically, fp32 mul / add
 __device__ __forceinline__ float2 resize_sample(const float2* __restrict__ s, int sw, const Lin& h, const Lin& v)
@@ -66,133 +68,6 @@ maps_down_kernel(const float2* __restrict__ xy, int N, int H, int W, int h4, int
     const Lin h = hcoef(c, w4, W), v = vcoef(r, h4, H);
     small[t] = resize_sample(xy + (size_t)n * H * W, W, h, v);
 }
-
-// cvRound(v) as x86 does it (cvtss2si: round half to even; out of range / NaN -> INT_MIN)
-__device__ __forceinline__ int cv_round(float v)
-{
-    return (fabsf(v) < 2147483648.0f) ? __float2int_rn(v) : (int)0x80000000;
-}
-
-// remapBilinear on 1/32-pixel fixed-point source coordinates: taps clamped to int16, 15-bit integer weights summing to 2^15,
-// constant border 0 (imgwarp.cpp); shared by cv2.remap (float maps) and cv2.warpPerspective (its own fixed-point maps)
-template <int C>
-__device__ __forceinline__ void bilinear_fixed_u8(const uint8_t* __restrict__ base, int H, int W, int sx, int sy, uint8_t* __restrict__ o)
-{
-    const int ix = min(max(sx >> 5, -32768), 32767), iy = min(max(sy >> 5, -32768), 32767);
-    const int fx = sx & 31, fy = sy & 31;
-    const int w00 = (32 - fx) * (32 - fy) * 32, w01 = fx * (32 - fy) * 32, w10 = (32 - fx) * fy * 32, w11 = fx * fy * 32;
-    const bool x0 = (unsigned)ix < (unsigned)W, x1 = (unsigned)(ix + 1) < (unsigned)W;
-    const bool y0 = (unsigned)iy < (unsigned)H, y1 = (unsigned)(iy + 1) < (unsigned)H;
-    const uint8_t* p00 = base + ((long long)iy * W + ix) * C;
-    int acc[C];
-#pragma unroll
-    for (int ch = 0; ch < C; ++ch) acc[ch] = 1 << 14;
-    if (y0 && x0) {
-#pragma unroll
-        for (int ch = 0; ch < C; ++ch) acc[ch] += w00 * (int)__ldg(p00 + ch);
-    }
-    if (y0 && x1) {
-#pragma unroll
-        for (int ch = 0; ch < C; ++ch) acc[ch] += w01 * (int)__ldg(p00 + C + ch);
-    }
-    if (y1 && x0) {
-#pragma unroll
-        for (int ch = 0; ch < C; ++ch) acc[ch] += w10 * (int)__ldg(p00 + (long long)W * C + ch);
-    }
-    if (y1 && x1) {
-#pragma unroll
-        for (int ch = 0; ch < C; ++ch) acc[ch] += w11 * (int)__ldg(p00 + (long long)W * C + C + ch);
-    }
-#pragma unroll
-    for (int ch = 0; ch < C; ++ch) o[ch] = (uint8_t)min(max(acc[ch] >> 15, 0), 255);
-}
-
-// warpRevBundle (deploy_bundle.py:148-173): output cell (i, j) = that region of cv2.warpPerspective(img, Hs_cvt[i][j],
-// WARP_INVERSE_MAP | INTER_LINEAR).  OpenCV walks the destination in blocks of bw columns and evaluates, in double,
-//   X0 = M0*bx + M1*y + M2 (left to right), W = W0 + M6*x1, W = W ? 32/W : 0, fX = clamp((X0 + M0*x1)*W), X = cvRound(fX)
-// with bx the block's first column and x1 = x - bx; restated operation by operation (no contraction: __dmul_rn / __dadd_rn).
-__device__ __forceinline__ int persp_fixed(double a, double b, double c, double bx, double y, double x1, double Wq)
-{
-    const double X0 = __dadd_rn(__dadd_rn(__dmul_rn(a, bx), __dmul_rn(b, y)), c);
-    double f = __dmul_rn(__dadd_rn(X0, __dmul_rn(a, x1)), Wq);
-    f = (f < 2147483647.0) ? f : 2147483647.0;                    // std::min((double)INT_MAX, f)
-    f = (-2147483648.0 < f) ? f : -2147483648.0;                  // std::max((double)INT_MIN, f)
-    return __double2int_rn(f);                                    // cvRound: round half to even
-}
-
-template <int C>
-__global__ void __launch_bounds__(256)
-warp_rev_bundle_kernel(const uint8_t* __restrict__ img, const double* __restrict__ Hc, int N, int H, int W, int gh, int gw, int bw,
-                       uint8_t* __restrict__ dst)
-{
-    const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= N * H * W) return;
-    const int x = t % W, y = (t / W) % H, n = t / (W * H);
-    const int ci = min(y / (H / gh), gh - 1), cj = min(x / (W / gw), gw - 1);       // the last cell takes the remainder (:162-165)
-    const double* M = Hc + ((size_t)(n * gh + ci) * gw + cj) * 9;
-    const int bxi = (x / bw) * bw;
-    const double bx = (double)bxi, x1 = (double)(x - bxi), yd = (double)y;
-    const double W0 = __dadd_rn(__dadd_rn(__dmul_rn(__ldg(M + 6), bx), __dmul_rn(__ldg(M + 7), yd)), __ldg(M + 8));
-    double Wq = __dadd_rn(W0, __dmul_rn(__ldg(M + 6), x1));
-    Wq = (Wq != 0.0) ? __ddiv_rn(32.0, Wq) : 0.0;
-    const int sx = persp_fixed(__ldg(M + 0), __ldg(M + 1), __ldg(M + 2), bx, yd, x1, Wq);
-    const int sy = persp_fixed(__ldg(M + 3), __ldg(M + 4), __ldg(M + 5), bx, yd, x1, Wq);
-    bilinear_fixed_u8<C>(img + (size_t)n * H * W * C, H, W, sx, sy, dst + (size_t)t * C);
-}
-
-template <int C>
-__global__ void __launch_bounds__(256)
-remap_up_kernel(const uint8_t* __restrict__ img, const float2* __restrict__ small, int N, int H, int W, int h4, int w4,
-                uint8_t* __restrict__ dst)
-{
-    const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= N * H * W) return;
-    const int c = t % W, r = (t / W) % H, n = t / (W * H);
-    const Lin h = hcoef(c, W, w4), v = vcoef(r, H, h4);
-    const float2 m = resize_sample(small + (size_t)n * h4 * w4, w4, h, v);
-    // (map + 1) / 2 * size in fp32 (deploy_bundle.py:142-143)
-    const float xp = __fmul_rn(__fmul_rn(__fadd_rn(m.x, 1.0f), 0.5f), (float)W);
-    const float yp = __fmul_rn(__fmul_rn(__fadd_rn(m.y, 1.0f), 0.5f), (float)H);
-    const int sx = cv_round(__fmul_rn(xp, 32.0f)), sy = cv_round(__fmul_rn(yp, 32.0f));
-    bilinear_fixed_u8<C>(img + (size_t)n * H * W * C, H, W, sx, sy, dst + (size_t)t * C);
-}
-
-}  // namespace
-
-size_t remap_bundle_workspace_bytes(int N, int H, int W) { return sizeof(float) * 2 * (size_t)N * (H / 4) * (W / 4); }
-
-int launch_remap_bundle_u8(const uint8_t* img, const float* xy, int N, int H, int W, int C, uint8_t* dst, void* workspace,
-                           cudaStream_t st)
-{
-    const int h4 = H / 4, w4 = W / 4;       // int(height / rate), int(width / rate)
-    float2* small = reinterpret_cast<float2*>(workspace);
-    const int t1 = N * h4 * w4, t2 = N * H * W;
-    maps_down_kernel<<<(t1 + 255) / 256, 256, 0, st>>>(reinterpret_cast<const float2*>(xy), N, H, W, h4, w4, small);
-    int rc = check_launch("maps_down");
-    if (rc != MGW_OK) return rc;
-    const int grid = (t2 + 255) / 256;
-    switch (C) {
-    case 1: remap_up_kernel<1><<<grid, 256, 0, st>>>(img, small, N, H, W, h4, w4, dst); break;
-    case 3: remap_up_kernel<3><<<grid, 256, 0, st>>>(img, small, N, H, W, h4, w4, dst); break;
-    case 4: remap_up_kernel<4><<<grid, 256, 0, st>>>(img, small, N, H, W, h4, w4, dst); break;
-    default: return set_error(MGW_ERR_UNSUPPORTED, "remap_bundle_u8: C must be 1, 3 or 4 (got %d)", C);
-    }
-    return check_launch("remap_up");
-}
-
-// ---------------------------------------------------------------------------------------------------------------------
-// cvt_img2train (config.py:6-21): BGR uint8 frame -> cv2 BGR2GRAY -> Pillow resize(BILINEAR) [-> crop] -> v*(1/255) - 0.5.
-// The host binding computes Pillow's 22-bit fixed-point coefficient tables (double arithmetic, Resample.c) once per shape
-// and slices them for the crop; the two passes below are Pillow's: horizontal first into a uint8 image, then vertical.
-// A batch of S frames of one size shares the tables; blockIdx.y is the frame (the stream index of a StreamBatch): each block
-// offsets its base pointers once, the per-pixel index arithmetic is the single-frame one, and S = 1 is the single-frame call.
-// The source frame is BGR (SRC_BGR) or YUV 4:2:0 in OpenCV's layout (MGW_YUV420_NV12 / MGW_YUV420_I420): the kernels then read
-// the BGR frame cv2.cvtColor would make of it, converted per pixel on the fly.
-// MIXED = per-slot source geometry (a batch of videos of different sizes): H, W are the batch's capacity, slot s owns the region
-// [s * frame_bytes(H, W), +frame_bytes(H, W)) of the source and its frame of size sizes[s] lies at the start of it, and the slot
-// has its own tables (kx [S,out_w,ks], ...) and tmp rows [S,H,out_w].  Block (., s) reads sizes[s] once, offsets its pointers to
-// the slot, and then runs the per-pixel code of the uniform batch at the slot's size with frame index 0.
-namespace {
 
 constexpr int SRC_BGR = 0;
 
@@ -234,6 +109,207 @@ __device__ __forceinline__ size_t src_frame_bytes(int H, int W)
 {
     return FMT == SRC_BGR ? (size_t)H * W * 3 : (size_t)H * W * 3 / 2;
 }
+
+// cvRound(v) as x86 does it (cvtss2si: round half to even; out of range / NaN -> INT_MIN)
+__device__ __forceinline__ int cv_round(float v)
+{
+    return (fabsf(v) < 2147483648.0f) ? __float2int_rn(v) : (int)0x80000000;
+}
+
+// a YUV 4:2:0 source (FMT = MGW_YUV420_*, C = 3) is read as the BGR frame cvtColor makes of it: each tap is converted
+template <int FMT>
+__device__ __forceinline__ int3 yuv_bgr_at(const uint8_t* __restrict__ f, int H, int W, int row, int x)
+{
+    return yuv_to_bgr(__ldg(f + (size_t)row * W + x), yuv_chroma_at<FMT>(f, H, W, row, x));
+}
+
+// remapBilinear on 1/32-pixel fixed-point source coordinates: taps clamped to int16, 15-bit integer weights summing to 2^15,
+// constant border 0 (imgwarp.cpp); shared by cv2.remap (float maps) and cv2.warpPerspective (its own fixed-point maps).
+// base: one frame [H,W,C] (SRC_BGR) or [3H/2,W] (YUV 4:2:0, C = 3: every tap converted as cvtColor converts it)
+template <int C, int FMT = SRC_BGR>
+__device__ __forceinline__ void bilinear_fixed_u8(const uint8_t* __restrict__ base, int H, int W, int sx, int sy, uint8_t* __restrict__ o)
+{
+    static_assert(FMT == SRC_BGR || C == 3, "a YUV 4:2:0 source is sampled as BGR");
+    const int ix = min(max(sx >> 5, -32768), 32767), iy = min(max(sy >> 5, -32768), 32767);
+    const int fx = sx & 31, fy = sy & 31;
+    const int w00 = (32 - fx) * (32 - fy) * 32, w01 = fx * (32 - fy) * 32, w10 = (32 - fx) * fy * 32, w11 = fx * fy * 32;
+    const bool x0 = (unsigned)ix < (unsigned)W, x1 = (unsigned)(ix + 1) < (unsigned)W;
+    const bool y0 = (unsigned)iy < (unsigned)H, y1 = (unsigned)(iy + 1) < (unsigned)H;
+    int acc[C];
+#pragma unroll
+    for (int ch = 0; ch < C; ++ch) acc[ch] = 1 << 14;
+    if constexpr (FMT == SRC_BGR) {
+        const uint8_t* p00 = base + ((long long)iy * W + ix) * C;
+        if (y0 && x0) {
+#pragma unroll
+            for (int ch = 0; ch < C; ++ch) acc[ch] += w00 * (int)__ldg(p00 + ch);
+        }
+        if (y0 && x1) {
+#pragma unroll
+            for (int ch = 0; ch < C; ++ch) acc[ch] += w01 * (int)__ldg(p00 + C + ch);
+        }
+        if (y1 && x0) {
+#pragma unroll
+            for (int ch = 0; ch < C; ++ch) acc[ch] += w10 * (int)__ldg(p00 + (long long)W * C + ch);
+        }
+        if (y1 && x1) {
+#pragma unroll
+            for (int ch = 0; ch < C; ++ch) acc[ch] += w11 * (int)__ldg(p00 + (long long)W * C + C + ch);
+        }
+    } else {
+        const auto add = [&](int w, int3 p) { acc[0] += w * p.x; acc[1] += w * p.y; acc[2] += w * p.z; };
+        if (y0 && x0) add(w00, yuv_bgr_at<FMT>(base, H, W, iy, ix));
+        if (y0 && x1) add(w01, yuv_bgr_at<FMT>(base, H, W, iy, ix + 1));
+        if (y1 && x0) add(w10, yuv_bgr_at<FMT>(base, H, W, iy + 1, ix));
+        if (y1 && x1) add(w11, yuv_bgr_at<FMT>(base, H, W, iy + 1, ix + 1));
+    }
+#pragma unroll
+    for (int ch = 0; ch < C; ++ch) o[ch] = (uint8_t)min(max(acc[ch] >> 15, 0), 255);
+}
+
+// warpRevBundle (deploy_bundle.py:148-173): output cell (i, j) = that region of cv2.warpPerspective(img, Hs_cvt[i][j],
+// WARP_INVERSE_MAP | INTER_LINEAR).  OpenCV walks the destination in blocks of bw columns and evaluates, in double,
+//   X0 = M0*bx + M1*y + M2 (left to right), W = W0 + M6*x1, W = W ? 32/W : 0, fX = clamp((X0 + M0*x1)*W), X = cvRound(fX)
+// with bx the block's first column and x1 = x - bx; restated operation by operation (no contraction: __dmul_rn / __dadd_rn).
+__device__ __forceinline__ int persp_fixed(double a, double b, double c, double bx, double y, double x1, double Wq)
+{
+    const double X0 = __dadd_rn(__dadd_rn(__dmul_rn(a, bx), __dmul_rn(b, y)), c);
+    double f = __dmul_rn(__dadd_rn(X0, __dmul_rn(a, x1)), Wq);
+    f = (f < 2147483647.0) ? f : 2147483647.0;                    // std::min((double)INT_MAX, f)
+    f = (-2147483648.0 < f) ? f : -2147483648.0;                  // std::max((double)INT_MIN, f)
+    return __double2int_rn(f);                                    // cvRound: round half to even
+}
+
+template <int C>
+__global__ void __launch_bounds__(256)
+warp_rev_bundle_kernel(const uint8_t* __restrict__ img, const double* __restrict__ Hc, int N, int H, int W, int gh, int gw, int bw,
+                       uint8_t* __restrict__ dst)
+{
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= N * H * W) return;
+    const int x = t % W, y = (t / W) % H, n = t / (W * H);
+    const int ci = min(y / (H / gh), gh - 1), cj = min(x / (W / gw), gw - 1);       // the last cell takes the remainder (:162-165)
+    const double* M = Hc + ((size_t)(n * gh + ci) * gw + cj) * 9;
+    const int bxi = (x / bw) * bw;
+    const double bx = (double)bxi, x1 = (double)(x - bxi), yd = (double)y;
+    const double W0 = __dadd_rn(__dadd_rn(__dmul_rn(__ldg(M + 6), bx), __dmul_rn(__ldg(M + 7), yd)), __ldg(M + 8));
+    double Wq = __dadd_rn(W0, __dmul_rn(__ldg(M + 6), x1));
+    Wq = (Wq != 0.0) ? __ddiv_rn(32.0, Wq) : 0.0;
+    const int sx = persp_fixed(__ldg(M + 0), __ldg(M + 1), __ldg(M + 2), bx, yd, x1, Wq);
+    const int sy = persp_fixed(__ldg(M + 3), __ldg(M + 4), __ldg(M + 5), bx, yd, x1, Wq);
+    bilinear_fixed_u8<C>(img + (size_t)n * H * W * C, H, W, sx, sy, dst + (size_t)t * C);
+}
+
+// K5b: output pixel (r, c) of frame n samples the /4 maps (h4 x w4) bilinearly at the output size H x W, turns them into pixel
+// coordinates of the frame and remaps the frame, which has the output's size.  Each thread takes a run of REMAP_RUN adjacent
+// pixels of the frame's row-major order (a run may cross rows), so that it stores whole words: C words of 4 pixels.  The
+// per-column and per-row map coefficients are the device functions of maps_down at the output size; their resize scales
+// (a double division each) are launch arguments.  blockIdx.y is the frame.
+constexpr int REMAP_RUN = 4;
+
+template <int C, int FMT>
+__global__ void __launch_bounds__(256)
+remap_up_kernel(const uint8_t* __restrict__ src, const float2* __restrict__ small, int H, int W, int h4, int w4, double xscale,
+                double yscale, uint8_t* __restrict__ dst)
+{
+    const int HW = H * W;
+    const int p0 = (blockIdx.x * blockDim.x + threadIdx.x) * REMAP_RUN;
+    if (p0 >= HW) return;
+    const size_t n = blockIdx.y;
+    const uint8_t* f = src + n * (FMT == SRC_BGR ? (size_t)HW * C : (size_t)HW * 3 / 2);
+    small += n * h4 * w4;
+    uint8_t* o = dst + (n * HW + p0) * C;
+    int r = p0 / W, c = p0 - r * W;
+    Lin v = vcoef_at(src_pos_s(r, yscale), h4);
+    uint8_t px[REMAP_RUN * C];
+#pragma unroll
+    for (int k = 0; k < REMAP_RUN; ++k) {
+        if (k > 0 && ++c == W) { c = 0; ++r; v = vcoef_at(src_pos_s(r, yscale), h4); }
+        // past the frame's last pixel r = H: its map rows clamp and its taps fall outside, and nothing of it is stored
+        const Lin h = hcoef_at(src_pos_s(c, xscale), w4);
+        const float2 m = resize_sample(small, w4, h, v);
+        // (map + 1) / 2 * size in fp32 (deploy_bundle.py:142-143)
+        const float xp = __fmul_rn(__fmul_rn(__fadd_rn(m.x, 1.0f), 0.5f), (float)W);
+        const float yp = __fmul_rn(__fmul_rn(__fadd_rn(m.y, 1.0f), 0.5f), (float)H);
+        const int sx = cv_round(__fmul_rn(xp, 32.0f)), sy = cv_round(__fmul_rn(yp, 32.0f));
+        bilinear_fixed_u8<C, FMT>(f, H, W, sx, sy, px + k * C);
+    }
+    if (p0 + REMAP_RUN <= HW && (reinterpret_cast<uintptr_t>(o) & 3) == 0) {
+#pragma unroll
+        for (int q = 0; q < C; ++q)
+            reinterpret_cast<uint32_t*>(o)[q] = (uint32_t)px[4 * q] | ((uint32_t)px[4 * q + 1] << 8) | ((uint32_t)px[4 * q + 2] << 16) |
+                                                ((uint32_t)px[4 * q + 3] << 24);
+    } else {
+        const int n_bytes = min(REMAP_RUN, HW - p0) * C;
+#pragma unroll
+        for (int i = 0; i < REMAP_RUN * C; ++i)
+            if (i < n_bytes) o[i] = px[i];
+    }
+}
+
+template <int C, int FMT>
+int launch_remap_up(const uint8_t* src, const float2* small, int N, int H, int W, int h4, int w4, uint8_t* dst, cudaStream_t st)
+{
+    const unsigned gx = (unsigned)((((long long)H * W + REMAP_RUN - 1) / REMAP_RUN + 255) / 256);
+    const double xscale = resize_scale(W, w4), yscale = resize_scale(H, h4);
+    // the frame index is gridDim.y: a batch of more than 65535 frames (mgw_remap_bundle_u8 allows it) takes several launches
+    for (int n0 = 0; n0 < N; n0 += 65535) {
+        const int n = min(N - n0, 65535);
+        remap_up_kernel<C, FMT><<<dim3(gx, n), 256, 0, st>>>(src + (size_t)n0 * (FMT == SRC_BGR ? (size_t)H * W * C : (size_t)H * W * 3 / 2),
+                                                             small + (size_t)n0 * h4 * w4, H, W, h4, w4, xscale, yscale,
+                                                             dst + (size_t)n0 * H * W * C);
+        if (int rc = check_launch("remap_up")) return rc;
+    }
+    return MGW_OK;
+}
+
+}  // namespace
+
+size_t remap_bundle_workspace_bytes(int N, int H, int W) { return sizeof(float) * 2 * (size_t)N * (H / 4) * (W / 4); }
+
+// K5a at the maps' size h x w, then K5b at the output size H x W; the frame src has the output's size
+int launch_remap_bundle(const uint8_t* src, int src_fmt, int C, const float* xy, int N, int h, int w, int H, int W, uint8_t* dst,
+                        void* workspace, cudaStream_t st)
+{
+    const int h4 = h / 4, w4 = w / 4;       // int(height / rate), int(width / rate)
+    float2* small = reinterpret_cast<float2*>(workspace);
+    const int t1 = N * h4 * w4;
+    maps_down_kernel<<<(t1 + 255) / 256, 256, 0, st>>>(reinterpret_cast<const float2*>(xy), N, h, w, h4, w4, small);
+    if (int rc = check_launch("maps_down")) return rc;
+    if (src_fmt != SRC_BGR && C != 3) return set_error(MGW_ERR_UNSUPPORTED, "remap_bundle: a YUV 4:2:0 source gives C = 3 (got %d)", C);
+    switch (src_fmt) {
+    case SRC_BGR:
+        switch (C) {
+        case 1: return launch_remap_up<1, SRC_BGR>(src, small, N, H, W, h4, w4, dst, st);
+        case 3: return launch_remap_up<3, SRC_BGR>(src, small, N, H, W, h4, w4, dst, st);
+        case 4: return launch_remap_up<4, SRC_BGR>(src, small, N, H, W, h4, w4, dst, st);
+        default: return set_error(MGW_ERR_UNSUPPORTED, "remap_bundle_u8: C must be 1, 3 or 4 (got %d)", C);
+        }
+    case MGW_YUV420_NV12: return launch_remap_up<3, MGW_YUV420_NV12>(src, small, N, H, W, h4, w4, dst, st);
+    case MGW_YUV420_I420: return launch_remap_up<3, MGW_YUV420_I420>(src, small, N, H, W, h4, w4, dst, st);
+    default: return set_error(MGW_ERR_INVALID, "remap_bundle: unknown source format %d", src_fmt);
+    }
+}
+
+int launch_remap_bundle_u8(const uint8_t* img, const float* xy, int N, int H, int W, int C, uint8_t* dst, void* workspace,
+                           cudaStream_t st)
+{
+    return launch_remap_bundle(img, SRC_BGR, C, xy, N, H, W, H, W, dst, workspace, st);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// cvt_img2train (config.py:6-21): BGR uint8 frame -> cv2 BGR2GRAY -> Pillow resize(BILINEAR) [-> crop] -> v*(1/255) - 0.5.
+// The host binding computes Pillow's 22-bit fixed-point coefficient tables (double arithmetic, Resample.c) once per shape
+// and slices them for the crop; the two passes below are Pillow's: horizontal first into a uint8 image, then vertical.
+// A batch of S frames of one size shares the tables; blockIdx.y is the frame (the stream index of a StreamBatch): each block
+// offsets its base pointers once, the per-pixel index arithmetic is the single-frame one, and S = 1 is the single-frame call.
+// The source frame is BGR (SRC_BGR) or YUV 4:2:0 in OpenCV's layout (MGW_YUV420_NV12 / MGW_YUV420_I420): the kernels then read
+// the BGR frame cv2.cvtColor would make of it, converted per pixel on the fly.
+// MIXED = per-slot source geometry (a batch of videos of different sizes): H, W are the batch's capacity, slot s owns the region
+// [s * frame_bytes(H, W), +frame_bytes(H, W)) of the source and its frame of size sizes[s] lies at the start of it, and the slot
+// has its own tables (kx [S,out_w,ks], ...) and tmp rows [S,H,out_w].  Block (., s) reads sizes[s] once, offsets its pointers to
+// the slot, and then runs the per-pixel code of the uniform batch at the slot's size with frame index 0.
+namespace {
 
 // A slot is idle -- its blocks return before they write anything -- when its size is 0, larger than the capacity, or odd for a
 // YUV format: never-joined slots, and a bad device-side size cannot move a read outside the slot's region.
@@ -365,13 +441,6 @@ int launch_cvt_img2train_mixed(const uint8_t* src, int src_fmt, int S, int max_h
 // ((b0*(S0>>4))>>16) + ((b1*(S1>>4))>>16) + 2) >> 2 vertically; an exact 2x2 decimation is OpenCV's INTER_AREA shortcut.
 // blockIdx.y is the frame of a batch of S frames of one size (as for cvt_img2train above).
 namespace {
-
-// a YUV 4:2:0 source (FMT = MGW_YUV420_*, C = 3) is resampled as the BGR frame cvtColor makes of it: each tap is converted
-template <int FMT>
-__device__ __forceinline__ int3 yuv_bgr_at(const uint8_t* __restrict__ f, int H, int W, int row, int x)
-{
-    return yuv_to_bgr(__ldg(f + (size_t)row * W + x), yuv_chroma_at<FMT>(f, H, W, row, x));
-}
 
 __device__ __forceinline__ int ch_of(const int3& p, int ch) { return ch == 0 ? p.x : (ch == 1 ? p.y : p.z); }
 

@@ -111,6 +111,10 @@ int launch_warp_fwd_pipe(const float* U, const float* Hs, const WarpShape& s, fl
 size_t remap_bundle_workspace_bytes(int N, int H, int W);
 int launch_remap_bundle_u8(const uint8_t* img, const float* xy, int N, int H, int W, int C, uint8_t* dst, void* workspace,
                            cudaStream_t st);
+// the same warp with maps xy [N,h,w,2] of the network's size applied to frames of the output's size H x W: BGR / C-channel
+// [N,H,W,C] (src_fmt 0) or YUV 4:2:0 [N,3H/2,W] (C = 3) -> dst [N,H,W,C]; the workspace is remap_bundle_workspace_bytes(N, h, w)
+int launch_remap_bundle(const uint8_t* src, int src_fmt, int C, const float* xy, int N, int h, int w, int H, int W, uint8_t* dst,
+                        void* workspace, cudaStream_t st);
 
 // S frames of one size ([S,H,W,C] -> [S,out_h,out_w,C]; S >= 1, the single-frame calls pass 1).  src_fmt: 0 for the BGR / C-channel
 // frames, MGW_YUV420_NV12 or MGW_YUV420_I420 for YUV 4:2:0 frames [S,3H/2,W] read as the BGR frames cvtColor makes of them (C = 3)

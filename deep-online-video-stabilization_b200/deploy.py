@@ -4,7 +4,8 @@
 
 `warpRevBundle2` keeps the reference signature -- one uint8 frame [H,W,3] and the operator's x_map / y_map [H,W] -- and
 accepts numpy arrays (as the reference's caller passes; the result comes back as a numpy array) or CUDA tensors (batched
-[N,H,W,C] / [N,H,W] too; the result stays on the device).  The work is one C-ABI call, mgw_remap_bundle_u8.
+[N,H,W,C] / [N,H,W] too; the result stays on the device).  The work is one C-ABI call, mgw_remap_bundle_u8; a frame of
+another size than the maps (1080p with the network's 288x512 maps) is stabilised at its own size by mgw_remap_bundle_frame.
 
 StreamBatch runs the whole per-frame loop for S videos of one size at once: one set of launches per frame, capturable as one
 CUDA graph, every video's result bit-identical to its own StreamState / CropState pipeline.  MixedStreamBatch does the same for
@@ -16,10 +17,14 @@ import torch
 from . import ops
 
 __all__ = ['warpRevBundle2', 'warpRevBundle', 'warpRev', 'cvt_theta_mat_bundle', 'cvt_img2train', 'cv2_resize', 'StreamState', 'CropState', 'StreamBatch',
-           'MixedStreamBatch', 'mixed_slot_tables']
+           'MixedStreamBatch', 'mixed_slot_tables', 'scale_rect']
 
 
-def warpRevBundle2(img, x_map, y_map, device=None):
+def warpRevBundle2(img, x_map, y_map, device=None, src_format='bgr'):
+    """The frame img, of any size, stabilised at its own size with the operator's x_map / y_map (network size): the reference's
+    expression with the size the colour frame is resized to taken from the frame instead of the network.  A frame at the maps'
+    size is exactly the reference's warpRevBundle2.  img: [H,W,C] or [N,H,W,C] uint8 BGR, or for src_format 'nv12' / 'i420' a
+    YUV 4:2:0 frame [3H/2,W] or batch [N,3H/2,W] (read as the BGR frame cv2.cvtColor makes of it; the result is BGR [H,W,3])."""
     as_numpy = isinstance(img, np.ndarray)
     dev = torch.device(device) if device is not None else (torch.device('cuda') if as_numpy else img.device)
 
@@ -27,16 +32,51 @@ def warpRevBundle2(img, x_map, y_map, device=None):
         t = torch.as_tensor(np.ascontiguousarray(a)) if isinstance(a, np.ndarray) else a
         return t.to(device=dev, dtype=dtype)
 
-    im, xm, ym = to_dev(img, torch.uint8), to_dev(x_map, torch.float32), to_dev(y_map, torch.float32)
-    single = im.dim() == 3
-    if single:
-        im = im.unsqueeze(0)
-    n, h, w, _ = im.shape
-    xy = torch.stack([xm.reshape(n, h, w), ym.reshape(n, h, w)], dim=-1)
-    dst = ops.remap_bundle_u8(im, xy)
+    xm, ym = to_dev(x_map, torch.float32), to_dev(y_map, torch.float32)
+    yuv = _yuv420_frames(img, src_format)
+    if yuv is not None:
+        im, single, H, W = yuv
+        im = im.to(device=dev).contiguous()
+    else:
+        im = to_dev(img, torch.uint8)
+        single = im.dim() == 3
+        if single:
+            im = im.unsqueeze(0)
+        H, W = int(im.shape[1]), int(im.shape[2])
+    n = int(im.shape[0])
+    if yuv is None and xm.numel() == n * H * W:
+        # the maps have the frame's size: the reference's call
+        xy = torch.stack([xm.reshape(n, H, W), ym.reshape(n, H, W)], dim=-1)
+        dst = ops.remap_bundle_u8(im, xy)
+    else:
+        shape = list(xm.shape)
+        while len(shape) > 2 and shape[-1] == 1:        # [1,h,w,1] as the network hands it out
+            shape.pop()
+        if len(shape) < 2 or xm.numel() != n * shape[-2] * shape[-1] or ym.numel() != xm.numel():
+            raise ValueError('x_map / y_map must be [h,w] maps, one per frame (got %s for %d frames)' % (tuple(xm.shape), n))
+        h, w = shape[-2], shape[-1]
+        xy = torch.stack([xm.reshape(n, h, w), ym.reshape(n, h, w)], dim=-1)
+        dst = ops.remap_bundle_frame(im.contiguous(), src_format, xy)
     if single:
         dst = dst[0]
     return dst.cpu().numpy() if as_numpy else dst
+
+
+def scale_rect(rect, from_size, to_size):
+    """A crop rectangle [top, left, bottom, right] (inclusive, as leave() / CropState.rect() give it on the network's lattice
+    from_size = (h, w)) carried to an output of to_size = (OH, OW) pixels with the centre alignment of the maps: output row R is
+    kept iff top <= (R + 0.5) * h / OH - 0.5 <= bottom (columns alike), in integers and clamped to the output.  The identity at
+    equal sizes."""
+    t, l, b, r = (int(v) for v in rect)
+    (h, w), (OH, OW) = (int(v) for v in from_size), (int(v) for v in to_size)
+
+    def first(lo, n, N):            # ceil(((2 lo + 1) N - n) / (2 n))
+        return min(max(-((n - (2 * lo + 1) * N) // (2 * n)), 0), N - 1)
+
+    def last(hi, n, N):             # floor(((2 hi + 1) N - n) / (2 n))
+        return min(max(((2 * hi + 1) * N - n) // (2 * n), 0), N - 1)
+
+    return [first(t, h, OH), first(l, w, OW), last(b, h, OH), last(r, w, OW)]
 
 
 def _pil_bilinear_windows(in_size, out_size):
@@ -365,13 +405,21 @@ class StreamBatch:
     Every slot is computed at every step.  A slot that carries no video (never joined, or left and not joined again) runs on
     whatever frame the caller puts there and its output means nothing: the caller decides which slots carry a video and
     ignores the others.  All buffers are allocated here and never reallocated, so a step can be captured once as a CUDA graph
-    (capture()) and replayed; join / leave between replays act on the same buffers."""
+    (capture()) and replayed; join / leave between replays act on the same buffers.
+
+    out_size=(OH, OW) sets the size of the stabilised colour frames (default: the network's (height, width), the reference's
+    output).  The network's maps warp the frame resized to that size; at out_size == src_size nothing is resized and the warp
+    reads the source batch (BGR or YUV 4:2:0) itself, so a 1080p video comes out at 1080p.  crop_rate does not act on the colour
+    frames, as in the reference; scale_rect() carries leave()'s rectangle to output pixels."""
 
     def __init__(self, S, src_size, height=288, width=512, depth=32, taps=(1, 2, 4, 8, 16, 32), use_masks=True, crop_rate=1, refine=1,
-                 device='cuda', src_format='bgr'):
+                 device='cuda', src_format='bgr', out_size=None):
         S, H, W, h, w = int(S), int(src_size[0]), int(src_size[1]), int(height), int(width)
         if S < 1 or refine < 1:
             raise ValueError('StreamBatch needs S >= 1 and refine >= 1 (got S=%d, refine=%d)' % (S, refine))
+        out = (h, w) if out_size is None else (int(out_size[0]), int(out_size[1]))
+        if not (1 <= out[0] <= 32767 and 1 <= out[1] <= 32767):
+            raise ValueError('out_size %s: each side in [1, 32767]' % (tuple(out_size),))
         if src_format == 'bgr':
             self.frame_shape = (H, W, 3)
         elif src_format in ops.YUV420_FORMATS:
@@ -386,6 +434,9 @@ class StreamBatch:
             raise ValueError('taps %s: 1 to 32 distances in [1, depth = %d]' % (self.taps, depth))
         dev = torch.device(device)
         self.S, self.src_size, self.height, self.width, self.depth = S, (H, W), h, w, int(depth)
+        self.out_size = out
+        # the remap reads the source batch itself when the output has its size; None keeps the network-size path as it was
+        self._direct = out_size is not None and out == (H, W)
         self.use_masks, self.crop_rate, self.refine = bool(use_masks), crop_rate, int(refine)
         self.nch = (2 if use_masks else 1) * len(self.taps) + 1
         f32 = dict(device=dev, dtype=torch.float32)
@@ -398,8 +449,8 @@ class StreamBatch:
         self.cur = torch.empty((S, h, w), **f32)
         self.cvt_tmp = torch.empty((S, H, w), device=dev, dtype=torch.uint8)
         self.in_x = torch.empty((S, h, w, self.nch), **f32)
-        self.small = torch.empty((S, h, w, 3), device=dev, dtype=torch.uint8)
-        self.colour = torch.empty((S, h, w, 3), device=dev, dtype=torch.uint8)
+        self.small = None if self._direct else torch.empty((S,) + out + (3,), device=dev, dtype=torch.uint8)
+        self.colour = torch.empty((S,) + out + (3,), device=dev, dtype=torch.uint8)
         self.remap_ws = torch.empty(ops.remap_bundle_workspace_floats(S, h, w), **f32)
         self._init_front_end(dev)
 
@@ -407,7 +458,7 @@ class StreamBatch:
         """the coefficient tables of the two stages that read the source frame: the uniform ones of src_size"""
         (H, W), h, w = self.src_size, self.height, self.width
         self._cvt = _cvt_tables(H, W, h, w, self.crop_rate, dev)
-        self._resize = _resize_tables(H, W, h, w, dev)
+        self._resize = _resize_tables(H, W, self.out_size[0], self.out_size[1], dev)
 
     def _slot(self, slot):
         if not isinstance(slot, (int, np.integer)) or not 0 <= slot < self.S:
@@ -454,8 +505,8 @@ class StreamBatch:
 
     def step(self, raw_bgr, net):
         """One frame of every slot from raw_bgr [S,H,W,3] uint8 on the device ([S,3H/2,W] for a YUV 4:2:0 batch): cvt_img2train,
-        advance(), cv2_resize of the colour frames and warpRevBundle2 with the last xy.  Returns the stabilised colour frames
-        [S,h,w,3] uint8 BGR (self.colour, overwritten by the next step)."""
+        advance(), cv2_resize of the colour frames to out_size (none at out_size == src_size) and warpRevBundle2 with the last xy.
+        Returns the stabilised colour frames [S,OH,OW,3] uint8 BGR (self.colour, overwritten by the next step)."""
         raw = ops._chk(raw_bgr, 'raw_bgr', torch.uint8)
         if tuple(raw.shape) != (self.S,) + self.frame_shape:
             raise ValueError('raw_bgr must be %s uint8 (got %s)' % ([self.S] + list(self.frame_shape), tuple(raw.shape)))
@@ -465,18 +516,25 @@ class StreamBatch:
         else:
             cur = ops.cvt_img2train_yuv420_batch(raw, self.src_format, self._cvt, h, w, out=self.cur, tmp=self.cvt_tmp)
         xy = self.advance(cur, net)
+        if self._direct:
+            return ops.remap_bundle_frame(raw, self.src_format, xy, out=self.colour, workspace=self.remap_ws)
+        oh, ow = self.out_size
         if self.src_format == 'bgr':
-            small = ops.resize_linear_u8_batch(raw, self._resize[0], self._resize[1], h, w, out=self.small)
+            small = ops.resize_linear_u8_batch(raw, self._resize[0], self._resize[1], oh, ow, out=self.small)
         else:
-            small = ops.resize_linear_yuv420_batch(raw, self.src_format, self._resize[0], self._resize[1], h, w, out=self.small)
-        return ops.remap_bundle_u8(small, xy, out=self.colour, workspace=self.remap_ws)
+            small = ops.resize_linear_yuv420_batch(raw, self.src_format, self._resize[0], self._resize[1], oh, ow, out=self.small)
+        if (oh, ow) == (h, w):
+            return ops.remap_bundle_u8(small, xy, out=self.colour, workspace=self.remap_ws)
+        return ops.remap_bundle_frame(small, 'bgr', xy, out=self.colour, workspace=self.remap_ws)
 
     def capture(self, raw_bgr, net, upload_from=None, download_to=None):
         """Records step(raw_bgr, net) as a CUDA graph and returns it: graph.replay() runs one step on whatever raw_bgr holds and
         leaves the frames in self.colour.  upload_from / download_to: optional host buffers ([S,H,W,3] or, for a YUV 4:2:0
-        batch, [S,3H/2,W] / [S,h,w,3] uint8, pinned) copied into raw_bgr before and out of self.colour after the step, inside the graph.  One eager step runs first
+        batch, [S,3H/2,W] / [S,OH,OW,3] uint8, pinned) copied into raw_bgr before and out of self.colour after the step, inside the graph.  One eager step runs first
         on a side stream as a warm-up (a network may select algorithms or allocate on its first call); the state it changed
         is restored, so capturing leaves every slot as it was."""
+        if download_to is not None and tuple(download_to.shape) != tuple(self.colour.shape):
+            raise ValueError('download_to must be %s (got %s)' % (list(self.colour.shape), tuple(download_to.shape)))
         state = (self.frames, self.masks, self.heads_dev, self.all_black)
         snap = [t.clone() for t in state]
         side = torch.cuda.Stream(device=self.frames.device)

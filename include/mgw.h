@@ -310,6 +310,17 @@ MGW_API int mgw_cvt_img2train_mixed(const uint8_t* src, int format, int S, int m
 MGW_API int mgw_resize_linear_mixed(const uint8_t* src, int format, int S, int max_h, int max_w, const int32_t* sizes,
                                const int32_t* xtab, const int32_t* ytab, int out_h, int out_w, uint8_t* dst, void* stream);
 
+/* ---- f1 at any output size: warpRevBundle2 of the frame at its own size ---------------------------------------------
+ * src [S,H,W,3] (MGW_BGR24) or [S,3H/2,W] (MGW_YUV420_NV12 / _I420), xy [S,h,w,2] (the operator's x_map,y_map at the network
+ * size) -> dst [S,H,W,3] BGR = cv2.remap of the frame with the /4 maps resized to (W, H) and scaled by (W, H), constant border 0
+ * (a YUV frame is read as the BGR frame cv2.cvtColor makes of it).  (H, W) == (h, w) with MGW_BGR24 is mgw_remap_bundle_u8, bit
+ * for bit.  workspace: device scratch of mgw_remap_bundle_frame_workspace_bytes() (the /4 maps), 8-byte aligned like xy.
+ * Checked in the order of the batch calls: sizes and format (0 <= S <= 65535, h, w >= 8, 1 <= H, W <= 32767, H and W even for
+ * YUV, S*H*W*3 < 2^31, S*h*w < 2^31), then S = 0 returns MGW_OK and launches nothing, then the pointers and their alignment. */
+MGW_API size_t mgw_remap_bundle_frame_workspace_bytes(int S, int h, int w, int H, int W);
+MGW_API int mgw_remap_bundle_frame(const uint8_t* src, int format, const float* xy, int S, int h, int w, int H, int W,
+                               uint8_t* dst, void* workspace, void* stream);
+
 /* ---- a6: interpolate(im, x, y, out_size), spatial_transformer.py:200-281 ------------------------------
  * im [N,IH,IW,C]; x,y [N,OH,OW] normalised coords -> out [N,OH,OW,C]. */
 MGW_API int mgw_interp_fwd(const float* im, const float* x, const float* y, int N, int IH, int IW, int C, int OH, int OW,
