@@ -534,6 +534,24 @@ int mgw_remap_bundle_frame(const uint8_t* src, int format, const float* xy, int 
     return launch_remap_bundle(src, format, 3, xy, S, h, w, H, W, dst, workspace, (cudaStream_t)stream);
 }
 
+// mgw_remap_bundle_frame's checks in its order, with H and W even for every source (a 4:2:0 result) and dst_format one of the two
+// YUV layouts (MGW_BGR24 is mgw_remap_bundle_frame)
+int mgw_remap_bundle_frame_yuv420(const uint8_t* src, int format, const float* xy, int S, int h, int w, int H, int W, int dst_format,
+                                  uint8_t* dst, void* workspace, void* stream)
+{
+    REQUIRE(S >= 0 && S <= 65535 && h >= 8 && w >= 8 && H >= 2 && W >= 2 && H <= 32766 && W <= 32766 && H % 2 == 0 && W % 2 == 0 &&
+            (long long)S * H * W * 3 < (1LL << 31) && (long long)S * h * w < (1LL << 31),
+            "mgw_remap_bundle_frame_yuv420: bad sizes (S=%d maps %dx%d frame %dx%d; h, w >= 8, H and W even)", S, h, w, H, W);
+    REQUIRE(format == MGW_BGR24 || format == MGW_YUV420_NV12 || format == MGW_YUV420_I420,
+            "mgw_remap_bundle_frame_yuv420: unknown format %d", format);
+    REQUIRE(dst_format == MGW_YUV420_NV12 || dst_format == MGW_YUV420_I420,
+            "mgw_remap_bundle_frame_yuv420: unknown destination format %d (NV12 or I420; BGR is mgw_remap_bundle_frame)", dst_format);
+    if (S == 0) return MGW_OK;
+    REQUIRE(src && xy && dst && workspace, "mgw_remap_bundle_frame_yuv420: null pointer");
+    REQUIRE(aligned(xy, 8) && aligned(workspace, 8), "mgw_remap_bundle_frame_yuv420: xy and workspace must be 8-byte aligned");
+    return launch_remap_bundle_yuv420(src, format, xy, S, h, w, H, W, dst_format, dst, workspace, (cudaStream_t)stream);
+}
+
 int mgw_stream_assemble(const float* frames, const float* masks, int depth, int head, const int* taps, int ntaps, int use_masks,
                         const float* cur, int H, int W, float* in_x, void* stream)
 {

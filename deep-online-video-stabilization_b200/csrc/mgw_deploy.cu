@@ -263,6 +263,118 @@ int launch_remap_up(const uint8_t* src, const float2* small, int N, int H, int W
     return MGW_OK;
 }
 
+// cv2.cvtColor(COLOR_BGR2YUV_I420), color_yuv.simd.hpp: BT.601 limited range in 20-bit fixed point.  Y of every pixel; U and V
+// of the top-left pixel of each 2x2 block only (no averaging).  Every sum lies in [16 << 20, 241 << 20): no clamp is needed.
+__device__ __forceinline__ int bgr_y(const uint8_t* p)
+{
+    return (269484 * p[2] + 528482 * p[1] + 102760 * p[0] + (16 << 20) + (1 << 19)) >> 20;
+}
+__device__ __forceinline__ int bgr_u(const uint8_t* p)
+{
+    return (-155188 * p[2] - 305135 * p[1] + 460324 * p[0] + (128 << 20) + (1 << 19)) >> 20;
+}
+__device__ __forceinline__ int bgr_v(const uint8_t* p)
+{
+    return (460324 * p[2] - 385875 * p[1] - 74448 * p[0] + (128 << 20) + (1 << 19)) >> 20;
+}
+
+// n (2 or 4) bytes b[0..n) to o: one word (or half word) where o is aligned, single bytes otherwise
+__device__ __forceinline__ void store_run(uint8_t* o, const uint8_t* b, int n)
+{
+    const uintptr_t a = reinterpret_cast<uintptr_t>(o);
+    if (n == 4 && (a & 3) == 0)
+        *reinterpret_cast<uint32_t*>(o) = (uint32_t)b[0] | ((uint32_t)b[1] << 8) | ((uint32_t)b[2] << 16) | ((uint32_t)b[3] << 24);
+    else if (n == 2 && (a & 1) == 0)
+        *reinterpret_cast<uint16_t*>(o) = (uint16_t)(b[0] | (b[1] << 8));
+    else {
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+            if (i < n) o[i] = b[i];
+    }
+}
+
+// K5b with the result as YUV 4:2:0 (DST_FMT = MGW_YUV420_NV12 / _I420, [3H/2,W] per frame; H and W even): each thread takes a
+// block of 2 rows x YUV_RUN columns of the output, the columns starting at a multiple of YUV_RUN inside one row pair (when W is
+// not a multiple of 4 the last block of a row is 2 columns wide).  Every pixel's BGR value is remap_up_kernel's, by the same
+// device functions; the column coefficients are shared by the two rows.  The thread writes the block's Y bytes and the U, V of
+// its two (or one) 2x2 chroma blocks, so the BGR frame never reaches memory.
+constexpr int YUV_RUN = 4;
+
+template <int SRC_FMT, int DST_FMT>
+__global__ void __launch_bounds__(256)
+remap_up_yuv_kernel(const uint8_t* __restrict__ src, const float2* __restrict__ small, int H, int W, int h4, int w4, double xscale,
+                    double yscale, uint8_t* __restrict__ dst)
+{
+    const int gw = (W + YUV_RUN - 1) / YUV_RUN;
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= (H >> 1) * gw) return;
+    const int r = (t / gw) * 2, c0 = (t % gw) * YUV_RUN;
+    const int ncol = min(YUV_RUN, W - c0);
+    const size_t n = blockIdx.y;
+    const uint8_t* f = src + n * src_frame_bytes<SRC_FMT>(H, W);
+    small += n * h4 * w4;
+    uint8_t* y = dst + n * ((size_t)H * W * 3 / 2);
+    uint8_t* uv = y + (size_t)H * W;
+    const Lin v0 = vcoef_at(src_pos_s(r, yscale), h4), v1 = vcoef_at(src_pos_s(r + 1, yscale), h4);
+    uint8_t ys[2][YUV_RUN], us[YUV_RUN / 2], vs[YUV_RUN / 2];
+#pragma unroll
+    for (int k = 0; k < YUV_RUN; ++k) {
+        // past the row's end (c0 + k >= W) the taps are computed as for any column and nothing of them is stored
+        const Lin hc = hcoef_at(src_pos_s(c0 + k, xscale), w4);
+#pragma unroll
+        for (int i = 0; i < 2; ++i) {
+            const float2 m = resize_sample(small, w4, hc, i ? v1 : v0);
+            // (map + 1) / 2 * size in fp32 (deploy_bundle.py:142-143)
+            const float xp = __fmul_rn(__fmul_rn(__fadd_rn(m.x, 1.0f), 0.5f), (float)W);
+            const float yp = __fmul_rn(__fmul_rn(__fadd_rn(m.y, 1.0f), 0.5f), (float)H);
+            const int sx = cv_round(__fmul_rn(xp, 32.0f)), sy = cv_round(__fmul_rn(yp, 32.0f));
+            uint8_t px[3];
+            bilinear_fixed_u8<3, SRC_FMT>(f, H, W, sx, sy, px);
+            ys[i][k] = (uint8_t)bgr_y(px);
+            if (i == 0 && (k & 1) == 0) { us[k >> 1] = (uint8_t)bgr_u(px); vs[k >> 1] = (uint8_t)bgr_v(px); }
+        }
+    }
+    store_run(y + (size_t)r * W + c0, ys[0], ncol);
+    store_run(y + (size_t)(r + 1) * W + c0, ys[1], ncol);
+    if constexpr (DST_FMT == MGW_YUV420_NV12) {
+        const uint8_t b[YUV_RUN] = {us[0], vs[0], us[1], vs[1]};
+        store_run(uv + (size_t)(r >> 1) * W + c0, b, ncol);
+    } else {
+        const size_t q = (size_t)(r >> 1) * (W >> 1) + (c0 >> 1);
+        store_run(uv + q, us, ncol >> 1);
+        store_run(uv + (size_t)(H >> 1) * (W >> 1) + q, vs, ncol >> 1);
+    }
+}
+
+template <int SRC_FMT, int DST_FMT>
+int launch_remap_up_yuv(const uint8_t* src, const float2* small, int N, int H, int W, int h4, int w4, uint8_t* dst, cudaStream_t st)
+{
+    const long long threads = (long long)(H / 2) * ((W + YUV_RUN - 1) / YUV_RUN);
+    remap_up_yuv_kernel<SRC_FMT, DST_FMT><<<dim3((unsigned)((threads + 255) / 256), N), 256, 0, st>>>(
+        src, small, H, W, h4, w4, resize_scale(W, w4), resize_scale(H, h4), dst);
+    return check_launch("remap_up_yuv");
+}
+
+template <int SRC_FMT>
+int launch_remap_up_yuv_to(int dst_fmt, const uint8_t* src, const float2* small, int N, int H, int W, int h4, int w4, uint8_t* dst,
+                           cudaStream_t st)
+{
+    switch (dst_fmt) {
+    case MGW_YUV420_NV12: return launch_remap_up_yuv<SRC_FMT, MGW_YUV420_NV12>(src, small, N, H, W, h4, w4, dst, st);
+    case MGW_YUV420_I420: return launch_remap_up_yuv<SRC_FMT, MGW_YUV420_I420>(src, small, N, H, W, h4, w4, dst, st);
+    default: return set_error(MGW_ERR_INVALID, "remap_bundle_yuv420: unknown destination format %d", dst_fmt);
+    }
+}
+
+// K5a: the /4 maps of every frame (h4 = int(height / rate), w4 = int(width / rate)) into the workspace
+float2* launch_maps_down(const float* xy, int N, int h, int w, void* workspace, cudaStream_t st)
+{
+    float2* small = reinterpret_cast<float2*>(workspace);
+    const int h4 = h / 4, w4 = w / 4, t1 = N * h4 * w4;
+    maps_down_kernel<<<(t1 + 255) / 256, 256, 0, st>>>(reinterpret_cast<const float2*>(xy), N, h, w, h4, w4, small);
+    return small;
+}
+
 }  // namespace
 
 size_t remap_bundle_workspace_bytes(int N, int H, int W) { return sizeof(float) * 2 * (size_t)N * (H / 4) * (W / 4); }
@@ -271,10 +383,8 @@ size_t remap_bundle_workspace_bytes(int N, int H, int W) { return sizeof(float) 
 int launch_remap_bundle(const uint8_t* src, int src_fmt, int C, const float* xy, int N, int h, int w, int H, int W, uint8_t* dst,
                         void* workspace, cudaStream_t st)
 {
-    const int h4 = h / 4, w4 = w / 4;       // int(height / rate), int(width / rate)
-    float2* small = reinterpret_cast<float2*>(workspace);
-    const int t1 = N * h4 * w4;
-    maps_down_kernel<<<(t1 + 255) / 256, 256, 0, st>>>(reinterpret_cast<const float2*>(xy), N, h, w, h4, w4, small);
+    const int h4 = h / 4, w4 = w / 4;
+    float2* small = launch_maps_down(xy, N, h, w, workspace, st);
     if (int rc = check_launch("maps_down")) return rc;
     if (src_fmt != SRC_BGR && C != 3) return set_error(MGW_ERR_UNSUPPORTED, "remap_bundle: a YUV 4:2:0 source gives C = 3 (got %d)", C);
     switch (src_fmt) {
@@ -295,6 +405,21 @@ int launch_remap_bundle_u8(const uint8_t* img, const float* xy, int N, int H, in
                            cudaStream_t st)
 {
     return launch_remap_bundle(img, SRC_BGR, C, xy, N, H, W, H, W, dst, workspace, st);
+}
+
+// launch_remap_bundle's warp (C = 3) with the result written as YUV 4:2:0: the same K5a, then the YUV variant of K5b
+int launch_remap_bundle_yuv420(const uint8_t* src, int src_fmt, const float* xy, int N, int h, int w, int H, int W, int dst_fmt,
+                               uint8_t* dst, void* workspace, cudaStream_t st)
+{
+    const int h4 = h / 4, w4 = w / 4;
+    float2* small = launch_maps_down(xy, N, h, w, workspace, st);
+    if (int rc = check_launch("maps_down")) return rc;
+    switch (src_fmt) {
+    case SRC_BGR: return launch_remap_up_yuv_to<SRC_BGR>(dst_fmt, src, small, N, H, W, h4, w4, dst, st);
+    case MGW_YUV420_NV12: return launch_remap_up_yuv_to<MGW_YUV420_NV12>(dst_fmt, src, small, N, H, W, h4, w4, dst, st);
+    case MGW_YUV420_I420: return launch_remap_up_yuv_to<MGW_YUV420_I420>(dst_fmt, src, small, N, H, W, h4, w4, dst, st);
+    default: return set_error(MGW_ERR_INVALID, "remap_bundle_yuv420: unknown source format %d", src_fmt);
+    }
 }
 
 // ---------------------------------------------------------------------------------------------------------------------

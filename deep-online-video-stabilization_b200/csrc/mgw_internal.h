@@ -115,6 +115,10 @@ int launch_remap_bundle_u8(const uint8_t* img, const float* xy, int N, int H, in
 // [N,H,W,C] (src_fmt 0) or YUV 4:2:0 [N,3H/2,W] (C = 3) -> dst [N,H,W,C]; the workspace is remap_bundle_workspace_bytes(N, h, w)
 int launch_remap_bundle(const uint8_t* src, int src_fmt, int C, const float* xy, int N, int h, int w, int H, int W, uint8_t* dst,
                         void* workspace, cudaStream_t st);
+// the same warp (C = 3, H and W even) with the result as YUV 4:2:0, dst [N,3H/2,W] in dst_fmt (MGW_YUV420_NV12 / _I420): Y, U, V as
+// cv2.cvtColor(COLOR_BGR2YUV_I420) computes them from the BGR result, converted inside the warp
+int launch_remap_bundle_yuv420(const uint8_t* src, int src_fmt, const float* xy, int N, int h, int w, int H, int W, int dst_fmt,
+                               uint8_t* dst, void* workspace, cudaStream_t st);
 
 // S frames of one size ([S,H,W,C] -> [S,out_h,out_w,C]; S >= 1, the single-frame calls pass 1).  src_fmt: 0 for the BGR / C-channel
 // frames, MGW_YUV420_NV12 or MGW_YUV420_I420 for YUV 4:2:0 frames [S,3H/2,W] read as the BGR frames cvtColor makes of them (C = 3)

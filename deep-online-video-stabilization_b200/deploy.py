@@ -20,11 +20,13 @@ __all__ = ['warpRevBundle2', 'warpRevBundle', 'warpRev', 'cvt_theta_mat_bundle',
            'MixedStreamBatch', 'mixed_slot_tables', 'scale_rect']
 
 
-def warpRevBundle2(img, x_map, y_map, device=None, src_format='bgr'):
+def warpRevBundle2(img, x_map, y_map, device=None, src_format='bgr', dst_format='bgr'):
     """The frame img, of any size, stabilised at its own size with the operator's x_map / y_map (network size): the reference's
     expression with the size the colour frame is resized to taken from the frame instead of the network.  A frame at the maps'
     size is exactly the reference's warpRevBundle2.  img: [H,W,C] or [N,H,W,C] uint8 BGR, or for src_format 'nv12' / 'i420' a
-    YUV 4:2:0 frame [3H/2,W] or batch [N,3H/2,W] (read as the BGR frame cv2.cvtColor makes of it; the result is BGR [H,W,3])."""
+    YUV 4:2:0 frame [3H/2,W] or batch [N,3H/2,W] (read as the BGR frame cv2.cvtColor makes of it; the result is BGR [H,W,3]).
+    dst_format 'nv12' / 'i420' (3-channel frames of even size): the result is YUV 4:2:0 [3H/2,W] ([N,3H/2,W]) for a video
+    encoder, cv2.cvtColor(COLOR_BGR2YUV_I420) of the BGR result (U and V interleaved for NV12), converted inside the warp."""
     as_numpy = isinstance(img, np.ndarray)
     dev = torch.device(device) if device is not None else (torch.device('cuda') if as_numpy else img.device)
 
@@ -44,7 +46,7 @@ def warpRevBundle2(img, x_map, y_map, device=None, src_format='bgr'):
             im = im.unsqueeze(0)
         H, W = int(im.shape[1]), int(im.shape[2])
     n = int(im.shape[0])
-    if yuv is None and xm.numel() == n * H * W:
+    if yuv is None and dst_format == 'bgr' and xm.numel() == n * H * W:
         # the maps have the frame's size: the reference's call
         xy = torch.stack([xm.reshape(n, H, W), ym.reshape(n, H, W)], dim=-1)
         dst = ops.remap_bundle_u8(im, xy)
@@ -56,7 +58,7 @@ def warpRevBundle2(img, x_map, y_map, device=None, src_format='bgr'):
             raise ValueError('x_map / y_map must be [h,w] maps, one per frame (got %s for %d frames)' % (tuple(xm.shape), n))
         h, w = shape[-2], shape[-1]
         xy = torch.stack([xm.reshape(n, h, w), ym.reshape(n, h, w)], dim=-1)
-        dst = ops.remap_bundle_frame(im.contiguous(), src_format, xy)
+        dst = ops.remap_bundle_frame(im.contiguous(), src_format, xy, out_format=dst_format)
     if single:
         dst = dst[0]
     return dst.cpu().numpy() if as_numpy else dst
@@ -410,16 +412,24 @@ class StreamBatch:
     out_size=(OH, OW) sets the size of the stabilised colour frames (default: the network's (height, width), the reference's
     output).  The network's maps warp the frame resized to that size; at out_size == src_size nothing is resized and the warp
     reads the source batch (BGR or YUV 4:2:0) itself, so a 1080p video comes out at 1080p.  crop_rate does not act on the colour
-    frames, as in the reference; scale_rect() carries leave()'s rectangle to output pixels."""
+    frames, as in the reference; scale_rect() carries leave()'s rectangle to output pixels.
+
+    out_format='nv12' or 'i420' hands the stabilised frames out as a video encoder takes them: self.colour, step() and the
+    captured download are YUV 4:2:0 [S,3OH/2,OW] uint8, cv2.cvtColor(COLOR_BGR2YUV_I420) of the BGR frames (U and V interleaved
+    for NV12), converted inside the warp -- half the bytes to download.  The output size must then be even."""
 
     def __init__(self, S, src_size, height=288, width=512, depth=32, taps=(1, 2, 4, 8, 16, 32), use_masks=True, crop_rate=1, refine=1,
-                 device='cuda', src_format='bgr', out_size=None):
+                 device='cuda', src_format='bgr', out_size=None, out_format='bgr'):
         S, H, W, h, w = int(S), int(src_size[0]), int(src_size[1]), int(height), int(width)
         if S < 1 or refine < 1:
             raise ValueError('StreamBatch needs S >= 1 and refine >= 1 (got S=%d, refine=%d)' % (S, refine))
         out = (h, w) if out_size is None else (int(out_size[0]), int(out_size[1]))
         if not (1 <= out[0] <= 32767 and 1 <= out[1] <= 32767):
             raise ValueError('out_size %s: each side in [1, 32767]' % (tuple(out_size),))
+        if out_format not in ('bgr',) + tuple(ops.YUV420_FORMATS):
+            raise ValueError("out_format must be 'bgr', 'nv12' or 'i420' (got %r)" % (out_format,))
+        if out_format != 'bgr' and (out[0] % 2 or out[1] % 2):
+            raise ValueError('a %s output needs an even size (got %dx%d)' % (out_format, out[0], out[1]))
         if src_format == 'bgr':
             self.frame_shape = (H, W, 3)
         elif src_format in ops.YUV420_FORMATS:
@@ -434,7 +444,7 @@ class StreamBatch:
             raise ValueError('taps %s: 1 to 32 distances in [1, depth = %d]' % (self.taps, depth))
         dev = torch.device(device)
         self.S, self.src_size, self.height, self.width, self.depth = S, (H, W), h, w, int(depth)
-        self.out_size = out
+        self.out_size, self.out_format = out, out_format
         # the remap reads the source batch itself when the output has its size; None keeps the network-size path as it was
         self._direct = out_size is not None and out == (H, W)
         self.use_masks, self.crop_rate, self.refine = bool(use_masks), crop_rate, int(refine)
@@ -450,7 +460,8 @@ class StreamBatch:
         self.cvt_tmp = torch.empty((S, H, w), device=dev, dtype=torch.uint8)
         self.in_x = torch.empty((S, h, w, self.nch), **f32)
         self.small = None if self._direct else torch.empty((S,) + out + (3,), device=dev, dtype=torch.uint8)
-        self.colour = torch.empty((S,) + out + (3,), device=dev, dtype=torch.uint8)
+        self.colour = torch.empty((S,) + out + (3,) if out_format == 'bgr' else (S, out[0] * 3 // 2, out[1]), device=dev,
+                                  dtype=torch.uint8)
         self.remap_ws = torch.empty(ops.remap_bundle_workspace_floats(S, h, w), **f32)
         self._init_front_end(dev)
 
@@ -506,7 +517,8 @@ class StreamBatch:
     def step(self, raw_bgr, net):
         """One frame of every slot from raw_bgr [S,H,W,3] uint8 on the device ([S,3H/2,W] for a YUV 4:2:0 batch): cvt_img2train,
         advance(), cv2_resize of the colour frames to out_size (none at out_size == src_size) and warpRevBundle2 with the last xy.
-        Returns the stabilised colour frames [S,OH,OW,3] uint8 BGR (self.colour, overwritten by the next step)."""
+        Returns the stabilised colour frames [S,OH,OW,3] uint8 BGR, or [S,3OH/2,OW] YUV 4:2:0 for out_format 'nv12' / 'i420'
+        (self.colour, overwritten by the next step)."""
         raw = ops._chk(raw_bgr, 'raw_bgr', torch.uint8)
         if tuple(raw.shape) != (self.S,) + self.frame_shape:
             raise ValueError('raw_bgr must be %s uint8 (got %s)' % ([self.S] + list(self.frame_shape), tuple(raw.shape)))
@@ -517,20 +529,25 @@ class StreamBatch:
             cur = ops.cvt_img2train_yuv420_batch(raw, self.src_format, self._cvt, h, w, out=self.cur, tmp=self.cvt_tmp)
         xy = self.advance(cur, net)
         if self._direct:
-            return ops.remap_bundle_frame(raw, self.src_format, xy, out=self.colour, workspace=self.remap_ws)
+            return ops.remap_bundle_frame(raw, self.src_format, xy, out=self.colour, workspace=self.remap_ws, out_format=self.out_format)
         oh, ow = self.out_size
         if self.src_format == 'bgr':
             small = ops.resize_linear_u8_batch(raw, self._resize[0], self._resize[1], oh, ow, out=self.small)
         else:
             small = ops.resize_linear_yuv420_batch(raw, self.src_format, self._resize[0], self._resize[1], oh, ow, out=self.small)
-        if (oh, ow) == (h, w):
+        return self._warp_small(small, xy)
+
+    def _warp_small(self, small, xy):
+        """warpRevBundle2 of the resized colour frames small [S,OH,OW,3] into self.colour"""
+        if self.out_size == (self.height, self.width) and self.out_format == 'bgr':
             return ops.remap_bundle_u8(small, xy, out=self.colour, workspace=self.remap_ws)
-        return ops.remap_bundle_frame(small, 'bgr', xy, out=self.colour, workspace=self.remap_ws)
+        return ops.remap_bundle_frame(small, 'bgr', xy, out=self.colour, workspace=self.remap_ws, out_format=self.out_format)
 
     def capture(self, raw_bgr, net, upload_from=None, download_to=None):
         """Records step(raw_bgr, net) as a CUDA graph and returns it: graph.replay() runs one step on whatever raw_bgr holds and
-        leaves the frames in self.colour.  upload_from / download_to: optional host buffers ([S,H,W,3] or, for a YUV 4:2:0
-        batch, [S,3H/2,W] / [S,OH,OW,3] uint8, pinned) copied into raw_bgr before and out of self.colour after the step, inside the graph.  One eager step runs first
+        leaves the frames in self.colour.  upload_from / download_to: optional host buffers (raw_bgr's shape / self.colour's:
+        [S,H,W,3] or, for a YUV 4:2:0 batch, [S,3H/2,W] / [S,OH,OW,3] or, for a YUV 4:2:0 output, [S,3OH/2,OW]; uint8, pinned)
+        copied into raw_bgr before and out of self.colour after the step, inside the graph.  One eager step runs first
         on a side stream as a warm-up (a network may select algorithms or allocate on its first call); the state it changed
         is restored, so capturing leaves every slot as it was."""
         if download_to is not None and tuple(download_to.shape) != tuple(self.colour.shape):
@@ -575,11 +592,13 @@ class MixedStreamBatch(StreamBatch):
     the whole pool, capacity bytes per slot whatever the slots' sizes.  A slot can join again at another size between replays of
     a captured graph: join writes the slot's size and tables with stream-ordered device copies, and the graph reads them.
     Slots that never joined are idle: the front end writes nothing for them and the network sees zero frames.  A slot that left
-    keeps its size and runs on whatever its region holds, as in StreamBatch."""
+    keeps its size and runs on whatever its region holds, as in StreamBatch.  out_format is StreamBatch's; the output stays at
+    the network's size."""
 
     def __init__(self, S, max_src_size, height=288, width=512, depth=32, taps=(1, 2, 4, 8, 16, 32), use_masks=True, crop_rate=1,
-                 refine=1, device='cuda', src_format='bgr'):
-        super().__init__(S, max_src_size, height, width, depth, taps, use_masks, crop_rate, refine, device, src_format)
+                 refine=1, device='cuda', src_format='bgr', out_format='bgr'):
+        super().__init__(S, max_src_size, height, width, depth, taps, use_masks, crop_rate, refine, device, src_format,
+                         out_format=out_format)
 
     def _init_front_end(self, dev):
         """per-slot sizes and tables, all zero (every slot idle) until a slot joins"""
@@ -642,8 +661,8 @@ class MixedStreamBatch(StreamBatch):
 
     def step(self, pool, net):
         """One frame of every slot from pool [S, frame_bytes(capacity)] uint8 on the device: cvt_img2train and cv2.resize of each
-        slot at its own size, and the StreamBatch step around them.  Returns the stabilised colour frames [S,h,w,3] uint8 BGR
-        (self.colour, overwritten by the next step)."""
+        slot at its own size, and the StreamBatch step around them.  Returns the stabilised colour frames [S,h,w,3] uint8 BGR, or
+        [S,3h/2,w] YUV 4:2:0 for out_format 'nv12' / 'i420' (self.colour, overwritten by the next step)."""
         if not isinstance(pool, torch.Tensor) or pool.dtype != torch.uint8 or tuple(pool.shape) != self.pool_shape:
             raise ValueError('pool must be a %s uint8 tensor (got %s %s)' % (list(self.pool_shape), tuple(getattr(pool, 'shape', ())),
                                                                            getattr(pool, 'dtype', type(pool))))
@@ -652,4 +671,4 @@ class MixedStreamBatch(StreamBatch):
         cur = ops.cvt_img2train_mixed(pool, self.src_format, self.sizes, self.tables, h, w, out=self.cur, tmp=self.cvt_tmp)
         xy = self.advance(cur, net)
         small = ops.resize_linear_mixed(pool, self.src_format, self.sizes, self.xtab, self.ytab, h, w, out=self.small)
-        return ops.remap_bundle_u8(small, xy, out=self.colour, workspace=self.remap_ws)
+        return self._warp_small(small, xy)

@@ -811,14 +811,18 @@ def resize_linear_mixed(pool, fmt, sizes, xtab, ytab, out_h, out_w, out=None):
 
 
 # ---- warpRevBundle2 at the frame's own size
-def remap_bundle_frame(src, src_format, xy, out=None, workspace=None):
+def remap_bundle_frame(src, src_format, xy, out=None, workspace=None, out_format='bgr'):
     """warpRevBundle2 of frames at any size: src [S,H,W,3] uint8 ('bgr') or [S,3H/2,W] ('nv12' / 'i420'), xy [S,h,w,2] fp32 (the
     operator's x_map,y_map at the network size) -> [S,H,W,3] BGR: the /4 maps resized to (W, H) and scaled by (W, H), then
     cv2.remap of the frame.  At (H, W) == (h, w) with 'bgr' this is remap_bundle_u8.  One C-ABI call (two launches).
+    out_format 'nv12' / 'i420' (H and W even): the result is [S,3H/2,W] YUV 4:2:0 instead, cv2.cvtColor(COLOR_BGR2YUV_I420) of
+    the BGR result (U and V interleaved for NV12), converted inside the warp (mgw_remap_bundle_frame_yuv420).
     out / workspace: optional preallocated result and fp32 scratch of remap_bundle_workspace_floats(S, h, w) (CUDA-graph capture)."""
     src, xy = _chk(src, 'src', torch.uint8), _chk(xy, 'xy')
     if src_format not in SRC_FORMATS:
         raise ValueError('source format must be one of %s (got %r)' % (sorted(SRC_FORMATS), src_format))
+    if out_format not in SRC_FORMATS:
+        raise ValueError('out_format must be one of %s (got %r)' % (sorted(SRC_FORMATS), out_format))
     if src_format == 'bgr':
         if src.dim() != 4 or src.shape[3] != 3:
             raise ValueError('a BGR batch must be [S,H,W,3] (got %s)' % (tuple(src.shape),))
@@ -828,12 +832,18 @@ def remap_bundle_frame(src, src_format, xy, out=None, workspace=None):
     if xy.dim() != 4 or xy.shape[0] != s or xy.shape[3] != 2:
         raise ValueError('xy must be [%d,h,w,2] (got %s)' % (s, tuple(xy.shape)))
     h, w = int(xy.shape[1]), int(xy.shape[2])
-    dst = _out(out, (s, H, W, 3), src.device, torch.uint8, 'out')
+    if out_format != 'bgr' and (H % 2 or W % 2):
+        raise ValueError('a %s result needs an even size (got %dx%d)' % (out_format, H, W))
+    dst = _out(out, (s, H, W, 3) if out_format == 'bgr' else (s, H * 3 // 2, W), src.device, torch.uint8, 'out')
     ws = (torch.empty(remap_bundle_workspace_floats(s, h, w), device=src.device, dtype=torch.float32) if workspace is None
           else _chk_out(workspace, 'workspace'))
     if ws.numel() < remap_bundle_workspace_floats(s, h, w):
         raise ValueError('workspace needs %d floats' % remap_bundle_workspace_floats(s, h, w))
     with torch.cuda.device(src.device):
-        check(lib.mgw_remap_bundle_frame(_p(src), SRC_FORMATS[src_format], _p(xy), s, h, w, H, W, _p(dst), _p(ws), _st()),
-              'mgw_remap_bundle_frame')
+        if out_format == 'bgr':
+            check(lib.mgw_remap_bundle_frame(_p(src), SRC_FORMATS[src_format], _p(xy), s, h, w, H, W, _p(dst), _p(ws), _st()),
+                  'mgw_remap_bundle_frame')
+        else:
+            check(lib.mgw_remap_bundle_frame_yuv420(_p(src), SRC_FORMATS[src_format], _p(xy), s, h, w, H, W, SRC_FORMATS[out_format],
+                                                    _p(dst), _p(ws), _st()), 'mgw_remap_bundle_frame_yuv420')
     return dst

@@ -321,6 +321,19 @@ MGW_API size_t mgw_remap_bundle_frame_workspace_bytes(int S, int h, int w, int H
 MGW_API int mgw_remap_bundle_frame(const uint8_t* src, int format, const float* xy, int S, int h, int w, int H, int W,
                                uint8_t* dst, void* workspace, void* stream);
 
+/* ---- f1 for the encoder: the stabilised frames as YUV 4:2:0 ------------------------------------------------------------
+ * mgw_remap_bundle_frame with the result written as dst [S,3H/2,W] uint8 in dst_format, MGW_YUV420_NV12 (what NVENC takes) or
+ * MGW_YUV420_I420 (yuv420p, what libx264 / libavcodec take), in the layouts above: byte for byte cv2.cvtColor(F,
+ * COLOR_BGR2YUV_I420) of the BGR frame F that mgw_remap_bundle_frame gives, its U and V planes interleaved for NV12.  That is
+ * BT.601 limited range in 20-bit fixed point, Y of every pixel and U, V of the top-left pixel of each 2x2 block (no chroma
+ * averaging); the conversion runs inside the warp and the BGR frame is never written.  Half the bytes of the BGR result.  The
+ * rows are packed (pitch W): a pitched encoder surface is the caller's copy.  Same workspace as mgw_remap_bundle_frame.
+ * Checked in the order of the batch calls: mgw_remap_bundle_frame's sizes and source format with H and W even for every source,
+ * and dst_format NV12 or I420 (MGW_BGR24 is rejected: that result is mgw_remap_bundle_frame's), then S = 0 returns MGW_OK and
+ * launches nothing, then the pointers and their alignment. */
+MGW_API int mgw_remap_bundle_frame_yuv420(const uint8_t* src, int format, const float* xy, int S, int h, int w, int H, int W,
+                               int dst_format, uint8_t* dst, void* workspace, void* stream);
+
 /* ---- a6: interpolate(im, x, y, out_size), spatial_transformer.py:200-281 ------------------------------
  * im [N,IH,IW,C]; x,y [N,OH,OW] normalised coords -> out [N,OH,OW,C]. */
 MGW_API int mgw_interp_fwd(const float* im, const float* x, const float* y, int N, int IH, int IW, int C, int OH, int OW,
