@@ -67,6 +67,7 @@ SIGNATURES = {
     'mgw_remap_bundle_frame_workspace_bytes': (ctypes.c_size_t, [c_i] * 5),
     'mgw_remap_bundle_frame': (c_i, [c_f, c_i, c_f, c_i, c_i, c_i, c_i, c_i, c_f, c_f, c_st]),
     'mgw_remap_bundle_frame_yuv420': (c_i, [c_f, c_i, c_f, c_i, c_i, c_i, c_i, c_i, c_i, c_f, c_f, c_st]),
+    'mgw_remap_bundle_frame_mixed': (c_i, [c_f, c_i, c_i, c_i, c_i, c_f, c_f, c_i, c_i, c_i, c_f, c_f, c_st]),
     'mgw_interp_fwd': (c_i, [c_f, c_f, c_f] + [c_i] * 6 + [c_f, c_st]),
     'mgw_interp_bwd': (c_i, [c_f, c_f, c_f, c_f] + [c_i] * 6 + [c_f, c_f, c_f, c_st]),
     'mgw_homography_warp_fwd': (c_i, [c_f, c_f] + [c_i] * 6 + [c_f, c_f, c_f, c_st]),

@@ -552,6 +552,25 @@ int mgw_remap_bundle_frame_yuv420(const uint8_t* src, int format, const float* x
     return launch_remap_bundle_yuv420(src, format, xy, S, h, w, H, W, dst_format, dst, workspace, (cudaStream_t)stream);
 }
 
+// mgw_remap_bundle_frame's checks over the capacity, in the batch calls' order; the capacity is even when either format is YUV
+int mgw_remap_bundle_frame_mixed(const uint8_t* src, int format, int S, int max_h, int max_w, const int32_t* sizes, const float* xy,
+                                 int h, int w, int dst_format, uint8_t* dst, void* workspace, void* stream)
+{
+    const auto known = [](int f) { return f == MGW_BGR24 || f == MGW_YUV420_NV12 || f == MGW_YUV420_I420; };
+    REQUIRE(known(format), "mgw_remap_bundle_frame_mixed: unknown format %d", format);
+    REQUIRE(known(dst_format), "mgw_remap_bundle_frame_mixed: unknown destination format %d", dst_format);
+    REQUIRE(S >= 0 && S <= 65535 && h >= 8 && w >= 8 && max_h >= 1 && max_w >= 1 && max_h <= 32767 && max_w <= 32767 &&
+            ((format == MGW_BGR24 && dst_format == MGW_BGR24) || (max_h % 2 == 0 && max_w % 2 == 0)) &&
+            (long long)S * max_h * max_w * 3 < (1LL << 31) && (long long)S * h * w < (1LL << 31),
+            "mgw_remap_bundle_frame_mixed: bad sizes (S=%d maps %dx%d capacity %dx%d; h, w >= 8, capacity even for YUV)", S, h, w,
+            max_h, max_w);
+    if (S == 0) return MGW_OK;
+    REQUIRE(src && sizes && xy && dst && workspace, "mgw_remap_bundle_frame_mixed: null pointer");
+    REQUIRE(aligned(xy, 8) && aligned(workspace, 8) && aligned(sizes, 8),
+            "mgw_remap_bundle_frame_mixed: xy, workspace and sizes must be 8-byte aligned");
+    return launch_remap_bundle_mixed(src, format, S, max_h, max_w, sizes, xy, h, w, dst_format, dst, workspace, (cudaStream_t)stream);
+}
+
 int mgw_stream_assemble(const float* frames, const float* masks, int depth, int head, const int* taps, int ntaps, int use_masks,
                         const float* cur, int H, int W, float* in_x, void* stream)
 {

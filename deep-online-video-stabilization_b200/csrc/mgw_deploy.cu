@@ -110,6 +110,15 @@ __device__ __forceinline__ size_t src_frame_bytes(int H, int W)
     return FMT == SRC_BGR ? (size_t)H * W * 3 : (size_t)H * W * 3 / 2;
 }
 
+// Per-slot geometry (MIXED kernels): a slot is idle -- its blocks return before they write anything -- when its size is 0, larger
+// than the capacity, or odd for a YUV format (the source's, or the result's in the warp): never-joined slots, and a bad
+// device-side size cannot move an access outside the slot's region.
+template <int FMT>
+__device__ __forceinline__ bool slot_active(int2 sz, int max_h, int max_w)
+{
+    return sz.x > 0 && sz.y > 0 && sz.x <= max_h && sz.y <= max_w && (FMT == SRC_BGR || ((sz.x | sz.y) & 1) == 0);
+}
+
 // cvRound(v) as x86 does it (cvtss2si: round half to even; out of range / NaN -> INT_MIN)
 __device__ __forceinline__ int cv_round(float v)
 {
@@ -205,17 +214,40 @@ warp_rev_bundle_kernel(const uint8_t* __restrict__ img, const double* __restrict
 // pixels of the frame's row-major order (a run may cross rows), so that it stores whole words: C words of 4 pixels.  The
 // per-column and per-row map coefficients are the device functions of maps_down at the output size; their resize scales
 // (a double division each) are launch arguments.  blockIdx.y is the frame.
+// MIXED = per-slot geometry (see cvt_img2train below): H, W are the capacity, slot s's source frame of size sizes[s] lies at the
+// start of its region [s * src_frame_bytes(H, W), ...) and its result at the start of [s * dst_frame_bytes(H, W), ...); block
+// (., s) reads the slot's size once, computes the slot's scales (bit for bit the host's launch arguments) and then runs the
+// per-pixel code of the uniform batch at the slot's size.
 constexpr int REMAP_RUN = 4;
 
-template <int C, int FMT>
+// a slot's two resize scales, computed by two threads of the block and broadcast through shared memory
+__device__ __forceinline__ void slot_scales(int H, int W, int h4, int w4, double& xscale, double& yscale)
+{
+    __shared__ double sc[2];
+    if (threadIdx.x < 2) sc[threadIdx.x] = threadIdx.x == 0 ? resize_scale(W, w4) : resize_scale(H, h4);
+    __syncthreads();
+    xscale = sc[0]; yscale = sc[1];
+}
+
+template <int C, int FMT, bool MIXED = false>
 __global__ void __launch_bounds__(256)
 remap_up_kernel(const uint8_t* __restrict__ src, const float2* __restrict__ small, int H, int W, int h4, int w4, double xscale,
-                double yscale, uint8_t* __restrict__ dst)
+                double yscale, uint8_t* __restrict__ dst, const int2* __restrict__ sizes)
 {
+    if constexpr (MIXED) {
+        static_assert(C == 3, "a slot's result is BGR");
+        const int2 sz = __ldg(sizes + blockIdx.y);
+        if (!slot_active<FMT>(sz, H, W)) return;            // block-uniform: before the barrier of slot_scales
+        src += (size_t)blockIdx.y * src_frame_bytes<FMT>(H, W);
+        small += (size_t)blockIdx.y * h4 * w4;
+        dst += (size_t)blockIdx.y * H * W * 3;
+        H = sz.x; W = sz.y;                                 // launched over the capacity's pixels: runs past the slot's return below
+        slot_scales(H, W, h4, w4, xscale, yscale);
+    }
     const int HW = H * W;
     const int p0 = (blockIdx.x * blockDim.x + threadIdx.x) * REMAP_RUN;
     if (p0 >= HW) return;
-    const size_t n = blockIdx.y;
+    const size_t n = MIXED ? 0 : blockIdx.y;
     const uint8_t* f = src + n * (FMT == SRC_BGR ? (size_t)HW * C : (size_t)HW * 3 / 2);
     small += n * h4 * w4;
     uint8_t* o = dst + (n * HW + p0) * C;
@@ -257,7 +289,7 @@ int launch_remap_up(const uint8_t* src, const float2* small, int N, int H, int W
         const int n = min(N - n0, 65535);
         remap_up_kernel<C, FMT><<<dim3(gx, n), 256, 0, st>>>(src + (size_t)n0 * (FMT == SRC_BGR ? (size_t)H * W * C : (size_t)H * W * 3 / 2),
                                                              small + (size_t)n0 * h4 * w4, H, W, h4, w4, xscale, yscale,
-                                                             dst + (size_t)n0 * H * W * C);
+                                                             dst + (size_t)n0 * H * W * C, nullptr);
         if (int rc = check_launch("remap_up")) return rc;
     }
     return MGW_OK;
@@ -297,20 +329,31 @@ __device__ __forceinline__ void store_run(uint8_t* o, const uint8_t* b, int n)
 // block of 2 rows x YUV_RUN columns of the output, the columns starting at a multiple of YUV_RUN inside one row pair (when W is
 // not a multiple of 4 the last block of a row is 2 columns wide).  Every pixel's BGR value is remap_up_kernel's, by the same
 // device functions; the column coefficients are shared by the two rows.  The thread writes the block's Y bytes and the U, V of
-// its two (or one) 2x2 chroma blocks, so the BGR frame never reaches memory.
+// its two (or one) 2x2 chroma blocks, so the BGR frame never reaches memory.  MIXED: as remap_up_kernel, with a YUV result region
+// of 3H/2*W bytes per slot; a slot of odd size is idle.
 constexpr int YUV_RUN = 4;
 
-template <int SRC_FMT, int DST_FMT>
+template <int SRC_FMT, int DST_FMT, bool MIXED = false>
 __global__ void __launch_bounds__(256)
 remap_up_yuv_kernel(const uint8_t* __restrict__ src, const float2* __restrict__ small, int H, int W, int h4, int w4, double xscale,
-                    double yscale, uint8_t* __restrict__ dst)
+                    double yscale, uint8_t* __restrict__ dst, const int2* __restrict__ sizes)
 {
+    if constexpr (MIXED) {
+        const int2 sz = __ldg(sizes + blockIdx.y);
+        // the result is 4:2:0, so every active slot is even (DST_FMT's rule covers an odd size from a BGR source)
+        if (!slot_active<SRC_FMT>(sz, H, W) || !slot_active<DST_FMT>(sz, H, W)) return;
+        src += (size_t)blockIdx.y * src_frame_bytes<SRC_FMT>(H, W);
+        small += (size_t)blockIdx.y * h4 * w4;
+        dst += (size_t)blockIdx.y * H * W * 3 / 2;
+        H = sz.x; W = sz.y;                                 // launched over the capacity's row pairs: blocks past the slot's return below
+        slot_scales(H, W, h4, w4, xscale, yscale);
+    }
     const int gw = (W + YUV_RUN - 1) / YUV_RUN;
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= (H >> 1) * gw) return;
     const int r = (t / gw) * 2, c0 = (t % gw) * YUV_RUN;
     const int ncol = min(YUV_RUN, W - c0);
-    const size_t n = blockIdx.y;
+    const size_t n = MIXED ? 0 : blockIdx.y;
     const uint8_t* f = src + n * src_frame_bytes<SRC_FMT>(H, W);
     small += n * h4 * w4;
     uint8_t* y = dst + n * ((size_t)H * W * 3 / 2);
@@ -351,7 +394,31 @@ int launch_remap_up_yuv(const uint8_t* src, const float2* small, int N, int H, i
 {
     const long long threads = (long long)(H / 2) * ((W + YUV_RUN - 1) / YUV_RUN);
     remap_up_yuv_kernel<SRC_FMT, DST_FMT><<<dim3((unsigned)((threads + 255) / 256), N), 256, 0, st>>>(
-        src, small, H, W, h4, w4, resize_scale(W, w4), resize_scale(H, h4), dst);
+        src, small, H, W, h4, w4, resize_scale(W, w4), resize_scale(H, h4), dst, nullptr);
+    return check_launch("remap_up_yuv");
+}
+
+// K5b over a pool of per-slot frames: the grid covers the capacity (max_h, max_w), gridDim.y is the slot
+template <int SRC_FMT>
+int launch_remap_up_mixed(int dst_fmt, const uint8_t* src, const float2* small, int S, int max_h, int max_w, int h4, int w4,
+                          const int2* sizes, uint8_t* dst, cudaStream_t st)
+{
+    if (dst_fmt == SRC_BGR) {
+        const unsigned gx = (unsigned)((((long long)max_h * max_w + REMAP_RUN - 1) / REMAP_RUN + 255) / 256);
+        remap_up_kernel<3, SRC_FMT, true><<<dim3(gx, S), 256, 0, st>>>(src, small, max_h, max_w, h4, w4, 0.0, 0.0, dst, sizes);
+        return check_launch("remap_up");
+    }
+    const long long threads = (long long)(max_h / 2) * ((max_w + YUV_RUN - 1) / YUV_RUN);
+    const dim3 grid((unsigned)((threads + 255) / 256), S);
+    switch (dst_fmt) {
+    case MGW_YUV420_NV12:
+        remap_up_yuv_kernel<SRC_FMT, MGW_YUV420_NV12, true><<<grid, 256, 0, st>>>(src, small, max_h, max_w, h4, w4, 0.0, 0.0, dst, sizes);
+        break;
+    case MGW_YUV420_I420:
+        remap_up_yuv_kernel<SRC_FMT, MGW_YUV420_I420, true><<<grid, 256, 0, st>>>(src, small, max_h, max_w, h4, w4, 0.0, 0.0, dst, sizes);
+        break;
+    default: return set_error(MGW_ERR_INVALID, "remap_bundle_frame_mixed: unknown destination format %d", dst_fmt);
+    }
     return check_launch("remap_up_yuv");
 }
 
@@ -422,6 +489,22 @@ int launch_remap_bundle_yuv420(const uint8_t* src, int src_fmt, const float* xy,
     }
 }
 
+// the same K5a, then K5b per slot at the slot's own size: src / dst are pools of capacity-sized regions, sizes [S,2]
+int launch_remap_bundle_mixed(const uint8_t* src, int src_fmt, int S, int max_h, int max_w, const int32_t* sizes, const float* xy,
+                              int h, int w, int dst_fmt, uint8_t* dst, void* workspace, cudaStream_t st)
+{
+    const int h4 = h / 4, w4 = w / 4;
+    float2* small = launch_maps_down(xy, S, h, w, workspace, st);
+    if (int rc = check_launch("maps_down")) return rc;
+    const int2* sz = reinterpret_cast<const int2*>(sizes);
+    switch (src_fmt) {
+    case SRC_BGR: return launch_remap_up_mixed<SRC_BGR>(dst_fmt, src, small, S, max_h, max_w, h4, w4, sz, dst, st);
+    case MGW_YUV420_NV12: return launch_remap_up_mixed<MGW_YUV420_NV12>(dst_fmt, src, small, S, max_h, max_w, h4, w4, sz, dst, st);
+    case MGW_YUV420_I420: return launch_remap_up_mixed<MGW_YUV420_I420>(dst_fmt, src, small, S, max_h, max_w, h4, w4, sz, dst, st);
+    default: return set_error(MGW_ERR_INVALID, "remap_bundle_frame_mixed: unknown source format %d", src_fmt);
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // cvt_img2train (config.py:6-21): BGR uint8 frame -> cv2 BGR2GRAY -> Pillow resize(BILINEAR) [-> crop] -> v*(1/255) - 0.5.
 // The host binding computes Pillow's 22-bit fixed-point coefficient tables (double arithmetic, Resample.c) once per shape
@@ -435,14 +518,6 @@ int launch_remap_bundle_yuv420(const uint8_t* src, int src_fmt, const float* xy,
 // has its own tables (kx [S,out_w,ks], ...) and tmp rows [S,H,out_w].  Block (., s) reads sizes[s] once, offsets its pointers to
 // the slot, and then runs the per-pixel code of the uniform batch at the slot's size with frame index 0.
 namespace {
-
-// A slot is idle -- its blocks return before they write anything -- when its size is 0, larger than the capacity, or odd for a
-// YUV format: never-joined slots, and a bad device-side size cannot move a read outside the slot's region.
-template <int FMT>
-__device__ __forceinline__ bool slot_active(int2 sz, int max_h, int max_w)
-{
-    return sz.x > 0 && sz.y > 0 && sz.x <= max_h && sz.y <= max_w && (FMT == SRC_BGR || ((sz.x | sz.y) & 1) == 0);
-}
 
 template <int FMT, bool MIXED = false>
 __global__ void __launch_bounds__(256)

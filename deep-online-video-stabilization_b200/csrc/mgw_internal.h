@@ -119,6 +119,11 @@ int launch_remap_bundle(const uint8_t* src, int src_fmt, int C, const float* xy,
 // cv2.cvtColor(COLOR_BGR2YUV_I420) computes them from the BGR result, converted inside the warp
 int launch_remap_bundle_yuv420(const uint8_t* src, int src_fmt, const float* xy, int N, int h, int w, int H, int W, int dst_fmt,
                                uint8_t* dst, void* workspace, cudaStream_t st);
+// the warp per slot at the slot's own size sizes[s] (int32 [S,2], 8-byte aligned): slot s's frame at src + s * frame_bytes(max_h,
+// max_w) in src_fmt, its result at dst + s * dst_frame_bytes(max_h, max_w) in dst_fmt (MGW_BGR24 or YUV 4:2:0); xy [S,h,w,2].
+// Slots with a size of 0, above the capacity or odd (either format YUV) write nothing.
+int launch_remap_bundle_mixed(const uint8_t* src, int src_fmt, int S, int max_h, int max_w, const int32_t* sizes, const float* xy,
+                              int h, int w, int dst_fmt, uint8_t* dst, void* workspace, cudaStream_t st);
 
 // S frames of one size ([S,H,W,C] -> [S,out_h,out_w,C]; S >= 1, the single-frame calls pass 1).  src_fmt: 0 for the BGR / C-channel
 // frames, MGW_YUV420_NV12 or MGW_YUV420_I420 for YUV 4:2:0 frames [S,3H/2,W] read as the BGR frames cvtColor makes of them (C = 3)

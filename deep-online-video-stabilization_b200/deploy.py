@@ -220,11 +220,12 @@ def _cvt_tables(H, W, height, width, crop_rate, device):
     return _CVT_TABLES[key]
 
 
-def mixed_slot_tables(src_size, max_src_size, height=288, width=512, crop_rate=1):
+def mixed_slot_tables(src_size, max_src_size, height=288, width=512, crop_rate=1, out_size=None):
     """One slot's tables for the per-slot calls (ops.cvt_img2train_mixed / ops.resize_linear_mixed), numpy int32:
-    (kx [width,ksx], x0, xn [width], ky [height,ksy], y0, yn [height], xtab [width,4], ytab [height,4]).  They are the uniform
+    (kx [width,ksx], x0, xn [width], ky [height,ksy], y0, yn [height], xtab [OW,4], ytab [OH,4]).  They are the uniform
     tables at the slot's size src_size = (H, W), with the Pillow windows zero-padded to the lengths ksx, ksy of the capacity
-    max_src_size; xtab / ytab are given even where the slot takes the 2x2 shortcut."""
+    max_src_size; xtab / ytab resize to out_size = (OH, OW) (default: the network's (height, width)) and are given even where
+    the slot takes the 2x2 shortcut."""
     (H, W), (mh, mw) = (int(v) for v in src_size), (int(v) for v in max_src_size)
     if not (0 < H <= mh and 0 < W <= mw):
         raise ValueError('source size %dx%d outside the capacity %dx%d' % (H, W, mh, mw))
@@ -235,8 +236,9 @@ def mixed_slot_tables(src_size, max_src_size, height=288, width=512, crop_rate=1
         raise ValueError('a %dx%d source needs longer windows than its capacity %dx%d' % (H, W, mh, mw))
     kxp, kyp = np.zeros((width, ksx), np.int32), np.zeros((height, ksy), np.int32)
     kxp[:, :kx.shape[1]], kyp[:, :ky.shape[1]] = kx, ky
+    oh, ow = (height, width) if out_size is None else (int(out_size[0]), int(out_size[1]))
     return (kxp, np.ascontiguousarray(x0), np.ascontiguousarray(xn), kyp, np.ascontiguousarray(y0), np.ascontiguousarray(yn),
-            _cv_linear_table(width, W, True), _cv_linear_table(height, H, False))
+            _cv_linear_table(ow, W, True), _cv_linear_table(oh, H, False))
 
 
 def cvt_img2train(img, crop_rate=1, height=288, width=512, device='cuda', as_numpy=False, src_format='bgr'):
@@ -592,13 +594,37 @@ class MixedStreamBatch(StreamBatch):
     the whole pool, capacity bytes per slot whatever the slots' sizes.  A slot can join again at another size between replays of
     a captured graph: join writes the slot's size and tables with stream-ordered device copies, and the graph reads them.
     Slots that never joined are idle: the front end writes nothing for them and the network sees zero frames.  A slot that left
-    keeps its size and runs on whatever its region holds, as in StreamBatch.  out_format is StreamBatch's; the output stays at
-    the network's size."""
+    keeps its size and runs on whatever its region holds, as in StreamBatch.
+
+    out_size sets the size of the stabilised colour frames, and out_format ('bgr', 'nv12', 'i420') their format, as in
+    StreamBatch:
+      None       the network's (height, width) for every slot: self.colour is [S,h,w,3] (or [S,3h/2,w]).
+      (OH, OW)   one size for every slot: each slot is resized to it with its own tables and warped; self.colour is [S,OH,OW,3]
+                 (or [S,3OH/2,OW]), each slot bit-identical to StreamBatch(1, (H_s, W_s), out_size=(OH, OW)).
+      'source'   each slot at its own size: the warp reads the pool itself and writes the output pool self.colour, of shape
+                 out_pool_shape = [S, dst_frame_bytes(capacity)] (3*H*W for BGR, 3H/2*W for YUV 4:2:0), slot s's frame at the
+                 start of its row; slot_output() gives that view of any buffer of that shape (device, or a pinned host buffer
+                 that capture(download_to=) fills -- the download copies the whole output pool).  Each slot is bit-identical
+                 to StreamBatch(1, (H_s, W_s), out_size=(H_s, W_s)).  With a YUV out_format, join() refuses a frame of odd size.
+    leave() gives the rectangle on the network's lattice; in output pixels it is scale_rect(mb.leave(s), (h, w),
+    mb.slot_sizes[s]) for 'source', or scale_rect(mb.leave(s), (h, w), (OH, OW)) for a common size."""
 
     def __init__(self, S, max_src_size, height=288, width=512, depth=32, taps=(1, 2, 4, 8, 16, 32), use_masks=True, crop_rate=1,
-                 refine=1, device='cuda', src_format='bgr', out_format='bgr'):
+                 refine=1, device='cuda', src_format='bgr', out_size=None, out_format='bgr'):
+        if isinstance(out_size, str) and out_size != 'source':
+            raise ValueError("out_size must be None, (OH, OW) or 'source' (got %r)" % (out_size,))
+        self._source_out = out_size == 'source'
+        # 'source': StreamBatch sizes its checks and its result at the capacity, which holds the output pool's bytes
         super().__init__(S, max_src_size, height, width, depth, taps, use_masks, crop_rate, refine, device, src_format,
-                         out_format=out_format)
+                         out_size=tuple(max_src_size) if self._source_out else out_size, out_format=out_format)
+        if self._source_out:
+            self.out_size = 'source'
+            self.colour = self.colour.view(self.S, -1)
+            self.out_pool_shape = tuple(self.colour.shape)
+        elif self._direct:
+            # a common output size equal to the capacity: the slots still go through the per-slot resize
+            self._direct = False
+            self.small = torch.zeros((self.S,) + self.out_size + (3,), device=self.frames.device, dtype=torch.uint8)
 
     def _init_front_end(self, dev):
         """per-slot sizes and tables, all zero (every slot idle) until a slot joins"""
@@ -610,10 +636,15 @@ class MixedStreamBatch(StreamBatch):
         self.tables = (torch.zeros((self.S, w, _pil_ksize(W, rw)), **i32), torch.zeros((self.S, w), **i32),
                        torch.zeros((self.S, w), **i32), torch.zeros((self.S, h, _pil_ksize(H, rh)), **i32),
                        torch.zeros((self.S, h), **i32), torch.zeros((self.S, h), **i32))
-        self.xtab, self.ytab = torch.zeros((self.S, w, 4), **i32), torch.zeros((self.S, h, 4), **i32)
+        if self._source_out:
+            self.xtab = self.ytab = None                    # the warp reads the pool: no resize
+        else:
+            oh, ow = self.out_size
+            self.xtab, self.ytab = torch.zeros((self.S, ow, 4), **i32), torch.zeros((self.S, oh, 4), **i32)
         self.slot_sizes = [None] * self.S
         self.cur.zero_()
-        self.small.zero_()
+        if self.small is not None:
+            self.small.zero_()
 
     def _frame_size(self, f):
         if not isinstance(f, torch.Tensor) or f.dtype != torch.uint8:
@@ -640,9 +671,13 @@ class MixedStreamBatch(StreamBatch):
         s = self._slot(slot)
         f = torch.as_tensor(np.ascontiguousarray(first)) if isinstance(first, np.ndarray) else first
         H, W = self._frame_size(f)
+        if self._source_out and self.out_format != 'bgr' and (H % 2 or W % 2):
+            raise ValueError('a %s output needs an even size (got a %dx%d frame)' % (self.out_format, H, W))
         # host-built tables (about 15 ms at 2160x3840), copied into the slot's rows on the current stream; nothing is kept per size
-        tabs = mixed_slot_tables((H, W), self.src_size, self.height, self.width, self.crop_rate)
-        for dst, src in zip((self.sizes,) + self.tables + (self.xtab, self.ytab), (np.array([H, W], np.int32),) + tabs):
+        tabs = mixed_slot_tables((H, W), self.src_size, self.height, self.width, self.crop_rate,
+                                 out_size=None if self._source_out else self.out_size)
+        dsts = (self.sizes,) + self.tables + (() if self._source_out else (self.xtab, self.ytab))
+        for dst, src in zip(dsts, (np.array([H, W], np.int32),) + tabs):
             dst[s].copy_(torch.as_tensor(src))
         self.slot_sizes[s] = (H, W)
         cur = cvt_img2train(f.to(self.frames.device), self.crop_rate, self.height, self.width, src_format=self.src_format)
@@ -659,10 +694,25 @@ class MixedStreamBatch(StreamBatch):
         shape = self._frame_shape_of(*self.slot_sizes[s])
         return buf[s, :int(np.prod(shape))].view(shape)
 
+    def slot_output(self, buf, slot):
+        """out_size='source': the view of slot `slot`'s stabilised frame inside a buffer buf of out_pool_shape uint8 (self.colour,
+        or a pinned host buffer it is downloaded into): BGR [H_s,W_s,3] or YUV 4:2:0 [3H_s/2,W_s] at the slot's size."""
+        if not self._source_out:
+            raise ValueError("slot_output needs out_size='source' (the output is self.colour[slot])")
+        s = self._slot(slot)
+        if self.slot_sizes[s] is None:
+            raise ValueError('slot %d carries no video' % s)
+        if tuple(buf.shape) != self.out_pool_shape or buf.dtype != torch.uint8:
+            raise ValueError('buf must be %s uint8 (got %s %s)' % (list(self.out_pool_shape), tuple(buf.shape), buf.dtype))
+        H, W = self.slot_sizes[s]
+        shape = (H, W, 3) if self.out_format == 'bgr' else (H * 3 // 2, W)
+        return buf[s, :int(np.prod(shape))].view(shape)
+
     def step(self, pool, net):
         """One frame of every slot from pool [S, frame_bytes(capacity)] uint8 on the device: cvt_img2train and cv2.resize of each
-        slot at its own size, and the StreamBatch step around them.  Returns the stabilised colour frames [S,h,w,3] uint8 BGR, or
-        [S,3h/2,w] YUV 4:2:0 for out_format 'nv12' / 'i420' (self.colour, overwritten by the next step)."""
+        slot at its own size (no resize for out_size='source'), and the StreamBatch step around them.  Returns the stabilised
+        colour frames (self.colour, overwritten by the next step): [S,OH,OW,3] uint8 BGR, or [S,3OH/2,OW] YUV 4:2:0 for out_format
+        'nv12' / 'i420', with (OH, OW) the network's size by default; the output pool out_pool_shape for out_size='source'."""
         if not isinstance(pool, torch.Tensor) or pool.dtype != torch.uint8 or tuple(pool.shape) != self.pool_shape:
             raise ValueError('pool must be a %s uint8 tensor (got %s %s)' % (list(self.pool_shape), tuple(getattr(pool, 'shape', ())),
                                                                            getattr(pool, 'dtype', type(pool))))
@@ -670,5 +720,9 @@ class MixedStreamBatch(StreamBatch):
         h, w = self.height, self.width
         cur = ops.cvt_img2train_mixed(pool, self.src_format, self.sizes, self.tables, h, w, out=self.cur, tmp=self.cvt_tmp)
         xy = self.advance(cur, net)
-        small = ops.resize_linear_mixed(pool, self.src_format, self.sizes, self.xtab, self.ytab, h, w, out=self.small)
+        if self._source_out:
+            return ops.remap_bundle_frame_mixed(pool, self.src_format, self.sizes, xy, self.out_format, out=self.colour,
+                                                workspace=self.remap_ws)
+        oh, ow = self.out_size
+        small = ops.resize_linear_mixed(pool, self.src_format, self.sizes, self.xtab, self.ytab, oh, ow, out=self.small)
         return self._warp_small(small, xy)

@@ -810,6 +810,37 @@ def resize_linear_mixed(pool, fmt, sizes, xtab, ytab, out_h, out_w, out=None):
     return dst
 
 
+def dst_frame_bytes(out_format, H, W):
+    """bytes of one result frame: 3*H*W for 'bgr', 3H/2*W for YUV 4:2:0"""
+    return H * W * 3 if out_format == 'bgr' else H * W * 3 // 2
+
+
+def remap_bundle_frame_mixed(pool, fmt, sizes, xy, out_format='bgr', out=None, workspace=None):
+    """warpRevBundle2 of every slot of a pool at the slot's own size (remap_bundle_frame of the slot's frame alone, with xy[s]):
+    pool as for cvt_img2train_mixed, xy [S,h,w,2] fp32 -> the output pool [S, dst_frame_bytes(capacity)] uint8, slot s's result
+    at the start of its row, BGR [H_s,W_s,3] or YUV 4:2:0 [3H_s/2,W_s] for out_format 'nv12' / 'i420' (the capacity must then be
+    even).  Bytes past a slot's result, and the rows of idle slots (size 0, above the capacity, odd with either format YUV), are
+    left as they were.  out / workspace: optional preallocated output pool and fp32 scratch of remap_bundle_workspace_floats(S, h, w)."""
+    pool, sizes, xy = _chk(pool, 'pool', torch.uint8), _chk(sizes, 'sizes', torch.int32), _chk(xy, 'xy')
+    code, s, mh, mw = _mixed_dims(pool, fmt, sizes)
+    if out_format not in SRC_FORMATS:
+        raise ValueError('out_format must be one of %s (got %r)' % (sorted(SRC_FORMATS), out_format))
+    if out_format != 'bgr' and (mh % 2 or mw % 2):
+        raise ValueError('a %s result needs an even capacity (got %dx%d)' % (out_format, mh, mw))
+    if xy.dim() != 4 or xy.shape[0] != s or xy.shape[3] != 2:
+        raise ValueError('xy must be [%d,h,w,2] (got %s)' % (s, tuple(xy.shape)))
+    h, w = int(xy.shape[1]), int(xy.shape[2])
+    dst = _out(out, (s, dst_frame_bytes(out_format, mh, mw)), pool.device, torch.uint8, 'out')
+    ws = (torch.empty(remap_bundle_workspace_floats(s, h, w), device=pool.device, dtype=torch.float32) if workspace is None
+          else _chk_out(workspace, 'workspace'))
+    if ws.numel() < remap_bundle_workspace_floats(s, h, w):
+        raise ValueError('workspace needs %d floats' % remap_bundle_workspace_floats(s, h, w))
+    with torch.cuda.device(pool.device):
+        check(lib.mgw_remap_bundle_frame_mixed(_p(pool), code, s, mh, mw, _p(sizes), _p(xy), h, w, SRC_FORMATS[out_format], _p(dst),
+                                               _p(ws), _st()), 'mgw_remap_bundle_frame_mixed')
+    return dst
+
+
 # ---- warpRevBundle2 at the frame's own size
 def remap_bundle_frame(src, src_format, xy, out=None, workspace=None, out_format='bgr'):
     """warpRevBundle2 of frames at any size: src [S,H,W,3] uint8 ('bgr') or [S,3H/2,W] ('nv12' / 'i420'), xy [S,h,w,2] fp32 (the

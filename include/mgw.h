@@ -334,6 +334,20 @@ MGW_API int mgw_remap_bundle_frame(const uint8_t* src, int format, const float* 
 MGW_API int mgw_remap_bundle_frame_yuv420(const uint8_t* src, int format, const float* xy, int S, int h, int w, int H, int W,
                                int dst_format, uint8_t* dst, void* workspace, void* stream);
 
+/* ---- f1 for a batch of videos of different source sizes, each stabilised at its own size -------------------------------
+ * src is a pool of the per-slot calls above (format, capacity (max_h, max_w), sizes [S,2] device int32, 8-byte aligned), xy
+ * [S,h,w,2] as for mgw_remap_bundle_frame.  dst holds S regions of dst_frame_bytes(max_h, max_w) (3*max_h*max_w for MGW_BGR24,
+ * 3*max_h*max_w/2 for YUV 4:2:0); slot s's result lies contiguous at the start of its region in the slot's own size: BGR
+ * [H_s,W_s,3] or, for dst_format MGW_YUV420_NV12 / _I420, [3H_s/2,W_s].  Every active slot's bytes are those of
+ * mgw_remap_bundle_frame (MGW_BGR24) or mgw_remap_bundle_frame_yuv420 on that slot's frame alone at (H_s, W_s) with xy[s].  Bytes
+ * past a slot's result inside its region are not written, nor is any byte of an idle slot's region: size 0, above the capacity,
+ * or odd when either format is YUV.  workspace: mgw_remap_bundle_frame_workspace_bytes(S, h, w, ., .).
+ * Checked in the order of the batch calls: both formats and the sizes (0 <= S <= 65535, h, w >= 8, 1 <= max_h, max_w <= 32767,
+ * the capacity even when either format is YUV, S*max_h*max_w*3 < 2^31, S*h*w < 2^31), then S = 0 returns MGW_OK and launches
+ * nothing, then the pointers and the 8-byte alignment of xy, workspace and sizes. */
+MGW_API int mgw_remap_bundle_frame_mixed(const uint8_t* src, int format, int S, int max_h, int max_w, const int32_t* sizes,
+                               const float* xy, int h, int w, int dst_format, uint8_t* dst, void* workspace, void* stream);
+
 /* ---- a6: interpolate(im, x, y, out_size), spatial_transformer.py:200-281 ------------------------------
  * im [N,IH,IW,C]; x,y [N,OH,OW] normalised coords -> out [N,OH,OW,C]. */
 MGW_API int mgw_interp_fwd(const float* im, const float* x, const float* y, int N, int IH, int IW, int C, int OH, int OW,
