@@ -68,6 +68,7 @@ SIGNATURES = {
     'mgw_remap_bundle_frame': (c_i, [c_f, c_i, c_f, c_i, c_i, c_i, c_i, c_i, c_f, c_f, c_st]),
     'mgw_remap_bundle_frame_yuv420': (c_i, [c_f, c_i, c_f, c_i, c_i, c_i, c_i, c_i, c_i, c_f, c_f, c_st]),
     'mgw_remap_bundle_frame_mixed': (c_i, [c_f, c_i, c_i, c_i, c_i, c_f, c_f, c_i, c_i, c_i, c_f, c_f, c_st]),
+    'mgw_copy_slots_mixed': (c_i, [c_f, c_f, c_i, c_i, c_i, c_i, c_f, c_st]),
     'mgw_interp_fwd': (c_i, [c_f, c_f, c_f] + [c_i] * 6 + [c_f, c_st]),
     'mgw_interp_bwd': (c_i, [c_f, c_f, c_f, c_f] + [c_i] * 6 + [c_f, c_f, c_f, c_st]),
     'mgw_homography_warp_fwd': (c_i, [c_f, c_f] + [c_i] * 6 + [c_f, c_f, c_f, c_st]),

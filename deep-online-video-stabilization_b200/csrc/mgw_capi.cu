@@ -571,6 +571,51 @@ int mgw_remap_bundle_frame_mixed(const uint8_t* src, int format, int S, int max_
     return launch_remap_bundle_mixed(src, format, S, max_h, max_w, sizes, xy, h, w, dst_format, dst, workspace, (cudaStream_t)stream);
 }
 
+// The address a kernel reaches the `bytes` bytes at p through: device or managed memory as it is, pinned host memory through its
+// mapped device address.  Both ends are looked up, so a buffer that runs past its allocation is refused; pageable memory has no
+// device address.
+static int device_address(const char* fn, const char* what, const void* p, size_t bytes, const void** dev)
+{
+    const char* q[2] = {static_cast<const char*>(p), static_cast<const char*>(p) + bytes - 1};
+    const char* d[2];
+    for (int k = 0; k < 2; ++k) {
+        cudaPointerAttributes a;
+        const cudaError_t e = cudaPointerGetAttributes(&a, q[k]);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            return set_error(MGW_ERR_CUDA, "%s: %s: %s", fn, what, cudaGetErrorString(e));
+        }
+        REQUIRE(a.type != cudaMemoryTypeUnregistered, "%s: %s is pageable host memory (pin it: cudaHostAlloc / cudaHostRegister)", fn, what);
+        REQUIRE(a.devicePointer, "%s: %s has no device address", fn, what);
+        d[k] = static_cast<const char*>(a.devicePointer);
+    }
+    REQUIRE(d[1] == d[0] + (bytes - 1), "%s: %s is not one mapped range of %zu bytes", fn, what, bytes);
+    *dev = d[0];
+    return MGW_OK;
+}
+
+// The batch calls' order: format and sizes, then S = 0, then pointers and alignment; then where src and dst live
+int mgw_copy_slots_mixed(const uint8_t* src, uint8_t* dst, int format, int S, int max_h, int max_w, const int32_t* sizes, void* stream)
+{
+    REQUIRE(format == MGW_BGR24 || format == MGW_YUV420_NV12 || format == MGW_YUV420_I420, "mgw_copy_slots_mixed: unknown format %d",
+            format);
+    const long long stride = format == MGW_BGR24 ? 3LL * max_h * max_w : 3LL * max_h * max_w / 2;
+    REQUIRE(S >= 0 && S <= 65535 && max_h >= 1 && max_w >= 1 && max_h <= 32767 && max_w <= 32767 &&
+            (format == MGW_BGR24 || (max_h % 2 == 0 && max_w % 2 == 0)) && S * stride < (1LL << 31),
+            "mgw_copy_slots_mixed: bad sizes (S=%d capacity %dx%d; capacity even for YUV, S * frame_bytes(capacity) < 2^31)", S, max_h,
+            max_w);
+    if (S == 0) return MGW_OK;
+    REQUIRE(src && dst && sizes, "mgw_copy_slots_mixed: null pointer");
+    REQUIRE(aligned(src, 16) && aligned(dst, 16), "mgw_copy_slots_mixed: src and dst must be 16-byte aligned");
+    REQUIRE(aligned(sizes, 8), "mgw_copy_slots_mixed: sizes must be 8-byte aligned");
+    const size_t bytes = (size_t)(S * stride);
+    const void *s_dev, *d_dev;
+    TRY(device_address("mgw_copy_slots_mixed", "src", src, bytes, &s_dev));
+    TRY(device_address("mgw_copy_slots_mixed", "dst", dst, bytes, &d_dev));
+    return launch_copy_slots_mixed(static_cast<const uint8_t*>(s_dev), static_cast<uint8_t*>(const_cast<void*>(d_dev)), format, S, max_h,
+                                   max_w, sizes, (cudaStream_t)stream);
+}
+
 int mgw_stream_assemble(const float* frames, const float* masks, int depth, int head, const int* taps, int ntaps, int use_masks,
                         const float* cur, int H, int W, float* in_x, void* stream)
 {

@@ -506,6 +506,70 @@ int launch_remap_bundle_mixed(const uint8_t* src, int src_fmt, int S, int max_h,
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
+// Exact-bytes transfer of a pool of per-slot frames (MIXED): slot s's frame_bytes(sizes[s]) bytes from src + s * stride to
+// dst + s * stride, stride = frame_bytes(max_h, max_w); nothing past them is read or written, and an idle slot (the MIXED rule)
+// moves nothing.  Either side may be pinned host memory reached through its mapped device address, so the kernel is the
+// upload, the download or a device copy; a copy-engine node of a captured graph has a fixed size, this kernel reads the sizes
+// at replay.  src and dst are 16-byte aligned, so both sides of a slot share the misalignment of s * stride: a head of under
+// 16 bytes up to the boundary, the body in 16-byte vectors (COPY_UNROLL independent loads in flight per thread, to cover
+// the round trip of a read across PCIe), a tail of under 16 bytes.  gridDim.y is the slot, gridDim.x blocks share its body.
+namespace {
+
+constexpr int COPY_THREADS = 256, COPY_UNROLL = 4;
+
+// FMT = SRC_BGR or MGW_YUV420_NV12 (I420 has NV12's bytes per frame and idle rule)
+template <int FMT>
+__global__ void __launch_bounds__(COPY_THREADS)
+copy_slots_kernel(const uint8_t* __restrict__ src, uint8_t* __restrict__ dst, int max_h, int max_w, const int2* __restrict__ sizes)
+{
+    const int2 sz = __ldg(sizes + blockIdx.y);
+    if (!slot_active<FMT>(sz, max_h, max_w)) return;
+    const size_t off = (size_t)blockIdx.y * src_frame_bytes<FMT>(max_h, max_w);
+    src += off;
+    dst += off;
+    const int n = (int)src_frame_bytes<FMT>(sz.x, sz.y);                  // < 2^31: the call checks S * stride
+    const int head = min((int)((16 - (off & 15)) & 15), n);
+    const int n16 = (n - head) >> 4, tail = head + (n16 << 4);
+    const int t = blockIdx.x * COPY_THREADS + threadIdx.x, nt = gridDim.x * COPY_THREADS;
+    if (t < head) dst[t] = __ldcs(src + t);
+    if (t < n - tail) dst[tail + t] = __ldcs(src + tail + t);
+    const uint4* s4 = reinterpret_cast<const uint4*>(src + head);
+    uint4* d4 = reinterpret_cast<uint4*>(dst + head);
+    int i = t;
+    for (; i + (COPY_UNROLL - 1) * nt < n16; i += COPY_UNROLL * nt) {
+        uint4 v[COPY_UNROLL];
+#pragma unroll
+        for (int k = 0; k < COPY_UNROLL; ++k) v[k] = __ldcs(s4 + i + k * nt);
+#pragma unroll
+        for (int k = 0; k < COPY_UNROLL; ++k) __stcs(d4 + i + k * nt, v[k]);
+    }
+    for (; i < n16; i += nt) __stcs(d4 + i, __ldcs(s4 + i));
+}
+
+}  // namespace
+
+// gridDim.x: COPY_BLOCKS_PER_SM blocks per SM spread over the slots, no more than one pass over a full slot needs
+int launch_copy_slots_mixed(const uint8_t* src, uint8_t* dst, int fmt, int S, int max_h, int max_w, const int32_t* sizes, cudaStream_t st)
+{
+    constexpr long long COPY_BLOCKS_PER_SM = 8;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const long long stride = fmt == SRC_BGR ? 3LL * max_h * max_w : 3LL * max_h * max_w / 2;
+    const long long pass = (long long)COPY_THREADS * COPY_UNROLL * 16;
+    const long long full = (stride + pass - 1) / pass, spread = (sms * COPY_BLOCKS_PER_SM + S - 1) / S;
+    const dim3 grid((unsigned)(full < spread ? full : spread), S);
+    const int2* sz = reinterpret_cast<const int2*>(sizes);
+    switch (fmt) {
+    case SRC_BGR: copy_slots_kernel<SRC_BGR><<<grid, COPY_THREADS, 0, st>>>(src, dst, max_h, max_w, sz); break;
+    case MGW_YUV420_NV12:
+    case MGW_YUV420_I420: copy_slots_kernel<MGW_YUV420_NV12><<<grid, COPY_THREADS, 0, st>>>(src, dst, max_h, max_w, sz); break;
+    default: return set_error(MGW_ERR_INVALID, "copy_slots_mixed: unknown format %d", fmt);
+    }
+    return check_launch("copy_slots");
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
 // cvt_img2train (config.py:6-21): BGR uint8 frame -> cv2 BGR2GRAY -> Pillow resize(BILINEAR) [-> crop] -> v*(1/255) - 0.5.
 // The host binding computes Pillow's 22-bit fixed-point coefficient tables (double arithmetic, Resample.c) once per shape
 // and slices them for the crop; the two passes below are Pillow's: horizontal first into a uint8 image, then vertical.

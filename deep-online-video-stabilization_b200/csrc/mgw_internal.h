@@ -124,6 +124,9 @@ int launch_remap_bundle_yuv420(const uint8_t* src, int src_fmt, const float* xy,
 // Slots with a size of 0, above the capacity or odd (either format YUV) write nothing.
 int launch_remap_bundle_mixed(const uint8_t* src, int src_fmt, int S, int max_h, int max_w, const int32_t* sizes, const float* xy,
                               int h, int w, int dst_fmt, uint8_t* dst, void* workspace, cudaStream_t st);
+// each active slot's frame_bytes(fmt, sizes[s]) bytes from src + s * stride to dst + s * stride (stride = frame_bytes(fmt, max_h,
+// max_w)); src / dst 16-byte aligned device addresses (a pinned host buffer's mapped one), sizes 8-byte aligned; idle slots as above
+int launch_copy_slots_mixed(const uint8_t* src, uint8_t* dst, int fmt, int S, int max_h, int max_w, const int32_t* sizes, cudaStream_t st);
 
 // S frames of one size ([S,H,W,C] -> [S,out_h,out_w,C]; S >= 1, the single-frame calls pass 1).  src_fmt: 0 for the BGR / C-channel
 // frames, MGW_YUV420_NV12 or MGW_YUV420_I420 for YUV 4:2:0 frames [S,3H/2,W] read as the BGR frames cvtColor makes of them (C = 3)

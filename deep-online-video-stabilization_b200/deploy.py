@@ -554,6 +554,12 @@ class StreamBatch:
         is restored, so capturing leaves every slot as it was."""
         if download_to is not None and tuple(download_to.shape) != tuple(self.colour.shape):
             raise ValueError('download_to must be %s (got %s)' % (list(self.colour.shape), tuple(download_to.shape)))
+        upload = None if upload_from is None else lambda: raw_bgr.copy_(upload_from, non_blocking=True)
+        download = None if download_to is None else lambda: download_to.copy_(self.colour, non_blocking=True)
+        return self._capture(raw_bgr, net, upload, download)
+
+    def _capture(self, raw_bgr, net, upload, download):
+        """capture() with the transfers as callables (or None) recorded before and after the step"""
         state = (self.frames, self.masks, self.heads_dev, self.all_black)
         snap = [t.clone() for t in state]
         side = torch.cuda.Stream(device=self.frames.device)
@@ -565,11 +571,11 @@ class StreamBatch:
             t.copy_(v)
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph):
-            if upload_from is not None:
-                raw_bgr.copy_(upload_from, non_blocking=True)
+            if upload is not None:
+                upload()
             self.step(raw_bgr, net)
-            if download_to is not None:
-                download_to.copy_(self.colour, non_blocking=True)
+            if download is not None:
+                download()
         return graph
 
 
@@ -591,8 +597,10 @@ class MixedStreamBatch(StreamBatch):
     pool: [S, frame_bytes(max_src_size)] uint8 (frame_bytes = 3*H*W for BGR, 3H/2*W for YUV 4:2:0); slot s's frame lies contiguous
     at the start of pool[s], BGR [H_s,W_s,3] or YUV [3H_s/2,W_s].  slot_frame() gives that view of any pool-shaped buffer (device
     or pinned host).  capture(pool, net, upload_from=, download_to=) is StreamBatch.capture: the upload inside the graph copies
-    the whole pool, capacity bytes per slot whatever the slots' sizes.  A slot can join again at another size between replays of
-    a captured graph: join writes the slot's size and tables with stream-ordered device copies, and the graph reads them.
+    the whole pool, capacity bytes per slot whatever the slots' sizes.  capture(..., exact_bytes=True) records the transfers as
+    one kernel each (ops.copy_slots_mixed) that moves every slot's frame at its size at replay and nothing else: the bytes past
+    each slot's frame, and idle slots' rows, are not copied in either direction.  A slot can join again at another size
+    between replays of a captured graph: join writes the slot's size and tables with stream-ordered device copies, and the graph reads them.
     Slots that never joined are idle: the front end writes nothing for them and the network sees zero frames.  A slot that left
     keeps its size and runs on whatever its region holds, as in StreamBatch.
 
@@ -604,7 +612,8 @@ class MixedStreamBatch(StreamBatch):
       'source'   each slot at its own size: the warp reads the pool itself and writes the output pool self.colour, of shape
                  out_pool_shape = [S, dst_frame_bytes(capacity)] (3*H*W for BGR, 3H/2*W for YUV 4:2:0), slot s's frame at the
                  start of its row; slot_output() gives that view of any buffer of that shape (device, or a pinned host buffer
-                 that capture(download_to=) fills -- the download copies the whole output pool).  Each slot is bit-identical
+                 that capture(download_to=) fills -- the download copies the whole output pool, or with exact_bytes=True
+                 each slot's frame).  Each slot is bit-identical
                  to StreamBatch(1, (H_s, W_s), out_size=(H_s, W_s)).  With a YUV out_format, join() refuses a frame of odd size.
     leave() gives the rectangle on the network's lattice; in output pixels it is scale_rect(mb.leave(s), (h, w),
     mb.slot_sizes[s]) for 'source', or scale_rect(mb.leave(s), (h, w), (OH, OW)) for a common size."""
@@ -726,3 +735,36 @@ class MixedStreamBatch(StreamBatch):
         oh, ow = self.out_size
         small = ops.resize_linear_mixed(pool, self.src_format, self.sizes, self.xtab, self.ytab, oh, ow, out=self.small)
         return self._warp_small(small, xy)
+
+    def capture(self, pool, net, upload_from=None, download_to=None, exact_bytes=False):
+        """StreamBatch.capture of step(pool, net).  exact_bytes=False copies the whole pool up (and, for out_size='source', the
+        whole output pool down).  exact_bytes=True records the transfers as ops.copy_slots_mixed, which moves each slot's frame at
+        the size it has at replay and nothing else: upload_from (pool_shape) and download_to (out_pool_shape for 'source') must
+        then be pinned host tensors.  The bytes past each slot's frame, and idle slots' rows, are not copied in either direction:
+        the device pool and the host output pool keep what they held there.  A uniform output ([S,OH,OW,3] or [S,3OH/2,OW]) is
+        downloaded whole either way: it has no bytes but the frames."""
+        if not exact_bytes:
+            return super().capture(pool, net, upload_from, download_to)
+        for name, t, shape in (('upload_from', upload_from, self.pool_shape),
+                               ('download_to', download_to, tuple(self.colour.shape))):
+            if t is None:
+                continue
+            if not isinstance(t, torch.Tensor) or t.is_cuda or not t.is_pinned():
+                raise ValueError('%s must be a pinned host tensor with exact_bytes=True' % name)
+            if tuple(t.shape) != shape:
+                raise ValueError('%s must be %s (got %s)' % (name, list(shape), tuple(t.shape)))
+        upload = download = None
+        if upload_from is not None:
+            src_view = (self.S,) + self.frame_shape
+            def upload():
+                ops.copy_slots_mixed(upload_from.view(src_view), pool.view(src_view), self.src_format, self.sizes)
+        if download_to is not None:
+            if self._source_out:
+                H, W = self.src_size                        # the output pool's capacity
+                out_view = (self.S, H, W, 3) if self.out_format == 'bgr' else (self.S, H * 3 // 2, W)
+                def download():
+                    ops.copy_slots_mixed(self.colour.view(out_view), download_to.view(out_view), self.out_format, self.sizes)
+            else:
+                def download():
+                    download_to.copy_(self.colour, non_blocking=True)
+        return self._capture(pool, net, upload, download)

@@ -841,6 +841,34 @@ def remap_bundle_frame_mixed(pool, fmt, sizes, xy, out_format='bgr', out=None, w
     return dst
 
 
+def copy_slots_mixed(src, dst, fmt, sizes):
+    """Each slot's own frame bytes of a pool, and nothing else, from src to dst: slot s's first frame_bytes(sizes[s]) bytes of
+    src[s] go to dst[s] (3*H_s*W_s for 'bgr', 3H_s/2*W_s for 'nv12' / 'i420'); bytes past them and the rows of idle slots (size 0,
+    above the capacity, odd for YUV) are neither read nor written.  src and dst have one shape, that of the pools of
+    cvt_img2train_mixed ([S,max_h,max_w,3] for 'bgr', [S,3max_h/2,max_w] for YUV 4:2:0, which gives the capacity), and each is
+    a contiguous CUDA tensor or a pinned CPU tensor: the kernel reads or writes pinned host memory across PCIe itself, so this
+    one call is an upload, a download or a device copy, and inside a captured graph it follows the sizes of the replay.
+    One C-ABI call (mgw_copy_slots_mixed)."""
+    if fmt not in SRC_FORMATS:
+        raise ValueError('format must be one of %s (got %r)' % (sorted(SRC_FORMATS), fmt))
+    for name, t in (('src', src), ('dst', dst)):
+        if not isinstance(t, torch.Tensor) or t.dtype != torch.uint8:
+            raise ValueError('%s must be a uint8 tensor' % name)
+    if tuple(src.shape) != tuple(dst.shape):
+        raise ValueError('src and dst must have one shape (got %s and %s)' % (tuple(src.shape), tuple(dst.shape)))
+    code, s, mh, mw = _mixed_dims(src, fmt, sizes)
+    for name, t in (('src', src), ('dst', dst)):
+        if not t.is_cuda and not t.is_pinned():
+            raise ValueError('%s is pageable host memory: the copy reaches host memory through its device address, which only pinned '
+                             'memory has' % name)
+        if not t.is_contiguous():
+            raise ValueError('%s must be contiguous' % name)
+    sizes = _chk(sizes, 'sizes', torch.int32)
+    with torch.cuda.device(sizes.device):
+        check(lib.mgw_copy_slots_mixed(_p(src), _p(dst), code, s, mh, mw, _p(sizes), _st()), 'mgw_copy_slots_mixed')
+    return dst
+
+
 # ---- warpRevBundle2 at the frame's own size
 def remap_bundle_frame(src, src_format, xy, out=None, workspace=None, out_format='bgr'):
     """warpRevBundle2 of frames at any size: src [S,H,W,3] uint8 ('bgr') or [S,3H/2,W] ('nv12' / 'i420'), xy [S,h,w,2] fp32 (the

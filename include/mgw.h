@@ -348,6 +348,22 @@ MGW_API int mgw_remap_bundle_frame_yuv420(const uint8_t* src, int format, const 
 MGW_API int mgw_remap_bundle_frame_mixed(const uint8_t* src, int format, int S, int max_h, int max_w, const int32_t* sizes,
                                const float* xy, int h, int w, int dst_format, uint8_t* dst, void* workspace, void* stream);
 
+/* ---- moving a pool of per-slot frames across PCIe: exactly each slot's bytes --------------------------------------------
+ * src and dst are pools of the per-slot calls above (format, capacity (max_h, max_w), sizes [S,2] device int32, 8-byte
+ * aligned).  For every active slot s the first frame_bytes(format, sizes[s]) bytes of src + s * frame_bytes(max_h, max_w) are
+ * copied to the same offset of dst; bytes past them, and every byte of an idle slot's region (size 0, above the capacity, odd
+ * for YUV), are neither read nor written.  One kernel, which reads the sizes when it runs, so a captured graph keeps working
+ * when a slot changes size.  Unlike every other call here, src and dst may each be pinned host memory (cudaHostAlloc /
+ * cudaHostRegister, read or written through its mapped device address across PCIe) as well as device or managed memory: the
+ * upload of a pinned host pool into the device pool, the download of an output pool, or a device copy.  Pageable host memory
+ * is refused (MGW_ERR_INVALID, "pageable" in mgw_last_error()) before anything is launched.
+ * Checked in the order of the batch calls: the format, the sizes (0 <= S <= 65535, 1 <= max_h, max_w <= 32767, even for YUV,
+ * S * frame_bytes(max_h, max_w) < 2^31), then S = 0 returns MGW_OK and launches nothing, then null pointers, src and dst 16-byte
+ * aligned, sizes 8-byte aligned, then the first and the last byte of src and of dst must be device, managed or pinned host
+ * memory (cudaPointerGetAttributes; legal inside a stream capture). */
+MGW_API int mgw_copy_slots_mixed(const uint8_t* src, uint8_t* dst, int format, int S, int max_h, int max_w, const int32_t* sizes,
+                               void* stream);
+
 /* ---- a6: interpolate(im, x, y, out_size), spatial_transformer.py:200-281 ------------------------------
  * im [N,IH,IW,C]; x,y [N,OH,OW] normalised coords -> out [N,OH,OW,C]. */
 MGW_API int mgw_interp_fwd(const float* im, const float* x, const float* y, int N, int IH, int IW, int C, int OH, int OW,
