@@ -12,8 +12,9 @@
 //             per thread they queued in the LSU for thousands of cycles).  dU is pre-accumulated in a shared-memory box in
 //             FIXED POINT with native integer shared atomics (ATOMS.ADD, ~1 cycle per warp instruction measured on B200,
 //             against ~4-6 cycles and a serialising ~300-cycle round trip for the CAS loop behind atomicAdd(float*)); the
-//             scale is a power of two chosen per tile from max|d_out|, kBits = 31 - ceil(log2(TH*TW)) <= 22 bits per term,
-//             so the int32 sums provably cannot overflow.  The box leaves as fp32 by 16-byte reductions
+//             scale is a power of two chosen per tile from max|d_out|, kBits = 30 - floor(log2(TH*TW)) <= 22 bits per term:
+//             a term rounds to at most 2^kBits and TH*TW of them stay below 2^31, so the int32 sums provably cannot
+//             overflow.  The box leaves as fp32 by 16-byte reductions
 //             (red.global.add.v4.f32, REDG; all-zero groups skipped) straight from the fixed-point words -- no conversion
 //             back into shared memory, no third barrier, no TMA read wait before the CTA exits.
 //             Launched programmatically behind the library's zero-fill of dU, the kernel runs next to it up to its first
@@ -67,7 +68,6 @@ struct Geo {
 struct TileInfo {
     int bx0, by0;                   // first column / row of the staged source box
     int interior;                   // every tap of every pixel of the tile is unclipped AND inside the staged box
-    int area_ok;                    // backward: the tile is not magnified beyond what the fixed-point headroom covers
     float wmax[kMaxWarps];          // backward: per-warp max|d_out|
 };
 
@@ -95,7 +95,7 @@ __device__ __forceinline__ Tile this_tile(const TileCfg& cfg)
 // to global memory for the ones outside the box.
 template <int C, int TW, int K, int NT>
 __device__ __forceinline__ void source_box(const TileCfg& cfg, const Tile& tl, const float (&Hc)[9], float stepx, float stepy,
-                                           int& bx0, int& by0, int& interior, int& area_ok, int* complete = nullptr)
+                                           int& bx0, int& by0, int& interior, int* complete = nullptr)
 {
     using G = Geo<C, TW, K, NT>;
     const int k4 = threadIdx.x & 3;
@@ -115,7 +115,7 @@ __device__ __forceinline__ void source_box(const TileCfg& cfg, const Tile& tl, c
         ok = ok && (__shfl_xor_sync(0xffffffffu, (int)ok, o) != 0);
     }
     ok = ok && (sgn == 4 || sgn == -4);
-    bx0 = 0; by0 = 0; interior = 0; area_ok = 0;
+    bx0 = 0; by0 = 0; interior = 0;
     if (complete) *complete = 0;
     if (ok) {
         const int ux0 = (int)floorf(xmin) - 1, ux1 = (int)floorf(xmax) + 2;      // unclipped tap range, 1 px of slack
@@ -132,8 +132,6 @@ __device__ __forceinline__ void source_box(const TileCfg& cfg, const Tile& tl, c
                     ux1 - bx0 < G::SBW && uy1 - by0 < G::SBH) ? 1 : 0;
         // every tap that survives clipping lies inside the box (the backward skips pixels with a clipped tap, see below)
         if (complete) *complete = (ix0 >= bx0 && ix1 - bx0 < G::SBW && iy0 >= by0 && iy1 - by0 < G::SBH) ? 1 : 0;
-        // magnification guard for the fixed-point accumulator: bbox area >= 1/16 of the tile area
-        area_ok = ((xmax - xmin + 1.0f) * (ymax - ymin + 1.0f) * 16.0f >= (float)(G::TH * TW)) ? 1 : 0;
     }
 }
 
@@ -194,8 +192,8 @@ warp_fwd_tma_kernel(const __grid_constant__ CUtensorMap mapU, const __grid_const
     const float stepx = cfg.stepx, stepy = cfg.stepy;
     __syncthreads();                                  // barrier initialised; nobody has waited on anything long yet
     if (tid < 32 && out) {
-        int bx0, by0, interior, area_ok;
-        source_box<C, TW, K, NT>(cfg, tl, Hc, stepx, stepy, bx0, by0, interior, area_ok);
+        int bx0, by0, interior;
+        source_box<C, TW, K, NT>(cfg, tl, Hc, stepx, stepy, bx0, by0, interior);
         if (tid == 0) {
             ti->bx0 = bx0; ti->by0 = by0; ti->interior = interior;
             tma::mbar_expect_tx(bar, (uint32_t)(G::kBoxF * sizeof(float)));     // release: publishes ti
@@ -305,6 +303,7 @@ constexpr float kMagic = 12582912.0f;          // 1.5 * 2^23
 constexpr int kMagicBits = 0x4B400000;
 __device__ __forceinline__ int fixed_of(float w, float gs) { return __float_as_int(__fmaf_rn(w, gs, kMagic)) - kMagicBits; }
 __device__ __forceinline__ float float_of_fixed(int v) { return (float)v; }      // sums of coincident taps may exceed 2^22: plain I2F
+constexpr int bit_width(int v) { return v > 0 ? 1 + bit_width(v >> 1) : 0; }       // floor(log2 v) + 1
 
 // dH terms of one pixel (SURVEY.md 8a-bwd) accumulated into the thread's 8 partial sums
 __device__ __forceinline__ void accumulate_dh(float (&dh)[8], float gxn, float gyn, float xn, float yn, float zs, float xt, float yt)
@@ -399,10 +398,10 @@ warp_bwd_tma_kernel(const __grid_constant__ CUtensorMap mapU, const __grid_const
     // the LSU for ~3500 cycles next to the other CTAs' shared-memory traffic: issued behind them, the box arrived ~4000 cycles
     // after the first barrier).  Thread 0 initialised the barrier itself; everybody else meets it after the __syncthreads below.
     if (tid < 32) {
-        int bx0, by0, interior, area_ok, complete;
-        source_box<C, TW, K, NT>(cfg, tl, Hc, stepx, stepy, bx0, by0, interior, area_ok, &complete);
+        int bx0, by0, interior, complete;
+        source_box<C, TW, K, NT>(cfg, tl, Hc, stepx, stepy, bx0, by0, interior, &complete);
         if (tid == 0) {
-            ti->bx0 = bx0; ti->by0 = by0; ti->interior = complete; ti->area_ok = area_ok;      // backward: "interior" = complete
+            ti->bx0 = bx0; ti->by0 = by0; ti->interior = complete;      // backward: "interior" = complete
             tma::mbar_expect_tx(bar, (uint32_t)(G::kBoxF * sizeof(float)));
             tma::load_3d(s_src, &mapU, bar, bx0 * C, by0, tl.n);
         }
@@ -482,14 +481,15 @@ warp_bwd_tma_kernel(const __grid_constant__ CUtensorMap mapU, const __grid_const
         for (int w = 0; w < NT / 32; ++w) mb = max(mb, (unsigned)__float_as_int(ti->wmax[w]));
         const float mm = __int_as_float((int)mb);
         const int e = (int)(mb >> 23) - 127;                                // floor(log2 mm) for normal mm; 128 for Inf/NaN
-        // |w*g*scale| < 2^kBits per term (tap weights are in [0,1] on this path).  A pixel adds at most ONE term to a word (its
-        // four taps are four different pixels), so a word receives at most TH*TW terms: with kBits = 31 - ceil(log2(TH*TW)) the
-        // int32 sum cannot overflow whatever the map does (no magnification heuristic); the quantum is 2^-kBits of the tile's
-        // max|d_out| (2^-20 for the 64 x 24 tile: a millionth, against a 1e-4 tolerance)
+        // |w*g*scale| < 2^kBits per term before rounding (tap weights are in [0,1] on this path), but fixed_of() rounds to
+        // nearest, so a term can reach 2^kBits exactly.  A pixel adds at most ONE term to a word (its four taps are four
+        // different pixels), so a word receives at most kTerms = TH*TW terms: with kBits = 31 - bit_width(kTerms), i.e.
+        // 30 - floor(log2 kTerms), their sum stays below 2^31 whatever the map does (no magnification heuristic).  Each term
+        // is exact to 2^-kBits of the tile's max|d_out| (2^-20 for the 64 x 24 tile: a millionth, against a 1e-4 tolerance)
         constexpr int kTerms = G::TH * TW;
+        constexpr int kBits = 31 - bit_width(kTerms);
         // (never more than 22: fixed_of()'s magic-number rounding holds |v| <= 2^22)
-        constexpr int kBits = 31 - (kTerms <= 512 ? 9 : kTerms <= 1024 ? 10 : kTerms <= 2048 ? 11 : 12);
-        static_assert(kTerms <= 4096 && kBits <= 22, "fixed-point headroom");
+        static_assert(kBits <= 22 && ((long long)kTerms << kBits) < (1LL << 31), "fixed-point headroom");
         fixed = (mm > 0.0f) && (e > -100) && (e < 100);
         scale = __int_as_float((kBits - 1 - e + 127) << 23);
         inv_scale = __int_as_float((e - (kBits - 1) + 127) << 23);
