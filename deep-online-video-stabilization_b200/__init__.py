@@ -10,7 +10,7 @@ from . import _lib, deploy, functional, losses, ops, parallel, spatial_transform
 from ._lib import MgwError, launch_count, set_impl  # noqa: F401
 from .losses import (feature_loss, get_4_pts, get_black_pos, get_black_pos_loss, get_consistency_loss, get_distortion_loss,  # noqa: F401
                      img_loss, loss_gates, pass_coef, temp_loss, total_loss, train_pass, transformer_img_loss, vertex_losses)
-from .deploy import CropState, MixedStreamBatch, StreamBatch, StreamState, warpRevBundle, warpRevBundle2  # noqa: F401
+from .deploy import CropState, MixedStreamBatch, PlaneTable, StreamBatch, StreamState, warpRevBundle, warpRevBundle2  # noqa: F401
 from .spatial_transformer import interpolate  # noqa: F401
 from .stabnet import StabNet, inference_stable_net, train_losses  # noqa: F401
 from .spatial_transformer3 import transformer  # noqa: F401

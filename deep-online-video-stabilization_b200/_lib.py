@@ -69,6 +69,9 @@ SIGNATURES = {
     'mgw_remap_bundle_frame_yuv420': (c_i, [c_f, c_i, c_f, c_i, c_i, c_i, c_i, c_i, c_i, c_f, c_f, c_st]),
     'mgw_remap_bundle_frame_mixed': (c_i, [c_f, c_i, c_i, c_i, c_i, c_f, c_f, c_i, c_i, c_i, c_f, c_f, c_st]),
     'mgw_copy_slots_mixed': (c_i, [c_f, c_f, c_i, c_i, c_i, c_i, c_f, c_st]),
+    'mgw_cvt_img2train_planes': (c_i, [c_f, c_i, c_i, c_i, c_i, c_f, c_f, c_f, c_i, c_f, c_f, c_f, c_i, c_i, c_i, c_f, c_f, c_st]),
+    'mgw_resize_linear_planes': (c_i, [c_f, c_i, c_i, c_i, c_i, c_f, c_f, c_i, c_i, c_f, c_st]),
+    'mgw_remap_bundle_frame_planes': (c_i, [c_f, c_i, c_f, c_i, c_i, c_i, c_i, c_i, c_f, c_i, c_f, c_st]),
     'mgw_interp_fwd': (c_i, [c_f, c_f, c_f] + [c_i] * 6 + [c_f, c_st]),
     'mgw_interp_bwd': (c_i, [c_f, c_f, c_f, c_f] + [c_i] * 6 + [c_f, c_f, c_f, c_st]),
     'mgw_homography_warp_fwd': (c_i, [c_f, c_f] + [c_i] * 6 + [c_f, c_f, c_f, c_st]),
@@ -80,6 +83,11 @@ SIGNATURES = {
     'mgw_temp_loss_fwd': (c_i, [c_f] * 5 + [c_i] * 4 + [c_f, c_st]),
     'mgw_temp_loss_bwd': (c_i, [c_f] * 6 + [c_fl, c_f] + [c_i] * 4 + [c_f, c_f, c_st]),
 }
+
+
+class mgw_planes(ctypes.Structure):
+    """include/mgw.h's mgw_planes: one frame's plane addresses (plane[0] == 0: the slot is idle) and row pitches in bytes"""
+    _fields_ = [('plane', ctypes.c_uint64 * 3), ('pitch', ctypes.c_int32 * 3), ('reserved', ctypes.c_int32 * 3)]
 
 
 class MgwError(RuntimeError):

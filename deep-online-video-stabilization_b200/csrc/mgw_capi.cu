@@ -814,6 +814,55 @@ int mgw_resize_linear_mixed(const uint8_t* src, int format, int S, int max_h, in
     return launch_resize_linear_mixed(src, format, S, max_h, max_w, sizes, xtab, ytab, out_h, out_w, dst, (cudaStream_t)stream);
 }
 
+static_assert(sizeof(mgw_planes) == 48 && offsetof(mgw_planes, pitch) == 24, "mgw_planes: 48-byte entries, pitches at 24");
+
+// Per-slot planes: the uniform calls' size limits at (H, W) for the format (validate_mixed with the frame size as the capacity);
+// a table is 16-byte aligned, the alignment of the two vector loads of each entry
+int mgw_cvt_img2train_planes(const void* src, int format, int S, int H, int W, const int32_t* kx, const int32_t* x0, const int32_t* xn,
+                             int ksx, const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h, int out_w, uint8_t* tmp,
+                             float* out, void* stream)
+{
+    TRY(validate_mixed("mgw_cvt_img2train_planes", format, S, H, W, out_h, out_w));
+    REQUIRE(ksx > 0 && ksy > 0, "mgw_cvt_img2train_planes: bad sizes (ksx=%d ksy=%d)", ksx, ksy);
+    if (S == 0) return MGW_OK;
+    REQUIRE(src && kx && x0 && xn && ky && y0 && yn && tmp && out, "mgw_cvt_img2train_planes: null pointer");
+    REQUIRE(aligned(src, 16), "mgw_cvt_img2train_planes: the planes table must be 16-byte aligned");
+    return launch_cvt_img2train_planes(static_cast<const mgw_planes*>(src), format, S, H, W, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w,
+                                       tmp, out, (cudaStream_t)stream);
+}
+
+int mgw_resize_linear_planes(const void* src, int format, int S, int H, int W, const int32_t* xtab, const int32_t* ytab, int out_h,
+                             int out_w, uint8_t* dst, void* stream)
+{
+    TRY(validate_mixed("mgw_resize_linear_planes", format, S, H, W, out_h, out_w));
+    if (S == 0) return MGW_OK;
+    REQUIRE(src && dst, "mgw_resize_linear_planes: null pointer");
+    REQUIRE((W == 2 * out_w && H == 2 * out_h) || (xtab && ytab), "mgw_resize_linear_planes: coefficient tables are required");
+    REQUIRE((!xtab || aligned(xtab, 16)) && (!ytab || aligned(ytab, 16)), "mgw_resize_linear_planes: tables must be 16-byte aligned");
+    REQUIRE(aligned(src, 16), "mgw_resize_linear_planes: the planes table must be 16-byte aligned");
+    return launch_resize_linear_planes(static_cast<const mgw_planes*>(src), format, S, H, W, xtab, ytab, out_h, out_w, dst,
+                                       (cudaStream_t)stream);
+}
+
+// mgw_remap_bundle_frame_mixed's checks at the frame size: H and W even when either format is YUV
+int mgw_remap_bundle_frame_planes(const void* src, int format, const float* xy, int S, int h, int w, int H, int W, const void* dst,
+                                  int dst_format, void* workspace, void* stream)
+{
+    const auto known = [](int f) { return f == MGW_BGR24 || f == MGW_YUV420_NV12 || f == MGW_YUV420_I420; };
+    REQUIRE(known(format), "mgw_remap_bundle_frame_planes: unknown format %d", format);
+    REQUIRE(known(dst_format), "mgw_remap_bundle_frame_planes: unknown destination format %d", dst_format);
+    REQUIRE(S >= 0 && S <= 65535 && h >= 8 && w >= 8 && H >= 1 && W >= 1 && H <= 32767 && W <= 32767 &&
+            ((format == MGW_BGR24 && dst_format == MGW_BGR24) || (H % 2 == 0 && W % 2 == 0)) &&
+            (long long)S * H * W * 3 < (1LL << 31) && (long long)S * h * w < (1LL << 31),
+            "mgw_remap_bundle_frame_planes: bad sizes (S=%d maps %dx%d frame %dx%d; h, w >= 8, H and W even for YUV)", S, h, w, H, W);
+    if (S == 0) return MGW_OK;
+    REQUIRE(src && xy && dst && workspace, "mgw_remap_bundle_frame_planes: null pointer");
+    REQUIRE(aligned(src, 16) && aligned(dst, 16), "mgw_remap_bundle_frame_planes: the planes tables must be 16-byte aligned");
+    REQUIRE(aligned(xy, 8) && aligned(workspace, 8), "mgw_remap_bundle_frame_planes: xy and workspace must be 8-byte aligned");
+    return launch_remap_bundle_planes(static_cast<const mgw_planes*>(src), format, xy, S, h, w, H, W, static_cast<const mgw_planes*>(dst),
+                                      dst_format, workspace, (cudaStream_t)stream);
+}
+
 static int validate_streams(const char* fn, int S, int depth, int H, int W, int nch)
 {
     REQUIRE(S >= 0 && S <= 65535 && depth > 0 && H > 0 && W > 0 && (long long)S * depth * H * W < (1LL << 31) &&

@@ -119,6 +119,58 @@ __device__ __forceinline__ bool slot_active(int2 sz, int max_h, int max_w)
     return sz.x > 0 && sz.y > 0 && sz.x <= max_h && sz.y <= max_w && (FMT == SRC_BGR || ((sz.x | sz.y) & 1) == 0);
 }
 
+// Per-slot planes (PLANES kernels): slot s's frame is described by entry s of a table of mgw_planes in device memory, each plane
+// at its own address with its own row pitch, row r of plane k at p[k] + (size_t)r * pitch[k].  Block (., s) loads the entry once
+// -- two 16-byte loads, a third for I420's V plane -- and the slot is idle (its blocks return before they write anything) when a
+// plane FMT uses is 0 or its pitch is below that plane's row bytes at the frame size H x W: a bad device-side entry cannot move an
+// access past the rows it describes.
+struct Planes { uint8_t* p[3]; size_t pitch[3]; };
+
+template <int FMT>
+__device__ __forceinline__ bool load_planes(const mgw_planes* __restrict__ tab, int s, int W, Planes& f)
+{
+    const uint4* e = reinterpret_cast<const uint4*>(tab + s);
+    const uint4 a = __ldg(e), b = __ldg(e + 1);
+    f.p[0] = reinterpret_cast<uint8_t*>(a.x | ((uint64_t)a.y << 32));
+    f.p[1] = reinterpret_cast<uint8_t*>(a.z | ((uint64_t)a.w << 32));
+    f.p[2] = reinterpret_cast<uint8_t*>(b.x | ((uint64_t)b.y << 32));
+    const int q0 = (int)b.z, q1 = (int)b.w;
+    f.pitch[0] = (size_t)(unsigned)q0; f.pitch[1] = (size_t)(unsigned)q1;
+    if constexpr (FMT == SRC_BGR) return f.p[0] && q0 >= 3 * W;
+    else if constexpr (FMT == MGW_YUV420_NV12) return f.p[0] && f.p[1] && q0 >= W && q1 >= W;
+    else {
+        const int q2 = (int)__ldg(e + 2).x;
+        f.pitch[2] = (size_t)(unsigned)q2;
+        return f.p[0] && f.p[1] && f.p[2] && q0 >= W && q1 >= (W >> 1) && q2 >= (W >> 1);
+    }
+}
+
+// yuv_chroma_at / yuv_bgr_at on pitched planes: NV12's UV rows in p[1], I420's U and V in p[1] and p[2]
+template <int FMT>
+__device__ __forceinline__ Chroma planes_chroma_at(const Planes& f, int row, int x)
+{
+    const size_t r = (size_t)(row >> 1);
+    if constexpr (FMT == MGW_YUV420_NV12) {
+        const uint8_t* p = f.p[1] + r * f.pitch[1] + (x & ~1);
+        return yuv_chroma(__ldg(p), __ldg(p + 1));
+    } else {
+        const size_t c = (size_t)(x >> 1);
+        return yuv_chroma(__ldg(f.p[1] + r * f.pitch[1] + c), __ldg(f.p[2] + r * f.pitch[2] + c));
+    }
+}
+
+// the BGR value of pixel (row, x) of a pitched source: the bytes of a BGR row, or the pixel cvtColor makes of a YUV 4:2:0 one
+template <int FMT>
+__device__ __forceinline__ int3 planes_bgr_at(const Planes& f, int row, int x)
+{
+    if constexpr (FMT == SRC_BGR) {
+        const uint8_t* p = f.p[0] + (size_t)row * f.pitch[0] + (size_t)x * 3;
+        return make_int3(__ldg(p), __ldg(p + 1), __ldg(p + 2));
+    } else {
+        return yuv_to_bgr(__ldg(f.p[0] + (size_t)row * f.pitch[0] + x), planes_chroma_at<FMT>(f, row, x));
+    }
+}
+
 // cvRound(v) as x86 does it (cvtss2si: round half to even; out of range / NaN -> INT_MIN)
 __device__ __forceinline__ int cv_round(float v)
 {
@@ -176,6 +228,25 @@ __device__ __forceinline__ void bilinear_fixed_u8(const uint8_t* __restrict__ ba
     for (int ch = 0; ch < C; ++ch) o[ch] = (uint8_t)min(max(acc[ch] >> 15, 0), 255);
 }
 
+// bilinear_fixed_u8 (C = 3) on a pitched source: the same taps, weights and order; a tap's row is addressed only when it is inside
+template <int FMT>
+__device__ __forceinline__ void bilinear_fixed_planes(const Planes& f, int H, int W, int sx, int sy, uint8_t* __restrict__ o)
+{
+    const int ix = min(max(sx >> 5, -32768), 32767), iy = min(max(sy >> 5, -32768), 32767);
+    const int fx = sx & 31, fy = sy & 31;
+    const int w00 = (32 - fx) * (32 - fy) * 32, w01 = fx * (32 - fy) * 32, w10 = (32 - fx) * fy * 32, w11 = fx * fy * 32;
+    const bool x0 = (unsigned)ix < (unsigned)W, x1 = (unsigned)(ix + 1) < (unsigned)W;
+    const bool y0 = (unsigned)iy < (unsigned)H, y1 = (unsigned)(iy + 1) < (unsigned)H;
+    int acc[3] = {1 << 14, 1 << 14, 1 << 14};
+    const auto add = [&](int w, int3 p) { acc[0] += w * p.x; acc[1] += w * p.y; acc[2] += w * p.z; };
+    if (y0 && x0) add(w00, planes_bgr_at<FMT>(f, iy, ix));
+    if (y0 && x1) add(w01, planes_bgr_at<FMT>(f, iy, ix + 1));
+    if (y1 && x0) add(w10, planes_bgr_at<FMT>(f, iy + 1, ix));
+    if (y1 && x1) add(w11, planes_bgr_at<FMT>(f, iy + 1, ix + 1));
+#pragma unroll
+    for (int ch = 0; ch < 3; ++ch) o[ch] = (uint8_t)min(max(acc[ch] >> 15, 0), 255);
+}
+
 // warpRevBundle (deploy_bundle.py:148-173): output cell (i, j) = that region of cv2.warpPerspective(img, Hs_cvt[i][j],
 // WARP_INVERSE_MAP | INTER_LINEAR).  OpenCV walks the destination in blocks of bw columns and evaluates, in double,
 //   X0 = M0*bx + M1*y + M2 (left to right), W = W0 + M6*x1, W = W ? 32/W : 0, fX = clamp((X0 + M0*x1)*W), X = cvRound(fX)
@@ -229,11 +300,56 @@ __device__ __forceinline__ void slot_scales(int H, int W, int h4, int w4, double
     xscale = sc[0]; yscale = sc[1];
 }
 
-template <int C, int FMT, bool MIXED = false>
+// pixel (c, r) of the output: its source position in 1/32 pixel from the /4 maps, as remap_up_kernel computes it
+__device__ __forceinline__ int2 remap_src_fixed(const float2* __restrict__ small, int w4, const Lin& h, const Lin& v, int H, int W)
+{
+    const float2 m = resize_sample(small, w4, h, v);
+    // (map + 1) / 2 * size in fp32 (deploy_bundle.py:142-143)
+    const float xp = __fmul_rn(__fmul_rn(__fadd_rn(m.x, 1.0f), 0.5f), (float)W);
+    const float yp = __fmul_rn(__fmul_rn(__fadd_rn(m.y, 1.0f), 0.5f), (float)H);
+    return make_int2(cv_round(__fmul_rn(xp, 32.0f)), cv_round(__fmul_rn(yp, 32.0f)));
+}
+
+// PLANES (C = 3): the source frame and the BGR result are slot blockIdx.y's entries of the tables sp (FMT) and dp (BGR), src and dst
+// unused.  A pitched row cannot be continued by the next one, so the threads are laid out over rows x ceil(W / REMAP_RUN) column
+// groups, as in remap_up_yuv_kernel: each stores the 3 * REMAP_RUN bytes of its group (fewer at the row's end) as 3 words where the
+// address is aligned and byte by byte otherwise.
+template <int C, int FMT, bool MIXED = false, bool PLANES = false>
 __global__ void __launch_bounds__(256)
 remap_up_kernel(const uint8_t* __restrict__ src, const float2* __restrict__ small, int H, int W, int h4, int w4, double xscale,
-                double yscale, uint8_t* __restrict__ dst, const int2* __restrict__ sizes)
+                double yscale, uint8_t* __restrict__ dst, const int2* __restrict__ sizes, const mgw_planes* __restrict__ sp,
+                const mgw_planes* __restrict__ dp)
 {
+    if constexpr (PLANES) {
+        static_assert(C == 3 && !MIXED, "a table's slot is a colour frame of the batch's size");
+        Planes f, d;
+        if (!load_planes<FMT>(sp, blockIdx.y, W, f) || !load_planes<SRC_BGR>(dp, blockIdx.y, W, d)) return;
+        const int gw = (W + REMAP_RUN - 1) / REMAP_RUN;
+        const int t = blockIdx.x * blockDim.x + threadIdx.x;
+        if (t >= H * gw) return;
+        const int r = t / gw, c0 = (t - r * gw) * REMAP_RUN, ncol = min(REMAP_RUN, W - c0);
+        small += (size_t)blockIdx.y * h4 * w4;
+        const Lin v = vcoef_at(src_pos_s(r, yscale), h4);
+        uint8_t px[REMAP_RUN * 3];
+#pragma unroll
+        for (int k = 0; k < REMAP_RUN; ++k) {
+            // past the row's end (c0 + k >= W) the pixel is computed as any other and not stored
+            const int2 q = remap_src_fixed(small, w4, hcoef_at(src_pos_s(c0 + k, xscale), w4), v, H, W);
+            bilinear_fixed_planes<FMT>(f, H, W, q.x, q.y, px + k * 3);
+        }
+        uint8_t* o = d.p[0] + (size_t)r * d.pitch[0] + (size_t)c0 * 3;
+        if (ncol == REMAP_RUN && (reinterpret_cast<uintptr_t>(o) & 3) == 0) {
+#pragma unroll
+            for (int q = 0; q < 3; ++q)
+                reinterpret_cast<uint32_t*>(o)[q] = (uint32_t)px[4 * q] | ((uint32_t)px[4 * q + 1] << 8) | ((uint32_t)px[4 * q + 2] << 16) |
+                                                    ((uint32_t)px[4 * q + 3] << 24);
+        } else {
+#pragma unroll
+            for (int i = 0; i < REMAP_RUN * 3; ++i)
+                if (i < ncol * 3) o[i] = px[i];
+        }
+        return;
+    }
     if constexpr (MIXED) {
         static_assert(C == 3, "a slot's result is BGR");
         const int2 sz = __ldg(sizes + blockIdx.y);
@@ -289,7 +405,7 @@ int launch_remap_up(const uint8_t* src, const float2* small, int N, int H, int W
         const int n = min(N - n0, 65535);
         remap_up_kernel<C, FMT><<<dim3(gx, n), 256, 0, st>>>(src + (size_t)n0 * (FMT == SRC_BGR ? (size_t)H * W * C : (size_t)H * W * 3 / 2),
                                                              small + (size_t)n0 * h4 * w4, H, W, h4, w4, xscale, yscale,
-                                                             dst + (size_t)n0 * H * W * C, nullptr);
+                                                             dst + (size_t)n0 * H * W * C, nullptr, nullptr, nullptr);
         if (int rc = check_launch("remap_up")) return rc;
     }
     return MGW_OK;
@@ -330,14 +446,22 @@ __device__ __forceinline__ void store_run(uint8_t* o, const uint8_t* b, int n)
 // not a multiple of 4 the last block of a row is 2 columns wide).  Every pixel's BGR value is remap_up_kernel's, by the same
 // device functions; the column coefficients are shared by the two rows.  The thread writes the block's Y bytes and the U, V of
 // its two (or one) 2x2 chroma blocks, so the BGR frame never reaches memory.  MIXED: as remap_up_kernel, with a YUV result region
-// of 3H/2*W bytes per slot; a slot of odd size is idle.
+// of 3H/2*W bytes per slot; a slot of odd size is idle.  PLANES: the source and the result are slot blockIdx.y's entries of the
+// tables sp (SRC_FMT) and dp (DST_FMT), src and dst unused; the same threads and arithmetic, pitched loads and stores.
 constexpr int YUV_RUN = 4;
 
-template <int SRC_FMT, int DST_FMT, bool MIXED = false>
+template <int SRC_FMT, int DST_FMT, bool MIXED = false, bool PLANES = false>
 __global__ void __launch_bounds__(256)
 remap_up_yuv_kernel(const uint8_t* __restrict__ src, const float2* __restrict__ small, int H, int W, int h4, int w4, double xscale,
-                    double yscale, uint8_t* __restrict__ dst, const int2* __restrict__ sizes)
+                    double yscale, uint8_t* __restrict__ dst, const int2* __restrict__ sizes, const mgw_planes* __restrict__ sp,
+                    const mgw_planes* __restrict__ dp)
 {
+    [[maybe_unused]] Planes sf, df;
+    if constexpr (PLANES) {
+        static_assert(!MIXED, "a table's slot is a frame of the batch's size");
+        if (!load_planes<SRC_FMT>(sp, blockIdx.y, W, sf) || !load_planes<DST_FMT>(dp, blockIdx.y, W, df)) return;
+        small += (size_t)blockIdx.y * h4 * w4;
+    }
     if constexpr (MIXED) {
         const int2 sz = __ldg(sizes + blockIdx.y);
         // the result is 4:2:0, so every active slot is even (DST_FMT's rule covers an odd size from a BGR source)
@@ -353,7 +477,7 @@ remap_up_yuv_kernel(const uint8_t* __restrict__ src, const float2* __restrict__ 
     if (t >= (H >> 1) * gw) return;
     const int r = (t / gw) * 2, c0 = (t % gw) * YUV_RUN;
     const int ncol = min(YUV_RUN, W - c0);
-    const size_t n = MIXED ? 0 : blockIdx.y;
+    const size_t n = (MIXED || PLANES) ? 0 : blockIdx.y;
     const uint8_t* f = src + n * src_frame_bytes<SRC_FMT>(H, W);
     small += n * h4 * w4;
     uint8_t* y = dst + n * ((size_t)H * W * 3 / 2);
@@ -372,10 +496,24 @@ remap_up_yuv_kernel(const uint8_t* __restrict__ src, const float2* __restrict__ 
             const float yp = __fmul_rn(__fmul_rn(__fadd_rn(m.y, 1.0f), 0.5f), (float)H);
             const int sx = cv_round(__fmul_rn(xp, 32.0f)), sy = cv_round(__fmul_rn(yp, 32.0f));
             uint8_t px[3];
-            bilinear_fixed_u8<3, SRC_FMT>(f, H, W, sx, sy, px);
+            if constexpr (PLANES) bilinear_fixed_planes<SRC_FMT>(sf, H, W, sx, sy, px);
+            else bilinear_fixed_u8<3, SRC_FMT>(f, H, W, sx, sy, px);
             ys[i][k] = (uint8_t)bgr_y(px);
             if (i == 0 && (k & 1) == 0) { us[k >> 1] = (uint8_t)bgr_u(px); vs[k >> 1] = (uint8_t)bgr_v(px); }
         }
+    }
+    if constexpr (PLANES) {
+        store_run(df.p[0] + (size_t)r * df.pitch[0] + c0, ys[0], ncol);
+        store_run(df.p[0] + (size_t)(r + 1) * df.pitch[0] + c0, ys[1], ncol);
+        const size_t cr = (size_t)(r >> 1);
+        if constexpr (DST_FMT == MGW_YUV420_NV12) {
+            const uint8_t b[YUV_RUN] = {us[0], vs[0], us[1], vs[1]};
+            store_run(df.p[1] + cr * df.pitch[1] + c0, b, ncol);
+        } else {
+            store_run(df.p[1] + cr * df.pitch[1] + (c0 >> 1), us, ncol >> 1);
+            store_run(df.p[2] + cr * df.pitch[2] + (c0 >> 1), vs, ncol >> 1);
+        }
+        return;
     }
     store_run(y + (size_t)r * W + c0, ys[0], ncol);
     store_run(y + (size_t)(r + 1) * W + c0, ys[1], ncol);
@@ -394,7 +532,7 @@ int launch_remap_up_yuv(const uint8_t* src, const float2* small, int N, int H, i
 {
     const long long threads = (long long)(H / 2) * ((W + YUV_RUN - 1) / YUV_RUN);
     remap_up_yuv_kernel<SRC_FMT, DST_FMT><<<dim3((unsigned)((threads + 255) / 256), N), 256, 0, st>>>(
-        src, small, H, W, h4, w4, resize_scale(W, w4), resize_scale(H, h4), dst, nullptr);
+        src, small, H, W, h4, w4, resize_scale(W, w4), resize_scale(H, h4), dst, nullptr, nullptr, nullptr);
     return check_launch("remap_up_yuv");
 }
 
@@ -405,19 +543,49 @@ int launch_remap_up_mixed(int dst_fmt, const uint8_t* src, const float2* small, 
 {
     if (dst_fmt == SRC_BGR) {
         const unsigned gx = (unsigned)((((long long)max_h * max_w + REMAP_RUN - 1) / REMAP_RUN + 255) / 256);
-        remap_up_kernel<3, SRC_FMT, true><<<dim3(gx, S), 256, 0, st>>>(src, small, max_h, max_w, h4, w4, 0.0, 0.0, dst, sizes);
+        remap_up_kernel<3, SRC_FMT, true><<<dim3(gx, S), 256, 0, st>>>(src, small, max_h, max_w, h4, w4, 0.0, 0.0, dst, sizes, nullptr,
+                                                                       nullptr);
         return check_launch("remap_up");
     }
     const long long threads = (long long)(max_h / 2) * ((max_w + YUV_RUN - 1) / YUV_RUN);
     const dim3 grid((unsigned)((threads + 255) / 256), S);
     switch (dst_fmt) {
     case MGW_YUV420_NV12:
-        remap_up_yuv_kernel<SRC_FMT, MGW_YUV420_NV12, true><<<grid, 256, 0, st>>>(src, small, max_h, max_w, h4, w4, 0.0, 0.0, dst, sizes);
+        remap_up_yuv_kernel<SRC_FMT, MGW_YUV420_NV12, true><<<grid, 256, 0, st>>>(src, small, max_h, max_w, h4, w4, 0.0, 0.0, dst, sizes,
+                                                                                  nullptr, nullptr);
         break;
     case MGW_YUV420_I420:
-        remap_up_yuv_kernel<SRC_FMT, MGW_YUV420_I420, true><<<grid, 256, 0, st>>>(src, small, max_h, max_w, h4, w4, 0.0, 0.0, dst, sizes);
+        remap_up_yuv_kernel<SRC_FMT, MGW_YUV420_I420, true><<<grid, 256, 0, st>>>(src, small, max_h, max_w, h4, w4, 0.0, 0.0, dst, sizes,
+                                                                                  nullptr, nullptr);
         break;
     default: return set_error(MGW_ERR_INVALID, "remap_bundle_frame_mixed: unknown destination format %d", dst_fmt);
+    }
+    return check_launch("remap_up_yuv");
+}
+
+// K5b between two tables of planes (S slots of one size H x W): BGR results over rows x column groups, YUV ones over row pairs
+template <int SRC_FMT>
+int launch_remap_up_planes(int dst_fmt, const mgw_planes* sp, const float2* small, int S, int H, int W, int h4, int w4,
+                           const mgw_planes* dp, cudaStream_t st)
+{
+    const double xscale = resize_scale(W, w4), yscale = resize_scale(H, h4);
+    const long long groups = (W + REMAP_RUN - 1) / REMAP_RUN;
+    if (dst_fmt == SRC_BGR) {
+        const dim3 grid((unsigned)(((long long)H * groups + 255) / 256), S);
+        remap_up_kernel<3, SRC_FMT, false, true><<<grid, 256, 0, st>>>(nullptr, small, H, W, h4, w4, xscale, yscale, nullptr, nullptr, sp, dp);
+        return check_launch("remap_up");
+    }
+    const dim3 grid((unsigned)(((long long)(H / 2) * ((W + YUV_RUN - 1) / YUV_RUN) + 255) / 256), S);
+    switch (dst_fmt) {
+    case MGW_YUV420_NV12:
+        remap_up_yuv_kernel<SRC_FMT, MGW_YUV420_NV12, false, true><<<grid, 256, 0, st>>>(nullptr, small, H, W, h4, w4, xscale, yscale, nullptr,
+                                                                                         nullptr, sp, dp);
+        break;
+    case MGW_YUV420_I420:
+        remap_up_yuv_kernel<SRC_FMT, MGW_YUV420_I420, false, true><<<grid, 256, 0, st>>>(nullptr, small, H, W, h4, w4, xscale, yscale, nullptr,
+                                                                                         nullptr, sp, dp);
+        break;
+    default: return set_error(MGW_ERR_INVALID, "remap_bundle_frame_planes: unknown destination format %d", dst_fmt);
     }
     return check_launch("remap_up_yuv");
 }
@@ -505,6 +673,21 @@ int launch_remap_bundle_mixed(const uint8_t* src, int src_fmt, int S, int max_h,
     }
 }
 
+// the same K5a, then K5b from the source table's planes into the destination table's
+int launch_remap_bundle_planes(const mgw_planes* src, int src_fmt, const float* xy, int S, int h, int w, int H, int W,
+                               const mgw_planes* dst, int dst_fmt, void* workspace, cudaStream_t st)
+{
+    const int h4 = h / 4, w4 = w / 4;
+    float2* small = launch_maps_down(xy, S, h, w, workspace, st);
+    if (int rc = check_launch("maps_down")) return rc;
+    switch (src_fmt) {
+    case SRC_BGR: return launch_remap_up_planes<SRC_BGR>(dst_fmt, src, small, S, H, W, h4, w4, dst, st);
+    case MGW_YUV420_NV12: return launch_remap_up_planes<MGW_YUV420_NV12>(dst_fmt, src, small, S, H, W, h4, w4, dst, st);
+    case MGW_YUV420_I420: return launch_remap_up_planes<MGW_YUV420_I420>(dst_fmt, src, small, S, H, W, h4, w4, dst, st);
+    default: return set_error(MGW_ERR_INVALID, "remap_bundle_frame_planes: unknown source format %d", src_fmt);
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // Exact-bytes transfer of a pool of per-slot frames (MIXED): slot s's frame_bytes(sizes[s]) bytes from src + s * stride to
 // dst + s * stride, stride = frame_bytes(max_h, max_w); nothing past them is read or written, and an idle slot (the MIXED rule)
@@ -581,14 +764,46 @@ int launch_copy_slots_mixed(const uint8_t* src, uint8_t* dst, int fmt, int S, in
 // [s * frame_bytes(H, W), +frame_bytes(H, W)) of the source and its frame of size sizes[s] lies at the start of it, and the slot
 // has its own tables (kx [S,out_w,ks], ...) and tmp rows [S,H,out_w].  Block (., s) reads sizes[s] once, offsets its pointers to
 // the slot, and then runs the per-pixel code of the uniform batch at the slot's size with frame index 0.
+// PLANES = per-slot planes (a uniform batch whose frames lie wherever a decoder put them): slot s's source is entry s of the table
+// `planes` (see load_planes), bgr is unused; the tables, tmp and out are the uniform batch's, and an idle slot writes no row of either.
 namespace {
 
-template <int FMT, bool MIXED = false>
+template <int FMT, bool MIXED = false, bool PLANES = false>
 __global__ void __launch_bounds__(256)
 gray_hpass_kernel(const uint8_t* __restrict__ bgr, int H, int W, const int32_t* __restrict__ kx, const int32_t* __restrict__ x0,
-                  const int32_t* __restrict__ xn, int ks, int out_w, uint8_t* __restrict__ tmp, const int2* __restrict__ sizes)
+                  const int32_t* __restrict__ xn, int ks, int out_w, uint8_t* __restrict__ tmp, const int2* __restrict__ sizes,
+                  const mgw_planes* __restrict__ planes)
 {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if constexpr (PLANES) {
+        static_assert(!MIXED, "a table's slot is a frame of the batch's size");
+        Planes f;
+        if (!load_planes<FMT>(planes, blockIdx.y, W, f)) return;
+        if (t >= H * out_w) return;
+        tmp += (size_t)blockIdx.y * H * out_w;
+        const int xx = t % out_w, row = t / out_w;
+        const int n = __ldg(xn + xx), xs = __ldg(x0 + xx);
+        int acc = 1 << 21;
+        if constexpr (FMT == SRC_BGR) {
+            const uint8_t* p = f.p[0] + (size_t)row * f.pitch[0] + (size_t)xs * 3;
+            for (int k = 0; k < n; ++k, p += 3) {
+                const int g = ((int)__ldg(p) * 3735 + (int)__ldg(p + 1) * 19235 + (int)__ldg(p + 2) * 9798 + (1 << 14)) >> 15;
+                acc += g * __ldg(kx + (size_t)xx * ks + k);
+            }
+        } else {
+            const uint8_t* py = f.p[0] + (size_t)row * f.pitch[0] + xs;
+            Chroma c;
+#pragma unroll 1
+            for (int k = 0; k < n; ++k) {
+                if (k == 0 || ((xs + k) & 1) == 0) c = planes_chroma_at<FMT>(f, row, xs + k);
+                const int3 p = yuv_to_bgr(__ldg(py + k), c);
+                const int g = (p.x * 3735 + p.y * 19235 + p.z * 9798 + (1 << 14)) >> 15;
+                acc += g * __ldg(kx + (size_t)xx * ks + k);
+            }
+        }
+        tmp[t] = (uint8_t)min(max(acc >> 22, 0), 255);
+        return;
+    }
     if constexpr (MIXED) {
         const int2 sz = __ldg(sizes + blockIdx.y);
         if (!slot_active<FMT>(sz, H, W)) return;
@@ -631,12 +846,18 @@ gray_hpass_kernel(const uint8_t* __restrict__ bgr, int H, int W, const int32_t* 
 }
 
 // MIXED: H is the capacity's height (the tmp rows of a slot), max_w its width; the slot's rows of ky / y0 / yn
-template <int FMT = SRC_BGR, bool MIXED = false>
+// PLANES: max_w is the source width; a slot that gray_hpass found idle is skipped by the same rule
+template <int FMT = SRC_BGR, bool MIXED = false, bool PLANES = false>
 __global__ void __launch_bounds__(256)
 vpass_norm_kernel(const uint8_t* __restrict__ tmp, int H, int out_w, const int32_t* __restrict__ ky, const int32_t* __restrict__ y0,
-                  const int32_t* __restrict__ yn, int ks, int out_h, float* __restrict__ out, const int2* __restrict__ sizes, int max_w)
+                  const int32_t* __restrict__ yn, int ks, int out_h, float* __restrict__ out, const int2* __restrict__ sizes, int max_w,
+                  const mgw_planes* __restrict__ planes)
 {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if constexpr (PLANES) {
+        Planes f;
+        if (!load_planes<FMT>(planes, blockIdx.y, max_w, f)) return;
+    }
     if constexpr (MIXED) {
         if (!slot_active<FMT>(__ldg(sizes + blockIdx.y), H, max_w)) return;
         ky += (size_t)blockIdx.y * out_h * ks;
@@ -664,14 +885,41 @@ int launch_cvt_img2train_u8(const uint8_t* bgr, int S, int H, int W, const int32
 {
     const dim3 g1((H * out_w + 255) / 256, S);
     switch (src_fmt) {
-    case SRC_BGR: gray_hpass_kernel<SRC_BGR><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp, nullptr); break;
-    case MGW_YUV420_NV12: gray_hpass_kernel<MGW_YUV420_NV12><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp, nullptr); break;
-    case MGW_YUV420_I420: gray_hpass_kernel<MGW_YUV420_I420><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp, nullptr); break;
+    case SRC_BGR: gray_hpass_kernel<SRC_BGR><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp, nullptr, nullptr); break;
+    case MGW_YUV420_NV12:
+        gray_hpass_kernel<MGW_YUV420_NV12><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp, nullptr, nullptr); break;
+    case MGW_YUV420_I420:
+        gray_hpass_kernel<MGW_YUV420_I420><<<g1, 256, 0, st>>>(bgr, H, W, kx, x0, xn, ksx, out_w, tmp, nullptr, nullptr); break;
     default: return set_error(MGW_ERR_INVALID, "cvt_img2train: unknown source format %d", src_fmt);
     }
     if (int rc = check_launch("gray_hpass")) return rc;
-    vpass_norm_kernel<<<dim3((out_h * out_w + 255) / 256, S), 256, 0, st>>>(tmp, H, out_w, ky, y0, yn, ksy, out_h, out, nullptr, 0);
+    vpass_norm_kernel<<<dim3((out_h * out_w + 255) / 256, S), 256, 0, st>>>(tmp, H, out_w, ky, y0, yn, ksy, out_h, out, nullptr, 0, nullptr);
     return check_launch("vpass_norm");
+}
+
+template <int FMT>
+static int cvt_planes(const mgw_planes* src, int S, int H, int W, const int32_t* kx, const int32_t* x0, const int32_t* xn, int ksx,
+                      const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h, int out_w, uint8_t* tmp, float* out,
+                      cudaStream_t st)
+{
+    gray_hpass_kernel<FMT, false, true><<<dim3((H * out_w + 255) / 256, S), 256, 0, st>>>(nullptr, H, W, kx, x0, xn, ksx, out_w, tmp,
+                                                                                        nullptr, src);
+    if (int rc = check_launch("gray_hpass")) return rc;
+    vpass_norm_kernel<FMT, false, true><<<dim3((out_h * out_w + 255) / 256, S), 256, 0, st>>>(tmp, H, out_w, ky, y0, yn, ksy, out_h, out,
+                                                                                            nullptr, W, src);
+    return check_launch("vpass_norm");
+}
+
+int launch_cvt_img2train_planes(const mgw_planes* src, int src_fmt, int S, int H, int W, const int32_t* kx, const int32_t* x0,
+                                const int32_t* xn, int ksx, const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h,
+                                int out_w, uint8_t* tmp, float* out, cudaStream_t st)
+{
+    switch (src_fmt) {
+    case SRC_BGR: return cvt_planes<SRC_BGR>(src, S, H, W, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w, tmp, out, st);
+    case MGW_YUV420_NV12: return cvt_planes<MGW_YUV420_NV12>(src, S, H, W, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w, tmp, out, st);
+    case MGW_YUV420_I420: return cvt_planes<MGW_YUV420_I420>(src, S, H, W, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w, tmp, out, st);
+    default: return set_error(MGW_ERR_INVALID, "cvt_img2train_planes: unknown source format %d", src_fmt);
+    }
 }
 
 template <int FMT>
@@ -679,10 +927,11 @@ static int cvt_mixed(const uint8_t* src, int S, int max_h, int max_w, const int2
                      const int32_t* xn, int ksx, const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h, int out_w,
                      uint8_t* tmp, float* out, cudaStream_t st)
 {
-    gray_hpass_kernel<FMT, true><<<dim3((max_h * out_w + 255) / 256, S), 256, 0, st>>>(src, max_h, max_w, kx, x0, xn, ksx, out_w, tmp, sizes);
+    gray_hpass_kernel<FMT, true><<<dim3((max_h * out_w + 255) / 256, S), 256, 0, st>>>(src, max_h, max_w, kx, x0, xn, ksx, out_w, tmp, sizes,
+                                                                                      nullptr);
     if (int rc = check_launch("gray_hpass")) return rc;
     vpass_norm_kernel<FMT, true><<<dim3((out_h * out_w + 255) / 256, S), 256, 0, st>>>(tmp, max_h, out_w, ky, y0, yn, ksy, out_h, out,
-                                                                                      sizes, max_w);
+                                                                                      sizes, max_w, nullptr);
     return check_launch("vpass_norm");
 }
 
@@ -709,13 +958,50 @@ namespace {
 __device__ __forceinline__ int ch_of(const int3& p, int ch) { return ch == 0 ? p.x : (ch == 1 ? p.y : p.z); }
 
 // MIXED: H, W are the capacity (see cvt_img2train above); xtab [S,out_w], ytab [S,out_h]; the 2x2 shortcut is the slot's own
-template <int C, int FMT = SRC_BGR, bool MIXED = false>
+// PLANES: slot s's source is entry s of the table `planes` (img unused), the uniform tables and dst; an idle slot writes nothing
+template <int C, int FMT = SRC_BGR, bool MIXED = false, bool PLANES = false>
 __global__ void __launch_bounds__(256)
 resize_u8_kernel(const uint8_t* __restrict__ img, int H, int W, const int4* __restrict__ xtab, const int4* __restrict__ ytab,
-                 int out_h, int out_w, int area2, uint8_t* __restrict__ dst, const int2* __restrict__ sizes)
+                 int out_h, int out_w, int area2, uint8_t* __restrict__ dst, const int2* __restrict__ sizes,
+                 const mgw_planes* __restrict__ planes)
 {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= out_h * out_w) return;
+    if constexpr (PLANES) {
+        static_assert(C == 3 && !MIXED, "a table's slot is a colour frame of the batch's size");
+        Planes f;
+        if (!load_planes<FMT>(planes, blockIdx.y, W, f)) return;
+        const int x = t % out_w, y = t / out_w;
+        uint8_t* o = dst + ((size_t)blockIdx.y * out_h * out_w + t) * 3;
+        int3 p00, p01, p10, p11;
+        if (area2) {
+            if constexpr (FMT == SRC_BGR) {
+                p00 = planes_bgr_at<FMT>(f, 2 * y, 2 * x); p01 = planes_bgr_at<FMT>(f, 2 * y, 2 * x + 1);
+                p10 = planes_bgr_at<FMT>(f, 2 * y + 1, 2 * x); p11 = planes_bgr_at<FMT>(f, 2 * y + 1, 2 * x + 1);
+            } else {
+                // the 2x2 block starts at even coordinates: four Y samples, one chroma sample
+                const uint8_t* py = f.p[0] + (size_t)(2 * y) * f.pitch[0] + 2 * x;
+                const Chroma c = planes_chroma_at<FMT>(f, 2 * y, 2 * x);
+                p00 = yuv_to_bgr(__ldg(py), c); p01 = yuv_to_bgr(__ldg(py + 1), c);
+                p10 = yuv_to_bgr(__ldg(py + f.pitch[0]), c); p11 = yuv_to_bgr(__ldg(py + f.pitch[0] + 1), c);
+            }
+            o[0] = (uint8_t)((p00.x + p01.x + p10.x + p11.x + 2) >> 2);
+            o[1] = (uint8_t)((p00.y + p01.y + p10.y + p11.y + 2) >> 2);
+            o[2] = (uint8_t)((p00.z + p01.z + p10.z + p11.z + 2) >> 2);
+            return;
+        }
+        const int4 xt = __ldg(xtab + x), yt = __ldg(ytab + y);        // {i0, i1, a0, a1}
+        p00 = planes_bgr_at<FMT>(f, yt.x, xt.x); p01 = planes_bgr_at<FMT>(f, yt.x, xt.y);
+        p10 = planes_bgr_at<FMT>(f, yt.y, xt.x); p11 = planes_bgr_at<FMT>(f, yt.y, xt.y);
+#pragma unroll
+        for (int ch = 0; ch < 3; ++ch) {
+            const int h0 = ch_of(p00, ch) * xt.z + ch_of(p01, ch) * xt.w;
+            const int h1 = ch_of(p10, ch) * xt.z + ch_of(p11, ch) * xt.w;
+            const int v = (((yt.z * (h0 >> 4)) >> 16) + ((yt.w * (h1 >> 4)) >> 16) + 2) >> 2;
+            o[ch] = (uint8_t)min(max(v, 0), 255);
+        }
+        return;
+    }
     if constexpr (MIXED) {
         static_assert(C == 3, "a slot's frame is BGR or YUV 4:2:0");
         const int2 sz = __ldg(sizes + blockIdx.y);
@@ -793,17 +1079,40 @@ int launch_resize_linear_u8(const uint8_t* img, int S, int H, int W, int C, cons
     if (src_fmt != SRC_BGR) {
         if (C != 3) return set_error(MGW_ERR_UNSUPPORTED, "resize_linear_u8: a YUV 4:2:0 source gives C = 3 (got %d)", C);
         switch (src_fmt) {
-        case MGW_YUV420_NV12: resize_u8_kernel<3, MGW_YUV420_NV12><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr); break;
-        case MGW_YUV420_I420: resize_u8_kernel<3, MGW_YUV420_I420><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr); break;
+        case MGW_YUV420_NV12:
+            resize_u8_kernel<3, MGW_YUV420_NV12><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr, nullptr); break;
+        case MGW_YUV420_I420:
+            resize_u8_kernel<3, MGW_YUV420_I420><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr, nullptr); break;
         default: return set_error(MGW_ERR_INVALID, "resize_linear_u8: unknown source format %d", src_fmt);
         }
         return check_launch("resize_u8");
     }
     switch (C) {
-    case 1: resize_u8_kernel<1><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr); break;
-    case 3: resize_u8_kernel<3><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr); break;
-    case 4: resize_u8_kernel<4><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr); break;
+    case 1: resize_u8_kernel<1><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr, nullptr); break;
+    case 3: resize_u8_kernel<3><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr, nullptr); break;
+    case 4: resize_u8_kernel<4><<<grid, 256, 0, st>>>(img, H, W, xt, yt, out_h, out_w, area2, dst, nullptr, nullptr); break;
     default: return set_error(MGW_ERR_UNSUPPORTED, "resize_linear_u8: C must be 1, 3 or 4 (got %d)", C);
+    }
+    return check_launch("resize_u8");
+}
+
+int launch_resize_linear_planes(const mgw_planes* src, int src_fmt, int S, int H, int W, const int32_t* xtab, const int32_t* ytab,
+                                int out_h, int out_w, uint8_t* dst, cudaStream_t st)
+{
+    const int area2 = (W == 2 * out_w && H == 2 * out_h) ? 1 : 0;
+    const dim3 grid((out_h * out_w + 255) / 256, S);
+    const int4* xt = reinterpret_cast<const int4*>(xtab);
+    const int4* yt = reinterpret_cast<const int4*>(ytab);
+    switch (src_fmt) {
+    case SRC_BGR:
+        resize_u8_kernel<3, SRC_BGR, false, true><<<grid, 256, 0, st>>>(nullptr, H, W, xt, yt, out_h, out_w, area2, dst, nullptr, src); break;
+    case MGW_YUV420_NV12:
+        resize_u8_kernel<3, MGW_YUV420_NV12, false, true><<<grid, 256, 0, st>>>(nullptr, H, W, xt, yt, out_h, out_w, area2, dst, nullptr, src);
+        break;
+    case MGW_YUV420_I420:
+        resize_u8_kernel<3, MGW_YUV420_I420, false, true><<<grid, 256, 0, st>>>(nullptr, H, W, xt, yt, out_h, out_w, area2, dst, nullptr, src);
+        break;
+    default: return set_error(MGW_ERR_INVALID, "resize_linear_planes: unknown source format %d", src_fmt);
     }
     return check_launch("resize_u8");
 }
@@ -816,11 +1125,11 @@ int launch_resize_linear_mixed(const uint8_t* src, int src_fmt, int S, int max_h
     const int4* xt = reinterpret_cast<const int4*>(xtab);
     const int4* yt = reinterpret_cast<const int4*>(ytab);
     switch (src_fmt) {
-    case SRC_BGR: resize_u8_kernel<3, SRC_BGR, true><<<grid, 256, 0, st>>>(src, max_h, max_w, xt, yt, out_h, out_w, 0, dst, sz); break;
+    case SRC_BGR: resize_u8_kernel<3, SRC_BGR, true><<<grid, 256, 0, st>>>(src, max_h, max_w, xt, yt, out_h, out_w, 0, dst, sz, nullptr); break;
     case MGW_YUV420_NV12:
-        resize_u8_kernel<3, MGW_YUV420_NV12, true><<<grid, 256, 0, st>>>(src, max_h, max_w, xt, yt, out_h, out_w, 0, dst, sz); break;
+        resize_u8_kernel<3, MGW_YUV420_NV12, true><<<grid, 256, 0, st>>>(src, max_h, max_w, xt, yt, out_h, out_w, 0, dst, sz, nullptr); break;
     case MGW_YUV420_I420:
-        resize_u8_kernel<3, MGW_YUV420_I420, true><<<grid, 256, 0, st>>>(src, max_h, max_w, xt, yt, out_h, out_w, 0, dst, sz); break;
+        resize_u8_kernel<3, MGW_YUV420_I420, true><<<grid, 256, 0, st>>>(src, max_h, max_w, xt, yt, out_h, out_w, 0, dst, sz, nullptr); break;
     default: return set_error(MGW_ERR_INVALID, "resize_linear_mixed: unknown source format %d", src_fmt);
     }
     return check_launch("resize_u8");

@@ -142,6 +142,15 @@ int launch_cvt_img2train_mixed(const uint8_t* src, int src_fmt, int S, int max_h
                                int ksy, int out_h, int out_w, uint8_t* tmp, float* out, cudaStream_t st);
 int launch_resize_linear_mixed(const uint8_t* src, int src_fmt, int S, int max_h, int max_w, const int32_t* sizes, const int32_t* xtab,
                                const int32_t* ytab, int out_h, int out_w, uint8_t* dst, cudaStream_t st);
+// per-slot planes: slot s's source frame (and, for the warp, its result) described by entry s of a device table of mgw_planes
+// (16-byte aligned); S frames of one size H x W, uniform tables; slots whose entry lacks a plane or has a short pitch write nothing
+int launch_cvt_img2train_planes(const mgw_planes* src, int src_fmt, int S, int H, int W, const int32_t* kx, const int32_t* x0,
+                                const int32_t* xn, int ksx, const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h,
+                                int out_w, uint8_t* tmp, float* out, cudaStream_t st);
+int launch_resize_linear_planes(const mgw_planes* src, int src_fmt, int S, int H, int W, const int32_t* xtab, const int32_t* ytab,
+                                int out_h, int out_w, uint8_t* dst, cudaStream_t st);
+int launch_remap_bundle_planes(const mgw_planes* src, int src_fmt, const float* xy, int S, int h, int w, int H, int W,
+                               const mgw_planes* dst, int dst_fmt, void* workspace, cudaStream_t st);
 int launch_warp_rev_bundle_u8(const uint8_t* img, const double* Hs_cvt, int N, int H, int W, int C, int gh, int gw, uint8_t* dst,
                               cudaStream_t st);
 

@@ -17,7 +17,7 @@ import torch
 from . import ops
 
 __all__ = ['warpRevBundle2', 'warpRevBundle', 'warpRev', 'cvt_theta_mat_bundle', 'cvt_img2train', 'cv2_resize', 'StreamState', 'CropState', 'StreamBatch',
-           'MixedStreamBatch', 'mixed_slot_tables', 'scale_rect']
+           'MixedStreamBatch', 'mixed_slot_tables', 'scale_rect', 'PlaneTable']
 
 
 def warpRevBundle2(img, x_map, y_map, device=None, src_format='bgr', dst_format='bgr'):
@@ -387,6 +387,125 @@ class CropState:
         return frame[..., t:b + 1, l:r + 1, :]
 
 
+_PLANES_DTYPE = np.dtype([('plane', '<u8', (3,)), ('pitch', '<i4', (3,)), ('reserved', '<i4', (3,))])     # mgw_planes, 48 bytes
+
+
+def _plane_rows(fmt, H, W):
+    """(rows, row bytes) of each plane of an H x W frame in fmt"""
+    if fmt == 'bgr':
+        return [(H, 3 * W)]
+    if fmt == 'nv12':
+        return [(H, W), (H // 2, W)]
+    return [(H, W), (H // 2, W // 2), (H // 2, W // 2)]
+
+
+class PlaneTable:
+    """Where the S frames of a batch of one size lie: per slot the device address and row pitch of each plane, as a decoder or an
+    encoder hands its surfaces out.  A pinned host mirror (host, int64 [S,6], one include/mgw.h mgw_planes per row) that set() /
+    clear() edit, and the device table (device) that the plane-table calls read, refreshed by upload().
+
+        src = PlaneTable(S, 'nv12', (1080, 1920))
+        src.set(0, (y_plane, uv_plane))                 # pitched uint8 CUDA views: [1080,>=1920] and [540,>=1920]
+        src.set(1, ((y_addr, pitch), (uv_addr, pitch))) # or raw (address, pitch) pairs from any decoder binding
+        src.clear(2)                                    # slot 2 is idle: nothing is read or written for it
+        src.upload()
+
+    fmt 'bgr': one plane of H rows of 3W bytes; 'nv12': Y (H rows of W) and interleaved UV (H/2 rows of W); 'i420': Y, U and V
+    (H/2 rows of W/2 each).  Pitches are in bytes, need no alignment, and planes need not be adjacent.  set() checks each entry:
+    every plane present and its pitch at least its row bytes.  The table holds addresses only: the caller keeps the surfaces
+    alive (views passed to set() are referenced until the slot is set again or cleared).
+
+    upload() is one cudaMemcpyAsync of the mirror on the current stream, followed by the event `uploaded`.  Inside a captured
+    graph (StreamBatch.capture_planes) the copy is recorded and reads the mirror at every replay, so the mirror must not be edited
+    while a replay that reads it is in flight: wait for `uploaded` (uploaded.synchronize()) after replaying before the next edit,
+    or alternate two tables, each with its own graph."""
+
+    def __init__(self, S, fmt, size, device='cuda'):
+        S, H, W = int(S), int(size[0]), int(size[1])
+        if fmt not in ops.SRC_FORMATS:
+            raise ValueError("fmt must be 'bgr', 'nv12' or 'i420' (got %r)" % (fmt,))
+        if not 1 <= S <= 65535 or not (1 <= H <= 32767 and 1 <= W <= 32767) or (fmt != 'bgr' and (H % 2 or W % 2)):
+            raise ValueError('PlaneTable needs 1 <= S <= 65535 and a size in [1, 32767], even for %s (got S=%d, %dx%d)' % (fmt, S, H, W))
+        dev = torch.device(device)
+        self.S, self.fmt, self.size = S, fmt, (H, W)
+        self.host = torch.zeros((S, ops.PLANES_ENTRY_BYTES // 8), dtype=torch.int64, pin_memory=dev.type == 'cuda')
+        self.device = torch.zeros((S, ops.PLANES_ENTRY_BYTES // 8), dtype=torch.int64, device=dev)
+        self.uploaded = torch.cuda.Event(external=True) if dev.type == 'cuda' else None
+        self._entries = self.host.numpy().view(_PLANES_DTYPE).reshape(S)
+        self._keep = [None] * S
+
+    @classmethod
+    def packed(cls, batch, fmt):
+        """The table of a contiguous batch [S,H,W,3] ('bgr') or [S,3H/2,W] ('nv12' / 'i420'): pitches are the row bytes.
+        Uploaded on the current stream."""
+        if fmt == 'bgr':
+            S, H, W = int(batch.shape[0]), int(batch.shape[1]), int(batch.shape[2])
+        else:
+            S, H, W = int(batch.shape[0]), int(batch.shape[1]) // 3 * 2, int(batch.shape[2])
+        if not batch.is_contiguous() or batch.dtype != torch.uint8:
+            raise ValueError('a packed batch must be a contiguous uint8 tensor')
+        t = cls(S, fmt, (H, W), device=batch.device)
+        base, frame = batch.data_ptr(), batch[0].numel()
+        for s in range(S):
+            a, off = base + s * frame, 0
+            planes = []
+            for rows, nbytes in _plane_rows(fmt, H, W):
+                planes.append((a + off, nbytes))
+                off += rows * nbytes
+            t.set(s, planes)
+        t._keep = [batch] * S
+        t.upload()
+        return t
+
+    def _slot(self, slot):
+        if not isinstance(slot, (int, np.integer)) or not 0 <= slot < self.S:
+            raise ValueError('slot %r outside [0, %d)' % (slot, self.S))
+        return int(slot)
+
+    def set(self, slot, planes):
+        """Slot `slot`'s frame: one plane for 'bgr', two for 'nv12', three for 'i420', each a pitched uint8 view on the device
+        ([rows, >= row bytes] with unit column stride, or [H,W,3] for 'bgr'; the pitch is its row stride) or an (address, pitch)
+        pair.  Edits the host mirror only (see upload())."""
+        s = self._slot(slot)
+        rows = _plane_rows(self.fmt, *self.size)
+        if len(planes) != len(rows):
+            raise ValueError('a %s frame has %d planes (got %d)' % (self.fmt, len(rows), len(planes)))
+        addr, pitch = [0, 0, 0], [0, 0, 0]
+        for k, (p, (n, nbytes)) in enumerate(zip(planes, rows)):
+            if isinstance(p, torch.Tensor):
+                if p.dtype != torch.uint8 or p.device != self.device.device:
+                    raise ValueError('plane %d must be a uint8 tensor on %s (got %s on %s)' % (k, self.device.device, p.dtype, p.device))
+                if p.dim() == 3 and self.fmt == 'bgr' and p.shape[2] == 3 and p.stride(2) == 1 and p.stride(1) == 3:
+                    cover = p.shape[0] >= n and p.shape[1] * 3 >= nbytes
+                else:
+                    cover = p.dim() == 2 and p.stride(1) == 1 and p.shape[0] >= n and p.shape[1] >= nbytes
+                if not cover:
+                    raise ValueError('plane %d must cover %d rows of %d bytes with unit column stride (got %s, strides %s)'
+                                     % (k, n, nbytes, tuple(p.shape), p.stride()))
+                a, q = p.data_ptr(), p.stride(0)
+            else:
+                a, q = int(p[0]), int(p[1])
+            if a == 0:
+                raise ValueError('plane %d of slot %d is missing (address 0)' % (k, s))
+            if not nbytes <= q < 2 ** 31:
+                raise ValueError('plane %d of slot %d: pitch %d is below its %d row bytes (or above 2^31)' % (k, s, q, nbytes))
+            addr[k], pitch[k] = a, q
+        self._entries[s] = (addr, pitch, (0, 0, 0))
+        self._keep[s] = [p for p in planes if isinstance(p, torch.Tensor)]
+
+    def clear(self, slot):
+        """Slot `slot` becomes idle: the plane-table calls read and write nothing for it (after the next upload())."""
+        s = self._slot(slot)
+        self._entries[s] = ((0, 0, 0), (0, 0, 0), (0, 0, 0))
+        self._keep[s] = None
+
+    def upload(self):
+        """One cudaMemcpyAsync of the host mirror into the device table on the current stream, then the event `uploaded`."""
+        self.device.copy_(self.host, non_blocking=True)
+        if self.uploaded is not None:
+            self.uploaded.record()
+
+
 class StreamBatch:
     """S videos of one source size stabilised side by side.  Slot s holds what StreamState + CropState hold for one video (the
     history rings, a device-resident ring head, `all_black`), and one step advances every slot by one frame with one set of
@@ -560,12 +679,19 @@ class StreamBatch:
 
     def _capture(self, raw_bgr, net, upload, download):
         """capture() with the transfers as callables (or None) recorded before and after the step"""
+        return self._record(lambda: self.step(raw_bgr, net), upload, download)
+
+    def _record(self, run, upload, download, warm_upload=False):
+        """run() (one step) as a CUDA graph with upload / download (callables or None) recorded before and after it, after one
+        eager warm-up run on a side stream (with the upload first when warm_upload) whose state changes are undone"""
         state = (self.frames, self.masks, self.heads_dev, self.all_black)
         snap = [t.clone() for t in state]
         side = torch.cuda.Stream(device=self.frames.device)
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side):
-            self.step(raw_bgr, net)
+            if warm_upload and upload is not None:
+                upload()
+            run()
         torch.cuda.current_stream().wait_stream(side)
         for t, v in zip(state, snap):
             t.copy_(v)
@@ -573,10 +699,68 @@ class StreamBatch:
         with torch.cuda.graph(graph):
             if upload is not None:
                 upload()
-            self.step(raw_bgr, net)
+            run()
             if download is not None:
                 download()
         return graph
+
+    def _check_table(self, table, fmt, size, name):
+        if not isinstance(table, PlaneTable):
+            raise ValueError('%s must be a PlaneTable' % name)
+        if (table.S, table.fmt, table.size) != (self.S, fmt, tuple(size)):
+            raise ValueError('%s must describe %d %s frames of %dx%d (got %d %s frames of %dx%d)'
+                             % ((name, self.S, fmt) + tuple(size) + (table.S, table.fmt) + table.size))
+        if table.device.device != self.frames.device:
+            raise ValueError('%s lives on %s, the batch on %s' % (name, table.device.device, self.frames.device))
+
+    def _packed_table(self, attr, buf, fmt):
+        """the table of one of the batch's own buffers (self.colour / self.small), built and uploaded once"""
+        t = getattr(self, attr, None)
+        if t is None:
+            t = PlaneTable.packed(buf, fmt)
+            setattr(self, attr, t)
+        return t
+
+    def step_planes(self, src_table, net, dst_table=None):
+        """step() on frames that lie wherever the decoder put them: src_table (a PlaneTable of src_format and src_size, uploaded)
+        gives each slot's source planes and pitches, and the stabilised frames are written into the surfaces of dst_table (a
+        PlaneTable of out_format and out_size), or into self.colour when dst_table is None.  Every slot's frames and rings are
+        those of step() on the packed frames; join, leave, the crop and the rings behave as in step().  At out_size == src_size
+        the warp reads the source planes itself, otherwise cv2.resize writes them into self.small first.
+        A slot whose source entry is empty (PlaneTable.clear) is idle in the front end: its network frame keeps what it held; with
+        out_size == src_size the warp also writes nothing for it, and with a resize its destination is only left alone when its
+        dst_table entry is cleared as well.  Returns self.colour (dst_table None) or dst_table."""
+        self._check_table(src_table, self.src_format, self.src_size, 'src_table')
+        dst = self._packed_table('_colour_table', self.colour, self.out_format) if dst_table is None else dst_table
+        self._check_table(dst, self.out_format, self.out_size, 'dst_table')
+        h, w = self.height, self.width
+        cur = ops.cvt_img2train_planes(src_table.device, self.src_format, self.src_size, self._cvt, h, w, out=self.cur, tmp=self.cvt_tmp)
+        xy = self.advance(cur, net)
+        if self._direct:
+            ops.remap_bundle_frame_planes(src_table.device, self.src_format, xy, self.src_size, dst.device, self.out_format,
+                                          workspace=self.remap_ws)
+        else:
+            oh, ow = self.out_size
+            ops.resize_linear_planes(src_table.device, self.src_format, self.src_size, self._resize[0], self._resize[1], oh, ow,
+                                     out=self.small)
+            ops.remap_bundle_frame_planes(self._packed_table('_small_table', self.small, 'bgr').device, 'bgr', xy, self.out_size,
+                                          dst.device, self.out_format, workspace=self.remap_ws)
+        return self.colour if dst_table is None else dst_table
+
+    def capture_planes(self, src_table, net, dst_table=None):
+        """Records step_planes(src_table, net, dst_table) as a CUDA graph with the uploads of both tables at its head: edit the
+        tables' host mirrors (set / clear) between replays and each replay reads the surfaces they name then -- one graph follows a
+        decoder's rotating surface pool and an encoder's input surfaces.  A replay's upload reads the mirror when the replay runs,
+        so do not edit a mirror before the replay that reads it has copied it: wait for the table's event (table.uploaded.
+        synchronize(), recorded right after the copy inside the graph), or alternate two tables, each captured in its own graph.
+        join / leave between replays act as with capture()."""
+        self._check_table(src_table, self.src_format, self.src_size, 'src_table')
+        tables = (src_table,) if dst_table is None else (src_table, dst_table)
+
+        def upload():
+            for t in tables:
+                t.upload()
+        return self._record(lambda: self.step_planes(src_table, net, dst_table), upload, None, warm_upload=True)
 
 
 class MixedStreamBatch(StreamBatch):
@@ -735,6 +919,12 @@ class MixedStreamBatch(StreamBatch):
         oh, ow = self.out_size
         small = ops.resize_linear_mixed(pool, self.src_format, self.sizes, self.xtab, self.ytab, oh, ow, out=self.small)
         return self._warp_small(small, xy)
+
+    def step_planes(self, src_table, net, dst_table=None):
+        """Plane tables take a batch of one source size (StreamBatch): a MixedStreamBatch reads its frames from the pool."""
+        raise TypeError('plane tables take a batch of one source size: use StreamBatch.step_planes')
+
+    capture_planes = step_planes
 
     def capture(self, pool, net, upload_from=None, download_to=None, exact_bytes=False):
         """StreamBatch.capture of step(pool, net).  exact_bytes=False copies the whole pool up (and, for out_size='source', the

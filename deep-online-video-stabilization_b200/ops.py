@@ -906,3 +906,80 @@ def remap_bundle_frame(src, src_format, xy, out=None, workspace=None, out_format
             check(lib.mgw_remap_bundle_frame_yuv420(_p(src), SRC_FORMATS[src_format], _p(xy), s, h, w, H, W, SRC_FORMATS[out_format],
                                                     _p(dst), _p(ws), _st()), 'mgw_remap_bundle_frame_yuv420')
     return dst
+
+
+# ---- a batch of one size whose frames lie in decoder / encoder surfaces (deploy.StreamBatch.step_planes): per-slot planes
+PLANES_ENTRY_BYTES = 48          # sizeof(mgw_planes)
+
+
+def _planes_table(t, name):
+    """a device table of mgw_planes: a contiguous CUDA tensor, uint8 [S,48] or int64 [S,6] (deploy.PlaneTable.device) -> S"""
+    if not isinstance(t, torch.Tensor) or not t.is_cuda:
+        raise ValueError('%s must be a CUDA tensor holding a table of mgw_planes' % name)
+    if t.dtype not in (torch.uint8, torch.int64) or t.dim() != 2 or t.shape[1] * t.element_size() != PLANES_ENTRY_BYTES:
+        raise ValueError('%s must be uint8 [S,%d] or int64 [S,%d] (got %s %s)' % (name, PLANES_ENTRY_BYTES, PLANES_ENTRY_BYTES // 8,
+                                                                                  t.dtype, tuple(t.shape)))
+    if not t.is_contiguous():
+        raise ValueError('%s must be contiguous' % name)
+    return int(t.shape[0])
+
+
+def cvt_img2train_planes(table, fmt, size, tables, out_h, out_w, out=None, tmp=None):
+    """cvt_img2train of S frames of one size (H, W) = size, each described by its entry of the planes table (fmt 'bgr', 'nv12' or
+    'i420') -> [S,out_h,out_w] fp32, byte for byte the uniform batch call on the packed frames; the uniform tables.  Idle slots
+    (a missing plane or a short pitch) leave their rows of out / tmp [S,H,out_w] untouched.  One C-ABI call."""
+    if fmt not in SRC_FORMATS:
+        raise ValueError('source format must be one of %s (got %r)' % (sorted(SRC_FORMATS), fmt))
+    s, (h, w) = _planes_table(table, 'table'), (int(size[0]), int(size[1]))
+    kx, x0, xn, ky, y0, yn = (_chk(t, 'table', torch.int32) for t in tables)
+    if kx.shape[0] != out_w or ky.shape[0] != out_h:
+        raise ValueError('the tables must cover the %dx%d output' % (out_h, out_w))
+    tmp = _out(tmp, (s, h, out_w), table.device, torch.uint8, 'tmp')
+    out = _out(out, (s, out_h, out_w), table.device, torch.float32, 'out')
+    with torch.cuda.device(table.device):
+        check(lib.mgw_cvt_img2train_planes(_p(table), SRC_FORMATS[fmt], s, h, w, _p(kx), _p(x0), _p(xn), kx.shape[1], _p(ky), _p(y0),
+                                           _p(yn), ky.shape[1], out_h, out_w, _p(tmp), _p(out), _st()), 'mgw_cvt_img2train_planes')
+    return out
+
+
+def resize_linear_planes(table, fmt, size, xtab, ytab, out_h, out_w, out=None):
+    """cv2.resize of S frames of one size described by the planes table -> [S,out_h,out_w,3] BGR, contiguous (the uniform
+    tables; None / None for the 2x2 shortcut).  Idle slots leave their rows of out untouched.  One C-ABI call."""
+    if fmt not in SRC_FORMATS:
+        raise ValueError('source format must be one of %s (got %r)' % (sorted(SRC_FORMATS), fmt))
+    s, (h, w) = _planes_table(table, 'table'), (int(size[0]), int(size[1]))
+    xtab = None if xtab is None else _chk(xtab, 'xtab', torch.int32)
+    ytab = None if ytab is None else _chk(ytab, 'ytab', torch.int32)
+    dst = _out(out, (s, out_h, out_w, 3), table.device, torch.uint8, 'out')
+    with torch.cuda.device(table.device):
+        check(lib.mgw_resize_linear_planes(_p(table), SRC_FORMATS[fmt], s, h, w, _p(xtab), _p(ytab), out_h, out_w, _p(dst), _st()),
+              'mgw_resize_linear_planes')
+    return dst
+
+
+def remap_bundle_frame_planes(src_table, src_format, xy, size, dst_table, dst_format, workspace=None):
+    """warpRevBundle2 of S frames of one size (H, W) = size from the surfaces of src_table into those of dst_table (dst_format
+    'bgr', 'nv12' or 'i420'; H and W even when either format is YUV), xy [S,h,w,2] fp32.  Each active slot's used bytes are
+    remap_bundle_frame's on the packed frame; pitch padding, bytes between planes and idle slots are not written.  workspace:
+    optional fp32 scratch of remap_bundle_workspace_floats(S, h, w).  Returns dst_table.  One C-ABI call (two launches)."""
+    for name, f in (('source format', src_format), ('dst_format', dst_format)):
+        if f not in SRC_FORMATS:
+            raise ValueError('%s must be one of %s (got %r)' % (name, sorted(SRC_FORMATS), f))
+    s, (H, W) = _planes_table(src_table, 'src_table'), (int(size[0]), int(size[1]))
+    if _planes_table(dst_table, 'dst_table') != s:
+        raise ValueError('src_table and dst_table must have one entry per slot (got %d and %d)' % (s, dst_table.shape[0]))
+    xy = _chk(xy, 'xy')
+    if xy.dim() != 4 or xy.shape[0] != s or xy.shape[3] != 2:
+        raise ValueError('xy must be [%d,h,w,2] (got %s)' % (s, tuple(xy.shape)))
+    h, w = int(xy.shape[1]), int(xy.shape[2])
+    ws = (torch.empty(remap_bundle_workspace_floats(s, h, w), device=xy.device, dtype=torch.float32) if workspace is None
+          else _chk_out(workspace, 'workspace'))
+    if ws.numel() < remap_bundle_workspace_floats(s, h, w):
+        raise ValueError('workspace needs %d floats' % remap_bundle_workspace_floats(s, h, w))
+    if not (src_table.device == dst_table.device == xy.device == ws.device):
+        raise ValueError('src_table, dst_table, xy and workspace must be on one device (got %s, %s, %s, %s)'
+                         % (src_table.device, dst_table.device, xy.device, ws.device))
+    with torch.cuda.device(xy.device):
+        check(lib.mgw_remap_bundle_frame_planes(_p(src_table), SRC_FORMATS[src_format], _p(xy), s, h, w, H, W, _p(dst_table),
+                                                SRC_FORMATS[dst_format], _p(ws), _st()), 'mgw_remap_bundle_frame_planes')
+    return dst_table

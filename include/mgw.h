@@ -274,7 +274,7 @@ MGW_API int mgw_streams_push(float* frames, float* masks, int S, int depth, int3
  * Each call gives byte for byte what its BGR batch call gives on cv2.cvtColor(yuv, COLOR_YUV2BGR_NV12 / _I420) of every frame:
  * OpenCV's BT.601 limited-range 20-bit fixed point, one chroma sample per 2x2 block, converted inside the kernels that read the
  * source.  The frame the network sees is BGR2GRAY of that BGR frame, not the Y plane.  (cv2.VideoCapture converts with FFmpeg's
- * swscale, which is not byte-identical to cvtColor.)  Pitched decoder surfaces are copied to contiguous frames by the caller.
+ * swscale, which is not byte-identical to cvtColor.)  Pitched decoder surfaces: the plane-table calls (mgw_*_planes) below.
  * mgw_cvt_img2train_yuv420_batch: -> out [S,out_h,out_w]; tables and tmp (S*H*out_w bytes) as for mgw_cvt_img2train_u8_batch.
  * mgw_resize_linear_yuv420_batch: -> dst [S,out_h,out_w,3] BGR; tables as for mgw_resize_linear_u8_batch.
  * Checked in the order of the BGR batch calls: sizes and format (S <= 65535, H, W even and positive, S*(3H/2)*W < 2^31), then
@@ -327,7 +327,8 @@ MGW_API int mgw_remap_bundle_frame(const uint8_t* src, int format, const float* 
  * COLOR_BGR2YUV_I420) of the BGR frame F that mgw_remap_bundle_frame gives, its U and V planes interleaved for NV12.  That is
  * BT.601 limited range in 20-bit fixed point, Y of every pixel and U, V of the top-left pixel of each 2x2 block (no chroma
  * averaging); the conversion runs inside the warp and the BGR frame is never written.  Half the bytes of the BGR result.  The
- * rows are packed (pitch W): a pitched encoder surface is the caller's copy.  Same workspace as mgw_remap_bundle_frame.
+ * rows are packed (pitch W); mgw_remap_bundle_frame_planes below writes pitched encoder surfaces.  Same workspace as
+ * mgw_remap_bundle_frame.
  * Checked in the order of the batch calls: mgw_remap_bundle_frame's sizes and source format with H and W even for every source,
  * and dst_format NV12 or I420 (MGW_BGR24 is rejected: that result is mgw_remap_bundle_frame's), then S = 0 returns MGW_OK and
  * launches nothing, then the pointers and their alignment. */
@@ -363,6 +364,41 @@ MGW_API int mgw_remap_bundle_frame_mixed(const uint8_t* src, int format, int S, 
  * memory (cudaPointerGetAttributes; legal inside a stream capture). */
 MGW_API int mgw_copy_slots_mixed(const uint8_t* src, uint8_t* dst, int format, int S, int max_h, int max_w, const int32_t* sizes,
                                void* stream);
+
+/* ---- f1/f2 straight from decoder surfaces into encoder surfaces: per-slot plane pointers and pitches ---------------------
+ * A batch of S frames of one size H x W whose frames lie wherever a decoder (or an encoder's input pool) put them: each slot is
+ * described by one mgw_planes entry of a table in device memory, [S] entries, 16-byte aligned (48 bytes each: every entry is).
+ * plane[k] is a device address and pitch[k] its row pitch in bytes (any value, aligned or not; planes need not be adjacent):
+ *   MGW_BGR24:       plane[0] holds H rows of 3W used bytes.
+ *   MGW_YUV420_NV12: plane[0] is Y (H rows of W bytes), plane[1] interleaved U,V (H/2 rows of W bytes); NVDEC's layout of a
+ *                    1080p surface is plane[1] = plane[0] + pitch * 1088.
+ *   MGW_YUV420_I420: plane[0] is Y, plane[1] / plane[2] are U / V (H/2 rows of W/2 bytes each), e.g. an AVFrame's data[0..2]
+ *                    with linesize[0..2].
+ * Unused planes, pitches and `reserved` are ignored.  A slot is idle when a plane its format needs is 0 or a needed pitch is below
+ * that plane's row bytes: its blocks return before writing anything (no tmp, out or dst rows, no byte of a destination surface),
+ * so clearing an entry stops a slot and a bad entry can only stop it, never move an access.  The tables are read when the
+ * kernels run, so a captured graph follows whatever surfaces the entries hold at each replay.  The tables travel as const void*.
+ * mgw_cvt_img2train_planes: src table in `format` -> out [S,out_h,out_w]; tables and tmp (S*H*out_w bytes) as for the uniform
+ *   batch call; byte for byte mgw_cvt_img2train_u8_batch / _yuv420_batch on the packed frames.
+ * mgw_resize_linear_planes: -> dst [S,out_h,out_w,3] BGR, contiguous; tables as for the uniform batch call (2x2 INTER_AREA shortcut
+ *   included); byte for byte mgw_resize_linear_u8_batch / _yuv420_batch on the packed frames.
+ * mgw_remap_bundle_frame_planes: xy [S,h,w,2]; src table in `format`, dst table in dst_format (MGW_BGR24, MGW_YUV420_NV12 or
+ *   _I420), both of frames H x W.  Each active slot's used bytes are mgw_remap_bundle_frame's (MGW_BGR24) or
+ *   mgw_remap_bundle_frame_yuv420's on the packed frame; pitch padding and anything between planes is never written.  A
+ *   contiguous buffer is the table whose pitches are the row bytes.  workspace: mgw_remap_bundle_frame_workspace_bytes().
+ * Checked in the order of the batch calls: formats and sizes as for the uniform calls (H and W even when a format is YUV), then
+ * S = 0 returns MGW_OK and launches nothing, then null pointers and alignment: the tables 16 bytes, xy and workspace 8 bytes, the
+ * coefficient tables as in the uniform calls. */
+/* 48 bytes: three 8-byte addresses and three 4-byte pitches take 36, and padding to 48 keeps every entry of a table 16-byte
+ * aligned, so a block reads BGR / NV12 entries in two 16-byte loads (I420's V pitch in a third). */
+typedef struct { uint64_t plane[3]; int32_t pitch[3]; int32_t reserved[3]; } mgw_planes;
+MGW_API int mgw_cvt_img2train_planes(const void* src, int format, int S, int H, int W, const int32_t* kx, const int32_t* x0,
+                               const int32_t* xn, int ksx, const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h,
+                               int out_w, uint8_t* tmp, float* out, void* stream);
+MGW_API int mgw_resize_linear_planes(const void* src, int format, int S, int H, int W, const int32_t* xtab, const int32_t* ytab,
+                               int out_h, int out_w, uint8_t* dst, void* stream);
+MGW_API int mgw_remap_bundle_frame_planes(const void* src, int format, const float* xy, int S, int h, int w, int H, int W,
+                               const void* dst, int dst_format, void* workspace, void* stream);
 
 /* ---- a6: interpolate(im, x, y, out_size), spatial_transformer.py:200-281 ------------------------------
  * im [N,IH,IW,C]; x,y [N,OH,OW] normalised coords -> out [N,OH,OW,C]. */
