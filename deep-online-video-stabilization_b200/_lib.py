@@ -72,6 +72,10 @@ SIGNATURES = {
     'mgw_cvt_img2train_planes': (c_i, [c_f, c_i, c_i, c_i, c_i, c_f, c_f, c_f, c_i, c_f, c_f, c_f, c_i, c_i, c_i, c_f, c_f, c_st]),
     'mgw_resize_linear_planes': (c_i, [c_f, c_i, c_i, c_i, c_i, c_f, c_f, c_i, c_i, c_f, c_st]),
     'mgw_remap_bundle_frame_planes': (c_i, [c_f, c_i, c_f, c_i, c_i, c_i, c_i, c_i, c_f, c_i, c_f, c_st]),
+    'mgw_cvt_img2train_mixed_planes': (c_i, [c_f, c_i, c_i, c_i, c_i, c_f, c_f, c_f, c_f, c_i, c_f, c_f, c_f, c_i, c_i, c_i, c_f, c_f,
+                                             c_st]),
+    'mgw_resize_linear_mixed_planes': (c_i, [c_f, c_i, c_i, c_i, c_i, c_f, c_f, c_f, c_i, c_i, c_f, c_st]),
+    'mgw_remap_bundle_frame_mixed_planes': (c_i, [c_f, c_i, c_i, c_i, c_i, c_f, c_f, c_i, c_i, c_f, c_i, c_f, c_st]),
     'mgw_interp_fwd': (c_i, [c_f, c_f, c_f] + [c_i] * 6 + [c_f, c_st]),
     'mgw_interp_bwd': (c_i, [c_f, c_f, c_f, c_f] + [c_i] * 6 + [c_f, c_f, c_f, c_st]),
     'mgw_homography_warp_fwd': (c_i, [c_f, c_f] + [c_i] * 6 + [c_f, c_f, c_f, c_st]),

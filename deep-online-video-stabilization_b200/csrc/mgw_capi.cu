@@ -863,6 +863,64 @@ int mgw_remap_bundle_frame_planes(const void* src, int format, const float* xy, 
                                       dst_format, workspace, (cudaStream_t)stream);
 }
 
+// Per-slot sizes and planes: validate_mixed with the pool gone.  The capacity's limits hold for one frame (validate_mixed at S = 1);
+// the limits on tmp [S,max_h,out_w] and out [S,out_h,out_w] hold for all S slots.
+static int validate_mixed_planes(const char* fn, int format, int S, int max_h, int max_w, int out_h, int out_w)
+{
+    TRY(validate_mixed(fn, format, 1, max_h, max_w, out_h, out_w));
+    REQUIRE(S >= 0 && S <= 65535 && (long long)S * max_h * out_w < (1LL << 31) && (long long)S * out_h * out_w < (1LL << 29),
+            "%s: bad sizes (S=%d capacity %dx%d out %dx%d)", fn, S, max_h, max_w, out_h, out_w);
+    return MGW_OK;
+}
+
+int mgw_cvt_img2train_mixed_planes(const void* src, int format, int S, int max_h, int max_w, const int32_t* sizes, const int32_t* kx,
+                                   const int32_t* x0, const int32_t* xn, int ksx, const int32_t* ky, const int32_t* y0, const int32_t* yn,
+                                   int ksy, int out_h, int out_w, uint8_t* tmp, float* out, void* stream)
+{
+    TRY(validate_mixed_planes("mgw_cvt_img2train_mixed_planes", format, S, max_h, max_w, out_h, out_w));
+    REQUIRE(ksx > 0 && ksy > 0, "mgw_cvt_img2train_mixed_planes: bad sizes (ksx=%d ksy=%d)", ksx, ksy);
+    if (S == 0) return MGW_OK;
+    REQUIRE(src && sizes && kx && x0 && xn && ky && y0 && yn && tmp && out, "mgw_cvt_img2train_mixed_planes: null pointer");
+    REQUIRE(aligned(sizes, 8), "mgw_cvt_img2train_mixed_planes: sizes must be 8-byte aligned");
+    REQUIRE(aligned(src, 16), "mgw_cvt_img2train_mixed_planes: the planes table must be 16-byte aligned");
+    return launch_cvt_img2train_mixed_planes(static_cast<const mgw_planes*>(src), format, S, max_h, max_w, sizes, kx, x0, xn, ksx, ky, y0,
+                                             yn, ksy, out_h, out_w, tmp, out, (cudaStream_t)stream);
+}
+
+int mgw_resize_linear_mixed_planes(const void* src, int format, int S, int max_h, int max_w, const int32_t* sizes, const int32_t* xtab,
+                                   const int32_t* ytab, int out_h, int out_w, uint8_t* dst, void* stream)
+{
+    TRY(validate_mixed_planes("mgw_resize_linear_mixed_planes", format, S, max_h, max_w, out_h, out_w));
+    if (S == 0) return MGW_OK;
+    REQUIRE(src && sizes && xtab && ytab && dst, "mgw_resize_linear_mixed_planes: null pointer");
+    REQUIRE(aligned(xtab, 16) && aligned(ytab, 16), "mgw_resize_linear_mixed_planes: tables must be 16-byte aligned");
+    REQUIRE(aligned(sizes, 8), "mgw_resize_linear_mixed_planes: sizes must be 8-byte aligned");
+    REQUIRE(aligned(src, 16), "mgw_resize_linear_mixed_planes: the planes table must be 16-byte aligned");
+    return launch_resize_linear_mixed_planes(static_cast<const mgw_planes*>(src), format, S, max_h, max_w, sizes, xtab, ytab, out_h, out_w,
+                                             dst, (cudaStream_t)stream);
+}
+
+// mgw_remap_bundle_frame_mixed's checks in its order without the pool's S*max_h*max_w*3 < 2^31 (one frame is bounded by the
+// capacity's 32767 x 32767); S*h*w < 2^31 bounds xy and the /4 maps
+int mgw_remap_bundle_frame_mixed_planes(const void* src, int format, int S, int max_h, int max_w, const int32_t* sizes, const float* xy,
+                                        int h, int w, const void* dst, int dst_format, void* workspace, void* stream)
+{
+    const auto known = [](int f) { return f == MGW_BGR24 || f == MGW_YUV420_NV12 || f == MGW_YUV420_I420; };
+    REQUIRE(known(format), "mgw_remap_bundle_frame_mixed_planes: unknown format %d", format);
+    REQUIRE(known(dst_format), "mgw_remap_bundle_frame_mixed_planes: unknown destination format %d", dst_format);
+    REQUIRE(S >= 0 && S <= 65535 && h >= 8 && w >= 8 && max_h >= 1 && max_w >= 1 && max_h <= 32767 && max_w <= 32767 &&
+            ((format == MGW_BGR24 && dst_format == MGW_BGR24) || (max_h % 2 == 0 && max_w % 2 == 0)) && (long long)S * h * w < (1LL << 31),
+            "mgw_remap_bundle_frame_mixed_planes: bad sizes (S=%d maps %dx%d capacity %dx%d; h, w >= 8, capacity even for YUV)", S, h, w,
+            max_h, max_w);
+    if (S == 0) return MGW_OK;
+    REQUIRE(src && sizes && xy && dst && workspace, "mgw_remap_bundle_frame_mixed_planes: null pointer");
+    REQUIRE(aligned(xy, 8) && aligned(workspace, 8) && aligned(sizes, 8),
+            "mgw_remap_bundle_frame_mixed_planes: xy, workspace and sizes must be 8-byte aligned");
+    REQUIRE(aligned(src, 16) && aligned(dst, 16), "mgw_remap_bundle_frame_mixed_planes: the planes tables must be 16-byte aligned");
+    return launch_remap_bundle_mixed_planes(static_cast<const mgw_planes*>(src), format, S, max_h, max_w, sizes, xy, h, w,
+                                            static_cast<const mgw_planes*>(dst), dst_format, workspace, (cudaStream_t)stream);
+}
+
 static int validate_streams(const char* fn, int S, int depth, int H, int W, int nch)
 {
     REQUIRE(S >= 0 && S <= 65535 && depth > 0 && H > 0 && W > 0 && (long long)S * depth * H * W < (1LL << 31) &&

@@ -145,6 +145,16 @@ __device__ __forceinline__ bool load_planes(const mgw_planes* __restrict__ tab, 
     }
 }
 
+// MIXED && PLANES: slot s's entry at the slot's size sz = sizes[s] (its width for the pitch rule), and only when the entry's own
+// frame size, reserved[0] x reserved[1] (the third 16-byte word of the entry), equals sz: a slot that re-joined at another size
+// while its entry still names the old surface is idle, so a stale entry cannot move an access past the surface it describes
+template <int FMT>
+__device__ __forceinline__ bool load_planes_at(const mgw_planes* __restrict__ tab, int s, int2 sz, Planes& f)
+{
+    const int4 c = __ldg(reinterpret_cast<const int4*>(tab + s) + 2);
+    return c.y == sz.x && c.z == sz.y && load_planes<FMT>(tab, s, sz.y, f);
+}
+
 // yuv_chroma_at / yuv_bgr_at on pitched planes: NV12's UV rows in p[1], I420's U and V in p[1] and p[2]
 template <int FMT>
 __device__ __forceinline__ Chroma planes_chroma_at(const Planes& f, int row, int x)
@@ -313,7 +323,8 @@ __device__ __forceinline__ int2 remap_src_fixed(const float2* __restrict__ small
 // PLANES (C = 3): the source frame and the BGR result are slot blockIdx.y's entries of the tables sp (FMT) and dp (BGR), src and dst
 // unused.  A pitched row cannot be continued by the next one, so the threads are laid out over rows x ceil(W / REMAP_RUN) column
 // groups, as in remap_up_yuv_kernel: each stores the 3 * REMAP_RUN bytes of its group (fewer at the row's end) as 3 words where the
-// address is aligned and byte by byte otherwise.
+// address is aligned and byte by byte otherwise.  MIXED && PLANES: H, W are the capacity; block (., s) applies the MIXED rule to
+// sizes[s], loads both entries at that size (load_planes_at) and runs the PLANES code at the slot's size and scales.
 template <int C, int FMT, bool MIXED = false, bool PLANES = false>
 __global__ void __launch_bounds__(256)
 remap_up_kernel(const uint8_t* __restrict__ src, const float2* __restrict__ small, int H, int W, int h4, int w4, double xscale,
@@ -321,9 +332,16 @@ remap_up_kernel(const uint8_t* __restrict__ src, const float2* __restrict__ smal
                 const mgw_planes* __restrict__ dp)
 {
     if constexpr (PLANES) {
-        static_assert(C == 3 && !MIXED, "a table's slot is a colour frame of the batch's size");
+        static_assert(C == 3, "a table's slot is a colour frame");
         Planes f, d;
-        if (!load_planes<FMT>(sp, blockIdx.y, W, f) || !load_planes<SRC_BGR>(dp, blockIdx.y, W, d)) return;
+        if constexpr (MIXED) {
+            const int2 sz = __ldg(sizes + blockIdx.y);
+            // block-uniform: before the barrier of slot_scales
+            if (!slot_active<FMT>(sz, H, W) || !load_planes_at<FMT>(sp, blockIdx.y, sz, f) || !load_planes_at<SRC_BGR>(dp, blockIdx.y, sz, d))
+                return;
+            H = sz.x; W = sz.y;                             // launched over the capacity's rows x column groups: the rest return below
+            slot_scales(H, W, h4, w4, xscale, yscale);
+        } else if (!load_planes<FMT>(sp, blockIdx.y, W, f) || !load_planes<SRC_BGR>(dp, blockIdx.y, W, d)) return;
         const int gw = (W + REMAP_RUN - 1) / REMAP_RUN;
         const int t = blockIdx.x * blockDim.x + threadIdx.x;
         if (t >= H * gw) return;
@@ -447,7 +465,8 @@ __device__ __forceinline__ void store_run(uint8_t* o, const uint8_t* b, int n)
 // device functions; the column coefficients are shared by the two rows.  The thread writes the block's Y bytes and the U, V of
 // its two (or one) 2x2 chroma blocks, so the BGR frame never reaches memory.  MIXED: as remap_up_kernel, with a YUV result region
 // of 3H/2*W bytes per slot; a slot of odd size is idle.  PLANES: the source and the result are slot blockIdx.y's entries of the
-// tables sp (SRC_FMT) and dp (DST_FMT), src and dst unused; the same threads and arithmetic, pitched loads and stores.
+// tables sp (SRC_FMT) and dp (DST_FMT), src and dst unused; the same threads and arithmetic, pitched loads and stores.  MIXED &&
+// PLANES: the MIXED rule on sizes[s], both entries loaded at that size (load_planes_at), then the PLANES code at the slot's size.
 constexpr int YUV_RUN = 4;
 
 template <int SRC_FMT, int DST_FMT, bool MIXED = false, bool PLANES = false>
@@ -458,11 +477,16 @@ remap_up_yuv_kernel(const uint8_t* __restrict__ src, const float2* __restrict__ 
 {
     [[maybe_unused]] Planes sf, df;
     if constexpr (PLANES) {
-        static_assert(!MIXED, "a table's slot is a frame of the batch's size");
-        if (!load_planes<SRC_FMT>(sp, blockIdx.y, W, sf) || !load_planes<DST_FMT>(dp, blockIdx.y, W, df)) return;
+        if constexpr (MIXED) {
+            const int2 sz = __ldg(sizes + blockIdx.y);
+            if (!slot_active<SRC_FMT>(sz, H, W) || !slot_active<DST_FMT>(sz, H, W) || !load_planes_at<SRC_FMT>(sp, blockIdx.y, sz, sf) ||
+                !load_planes_at<DST_FMT>(dp, blockIdx.y, sz, df))
+                return;                                     // block-uniform: before the barrier of slot_scales
+            H = sz.x; W = sz.y;
+            slot_scales(H, W, h4, w4, xscale, yscale);
+        } else if (!load_planes<SRC_FMT>(sp, blockIdx.y, W, sf) || !load_planes<DST_FMT>(dp, blockIdx.y, W, df)) return;
         small += (size_t)blockIdx.y * h4 * w4;
-    }
-    if constexpr (MIXED) {
+    } else if constexpr (MIXED) {
         const int2 sz = __ldg(sizes + blockIdx.y);
         // the result is 4:2:0, so every active slot is even (DST_FMT's rule covers an odd size from a BGR source)
         if (!slot_active<SRC_FMT>(sz, H, W) || !slot_active<DST_FMT>(sz, H, W)) return;
@@ -590,6 +614,32 @@ int launch_remap_up_planes(int dst_fmt, const mgw_planes* sp, const float2* smal
     return check_launch("remap_up_yuv");
 }
 
+// K5b of a batch of per-slot sizes between two tables of planes: the grid covers the capacity, gridDim.y is the slot
+template <int SRC_FMT>
+int launch_remap_up_mixed_planes(int dst_fmt, const mgw_planes* sp, const float2* small, int S, int max_h, int max_w, int h4, int w4,
+                                 const int2* sizes, const mgw_planes* dp, cudaStream_t st)
+{
+    if (dst_fmt == SRC_BGR) {
+        const long long groups = (max_w + REMAP_RUN - 1) / REMAP_RUN;
+        const dim3 grid((unsigned)(((long long)max_h * groups + 255) / 256), S);
+        remap_up_kernel<3, SRC_FMT, true, true><<<grid, 256, 0, st>>>(nullptr, small, max_h, max_w, h4, w4, 0.0, 0.0, nullptr, sizes, sp, dp);
+        return check_launch("remap_up");
+    }
+    const dim3 grid((unsigned)(((long long)(max_h / 2) * ((max_w + YUV_RUN - 1) / YUV_RUN) + 255) / 256), S);
+    switch (dst_fmt) {
+    case MGW_YUV420_NV12:
+        remap_up_yuv_kernel<SRC_FMT, MGW_YUV420_NV12, true, true><<<grid, 256, 0, st>>>(nullptr, small, max_h, max_w, h4, w4, 0.0, 0.0,
+                                                                                        nullptr, sizes, sp, dp);
+        break;
+    case MGW_YUV420_I420:
+        remap_up_yuv_kernel<SRC_FMT, MGW_YUV420_I420, true, true><<<grid, 256, 0, st>>>(nullptr, small, max_h, max_w, h4, w4, 0.0, 0.0,
+                                                                                        nullptr, sizes, sp, dp);
+        break;
+    default: return set_error(MGW_ERR_INVALID, "remap_bundle_frame_mixed_planes: unknown destination format %d", dst_fmt);
+    }
+    return check_launch("remap_up_yuv");
+}
+
 template <int SRC_FMT>
 int launch_remap_up_yuv_to(int dst_fmt, const uint8_t* src, const float2* small, int N, int H, int W, int h4, int w4, uint8_t* dst,
                            cudaStream_t st)
@@ -688,6 +738,22 @@ int launch_remap_bundle_planes(const mgw_planes* src, int src_fmt, const float* 
     }
 }
 
+// the same K5a, then K5b per slot at the slot's own size from the source table's planes into the destination table's
+int launch_remap_bundle_mixed_planes(const mgw_planes* src, int src_fmt, int S, int max_h, int max_w, const int32_t* sizes,
+                                     const float* xy, int h, int w, const mgw_planes* dst, int dst_fmt, void* workspace, cudaStream_t st)
+{
+    const int h4 = h / 4, w4 = w / 4;
+    float2* small = launch_maps_down(xy, S, h, w, workspace, st);
+    if (int rc = check_launch("maps_down")) return rc;
+    const int2* sz = reinterpret_cast<const int2*>(sizes);
+    switch (src_fmt) {
+    case SRC_BGR: return launch_remap_up_mixed_planes<SRC_BGR>(dst_fmt, src, small, S, max_h, max_w, h4, w4, sz, dst, st);
+    case MGW_YUV420_NV12: return launch_remap_up_mixed_planes<MGW_YUV420_NV12>(dst_fmt, src, small, S, max_h, max_w, h4, w4, sz, dst, st);
+    case MGW_YUV420_I420: return launch_remap_up_mixed_planes<MGW_YUV420_I420>(dst_fmt, src, small, S, max_h, max_w, h4, w4, sz, dst, st);
+    default: return set_error(MGW_ERR_INVALID, "remap_bundle_frame_mixed_planes: unknown source format %d", src_fmt);
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // Exact-bytes transfer of a pool of per-slot frames (MIXED): slot s's frame_bytes(sizes[s]) bytes from src + s * stride to
 // dst + s * stride, stride = frame_bytes(max_h, max_w); nothing past them is read or written, and an idle slot (the MIXED rule)
@@ -766,6 +832,7 @@ int launch_copy_slots_mixed(const uint8_t* src, uint8_t* dst, int fmt, int S, in
 // the slot, and then runs the per-pixel code of the uniform batch at the slot's size with frame index 0.
 // PLANES = per-slot planes (a uniform batch whose frames lie wherever a decoder put them): slot s's source is entry s of the table
 // `planes` (see load_planes), bgr is unused; the tables, tmp and out are the uniform batch's, and an idle slot writes no row of either.
+// MIXED && PLANES: the MIXED slot (its size, tables and tmp / out rows at the capacity) read from its entry (load_planes_at).
 namespace {
 
 template <int FMT, bool MIXED = false, bool PLANES = false>
@@ -776,11 +843,18 @@ gray_hpass_kernel(const uint8_t* __restrict__ bgr, int H, int W, const int32_t* 
 {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if constexpr (PLANES) {
-        static_assert(!MIXED, "a table's slot is a frame of the batch's size");
         Planes f;
-        if (!load_planes<FMT>(planes, blockIdx.y, W, f)) return;
+        if constexpr (MIXED) {
+            const int2 sz = __ldg(sizes + blockIdx.y);
+            if (!slot_active<FMT>(sz, H, W) || !load_planes_at<FMT>(planes, blockIdx.y, sz, f)) return;
+            tmp += (size_t)blockIdx.y * H * out_w;          // the slot's tmp rows, laid out at the capacity
+            kx += (size_t)blockIdx.y * out_w * ks;
+            x0 += (size_t)blockIdx.y * out_w;
+            xn += (size_t)blockIdx.y * out_w;
+            H = sz.x;
+        } else if (!load_planes<FMT>(planes, blockIdx.y, W, f)) return;
         if (t >= H * out_w) return;
-        tmp += (size_t)blockIdx.y * H * out_w;
+        if constexpr (!MIXED) tmp += (size_t)blockIdx.y * H * out_w;
         const int xx = t % out_w, row = t / out_w;
         const int n = __ldg(xn + xx), xs = __ldg(x0 + xx);
         int acc = 1 << 21;
@@ -846,7 +920,7 @@ gray_hpass_kernel(const uint8_t* __restrict__ bgr, int H, int W, const int32_t* 
 }
 
 // MIXED: H is the capacity's height (the tmp rows of a slot), max_w its width; the slot's rows of ky / y0 / yn
-// PLANES: max_w is the source width; a slot that gray_hpass found idle is skipped by the same rule
+// PLANES: max_w is the source width; a slot that gray_hpass found idle is skipped by the same rule (MIXED && PLANES: at the slot's size)
 template <int FMT = SRC_BGR, bool MIXED = false, bool PLANES = false>
 __global__ void __launch_bounds__(256)
 vpass_norm_kernel(const uint8_t* __restrict__ tmp, int H, int out_w, const int32_t* __restrict__ ky, const int32_t* __restrict__ y0,
@@ -856,10 +930,13 @@ vpass_norm_kernel(const uint8_t* __restrict__ tmp, int H, int out_w, const int32
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if constexpr (PLANES) {
         Planes f;
-        if (!load_planes<FMT>(planes, blockIdx.y, max_w, f)) return;
+        if constexpr (MIXED) {
+            const int2 sz = __ldg(sizes + blockIdx.y);
+            if (!slot_active<FMT>(sz, H, max_w) || !load_planes_at<FMT>(planes, blockIdx.y, sz, f)) return;
+        } else if (!load_planes<FMT>(planes, blockIdx.y, max_w, f)) return;
     }
     if constexpr (MIXED) {
-        if (!slot_active<FMT>(__ldg(sizes + blockIdx.y), H, max_w)) return;
+        if (!PLANES && !slot_active<FMT>(__ldg(sizes + blockIdx.y), H, max_w)) return;
         ky += (size_t)blockIdx.y * out_h * ks;
         y0 += (size_t)blockIdx.y * out_h;
         yn += (size_t)blockIdx.y * out_h;
@@ -948,6 +1025,36 @@ int launch_cvt_img2train_mixed(const uint8_t* src, int src_fmt, int S, int max_h
     }
 }
 
+template <int FMT>
+static int cvt_mixed_planes(const mgw_planes* src, int S, int max_h, int max_w, const int2* sizes, const int32_t* kx, const int32_t* x0,
+                            const int32_t* xn, int ksx, const int32_t* ky, const int32_t* y0, const int32_t* yn, int ksy, int out_h,
+                            int out_w, uint8_t* tmp, float* out, cudaStream_t st)
+{
+    gray_hpass_kernel<FMT, true, true><<<dim3((max_h * out_w + 255) / 256, S), 256, 0, st>>>(nullptr, max_h, max_w, kx, x0, xn, ksx, out_w,
+                                                                                           tmp, sizes, src);
+    if (int rc = check_launch("gray_hpass")) return rc;
+    vpass_norm_kernel<FMT, true, true><<<dim3((out_h * out_w + 255) / 256, S), 256, 0, st>>>(tmp, max_h, out_w, ky, y0, yn, ksy, out_h,
+                                                                                           out, sizes, max_w, src);
+    return check_launch("vpass_norm");
+}
+
+int launch_cvt_img2train_mixed_planes(const mgw_planes* src, int src_fmt, int S, int max_h, int max_w, const int32_t* sizes,
+                                      const int32_t* kx, const int32_t* x0, const int32_t* xn, int ksx, const int32_t* ky,
+                                      const int32_t* y0, const int32_t* yn, int ksy, int out_h, int out_w, uint8_t* tmp, float* out,
+                                      cudaStream_t st)
+{
+    const int2* sz = reinterpret_cast<const int2*>(sizes);
+    switch (src_fmt) {
+    case SRC_BGR:
+        return cvt_mixed_planes<SRC_BGR>(src, S, max_h, max_w, sz, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w, tmp, out, st);
+    case MGW_YUV420_NV12:
+        return cvt_mixed_planes<MGW_YUV420_NV12>(src, S, max_h, max_w, sz, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w, tmp, out, st);
+    case MGW_YUV420_I420:
+        return cvt_mixed_planes<MGW_YUV420_I420>(src, S, max_h, max_w, sz, kx, x0, xn, ksx, ky, y0, yn, ksy, out_h, out_w, tmp, out, st);
+    default: return set_error(MGW_ERR_INVALID, "cvt_img2train_mixed_planes: unknown source format %d", src_fmt);
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // cv2.resize(frame, (width, height)) of the uint8 colour frame (deploy_bundle.py:301; INTER_LINEAR): OpenCV's 8-bit path --
 // 11-bit fixed-point weights (tables from the host binding: x0, x1, a0, a1 per output column / row), int32 horizontal sums,
@@ -959,6 +1066,7 @@ __device__ __forceinline__ int ch_of(const int3& p, int ch) { return ch == 0 ? p
 
 // MIXED: H, W are the capacity (see cvt_img2train above); xtab [S,out_w], ytab [S,out_h]; the 2x2 shortcut is the slot's own
 // PLANES: slot s's source is entry s of the table `planes` (img unused), the uniform tables and dst; an idle slot writes nothing
+// MIXED && PLANES: the MIXED slot (size rule, tables, its own 2x2 shortcut) read from its entry (load_planes_at)
 template <int C, int FMT = SRC_BGR, bool MIXED = false, bool PLANES = false>
 __global__ void __launch_bounds__(256)
 resize_u8_kernel(const uint8_t* __restrict__ img, int H, int W, const int4* __restrict__ xtab, const int4* __restrict__ ytab,
@@ -968,9 +1076,15 @@ resize_u8_kernel(const uint8_t* __restrict__ img, int H, int W, const int4* __re
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= out_h * out_w) return;
     if constexpr (PLANES) {
-        static_assert(C == 3 && !MIXED, "a table's slot is a colour frame of the batch's size");
+        static_assert(C == 3, "a table's slot is a colour frame");
         Planes f;
-        if (!load_planes<FMT>(planes, blockIdx.y, W, f)) return;
+        if constexpr (MIXED) {
+            const int2 sz = __ldg(sizes + blockIdx.y);
+            if (!slot_active<FMT>(sz, H, W) || !load_planes_at<FMT>(planes, blockIdx.y, sz, f)) return;
+            xtab += (size_t)blockIdx.y * out_w;
+            ytab += (size_t)blockIdx.y * out_h;
+            area2 = sz.y == 2 * out_w && sz.x == 2 * out_h;
+        } else if (!load_planes<FMT>(planes, blockIdx.y, W, f)) return;
         const int x = t % out_w, y = t / out_w;
         uint8_t* o = dst + ((size_t)blockIdx.y * out_h * out_w + t) * 3;
         int3 p00, p01, p10, p11;
@@ -1131,6 +1245,27 @@ int launch_resize_linear_mixed(const uint8_t* src, int src_fmt, int S, int max_h
     case MGW_YUV420_I420:
         resize_u8_kernel<3, MGW_YUV420_I420, true><<<grid, 256, 0, st>>>(src, max_h, max_w, xt, yt, out_h, out_w, 0, dst, sz, nullptr); break;
     default: return set_error(MGW_ERR_INVALID, "resize_linear_mixed: unknown source format %d", src_fmt);
+    }
+    return check_launch("resize_u8");
+}
+
+int launch_resize_linear_mixed_planes(const mgw_planes* src, int src_fmt, int S, int max_h, int max_w, const int32_t* sizes,
+                                      const int32_t* xtab, const int32_t* ytab, int out_h, int out_w, uint8_t* dst, cudaStream_t st)
+{
+    const dim3 grid((out_h * out_w + 255) / 256, S);
+    const int2* sz = reinterpret_cast<const int2*>(sizes);
+    const int4* xt = reinterpret_cast<const int4*>(xtab);
+    const int4* yt = reinterpret_cast<const int4*>(ytab);
+    switch (src_fmt) {
+    case SRC_BGR:
+        resize_u8_kernel<3, SRC_BGR, true, true><<<grid, 256, 0, st>>>(nullptr, max_h, max_w, xt, yt, out_h, out_w, 0, dst, sz, src); break;
+    case MGW_YUV420_NV12:
+        resize_u8_kernel<3, MGW_YUV420_NV12, true, true><<<grid, 256, 0, st>>>(nullptr, max_h, max_w, xt, yt, out_h, out_w, 0, dst, sz, src);
+        break;
+    case MGW_YUV420_I420:
+        resize_u8_kernel<3, MGW_YUV420_I420, true, true><<<grid, 256, 0, st>>>(nullptr, max_h, max_w, xt, yt, out_h, out_w, 0, dst, sz, src);
+        break;
+    default: return set_error(MGW_ERR_INVALID, "resize_linear_mixed_planes: unknown source format %d", src_fmt);
     }
     return check_launch("resize_u8");
 }

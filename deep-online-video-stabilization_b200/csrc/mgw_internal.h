@@ -151,6 +151,16 @@ int launch_resize_linear_planes(const mgw_planes* src, int src_fmt, int S, int H
                                 int out_h, int out_w, uint8_t* dst, cudaStream_t st);
 int launch_remap_bundle_planes(const mgw_planes* src, int src_fmt, const float* xy, int S, int h, int w, int H, int W,
                                const mgw_planes* dst, int dst_fmt, void* workspace, cudaStream_t st);
+// per-slot sizes and planes: the _mixed calls with slot s's frame (and the warp's result) in entry s of a table, read at sizes[s];
+// a slot is idle under the MIXED rule, the PLANES rule, or when the entry's own size (reserved[0], reserved[1]) is not sizes[s]
+int launch_cvt_img2train_mixed_planes(const mgw_planes* src, int src_fmt, int S, int max_h, int max_w, const int32_t* sizes,
+                                      const int32_t* kx, const int32_t* x0, const int32_t* xn, int ksx, const int32_t* ky,
+                                      const int32_t* y0, const int32_t* yn, int ksy, int out_h, int out_w, uint8_t* tmp, float* out,
+                                      cudaStream_t st);
+int launch_resize_linear_mixed_planes(const mgw_planes* src, int src_fmt, int S, int max_h, int max_w, const int32_t* sizes,
+                                      const int32_t* xtab, const int32_t* ytab, int out_h, int out_w, uint8_t* dst, cudaStream_t st);
+int launch_remap_bundle_mixed_planes(const mgw_planes* src, int src_fmt, int S, int max_h, int max_w, const int32_t* sizes,
+                                     const float* xy, int h, int w, const mgw_planes* dst, int dst_fmt, void* workspace, cudaStream_t st);
 int launch_warp_rev_bundle_u8(const uint8_t* img, const double* Hs_cvt, int N, int H, int W, int C, int gh, int gw, uint8_t* dst,
                               cudaStream_t st);
 

@@ -17,7 +17,7 @@ import torch
 from . import ops
 
 __all__ = ['warpRevBundle2', 'warpRevBundle', 'warpRev', 'cvt_theta_mat_bundle', 'cvt_img2train', 'cv2_resize', 'StreamState', 'CropState', 'StreamBatch',
-           'MixedStreamBatch', 'mixed_slot_tables', 'scale_rect', 'PlaneTable']
+           'MixedStreamBatch', 'mixed_slot_tables', 'scale_rect', 'PlaneTable', 'MixedPlaneTable']
 
 
 def warpRevBundle2(img, x_map, y_map, device=None, src_format='bgr', dst_format='bgr'):
@@ -399,75 +399,44 @@ def _plane_rows(fmt, H, W):
     return [(H, W), (H // 2, W // 2), (H // 2, W // 2)]
 
 
-class PlaneTable:
-    """Where the S frames of a batch of one size lie: per slot the device address and row pitch of each plane, as a decoder or an
-    encoder hands its surfaces out.  A pinned host mirror (host, int64 [S,6], one include/mgw.h mgw_planes per row) that set() /
-    clear() edit, and the device table (device) that the plane-table calls read, refreshed by upload().
+def _packed_planes(fmt, base, H, W):
+    """the (address, pitch) pairs of an H x W frame packed at address base: each plane after the previous one, pitch = row bytes"""
+    planes, off = [], 0
+    for rows, nbytes in _plane_rows(fmt, H, W):
+        planes.append((base + off, nbytes))
+        off += rows * nbytes
+    return planes
 
-        src = PlaneTable(S, 'nv12', (1080, 1920))
-        src.set(0, (y_plane, uv_plane))                 # pitched uint8 CUDA views: [1080,>=1920] and [540,>=1920]
-        src.set(1, ((y_addr, pitch), (uv_addr, pitch))) # or raw (address, pitch) pairs from any decoder binding
-        src.clear(2)                                    # slot 2 is idle: nothing is read or written for it
-        src.upload()
 
-    fmt 'bgr': one plane of H rows of 3W bytes; 'nv12': Y (H rows of W) and interleaved UV (H/2 rows of W); 'i420': Y, U and V
-    (H/2 rows of W/2 each).  Pitches are in bytes, need no alignment, and planes need not be adjacent.  set() checks each entry:
-    every plane present and its pitch at least its row bytes.  The table holds addresses only: the caller keeps the surfaces
-    alive (views passed to set() are referenced until the slot is set again or cleared).
+class _PlaneMirror:
+    """What PlaneTable and MixedPlaneTable share: the pinned host mirror of S mgw_planes entries, the device table, the checks of
+    one entry's planes against a frame size, clear() and upload()."""
 
-    upload() is one cudaMemcpyAsync of the mirror on the current stream, followed by the event `uploaded`.  Inside a captured
-    graph (StreamBatch.capture_planes) the copy is recorded and reads the mirror at every replay, so the mirror must not be edited
-    while a replay that reads it is in flight: wait for `uploaded` (uploaded.synchronize()) after replaying before the next edit,
-    or alternate two tables, each with its own graph."""
-
-    def __init__(self, S, fmt, size, device='cuda'):
+    def __init__(self, S, fmt, size, device, what):
+        """S entries of fmt for frames up to size (H, W); what names the size in the error"""
         S, H, W = int(S), int(size[0]), int(size[1])
         if fmt not in ops.SRC_FORMATS:
             raise ValueError("fmt must be 'bgr', 'nv12' or 'i420' (got %r)" % (fmt,))
         if not 1 <= S <= 65535 or not (1 <= H <= 32767 and 1 <= W <= 32767) or (fmt != 'bgr' and (H % 2 or W % 2)):
-            raise ValueError('PlaneTable needs 1 <= S <= 65535 and a size in [1, 32767], even for %s (got S=%d, %dx%d)' % (fmt, S, H, W))
+            raise ValueError('%s needs 1 <= S <= 65535 and a %s in [1, 32767], even for %s (got S=%d, %dx%d)'
+                             % (type(self).__name__, what, fmt, S, H, W))
         dev = torch.device(device)
-        self.S, self.fmt, self.size = S, fmt, (H, W)
+        self.S, self.fmt = S, fmt
         self.host = torch.zeros((S, ops.PLANES_ENTRY_BYTES // 8), dtype=torch.int64, pin_memory=dev.type == 'cuda')
         self.device = torch.zeros((S, ops.PLANES_ENTRY_BYTES // 8), dtype=torch.int64, device=dev)
         self.uploaded = torch.cuda.Event(external=True) if dev.type == 'cuda' else None
         self._entries = self.host.numpy().view(_PLANES_DTYPE).reshape(S)
         self._keep = [None] * S
 
-    @classmethod
-    def packed(cls, batch, fmt):
-        """The table of a contiguous batch [S,H,W,3] ('bgr') or [S,3H/2,W] ('nv12' / 'i420'): pitches are the row bytes.
-        Uploaded on the current stream."""
-        if fmt == 'bgr':
-            S, H, W = int(batch.shape[0]), int(batch.shape[1]), int(batch.shape[2])
-        else:
-            S, H, W = int(batch.shape[0]), int(batch.shape[1]) // 3 * 2, int(batch.shape[2])
-        if not batch.is_contiguous() or batch.dtype != torch.uint8:
-            raise ValueError('a packed batch must be a contiguous uint8 tensor')
-        t = cls(S, fmt, (H, W), device=batch.device)
-        base, frame = batch.data_ptr(), batch[0].numel()
-        for s in range(S):
-            a, off = base + s * frame, 0
-            planes = []
-            for rows, nbytes in _plane_rows(fmt, H, W):
-                planes.append((a + off, nbytes))
-                off += rows * nbytes
-            t.set(s, planes)
-        t._keep = [batch] * S
-        t.upload()
-        return t
-
     def _slot(self, slot):
         if not isinstance(slot, (int, np.integer)) or not 0 <= slot < self.S:
             raise ValueError('slot %r outside [0, %d)' % (slot, self.S))
         return int(slot)
 
-    def set(self, slot, planes):
-        """Slot `slot`'s frame: one plane for 'bgr', two for 'nv12', three for 'i420', each a pitched uint8 view on the device
-        ([rows, >= row bytes] with unit column stride, or [H,W,3] for 'bgr'; the pitch is its row stride) or an (address, pitch)
-        pair.  Edits the host mirror only (see upload())."""
+    def _write(self, slot, planes, H, W, reserved):
+        """entry `slot` = the planes of an H x W frame (checked as set() documents) and the words `reserved`, into the mirror"""
         s = self._slot(slot)
-        rows = _plane_rows(self.fmt, *self.size)
+        rows = _plane_rows(self.fmt, H, W)
         if len(planes) != len(rows):
             raise ValueError('a %s frame has %d planes (got %d)' % (self.fmt, len(rows), len(planes)))
         addr, pitch = [0, 0, 0], [0, 0, 0]
@@ -490,7 +459,7 @@ class PlaneTable:
             if not nbytes <= q < 2 ** 31:
                 raise ValueError('plane %d of slot %d: pitch %d is below its %d row bytes (or above 2^31)' % (k, s, q, nbytes))
             addr[k], pitch[k] = a, q
-        self._entries[s] = (addr, pitch, (0, 0, 0))
+        self._entries[s] = (addr, pitch, reserved)
         self._keep[s] = [p for p in planes if isinstance(p, torch.Tensor)]
 
     def clear(self, slot):
@@ -504,6 +473,106 @@ class PlaneTable:
         self.device.copy_(self.host, non_blocking=True)
         if self.uploaded is not None:
             self.uploaded.record()
+
+
+class PlaneTable(_PlaneMirror):
+    """Where the S frames of a batch of one size lie: per slot the device address and row pitch of each plane, as a decoder or an
+    encoder hands its surfaces out.  A pinned host mirror (host, int64 [S,6], one include/mgw.h mgw_planes per row) that set() /
+    clear() edit, and the device table (device) that the plane-table calls read, refreshed by upload().
+
+        src = PlaneTable(S, 'nv12', (1080, 1920))
+        src.set(0, (y_plane, uv_plane))                 # pitched uint8 CUDA views: [1080,>=1920] and [540,>=1920]
+        src.set(1, ((y_addr, pitch), (uv_addr, pitch))) # or raw (address, pitch) pairs from any decoder binding
+        src.clear(2)                                    # slot 2 is idle: nothing is read or written for it
+        src.upload()
+
+    fmt 'bgr': one plane of H rows of 3W bytes; 'nv12': Y (H rows of W) and interleaved UV (H/2 rows of W); 'i420': Y, U and V
+    (H/2 rows of W/2 each).  Pitches are in bytes, need no alignment, and planes need not be adjacent.  set() checks each entry:
+    every plane present and its pitch at least its row bytes.  The table holds addresses only: the caller keeps the surfaces
+    alive (views passed to set() are referenced until the slot is set again or cleared).
+
+    upload() is one cudaMemcpyAsync of the mirror on the current stream, followed by the event `uploaded`.  Inside a captured
+    graph (StreamBatch.capture_planes) the copy is recorded and reads the mirror at every replay, so the mirror must not be edited
+    while a replay that reads it is in flight: wait for `uploaded` (uploaded.synchronize()) after replaying before the next edit,
+    or alternate two tables, each with its own graph."""
+
+    def __init__(self, S, fmt, size, device='cuda'):
+        super().__init__(S, fmt, size, device, 'size')
+        self.size = (int(size[0]), int(size[1]))
+
+    @classmethod
+    def packed(cls, batch, fmt):
+        """The table of a contiguous batch [S,H,W,3] ('bgr') or [S,3H/2,W] ('nv12' / 'i420'): pitches are the row bytes.
+        Uploaded on the current stream."""
+        if fmt == 'bgr':
+            S, H, W = int(batch.shape[0]), int(batch.shape[1]), int(batch.shape[2])
+        else:
+            S, H, W = int(batch.shape[0]), int(batch.shape[1]) // 3 * 2, int(batch.shape[2])
+        if not batch.is_contiguous() or batch.dtype != torch.uint8:
+            raise ValueError('a packed batch must be a contiguous uint8 tensor')
+        t = cls(S, fmt, (H, W), device=batch.device)
+        base, frame = batch.data_ptr(), batch[0].numel()
+        for s in range(S):
+            t.set(s, _packed_planes(fmt, base + s * frame, H, W))
+        t._keep = [batch] * S
+        t.upload()
+        return t
+
+    def set(self, slot, planes):
+        """Slot `slot`'s frame: one plane for 'bgr', two for 'nv12', three for 'i420', each a pitched uint8 view on the device
+        ([rows, >= row bytes] with unit column stride, or [H,W,3] for 'bgr'; the pitch is its row stride) or an (address, pitch)
+        pair.  Edits the host mirror only (see upload())."""
+        self._write(slot, planes, *self.size, (0, 0, 0))
+
+
+class MixedPlaneTable(_PlaneMirror):
+    """PlaneTable for a MixedStreamBatch: the S frames have sizes of their own up to the capacity (H, W), and each entry names
+    the size of the frame it describes (mgw_planes.reserved[0], reserved[1] = height, width).  The mixed plane-table calls read
+    slot s only when its entry's size equals the batch's sizes[s]; otherwise the slot is idle.  host / device / uploaded, clear()
+    and upload() are PlaneTable's, and so is the rule on editing the mirror while a captured replay may still copy it.
+
+        src = MixedPlaneTable(S, 'nv12', (2160, 3840))
+        src.set(0, (y_plane, uv_plane), (1080, 1920))  # slot 0's surface holds a 1080p frame
+        src.set(1, ((y_addr, pitch), (uv_addr, pitch)), (720, 1280))
+        src.upload()
+
+    A slot that joins the batch again at another size stays idle until its entries are set at the new size and uploaded: a
+    stale entry can only stop the slot, never let it read or write past the surface it names.  Not a PlaneTable: a uniform
+    batch (StreamBatch.step_planes) refuses it."""
+
+    def __init__(self, S, fmt, capacity, device='cuda'):
+        super().__init__(S, fmt, capacity, device, 'capacity')
+        self.capacity = (int(capacity[0]), int(capacity[1]))
+
+    @classmethod
+    def pool(cls, buf, fmt, capacity, sizes):
+        """The table of a pool-shaped buffer buf (contiguous uint8, S rows of frame_bytes(capacity) bytes, e.g. MixedStreamBatch's
+        pool or its output pool): slot s's frame lies packed at the start of its row at sizes[s] = (H_s, W_s), or is idle for
+        None.  Uploaded on the current stream."""
+        H, W = int(capacity[0]), int(capacity[1])
+        if not isinstance(buf, torch.Tensor) or buf.dtype != torch.uint8 or not buf.is_contiguous():
+            raise ValueError('a pool must be a contiguous uint8 tensor')
+        S = int(buf.shape[0])
+        if len(sizes) != S or buf[0].numel() != ops.dst_frame_bytes(fmt, H, W):
+            raise ValueError('a %s pool of capacity %dx%d is [%d, %d] bytes with one size per slot (got %s and %d sizes)'
+                             % (fmt, H, W, S, ops.dst_frame_bytes(fmt, H, W), tuple(buf.shape), len(sizes)))
+        t = cls(S, fmt, (H, W), device=buf.device)
+        row = buf[0].numel()
+        for s, size in enumerate(sizes):
+            if size is not None:
+                t.set(s, _packed_planes(fmt, buf.data_ptr() + s * row, *size), size)
+        t._keep = [buf] * S
+        t.upload()
+        return t
+
+    def set(self, slot, planes, size):
+        """Slot `slot`'s frame of size (H_s, W_s) = size: within the capacity, even for 'nv12' / 'i420'.  planes as for
+        PlaneTable.set, each checked against that size; the size goes into the entry's reserved[0:2].  Edits the host mirror only."""
+        H, W = int(size[0]), int(size[1])
+        if not (1 <= H <= self.capacity[0] and 1 <= W <= self.capacity[1]) or (self.fmt != 'bgr' and (H % 2 or W % 2)):
+            raise ValueError('a slot of a %s table of capacity %dx%d takes a size within it, even for YUV (got %dx%d)'
+                             % ((self.fmt,) + self.capacity + (H, W)))
+        self._write(slot, planes, H, W, (H, W, 0))
 
 
 class StreamBatch:
@@ -755,6 +824,10 @@ class StreamBatch:
         synchronize(), recorded right after the copy inside the graph), or alternate two tables, each captured in its own graph.
         join / leave between replays act as with capture()."""
         self._check_table(src_table, self.src_format, self.src_size, 'src_table')
+        return self._record_planes(src_table, net, dst_table)
+
+    def _record_planes(self, src_table, net, dst_table):
+        """step_planes(src_table, net, dst_table) as a CUDA graph with the uploads of the tables at its head"""
         tables = (src_table,) if dst_table is None else (src_table, dst_table)
 
         def upload():
@@ -814,6 +887,8 @@ class MixedStreamBatch(StreamBatch):
             self.out_size = 'source'
             self.colour = self.colour.view(self.S, -1)
             self.out_pool_shape = tuple(self.colour.shape)
+            # the output pool's planes for step_planes, every slot idle until it joins (join writes its entry on the device)
+            self._colour_mtable = MixedPlaneTable.pool(self.colour, self.out_format, self.src_size, [None] * self.S)
         elif self._direct:
             # a common output size equal to the capacity: the slots still go through the per-slot resize
             self._direct = False
@@ -873,6 +948,11 @@ class MixedStreamBatch(StreamBatch):
         for dst, src in zip(dsts, (np.array([H, W], np.int32),) + tabs):
             dst[s].copy_(torch.as_tensor(src))
         self.slot_sizes[s] = (H, W)
+        if self._source_out:
+            # the output pool's entry at the new size, by a stream-ordered copy from pageable memory (as sizes): no wait on a replay
+            ct = self._colour_mtable
+            ct.set(s, _packed_planes(self.out_format, self.colour[s].data_ptr(), H, W), (H, W))
+            ct.device[s].copy_(torch.as_tensor(ct.host[s].numpy().copy()))
         cur = cvt_img2train(f.to(self.frames.device), self.crop_rate, self.height, self.width, src_format=self.src_format)
         super().join(s, cur.reshape(self.height, self.width))
 
@@ -920,11 +1000,56 @@ class MixedStreamBatch(StreamBatch):
         small = ops.resize_linear_mixed(pool, self.src_format, self.sizes, self.xtab, self.ytab, oh, ow, out=self.small)
         return self._warp_small(small, xy)
 
-    def step_planes(self, src_table, net, dst_table=None):
-        """Plane tables take a batch of one source size (StreamBatch): a MixedStreamBatch reads its frames from the pool."""
-        raise TypeError('plane tables take a batch of one source size: use StreamBatch.step_planes')
+    def _check_mixed_table(self, table, fmt, name):
+        if not isinstance(table, MixedPlaneTable):
+            raise TypeError('%s must be a MixedPlaneTable: a PlaneTable describes frames of one size (StreamBatch.step_planes)' % name)
+        if (table.S, table.fmt, table.capacity) != (self.S, fmt, self.src_size):
+            raise ValueError('%s must describe %d %s frames of capacity %dx%d (got %d %s frames of capacity %dx%d)'
+                             % ((name, self.S, fmt) + self.src_size + (table.S, table.fmt) + table.capacity))
+        if table.device.device != self.frames.device:
+            raise ValueError('%s lives on %s, the batch on %s' % (name, table.device.device, self.frames.device))
 
-    capture_planes = step_planes
+    def step_planes(self, src_table, net, dst_table=None):
+        """step() on frames that lie wherever the decoder put them: src_table is a MixedPlaneTable of src_format and the batch's
+        capacity (uploaded), whose entry s names slot s's surface at the slot's current size; a uniform PlaneTable is a TypeError.
+        Every slot's frames and rings are those of step() on the packed pool; join, leave, the crop and the rings are step()'s.
+          'source'    the warp reads the source planes and writes each slot at its own size into dst_table, a MixedPlaneTable of
+                      out_format and the capacity whose entries carry the slots' sizes, or into the output pool self.colour
+                      (dst_table None: the batch keeps that pool's table, and join updates a slot's entry on the device).
+          None / (OH, OW)  each slot is resized into self.small at its own size, then warped into dst_table, a PlaneTable of
+                      out_format and out_size, or into self.colour.
+        A slot is idle in the front end when its source entry is cleared, or names another size than the slot's (after a join at
+        a new size, until the entry is set at that size): its network frame keeps what it held.  With 'source' the warp then
+        writes nothing for it either, and a destination entry of another size idles it too; through the resize its destination
+        is left alone only when its dst_table entry is cleared as well.  Returns self.colour (dst_table None) or dst_table."""
+        self._check_mixed_table(src_table, self.src_format, 'src_table')
+        h, w = self.height, self.width
+        if self._source_out:
+            dst = self._colour_mtable if dst_table is None else dst_table
+            self._check_mixed_table(dst, self.out_format, 'dst_table')
+        else:
+            dst = self._packed_table('_colour_table', self.colour, self.out_format) if dst_table is None else dst_table
+            self._check_table(dst, self.out_format, self.out_size, 'dst_table')
+        cur = ops.cvt_img2train_mixed_planes(src_table.device, self.src_format, self.sizes, self.src_size, self.tables, h, w,
+                                             out=self.cur, tmp=self.cvt_tmp)
+        xy = self.advance(cur, net)
+        if self._source_out:
+            ops.remap_bundle_frame_mixed_planes(src_table.device, self.src_format, self.sizes, xy, self.src_size, dst.device,
+                                                self.out_format, workspace=self.remap_ws)
+        else:
+            oh, ow = self.out_size
+            ops.resize_linear_mixed_planes(src_table.device, self.src_format, self.sizes, self.src_size, self.xtab, self.ytab, oh, ow,
+                                           out=self.small)
+            ops.remap_bundle_frame_planes(self._packed_table('_small_table', self.small, 'bgr').device, 'bgr', xy, self.out_size,
+                                          dst.device, self.out_format, workspace=self.remap_ws)
+        return self.colour if dst_table is None else dst_table
+
+    def capture_planes(self, src_table, net, dst_table=None):
+        """StreamBatch.capture_planes for a MixedPlaneTable: step_planes(src_table, net, dst_table) as a CUDA graph with the uploads
+        of both tables at its head.  A slot may join again at another size between replays: it is idle until its entries are set
+        at the new size and uploaded by the next replay (the batch's own output pool table follows the join by itself)."""
+        self._check_mixed_table(src_table, self.src_format, 'src_table')
+        return self._record_planes(src_table, net, dst_table)
 
     def capture(self, pool, net, upload_from=None, download_to=None, exact_bytes=False):
         """StreamBatch.capture of step(pool, net).  exact_bytes=False copies the whole pool up (and, for out_size='source', the

@@ -983,3 +983,78 @@ def remap_bundle_frame_planes(src_table, src_format, xy, size, dst_table, dst_fo
         check(lib.mgw_remap_bundle_frame_planes(_p(src_table), SRC_FORMATS[src_format], _p(xy), s, h, w, H, W, _p(dst_table),
                                                 SRC_FORMATS[dst_format], _p(ws), _st()), 'mgw_remap_bundle_frame_planes')
     return dst_table
+
+
+# ---- videos of different sizes whose frames lie in decoder / encoder surfaces (deploy.MixedStreamBatch.step_planes)
+def _mixed_planes_dims(table, fmt, sizes, max_size, name='table'):
+    """a table of mgw_planes (deploy.MixedPlaneTable.device) of S slots in fmt, sizes int32 [S,2] on its device, the capacity
+    max_size = (max_h, max_w) -> (format constant, S, max_h, max_w, sizes)"""
+    if fmt not in SRC_FORMATS:
+        raise ValueError('source format must be one of %s (got %r)' % (sorted(SRC_FORMATS), fmt))
+    s = _planes_table(table, name)
+    sizes = _chk(sizes, 'sizes', torch.int32)
+    if tuple(sizes.shape) != (s, 2):
+        raise ValueError('sizes must be [%d,2] (got %s)' % (s, tuple(sizes.shape)))
+    if sizes.device != table.device:
+        raise ValueError('%s and sizes must be on one device (got %s and %s)' % (name, table.device, sizes.device))
+    return SRC_FORMATS[fmt], s, int(max_size[0]), int(max_size[1]), sizes
+
+
+def cvt_img2train_mixed_planes(table, fmt, sizes, max_size, tables, out_h, out_w, out=None, tmp=None):
+    """cvt_img2train_mixed with slot s's frame of size sizes[s] read from entry s of the planes table instead of a pool; the
+    capacity max_size = (max_h, max_w) sizes the per-slot tables and tmp [S,max_h,out_w] as in cvt_img2train_mixed.  Byte for
+    byte cvt_img2train_mixed on the packed pool.  Idle slots -- the _mixed rule, a missing plane or short pitch, or an entry whose
+    own size (its reserved[0:2]) is not sizes[s] -- leave their rows of out / tmp untouched.  One C-ABI call."""
+    code, s, mh, mw, sizes = _mixed_planes_dims(table, fmt, sizes, max_size)
+    kx, x0, xn, ky, y0, yn = (_chk(t, 'table', torch.int32) for t in tables)
+    if (kx.dim() != 3 or tuple(kx.shape[:2]) != (s, out_w) or ky.dim() != 3 or tuple(ky.shape[:2]) != (s, out_h) or
+            any(tuple(t.shape) != (s, out_w) for t in (x0, xn)) or any(tuple(t.shape) != (s, out_h) for t in (y0, yn))):
+        raise ValueError('the tables must be [%d,%d,ksx], [%d,%d] x2, [%d,%d,ksy], [%d,%d] x2' % (s, out_w, s, out_w, s, out_h, s, out_h))
+    tmp = _out(tmp, (s, mh, out_w), table.device, torch.uint8, 'tmp')
+    out = _out(out, (s, out_h, out_w), table.device, torch.float32, 'out')
+    with torch.cuda.device(table.device):
+        check(lib.mgw_cvt_img2train_mixed_planes(_p(table), code, s, mh, mw, _p(sizes), _p(kx), _p(x0), _p(xn), kx.shape[2], _p(ky),
+                                                 _p(y0), _p(yn), ky.shape[2], out_h, out_w, _p(tmp), _p(out), _st()),
+              'mgw_cvt_img2train_mixed_planes')
+    return out
+
+
+def resize_linear_mixed_planes(table, fmt, sizes, max_size, xtab, ytab, out_h, out_w, out=None):
+    """resize_linear_mixed with each slot read from its entry of the planes table -> [S,out_h,out_w,3] BGR, packed; xtab
+    [S,out_w,4], ytab [S,out_h,4] int32.  Idle slots (as for cvt_img2train_mixed_planes) leave their rows of out untouched."""
+    code, s, mh, mw, sizes = _mixed_planes_dims(table, fmt, sizes, max_size)
+    xtab, ytab = _chk(xtab, 'xtab', torch.int32), _chk(ytab, 'ytab', torch.int32)
+    if tuple(xtab.shape) != (s, out_w, 4) or tuple(ytab.shape) != (s, out_h, 4):
+        raise ValueError('xtab / ytab must be [%d,%d,4] / [%d,%d,4]' % (s, out_w, s, out_h))
+    dst = _out(out, (s, out_h, out_w, 3), table.device, torch.uint8, 'out')
+    with torch.cuda.device(table.device):
+        check(lib.mgw_resize_linear_mixed_planes(_p(table), code, s, mh, mw, _p(sizes), _p(xtab), _p(ytab), out_h, out_w, _p(dst),
+                                                 _st()), 'mgw_resize_linear_mixed_planes')
+    return dst
+
+
+def remap_bundle_frame_mixed_planes(src_table, src_format, sizes, xy, max_size, dst_table, dst_format, workspace=None):
+    """remap_bundle_frame_mixed from the surfaces of src_table into those of dst_table: slot s at its own size sizes[s], which both
+    of its entries must carry (their reserved[0:2]); xy [S,h,w,2] fp32; max_size = (max_h, max_w) the capacity (even when either
+    format is YUV).  Each active slot's used bytes are remap_bundle_frame_mixed's on the packed pool; pitch padding, bytes between
+    planes and idle slots are not written.  Returns dst_table.  One C-ABI call (two launches)."""
+    if dst_format not in SRC_FORMATS:
+        raise ValueError('dst_format must be one of %s (got %r)' % (sorted(SRC_FORMATS), dst_format))
+    code, s, mh, mw, sizes = _mixed_planes_dims(src_table, src_format, sizes, max_size, 'src_table')
+    if _planes_table(dst_table, 'dst_table') != s:
+        raise ValueError('src_table and dst_table must have one entry per slot (got %d and %d)' % (s, dst_table.shape[0]))
+    xy = _chk(xy, 'xy')
+    if xy.dim() != 4 or xy.shape[0] != s or xy.shape[3] != 2:
+        raise ValueError('xy must be [%d,h,w,2] (got %s)' % (s, tuple(xy.shape)))
+    h, w = int(xy.shape[1]), int(xy.shape[2])
+    ws = (torch.empty(remap_bundle_workspace_floats(s, h, w), device=xy.device, dtype=torch.float32) if workspace is None
+          else _chk_out(workspace, 'workspace'))
+    if ws.numel() < remap_bundle_workspace_floats(s, h, w):
+        raise ValueError('workspace needs %d floats' % remap_bundle_workspace_floats(s, h, w))
+    if not (src_table.device == dst_table.device == xy.device == ws.device):
+        raise ValueError('src_table, dst_table, xy and workspace must be on one device (got %s, %s, %s, %s)'
+                         % (src_table.device, dst_table.device, xy.device, ws.device))
+    with torch.cuda.device(xy.device):
+        check(lib.mgw_remap_bundle_frame_mixed_planes(_p(src_table), code, s, mh, mw, _p(sizes), _p(xy), h, w, _p(dst_table),
+                                                      SRC_FORMATS[dst_format], _p(ws), _st()), 'mgw_remap_bundle_frame_mixed_planes')
+    return dst_table

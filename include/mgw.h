@@ -400,6 +400,32 @@ MGW_API int mgw_resize_linear_planes(const void* src, int format, int S, int H, 
 MGW_API int mgw_remap_bundle_frame_planes(const void* src, int format, const float* xy, int S, int h, int w, int H, int W,
                                const void* dst, int dst_format, void* workspace, void* stream);
 
+/* ---- f1/f2 for a batch of videos of different source sizes, straight from decoder surfaces into encoder surfaces -----------
+ * The _mixed calls above with the pool replaced by a table of mgw_planes (the layouts of the plane-table calls): slot s's frame
+ * has the size sizes[s] (device int32 [S,2], 8-byte aligned) and lies in the planes of entry s.  That entry also names the size
+ * of the frame it describes: reserved[0] = its height, reserved[1] = its width (the plane-table calls above ignore `reserved`).
+ * The capacity (max_h, max_w) and the per-slot tables, tmp [S,max_h,out_w] and out rows are those of the _mixed calls.
+ * mgw_cvt_img2train_mixed_planes: -> out [S,out_h,out_w], as mgw_cvt_img2train_mixed.
+ * mgw_resize_linear_mixed_planes: -> dst [S,out_h,out_w,3] BGR, packed, as mgw_resize_linear_mixed.
+ * mgw_remap_bundle_frame_mixed_planes: xy [S,h,w,2]; each slot's result goes into entry s of the dst table (dst_format) at the
+ *   slot's own size sizes[s], which that entry must carry too; pitch padding and anything between planes is never written.
+ * Every active slot's bytes are bit-identical to the _mixed call on the packed pool of the same frames.  A slot is idle when
+ * sizes[s] is idle under the _mixed rule (0, above the capacity, odd when a format is YUV), when a plane its format needs is 0 or
+ * a needed pitch is below the plane's row bytes at the slot's width, or when an entry's size (reserved[0], reserved[1]) is not
+ * sizes[s]: an idle slot writes no tmp / out / dst row and no byte of a destination surface.  So a slot that joins again at
+ * another size stops until its entries name surfaces of the new size: a stale entry cannot move an access past its surface.
+ * Checked in the order of the _mixed calls, with their checks except the limits on the pool's offsets: the capacity's 32-bit
+ * limits hold for one frame (max_h*max_w < 2^29 for BGR, (3max_h/2)*max_w < 2^31 for YUV; 1 <= max_h, max_w <= 32767 for the
+ * warp), the limits on tmp (S*max_h*out_w < 2^31), out (S*out_h*out_w < 2^29) and xy (S*h*w < 2^31) for all S; then S = 0
+ * returns MGW_OK and launches nothing, then the pointers and their alignment, the tables last (16 bytes). */
+MGW_API int mgw_cvt_img2train_mixed_planes(const void* src, int format, int S, int max_h, int max_w, const int32_t* sizes,
+                               const int32_t* kx, const int32_t* x0, const int32_t* xn, int ksx, const int32_t* ky, const int32_t* y0,
+                               const int32_t* yn, int ksy, int out_h, int out_w, uint8_t* tmp, float* out, void* stream);
+MGW_API int mgw_resize_linear_mixed_planes(const void* src, int format, int S, int max_h, int max_w, const int32_t* sizes,
+                               const int32_t* xtab, const int32_t* ytab, int out_h, int out_w, uint8_t* dst, void* stream);
+MGW_API int mgw_remap_bundle_frame_mixed_planes(const void* src, int format, int S, int max_h, int max_w, const int32_t* sizes,
+                               const float* xy, int h, int w, const void* dst, int dst_format, void* workspace, void* stream);
+
 /* ---- a6: interpolate(im, x, y, out_size), spatial_transformer.py:200-281 ------------------------------
  * im [N,IH,IW,C]; x,y [N,OH,OW] normalised coords -> out [N,OH,OW,C]. */
 MGW_API int mgw_interp_fwd(const float* im, const float* x, const float* y, int N, int IH, int IW, int C, int OH, int OW,

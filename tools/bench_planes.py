@@ -80,7 +80,8 @@ def main():
             def copies_out():
                 for s in active:
                     dst[s][1].copy_(sb.colour[s, :H]); dst[s][2].copy_(sb.colour[s, H:])
-            g_b = sb._record(lambda: sb.step(raw, fixed_mesh_net(sb)), copies_in, copies_out if pitched_out else None, warm_upload=True)
+            net_b = fixed_mesh_net(sb)                          # built outside the capture: it copies a host mesh to the device
+            g_b = sb._record(lambda: sb.step(raw, net_b), copies_in, copies_out if pitched_out else None, warm_upload=True)
             # one replay of each on the same frames and state: the same output bytes
             g_a.replay(); g_b.replay(); torch.cuda.synchronize()
             for s in active:
